@@ -14,6 +14,10 @@ no data-path collective, weak scaling): every rank verifies its own batch.
   cpu_baseline : the CPU oracle restating the reference's per-signature core_verify, timed on a bounded sample
 
 `--impl reference` times the reference's CPU path (oracle restatement: blsful itself needs cargo + un-vendored crates).
+`--dump-outputs DIR` writes the status vectors of the last timed step of each leg as DIR/<name>.npy (float32); the inputs
+are seeded, so two builds run with the same arguments can be compared output for output.  The benchmark batch is all
+valid, so those vectors are all zero; planted_status.npy adds the statuses of the same device call, untimed, on a copy of
+the batch with a seeded set of planted rejections (see plant_rejections).
 """
 import argparse
 import gc
@@ -27,6 +31,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "agora-blsful_b200")):
     if p not in sys.path:
         sys.path.insert(0, p)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it
 
 import numpy as np
 
@@ -281,10 +286,54 @@ def emit(line: dict):
         os.write(_RESULT_FD, data)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """Writes each array as dirname/<name>.npy in float32.  If they would take more than DUMP_BYTES together, every array
+    is cut to the same fixed, seeded sample of positions, written beside it as <name>_index.npy (float64)."""
+    os.makedirs(dirname, exist_ok=True)
+    total = sum(a.size for a in arrays.values()) * 4
+    for i, (name, a) in enumerate(arrays.items()):
+        a = np.asarray(a).reshape(-1)
+        if total > DUMP_BYTES:
+            k = min(a.size, DUMP_BYTES // (len(arrays) * 12))   # 4 B per value + 8 B per index
+            idx = np.sort(np.random.default_rng(i).choice(a.size, k, replace=False))
+            np.save(os.path.join(dirname, f"{name}_index.npy"), idx.astype(np.float64))
+            a = a[idx]
+        np.save(os.path.join(dirname, f"{name}.npy"), a.astype(np.float32))
+
+
+def plant_rejections(pks, sigs, n, seed=7):
+    """A copy of a G2Impl batch (48 B keys, 96 B signatures) with k = min(64, n // 8) items of each kind the verifier must
+    reject, at fixed, seeded positions, and the statuses it must return: another item's signature (1), the identity
+    signature (2), the identity public key (3), an undecodable public key (4).  Everything else keeps status 0."""
+    k = min(64, n // 8)
+    pos = np.random.default_rng(seed).choice(n, 4 * k, replace=False).reshape(4, k)
+    p, s = pks.reshape(n, 48).copy(), sigs.reshape(n, 96).copy()
+    s[pos[0]] = sigs.reshape(n, 96)[(pos[0] + 1) % n]
+    s[pos[1]] = 0
+    s[pos[1], 0] = 0xC0
+    p[pos[2]] = 0
+    p[pos[2], 0] = 0xC0
+    p[pos[3]] = 0
+    want = np.zeros(n, dtype=np.uint8)
+    for status, idx in enumerate(pos, 1):
+        want[idx] = status
+    return p.reshape(-1), s.reshape(-1), want
+
+
+def _positive(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=_positive, default=3, help="timed steps of every leg")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="engine", choices=["engine", "reference"])
     ap.add_argument("--n", type=int, default=int(os.environ.get("BLSGPU_BENCH_N", 1_000_000)), help="signatures per batch per GPU")
@@ -293,6 +342,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the other BASELINE.json configs (cfg 1, 3, 4, 5, failure path)")
     ap.add_argument("--quorums", type=int, default=int(os.environ.get("BLSGPU_BENCH_QUORUMS", 10_000)), help="cfg 5 quorums of 400 members")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the status vectors of the last timed step of each leg, and of one untimed call on the batch "
+                         "with planted rejections, as DIR/<name>.npy (float32)")
     args = ap.parse_args()
     _claim_stdout()
 
@@ -301,6 +353,8 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs applies to the engine (--impl engine)")
         run_reference(args, rank, world)
         return
 
@@ -339,12 +393,14 @@ def main():
     np_pk, np_sig, np_msg, np_off = h_pk.numpy(), h_sig.numpy(), h_msg.numpy(), h_off.numpy().view(np.uint64)
 
     host_ms, host_dev_ms = [], []
+    last = {}  # the statuses each leg returned in its latest step (--dump-outputs)
 
     def step_host():
         t0 = time.perf_counter()
         st = eng.verify_batch_packed(impl, scheme, np_pk, np_sig, np_msg, np_off)
         host_ms.append((time.perf_counter() - t0) * 1e3)
         host_dev_ms.append(sum(eng.last_stage_ms().values()))
+        last["e2e_status"] = st
         return st
 
     def barrier():
@@ -386,13 +442,14 @@ def main():
     kernels = eng.last_kernel_ms()
     sampler.stop_flag = True
     sampler.join(timeout=2)
-    assert int(d_status.max().item()) == 0
+    last["verify_status"] = d_status.cpu().numpy()
+    assert int(last["verify_status"].max()) == 0
 
     # e2e through the host-buffer call
     for _ in range(max(1, args.warmup)):  # the same W warm-up calls as the device leg (the first calls grow the arena)
         st = step_host()
     assert int(st.max()) == 0
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
     ms_e2e = timed(step_host, e2e_steps)
 
     value = world * n * args.steps / (ms_total * 1e-3)
@@ -462,7 +519,9 @@ def main():
         s_pk, s_sig, s_msg, s_off = synth_batch(eng, n, seed=1000)
 
     def step_strong():
-        return B.verify_batch_folded(eng, impl, scheme, s_pk, s_sig, s_msg, s_off, rank, world, all_gather_parts)
+        r = B.verify_batch_folded(eng, impl, scheme, s_pk, s_sig, s_msg, s_off, rank, world, all_gather_parts)
+        last["strong_status"] = r[1]
+        return r
 
     lo_s, st = step_strong()
     assert int(st.max()) == 0
@@ -470,6 +529,18 @@ def main():
     line["strong_scaling"] = {"batch": n, "n_gpus": world, "ms_per_batch": ms_strong / e2e_steps, "value": n * e2e_steps / (ms_strong * 1e-3),
                               "unit": UNIT, "exchange_bytes_per_rank": 672,
                               "what": "ONE batch cut over the ranks: per-rank partial Fp12 + partial sum, all_gather, single final exponentiation"}
+    if rank == 0 and args.dump_outputs:
+        # the timed batch is all valid, so its statuses cannot tell a correct build from one that accepts everything:
+        # the same device call, after the timed legs, on a copy with planted rejections
+        p_pk, p_sig, want = plant_rejections(pks, sigs, n)
+        d_ppk, d_psig = torch.from_numpy(p_pk).to(dev), torch.from_numpy(p_sig).to(dev)
+        d_pstatus = torch.empty(n, dtype=torch.uint8, device=dev)
+        torch.cuda.synchronize()
+        eng.verify_batch_dev(impl, scheme, n, d_ppk.data_ptr(), d_psig.data_ptr(), d_msg.data_ptr(), d_off.data_ptr(), d_pstatus.data_ptr())
+        stream.synchronize()
+        last["planted_status"] = d_pstatus.cpu().numpy()
+        dump_outputs(args.dump_outputs, last)
+        assert np.array_equal(last["planted_status"], want), "the planted rejections must be found exactly"
     if rank == 0 and world == 1 and not args.no_configs:
         line["configs"] = other_configs(eng, B, (pks, sigs, msgs, off), peak_mac, args.quorums)
     if rank == 0 and not args.no_cpu_baseline and world == 1:

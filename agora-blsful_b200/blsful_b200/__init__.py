@@ -7,6 +7,7 @@ argument meaning and error behaviour:
   Signature::verify            -> verify_batch            (reference src/signature.rs:130-138)
   ProofOfPossession::verify    -> pop_verify_batch        (src/proof_of_possession.rs:77-81)
   AggregateSignature::verify   -> aggregate_verify        (src/aggregate_signature.rs:230-239)
+                               -> aggregate_verify_batch_status (q aggregates in one call)
   MultiSignature / AggregateSignature::from_signatures, MultiPublicKey::from_public_keys
                                -> sum_signatures / sum_public_keys (src/multi_signature.rs:80-107, multi_public_key.rs:79-83)
   Signature::verify_secure[_with_mode] -> verify_secure_batch   (src/signature.rs:177-197,256-276)
@@ -115,6 +116,7 @@ def load_library() -> ctypes.CDLL:
         "blsgpu_partial_finish": (c.c_int, [vp, c.c_int, u8p]),
         "blsgpu_pop_verify_batch": (c.c_int, [vp, c.c_int, c.c_int, c.c_size_t, u8p, u8p, u8p]),
         "blsgpu_aggregate_verify": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u8p, u8p, u64p, u8p, u8p, i64p]),
+        "blsgpu_aggregate_verify_batch": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u64p, u8p, u8p, u64p, u8p, u8p, i64p]),
         "blsgpu_sum_points": (c.c_int, [vp, c.c_int, c.c_int, c.c_size_t, u8p, u8p, u8p, i64p]),
         "blsgpu_verify_secure_batch": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u64p, u8p, u8p, u8p, u64p, u8p]),
         "blsgpu_aggregate_secure_batch": (c.c_int, [vp, c.c_int, c.c_int, c.c_size_t, u64p, u8p, u8p, u8p, u8p]),
@@ -151,7 +153,7 @@ EXPORTED_SYMBOLS = [
     "blsgpu_ctx_set_stream",
     "blsgpu_verify_batch",
     "blsgpu_miller_partial", "blsgpu_final_exp_is_one", "blsgpu_partial_finish",
-    "blsgpu_verify_batch_dev", "blsgpu_pop_verify_batch", "blsgpu_aggregate_verify", "blsgpu_sum_points",
+    "blsgpu_verify_batch_dev", "blsgpu_pop_verify_batch", "blsgpu_aggregate_verify", "blsgpu_aggregate_verify_batch", "blsgpu_sum_points",
     "blsgpu_verify_secure_batch", "blsgpu_aggregate_secure_batch", "blsgpu_hash_to_curve_batch", "blsgpu_recode_points",
     "blsgpu_fp_mul_batch", "blsgpu_pairing_product_is_one", "blsgpu_testdata_sign", "blsgpu_imad_peak",
     "blsgpu_combine_shares_batch", "blsgpu_verify_batch_wire", "blsgpu_pairing_check_batch",
@@ -367,6 +369,45 @@ class Engine:
                                                _ptr(status), _ptr(idx))
         self._check(rc, "blsgpu_aggregate_verify")
         return int(status[0]), (int(idx[0]), int(idx[1]))
+
+    def aggregate_verify_batch_status(self, impl_id: int, scheme: int, sets: Sequence[Tuple[Sequence[bytes], Sequence[bytes]]],
+                                      sigs, fmt: int = SerializationFormat.Modern) -> Tuple[np.ndarray, np.ndarray]:
+        """q x aggregate_verify_status in one engine call: sets[j] = (pks, msgs) of aggregate j, sigs[j] its signature.
+        Returns (status uint8[q], index int64[q, 2]) with the meaning aggregate_verify_status gives each aggregate alone."""
+        q = len(sets)
+        pl = pk_len(impl_id)
+        flat_pks, flat_msgs = [], []
+        soff = np.zeros(q + 1, dtype=np.uint64)
+        for j, (pks, msgs) in enumerate(sets):
+            pk = _pack_points(pks, pl, "public key")
+            if len(msgs) != pk.size // pl:
+                raise BlsError(ST_MISMATCHED_LENGTHS)
+            flat_pks.append(pk)
+            flat_msgs.extend(msgs)
+            soff[j + 1] = soff[j] + pk.size // pl
+        if isinstance(sigs, np.ndarray):
+            sg = _pack_points(sigs, sig_len(impl_id), "signature")
+        else:
+            for s in sigs:
+                if len(s) != sig_len(impl_id):
+                    raise BlsError(ST_INVALID_LENGTH, "signature")
+            sg = np.frombuffer(b"".join(bytes(s) for s in sigs), dtype=np.uint8)
+        if sg.size // sig_len(impl_id) != q:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        pk = np.concatenate(flat_pks) if flat_pks else np.zeros(0, dtype=np.uint8)
+        data, off = pack_messages(flat_msgs)
+        return self.aggregate_verify_batch_packed(impl_id, scheme, soff, pk, data, off, sg, fmt)
+
+    def aggregate_verify_batch_packed(self, impl_id, scheme, set_off: np.ndarray, pk: np.ndarray, data: np.ndarray, off: np.ndarray,
+                                      sg: np.ndarray, fmt: int = SerializationFormat.Modern) -> Tuple[np.ndarray, np.ndarray]:
+        """Flat-buffer form: set_off[q + 1] pair offsets per aggregate, pk / data / off over all pairs, sg q signatures."""
+        q = set_off.size - 1
+        status = np.zeros(q, dtype=np.uint8)
+        idx = np.full((q, 2), -1, dtype=np.int64)
+        rc = self._lib.blsgpu_aggregate_verify_batch(self._ctx, impl_id, scheme, fmt, q, _ptr(set_off), _ptr(pk), _ptr(data), _ptr(off),
+                                                     _ptr(sg), _ptr(status), _ptr(idx))
+        self._check(rc, "blsgpu_aggregate_verify_batch")
+        return status, idx
 
     # ---- point sums -------------------------------------------------------------------------------------------------
     def sum_points(self, group: int, points, fmt: int = SerializationFormat.Modern) -> bytes:

@@ -409,6 +409,57 @@ int probe_level(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, const std::vector<uint32_t>
   return BLSGPU_OK;
 }
 
+// The Miller stage over n items: F[g] = prod over the items of group g of ML(r pk, H), after ctx->ev_fork.  prep(stream, cn,
+// base, args) launches the kernel that fills the M6Arg records of items [base, base + cn).  The line stream is 39 KB per item:
+// batches beyond one pass (ctx->m6_chunk) go through in chunks with two line buffers, chunk c's lines produced on side
+// stream 0 while chunk c-1's accumulator consumes the other buffer on side stream 1.  Line buffer 0 is left in P.big_* for
+// the probes of the failure path.
+template <class PkA, class SigA, class Prep>
+int miller_stage(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t n, const PkA* d_pk, const SigA* d_h, const uint8_t* d_status, Fp12* d_F,
+                 const Prep& prep) {
+  const size_t M6_CHUNK = ctx->m6_chunk;  // planned by the entry point together with the arena size (plan_m6_chunk)
+  const size_t chunk = std::max<size_t>(std::min(n, M6_CHUNK), 6 * PROBE_SMALL);
+  const int nbuf = n > M6_CHUNK ? 2 : 1;
+  M6Arg* d_args[2];
+  SLineRec* d_lines[2];
+  for (int b = 0; b < nbuf; b++) {
+    d_args[b] = ctx->arena.take<M6Arg>(chunk);
+    d_lines[b] = ctx->arena.take<SLineRec>(chunk * M6_LINE_RECS);
+  }
+  P.big_args = d_args[0];
+  P.big_lines = d_lines[0];
+  P.big_items = chunk;
+  ARENA_OK();
+  CK(cudaStreamWaitEvent(ctx->side[0], ctx->ev_fork, 0));
+  CK(cudaStreamWaitEvent(ctx->side[1], ctx->ev_fork, 0));
+  size_t ci = 0;
+  for (size_t base = 0; base < n; base += M6_CHUNK, ci++) {
+    const size_t cn = std::min(M6_CHUNK, n - base);
+    const int b = (int)(ci % nbuf);
+    if (ci >= (size_t)nbuf) CK(cudaStreamWaitEvent(ctx->side[0], ctx->ev_accum[b], 0));  // the buffer's previous reader is done
+    size_t km = kernel_begin(ctx, BLSGPU_KERNEL_M6_PREP, ctx->side[0]);
+    prep(ctx->side[0], cn, base, d_args[b]);
+    kernel_end(ctx, km, ctx->side[0]);
+    CKR(check_launch(ctx, "k_m6_prep"));
+    km = kernel_begin(ctx, BLSGPU_KERNEL_M6_LINES, ctx->side[0]);
+    k_m6_lines<PkA, SigA><<<blocks_for(cn, M6_LINES_PAIRS), M6_LINES_TPB, M6_LINES_SMEM, ctx->side[0]>>>(
+        cn, base, d_args[b], d_pk, d_h, d_status, d_lines[b]);
+    kernel_end(ctx, km, ctx->side[0]);
+    CKR(check_launch(ctx, "k_m6_lines"));
+    CK(cudaEventRecord(ctx->ev_lines[b], ctx->side[0]));
+    CK(cudaStreamWaitEvent(ctx->side[1], ctx->ev_lines[b], 0));
+    km = kernel_begin(ctx, BLSGPU_KERNEL_M6_ACCUM, ctx->side[1]);
+    k_m6_accum<<<blocks_for(cn, M6_ITEMS_PER_BLOCK), 128, M6_ACCUM_SMEM, ctx->side[1]>>>(cn, base, d_status, d_lines[b], d_F);
+    kernel_end(ctx, km, ctx->side[1]);
+    CKR(check_launch(ctx, "k_m6_accum"));
+    CK(cudaEventRecord(ctx->ev_accum[b], ctx->side[1]));
+  }
+  // join: everything later on the caller's stream waits for the last accumulator (which waited for every line kernel)
+  CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_accum[(ci - 1) % nbuf], 0));
+  if (ci >= 2) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_accum[(ci - 2) % nbuf], 0));
+  return BLSGPU_OK;
+}
+
 template <class PkA, class SigA>
 int pipeline_partials(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t n, const PkA* d_pk, const SigA* d_sig, const SigA* d_h, uint8_t* d_status,
                       bool use_rlc) {
@@ -499,51 +550,9 @@ int pipeline_partials(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t n, const PkA* 
     P.root_T_ready = true;
   }
   stage_mark(ctx, BLSGPU_STAGE_MILLER);
-  {
-    // The line stream is 39 KB per item.  Batches beyond one pass (ctx->m6_chunk) go through in chunks with two line buffers:
-    // chunk c's lines are produced on side stream 0 while chunk c-1's accumulator consumes the other buffer on side stream 1.
-    const size_t M6_CHUNK = ctx->m6_chunk;  // planned by the entry point together with the arena size (plan_m6_chunk)
-    const size_t chunk = std::max<size_t>(std::min(n, M6_CHUNK), 6 * PROBE_SMALL);
-    const int nbuf = n > M6_CHUNK ? 2 : 1;
-    M6Arg* d_args[2];
-    SLineRec* d_lines[2];
-    for (int b = 0; b < nbuf; b++) {
-      d_args[b] = ctx->arena.take<M6Arg>(chunk);
-      d_lines[b] = ctx->arena.take<SLineRec>(chunk * M6_LINE_RECS);
-    }
-    P.big_args = d_args[0];
-    P.big_lines = d_lines[0];
-    P.big_items = chunk;
-    ARENA_OK();
-    CK(cudaStreamWaitEvent(ctx->side[0], ctx->ev_fork, 0));
-    CK(cudaStreamWaitEvent(ctx->side[1], ctx->ev_fork, 0));
-    size_t ci = 0;
-    for (size_t base = 0; base < n; base += M6_CHUNK, ci++) {
-      const size_t cn = std::min(M6_CHUNK, n - base);
-      const int b = (int)(ci % nbuf);
-      if (ci >= (size_t)nbuf) CK(cudaStreamWaitEvent(ctx->side[0], ctx->ev_accum[b], 0));  // the buffer's previous reader is done
-      size_t km = kernel_begin(ctx, BLSGPU_KERNEL_M6_PREP, ctx->side[0]);
-      k_m6_prep<PkA, SigA><<<blocks_for(cn), TPB, 0, ctx->side[0]>>>(cn, base, d_pk, d_h, (const uint8_t*)d_status, (const Digest*)d_root,
-                                                                      rbits, d_args[b]);
-      kernel_end(ctx, km, ctx->side[0]);
-      CKR(check_launch(ctx, "k_m6_prep"));
-      km = kernel_begin(ctx, BLSGPU_KERNEL_M6_LINES, ctx->side[0]);
-      k_m6_lines<PkA, SigA><<<blocks_for(cn, M6_LINES_PAIRS), M6_LINES_TPB, M6_LINES_SMEM, ctx->side[0]>>>(
-          cn, base, d_args[b], d_pk, d_h, d_status, d_lines[b]);
-      kernel_end(ctx, km, ctx->side[0]);
-      CKR(check_launch(ctx, "k_m6_lines"));
-      CK(cudaEventRecord(ctx->ev_lines[b], ctx->side[0]));
-      CK(cudaStreamWaitEvent(ctx->side[1], ctx->ev_lines[b], 0));
-      km = kernel_begin(ctx, BLSGPU_KERNEL_M6_ACCUM, ctx->side[1]);
-      k_m6_accum<<<blocks_for(cn, M6_ITEMS_PER_BLOCK), 128, M6_ACCUM_SMEM, ctx->side[1]>>>(cn, base, d_status, d_lines[b], d_F);
-      kernel_end(ctx, km, ctx->side[1]);
-      CKR(check_launch(ctx, "k_m6_accum"));
-      CK(cudaEventRecord(ctx->ev_accum[b], ctx->side[1]));
-    }
-    // join: everything later on the caller's stream waits for the last accumulator (which waited for every line kernel)
-    CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_accum[(ci - 1) % nbuf], 0));
-    if (ci >= 2) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_accum[(ci - 2) % nbuf], 0));
-  }
+  CKR((miller_stage<PkA, SigA>(ctx, P, n, d_pk, d_h, d_status, d_F, [&](cudaStream_t s, size_t cn, size_t base, M6Arg* args) {
+    k_m6_prep<PkA, SigA><<<blocks_for(cn), TPB, 0, s>>>(cn, base, d_pk, d_h, (const uint8_t*)d_status, (const Digest*)d_root, rbits, args);
+  })));
   if (use_msm) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_aux, 0));  // T = ML(-g, S) ran beside the Miller stage
   if (use_rlc && !use_msm) {
     LAUNCH((k_scale_sig<SigA>), blocks_for(n), TPB, n, d_sig, d_status, d_root, rbits, P.d_Sitem);
@@ -578,6 +587,46 @@ int pipeline_check(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, bool* ok_out) {
   return BLSGPU_OK;
 }
 
+// Walks a failing tree (P.lv over P.d_F / P.d_S, root failed) down to its failing leaves: bad = the leaf indices whose node
+// probe fails.  Children of node j at level k+1 are {j + m * cnt(k+1)} at level k.  A round of probes costs ~9 ms whatever
+// its size (one cooperative Miller pass + one final-exponentiation launch, both latency), so a round goes down as many levels
+// as it can while the candidates stay below BISECT_FANOUT: one bad signature in 1M is found in 3 rounds instead of 6.
+// before_leaves(cand) runs once, before the probes of the leaf level (it may fill in leaf sums of P.d_S).
+template <class PkA, class SigA, class BeforeLeaves>
+int descend_tree(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, std::vector<uint32_t>& bad, const BeforeLeaves& before_leaves) {
+  const std::vector<Level>& lv = P.lv;
+  const size_t one_round = P.big_items >= 6 * PROBE_SMALL ? std::min(P.x_cap, P.big_items / 6) : PROBE_SMALL;  // what probe_level takes at once
+  const size_t BISECT_FANOUT = std::min<size_t>(1024, one_round);
+  auto children = [&](const std::vector<uint32_t>& nodes, size_t level) {  // nodes at `level` -> their children at level - 1
+    std::vector<uint32_t> out;
+    const size_t cn = lv[level].cnt;
+    for (uint32_t j : nodes)
+      for (int m = 0; m < 16; m++) {
+        size_t idx = (size_t)j + (size_t)m * cn;
+        if (idx < lv[level - 1].cnt) out.push_back((uint32_t)idx);
+      }
+    return out;
+  };
+  bad.assign(1, 0);
+  std::vector<uint8_t> res;
+  for (size_t k = lv.size() - 1; k > 0;) {
+    std::vector<uint32_t> cand = children(bad, k);
+    k--;
+    while (k > 0 && cand.size() * 16 <= BISECT_FANOUT) {
+      cand = children(cand, k);
+      k--;
+    }
+    if (cand.empty()) break;
+    if (k == 0) CKR(before_leaves(cand));
+    CKR((probe_level<PkA, SigA>(ctx, P, cand, P.d_F + lv[k].off, P.d_S + lv[k].off, res)));
+    bad.clear();
+    for (size_t c = 0; c < cand.size(); c++)
+      if (!res[c]) bad.push_back(cand[c]);
+    if (bad.empty()) break;  // cannot happen for a failing parent; defensive
+  }
+  return BLSGPU_OK;
+}
+
 // the slice's check failed: per-group sums, descent of the 16-ary tree, exact per-item checks of the failing groups
 template <class PkA, class SigA>
 int pipeline_bisect(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P) {
@@ -603,54 +652,25 @@ int pipeline_bisect(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P) {
     for (size_t k = 1; k + 1 < lv.size(); k++)
       REDUCE_JAC(SigJ, lv[k].cnt, (const SigJ*)(P.d_S + lv[k].off), lv[k + 1].cnt, P.d_S + lv[k + 1].off);
   }
-  // walk down the 16-ary tree to the failing groups: children of node j at level k+1 are {j + m * cnt(k+1)} at level k
-  // A round of probes costs ~9 ms whatever its size (one cooperative Miller pass + one final-exponentiation launch, both
-  // latency), so a round goes down as many levels as it can while the candidates stay below BISECT_FANOUT: one bad signature
-  // in 1M is found in 3 rounds instead of 6.
-  const size_t one_round = P.big_items >= 6 * PROBE_SMALL ? std::min(P.x_cap, P.big_items / 6) : PROBE_SMALL;  // what probe_level takes at once
-  const size_t BISECT_FANOUT = std::min<size_t>(1024, one_round);
-  auto children = [&](const std::vector<uint32_t>& nodes, size_t level) {  // nodes at `level` -> their children at level - 1
-    std::vector<uint32_t> out;
-    const size_t cn = lv[level].cnt;
-    for (uint32_t j : nodes)
-      for (int m = 0; m < 16; m++) {
-        size_t idx = (size_t)j + (size_t)m * cn;
-        if (idx < lv[level - 1].cnt) out.push_back((uint32_t)idx);
-      }
-    return out;
-  };
-  std::vector<uint32_t> bad{0};
-  std::vector<uint8_t> res;
-  for (size_t k = lv.size() - 1; k > 0;) {
-    std::vector<uint32_t> cand = children(bad, k);
-    k--;
-    while (k > 0 && cand.size() * 16 <= BISECT_FANOUT) {
-      cand = children(cand, k);
-      k--;
-    }
-    if (cand.empty()) break;
-    if (k == 0 && by_nodes) {
-      // the candidate groups (children of failing level-1 nodes) get their sums now: r_i sig_i for their items only
-      std::vector<uint32_t> its;
-      for (uint32_t g : cand)
-        for (int m = 0; m < M6_GROUP; m++)
-          if ((size_t)g * M6_GROUP + m < n) its.push_back(g * M6_GROUP + m);
-      uint32_t* d_list = ctx->arena.take<uint32_t>(its.size() + cand.size());
-      ARENA_OK();
-      CK(cudaMemcpyAsync(d_list, its.data(), its.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-      CK(cudaMemcpyAsync(d_list + its.size(), cand.data(), cand.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-      LAUNCH((k_scale_sig_list<SigA>), blocks_for(its.size()), TPB, its.size(), (const uint32_t*)d_list, P.d_sig, (const uint8_t*)P.d_status,
-             (const Digest*)P.d_root, P.rbits, P.d_Sitem);
-      LAUNCH((k_group_sum_list<SigJ>), blocks_for(cand.size()), TPB, cand.size(), (const uint32_t*)(d_list + its.size()), n, (const SigJ*)P.d_Sitem,
-             P.d_S + lv[0].off);
-      CK(cudaStreamSynchronize(ctx->stream));  // the host vectors go out of scope
-    }
-    CKR((probe_level<PkA, SigA>(ctx, P, cand, P.d_F + lv[k].off, P.d_S + lv[k].off, res)));
-    bad.clear();
-    for (size_t c = 0; c < cand.size(); c++)
-      if (!res[c]) bad.push_back(cand[c]);
-    if (bad.empty()) break;  // cannot happen for a failing parent; defensive
-  }
+  std::vector<uint32_t> bad;
+  CKR((descend_tree<PkA, SigA>(ctx, P, bad, [&](const std::vector<uint32_t>& cand) -> int {
+    if (!by_nodes) return BLSGPU_OK;
+    // the candidate groups (children of failing level-1 nodes) get their sums now: r_i sig_i for their items only
+    std::vector<uint32_t> its;
+    for (uint32_t g : cand)
+      for (int m = 0; m < M6_GROUP; m++)
+        if ((size_t)g * M6_GROUP + m < n) its.push_back(g * M6_GROUP + m);
+    uint32_t* d_list = ctx->arena.take<uint32_t>(its.size() + cand.size());
+    ARENA_OK();
+    CK(cudaMemcpyAsync(d_list, its.data(), its.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_list + its.size(), cand.data(), cand.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+    LAUNCH((k_scale_sig_list<SigA>), blocks_for(its.size()), TPB, its.size(), (const uint32_t*)d_list, P.d_sig, (const uint8_t*)P.d_status,
+           (const Digest*)P.d_root, P.rbits, P.d_Sitem);
+    LAUNCH((k_group_sum_list<SigJ>), blocks_for(cand.size()), TPB, cand.size(), (const uint32_t*)(d_list + its.size()), n, (const SigJ*)P.d_Sitem,
+           P.d_S + lv[0].off);
+    CK(cudaStreamSynchronize(ctx->stream));  // the host vectors go out of scope
+    return BLSGPU_OK;
+  })));
   // every item of a failing group is decided by its own exact equation e(pk_i, H_i) e(-g, sig_i) == 1
   std::vector<uint32_t> items;
   for (uint32_t gidx : bad)
@@ -1598,6 +1618,263 @@ int blsgpu_aggregate_verify(blsgpu_ctx* ctx, int impl_id, int scheme, int format
                         : aggregate_verify_multi<1>(ctx, scheme, format, n, pks, msgs, msg_off, sig, status_out, index_out);
   return impl_id == 2 ? aggregate_verify_impl<2>(ctx, scheme, format, n, pks, msgs, msg_off, sig, status_out, index_out)
                       : aggregate_verify_impl<1>(ctx, scheme, format, n, pks, msgs, msg_off, sig, status_out, index_out);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// q x AggregateSignature::verify in one pipeline.  The host applies agg_host_checks per aggregate; the live aggregates share
+// one Miller stage in which aggregate j fills whole groups of slots and every pair of it is scaled by ONE scalar r_j, so
+//   F_j = prod_{i in j} ML(r_j pk_i, H_i)          (segmented product of its groups' values)
+//   S_j = r_j sig_j                                   (k_scale_sig with the aggregate as the item)
+// and a 16-ary tree over the q leaves (F_j, S_j) is checked at its root and descended with node probes on failure.
+// set_off / msg_off start at 0 here (the entry point rebases them).
+template <int IMPL>
+static int aggregate_batch_impl(blsgpu_ctx* ctx, int scheme, int format, size_t q, const uint64_t* set_off, const uint8_t* pks,
+                                const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* sigs, uint8_t* status_out, int64_t* index_out) {
+  typedef typename ImplT<IMPL>::PkAff PkA;
+  typedef typename ImplT<IMPL>::SigAff SigA;
+  typedef typename PtInfo<SigA>::Jac SigJ;
+  const size_t Lp = PtInfo<PkA>::LEN, Ls = PtInfo<SigA>::LEN;
+  const size_t np = (size_t)set_off[q], msg_bytes = (size_t)msg_off[np];
+  // layout: aggregate j owns groups g_first[j] .. g_first[j+1]-1, at least one (an empty or decided aggregate's group is all
+  // padding, so its F_j is 1)
+  std::vector<size_t> g_first(q + 1, 0);
+  for (size_t j = 0; j < q; j++) g_first[j + 1] = g_first[j] + std::max<size_t>(1, (size_t)(set_off[j + 1] - set_off[j] + M6_GROUP - 1) / M6_GROUP);
+  const size_t ng = g_first[q], nslots = ng * M6_GROUP;
+  // the segmented product: levels of ranges of <= 16 consecutive nodes of one aggregate, until one node per aggregate
+  std::vector<uint32_t> seg_off;       // every level's n_out + 1 range offsets, concatenated
+  std::vector<size_t> seg_n{ng};       // nodes per level (level 0: the groups)
+  {
+    std::vector<size_t> cnt(q);
+    for (size_t j = 0; j < q; j++) cnt[j] = g_first[j + 1] - g_first[j];
+    while (seg_n.back() > q) {
+      uint32_t in = 0;
+      size_t outs = 0;
+      seg_off.push_back(0);
+      for (size_t j = 0; j < q; j++) {
+        const size_t o = (cnt[j] + 15) / 16;
+        for (size_t k = 0; k < o; k++) {
+          in += (uint32_t)std::min<size_t>(16, cnt[j] - 16 * k);
+          seg_off.push_back(in);
+        }
+        cnt[j] = o;
+        outs += o;
+      }
+      seg_n.push_back(outs);
+    }
+  }
+  size_t seg_total = 0;
+  for (size_t k = 0; k + 1 < seg_n.size(); k++) seg_total += seg_n[k];  // every level but the last (which is the set tree's)
+  Pipe<PkA, SigA> P;
+  P.lv = make_levels(q);
+  const size_t qtotal = levels_total(P.lv), ndig = levels_total(make_levels(np + q));
+  P.x_cap = std::max<size_t>(PROBE_SMALL, std::min<size_t>(q, 4096) + 16);
+  size_t head = np * (Lp + sizeof(PkA) + sizeof(SigA) + 2) + msg_bytes + (np + 1) * 8 + q * (Ls + sizeof(SigA) + 2) + (q + 1) * 8 +
+                np * sizeof(SigJ) + (ndig + 2) * sizeof(Digest) + nslots * (sizeof(PkA) + sizeof(SigA) + 1 + 4) + ng * 4 +
+                seg_off.size() * 4 + seg_total * sizeof(Fp12) + qtotal * (sizeof(Fp12) + sizeof(SigJ)) + P.x_cap * 5 +
+                P.x_cap * (6 * (sizeof(PkA) + sizeof(SigA) + 1) + sizeof(Fp12)) + 6 * PROBE_SMALL * M6_ITEM_BYTES + 40 * 256;
+  CKR((ensure_pipeline_arena<PkA, SigA>(ctx, nslots, head)));
+  stage_reset(ctx);
+  uint8_t *d_pkb, *d_sigb, *d_msgs;
+  uint64_t *d_moff, *d_soff;
+  CKR(upload(ctx, d_pkb, pks, np * Lp));
+  CKR(upload(ctx, d_sigb, sigs, q * Ls));
+  CKR(upload(ctx, d_msgs, msgs, msg_bytes));
+  CKR(upload(ctx, d_moff, msg_off, np + 1));
+  CKR(upload(ctx, d_soff, set_off, q + 1));
+  PkA* d_pk = ctx->arena.take<PkA>(std::max<size_t>(np, 1));
+  SigA* d_sig = ctx->arena.take<SigA>(q);
+  uint8_t* d_st = ctx->arena.take<uint8_t>(np + q);  // decode statuses: the pks, then the signatures
+  ARENA_OK();
+  stage_mark(ctx, BLSGPU_STAGE_DECODE_PK);
+  if (np) CKR((decode_points<PkA>(ctx, np, (const uint8_t*)d_pkb, format, d_pk, d_st, BLSGPU_KERNEL_DECODE_PK)));
+  stage_mark(ctx, BLSGPU_STAGE_DECODE_SIG);
+  CKR((decode_points<SigA>(ctx, q, (const uint8_t*)d_sigb, format, d_sig, d_st + np, BLSGPU_KERNEL_DECODE_SIG)));
+  std::vector<uint8_t> st(np + q);
+  std::vector<uint32_t> inf(np + q);
+  CK(cudaMemcpyAsync(st.data(), d_st, np + q, cudaMemcpyDeviceToHost, ctx->stream));
+  if (np) CK(cudaMemcpy2DAsync(inf.data(), 4, reinterpret_cast<const uint8_t*>(d_pk) + offsetof(PkA, inf), sizeof(PkA), 4, np, cudaMemcpyDeviceToHost,
+                               ctx->stream));
+  CK(cudaMemcpy2DAsync(inf.data() + np, 4, reinterpret_cast<const uint8_t*>(d_sig) + offsetof(SigA, inf), sizeof(SigA), 4, q, cudaMemcpyDeviceToHost,
+                       ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  // the reference's checks per aggregate, in its order; a decided aggregate takes no part in the pairing work
+  std::vector<uint8_t> agg_pre(q, BLSGPU_ST_OK), pair_pre(np, PROBE_SKIP);
+  std::vector<uint32_t> slot_src(nslots, 0xffffffffu), g_set(ng);
+  size_t live = 0;
+  {
+    std::vector<uint8_t> st_j;
+    std::vector<uint32_t> inf_j;
+    for (size_t j = 0; j < q; j++) {
+      const size_t lo = (size_t)set_off[j], n = (size_t)set_off[j + 1] - lo;
+      st_j.assign(st.begin() + lo, st.begin() + lo + n);
+      st_j.push_back(st[np + j]);
+      inf_j.assign(inf.begin() + lo, inf.begin() + lo + n);
+      inf_j.push_back(inf[np + j]);
+      for (size_t g = g_first[j]; g < g_first[j + 1]; g++) g_set[g] = (uint32_t)j;
+      if (agg_host_checks(scheme, n, st_j.data(), inf_j.data(), msgs, msg_off + lo, status_out + j, index_out + 2 * j)) {
+        agg_pre[j] = PROBE_SKIP;
+        continue;
+      }
+      live++;
+      for (size_t i = 0; i < n; i++) {
+        pair_pre[lo + i] = BLSGPU_ST_OK;
+        slot_src[g_first[j] * M6_GROUP + i] = (uint32_t)(lo + i);
+      }
+    }
+  }
+  if (live == 0) {
+    stage_collect(ctx);
+    return BLSGPU_OK;
+  }
+  uint8_t *d_pair_pre, *d_agg_pre;
+  uint32_t *d_src, *d_gset, *d_segoff;
+  CKR(upload(ctx, d_pair_pre, pair_pre.data(), np));
+  CKR(upload(ctx, d_agg_pre, agg_pre.data(), q));
+  CKR(upload(ctx, d_src, slot_src.data(), nslots));
+  CKR(upload(ctx, d_gset, g_set.data(), ng));
+  CKR(upload(ctx, d_segoff, seg_off.data(), seg_off.size()));
+  DstParam dst;
+  make_dst(dst, IMPL, scheme, false);
+  SigA* d_h = ctx->arena.take<SigA>(std::max<size_t>(np, 1));
+  stage_mark(ctx, BLSGPU_STAGE_HASH);
+  CKR((hash_points<SigA, PkA>(ctx, np, (const uint8_t*)d_msgs, (const uint64_t*)d_moff, scheme == 1 ? 1 : 0, (const PkA*)d_pk,
+                              (const uint8_t*)d_pair_pre, dst, d_h)));
+  // the scalars: r_j = rlc_scalar(root, j), root = 16-ary SHA-256 tree over every pk, hashed message, signature and range
+  Digest* d_dig = ctx->arena.take<Digest>(ndig + 2);
+  Digest* d_root = d_dig + ndig;  // [root, salt]
+  CKR(fresh_salt(ctx));
+  {
+    const std::vector<Level> ld = make_levels(np + q);
+    LAUNCH((k_agg_leaf_digest<PkA, SigA>), blocks_for(np + q), TPB, np, q, (const PkA*)d_pk, (const SigA*)d_h, (const SigA*)d_sig,
+           (const uint64_t*)d_soff, d_dig);
+    for (size_t k = 0; k + 1 < ld.size(); k++)
+      LAUNCH(k_digest_reduce, blocks_for(ld[k + 1].cnt), TPB, ld[k].cnt, d_dig + ld[k].off, ld[k + 1].cnt, d_dig + ld[k + 1].off);
+    CK(cudaMemcpyAsync(d_root, d_dig + ld.back().off, sizeof(Digest), cudaMemcpyDeviceToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_root + 1, ctx->salt, 32, cudaMemcpyHostToDevice, ctx->stream));
+  }
+  PkA* d_pks = ctx->arena.take<PkA>(nslots);
+  SigA* d_hs = ctx->arena.take<SigA>(nslots);
+  uint8_t* d_pres = ctx->arena.take<uint8_t>(nslots);
+  LAUNCH((k_agg_slots<PkA, SigA>), blocks_for(nslots), TPB, nslots, (const uint32_t*)d_src, (const PkA*)d_pk, (const SigA*)d_h, d_pks, d_hs, d_pres);
+  // the pipe of the set tree: leaves (F_j, S_j), probe scratch
+  P.n = nslots;
+  P.ng = q;
+  P.use_rlc = true;
+  P.use_msm = false;
+  const int rbits = P.rbits = ctx->rlc_bits;
+  P.d_pk = d_pks;
+  P.d_h = d_hs;
+  P.d_status = d_pres;
+  P.d_root = d_root;
+  P.d_F = ctx->arena.take<Fp12>(qtotal);
+  P.d_S = ctx->arena.take<SigJ>(qtotal);
+  P.d_ok = ctx->arena.take<uint8_t>(P.x_cap);
+  P.d_idx = ctx->arena.take<uint32_t>(P.x_cap);
+  P.x_pk = ctx->arena.take<PkA>(6 * P.x_cap);
+  P.x_h = ctx->arena.take<SigA>(6 * P.x_cap);
+  P.x_pre = ctx->arena.take<uint8_t>(6 * P.x_cap);
+  P.x_T = ctx->arena.take<Fp12>(P.x_cap);
+  P.x_args = ctx->arena.take<M6Arg>(6 * PROBE_SMALL);
+  P.x_lines = ctx->arena.take<SLineRec>(6 * PROBE_SMALL * M6_LINE_RECS);
+  Fp12* d_Fseg = ctx->arena.take<Fp12>(std::max<size_t>(seg_total, 1));
+  CK(cudaFuncSetAttribute(k_m6_lines<PkA, SigA>, cudaFuncAttributeMaxDynamicSharedMemorySize, M6_LINES_SMEM));
+  CK(cudaFuncSetAttribute(k_m6_accum, cudaFuncAttributeMaxDynamicSharedMemorySize, M6_ACCUM_SMEM));
+  CK(cudaFuncSetAttribute(k_final6, cudaFuncAttributeMaxDynamicSharedMemorySize, FE6_SMEM));
+  stage_mark(ctx, BLSGPU_STAGE_SCALE_SIG);
+  LAUNCH((k_scale_sig<SigA>), blocks_for(q), TPB, q, (const SigA*)d_sig, (const uint8_t*)d_agg_pre, (const Digest*)d_root, rbits, P.d_S);
+  CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
+  P.root_T_ready = false;
+  stage_mark(ctx, BLSGPU_STAGE_MILLER);
+  const bool segmented = seg_n.size() > 1;  // some aggregate spans more than one group
+  CKR((miller_stage<PkA, SigA>(ctx, P, nslots, d_pks, d_hs, d_pres, segmented ? d_Fseg : P.d_F,
+                               [&](cudaStream_t s, size_t cn, size_t base, M6Arg* args) {
+                                 k_m6_prep_sets<PkA, SigA><<<blocks_for(cn), TPB, 0, s>>>(cn, base, d_pks, d_hs, (const uint8_t*)d_pres,
+                                                                                          (const uint32_t*)d_gset, (const Digest*)d_root, rbits, args);
+                               })));
+  stage_mark(ctx, BLSGPU_STAGE_REDUCE);
+  {
+    size_t in_off = 0, out_off = seg_n[0], o = 0;
+    for (size_t k = 1; k < seg_n.size(); k++) {
+      const size_t n_out = seg_n[k];
+      const Fp12* in = d_Fseg + in_off;
+      Fp12* out = k + 1 == seg_n.size() ? P.d_F : d_Fseg + out_off;
+      if (n_out <= REDUCE_WIDE_MAX)
+        LAUNCH(k_seg_reduce_fp12_w, blocks_for(n_out * 16), TPB, n_out, (const uint32_t*)(d_segoff + o), in, out);
+      else
+        LAUNCH(k_seg_reduce_fp12, blocks_for(n_out), TPB, n_out, (const uint32_t*)(d_segoff + o), in, out);
+      o += n_out + 1;
+      in_off = out_off;
+      out_off += n_out;
+    }
+  }
+  const std::vector<Level>& lv = P.lv;
+  for (size_t k = 0; k + 1 < lv.size(); k++) {
+    REDUCE_FP12(lv[k].cnt, (const Fp12*)(P.d_F + lv[k].off), lv[k + 1].cnt, P.d_F + lv[k + 1].off);
+    REDUCE_JAC(SigJ, lv[k].cnt, (const SigJ*)(P.d_S + lv[k].off), lv[k + 1].cnt, P.d_S + lv[k + 1].off);
+  }
+  bool ok = false;
+  CKR((pipeline_check<PkA, SigA>(ctx, P, &ok)));
+  for (size_t j = 0; j < q; j++)
+    if (agg_pre[j] == BLSGPU_ST_OK) status_out[j] = BLSGPU_ST_OK;
+  if (!ok) {
+    std::vector<uint32_t> bad;
+    CKR((descend_tree<PkA, SigA>(ctx, P, bad, [](const std::vector<uint32_t>&) { return (int)BLSGPU_OK; })));
+    // Leaf j is exact, not a probabilistic verdict: its probe is final_exp(F_j * ML(-g, r_j sig_j)) =
+    // (prod_i e(pk_i, H_i) * e(-g, sig_j))^(3 r_j).  rlc_scalar never returns 0 and r_j < 2^128 < r, so gcd(3 r_j, r) = 1,
+    // and Gt has prime order r: the leaf is 1 exactly when aggregate j is valid.  Only an ACCEPT rests on the combination
+    // (probability >= 1 - 2^-bits per call, as for blsgpu_verify_batch).
+    for (uint32_t j : bad) status_out[j] = BLSGPU_ST_INVALID_SIGNATURE;
+  }
+  stage_mark(ctx, BLSGPU_STAGE_COUNT);
+  stage_collect(ctx);
+  return BLSGPU_OK;
+}
+
+int blsgpu_aggregate_verify_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t q, const uint64_t* set_off, const uint8_t* pks,
+                                  const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* sigs, uint8_t* status_out, int64_t* index_out) {
+  NVTX_RANGE("blsgpu_aggregate_verify_batch");
+  if (!ctx) return BLSGPU_E_ARG;
+  if (!args_ok(impl_id, scheme, format) || (q && (!set_off || !msg_off || !sigs || !status_out))) {
+    ctx->err = "blsgpu_aggregate_verify_batch: bad arguments";
+    return BLSGPU_E_ARG;
+  }
+  if (q == 0) return BLSGPU_OK;
+  CHECK_OFFSETS(set_off, q, "blsgpu_aggregate_verify_batch (set_off)");
+  const size_t p0 = (size_t)set_off[0], np = (size_t)set_off[q] - p0;
+  if (np > 0xfffffff0ull) {
+    ctx->err = "blsgpu_aggregate_verify_batch: at most 2^32 - 16 pairs per call";
+    return BLSGPU_E_ARG;
+  }
+  CHECK_OFFSETS(msg_off + p0, np, "blsgpu_aggregate_verify_batch (msg_off)");
+  if ((np && !pks) || (msg_off[p0 + np] > msg_off[p0] && !msgs)) {
+    ctx->err = "blsgpu_aggregate_verify_batch: pks or msgs is null";
+    return BLSGPU_E_ARG;
+  }
+  CKR(set_device(ctx));
+  std::vector<int64_t> idx_scratch;
+  if (!index_out) {
+    idx_scratch.resize(2 * q);
+    index_out = idx_scratch.data();
+  }
+  const size_t pk_len = impl_id == 2 ? 48 : 96, sig_len = impl_id == 2 ? 96 : 48;
+  // aggregates lo .. hi-1 on context c, with their pair and message offsets rebased to 0
+  auto run = [&](blsgpu_ctx* c, size_t lo, size_t hi) -> int {
+    const size_t a = (size_t)set_off[lo], b = (size_t)set_off[hi];
+    std::vector<uint64_t> so(hi - lo + 1), mo(b - a + 1);
+    for (size_t j = lo; j <= hi; j++) so[j - lo] = set_off[j] - a;
+    for (size_t i = a; i <= b; i++) mo[i - a] = msg_off[i] - msg_off[a];
+    const uint8_t* pk = pks ? pks + a * pk_len : nullptr;
+    const uint8_t* ms = msgs ? msgs + msg_off[a] : nullptr;
+    return impl_id == 2 ? aggregate_batch_impl<2>(c, scheme, format, hi - lo, so.data(), pk, ms, mo.data(), sigs + lo * sig_len, status_out + lo,
+                                                  index_out + 2 * lo)
+                        : aggregate_batch_impl<1>(c, scheme, format, hi - lo, so.data(), pk, ms, mo.data(), sigs + lo * sig_len, status_out + lo,
+                                                  index_out + 2 * lo);
+  };
+  const size_t ndev = 1 + ctx->peers.size();
+  if (ndev == 1 || np < ndev * SHARD_MIN_ITEMS) return run(ctx, 0, q);
+  // aggregates are independent: contiguous runs per device, balanced by pair count, nothing to fold
+  const std::vector<size_t> cut = balanced_cuts(q, set_off, ndev);
+  return run_on_devices(ctx, [&](blsgpu_ctx* c, size_t d) { return cut[d] == cut[d + 1] ? (int)BLSGPU_OK : run(c, cut[d], cut[d + 1]); });
 }
 
 // ---------------------------------------------------------------------------------------------------------------------

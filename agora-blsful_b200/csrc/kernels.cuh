@@ -1341,6 +1341,102 @@ __global__ void k_and_flags(size_t n, const uint8_t* flag, uint8_t* ok) {
   ok[i] = ok[i] && flag[i];
 }
 
+// ---- many aggregate signatures in one call (blsgpu_aggregate_verify_batch) ------------------------------------------------
+// Aggregate j owns pairs set_off[j] .. set_off[j+1]-1 and whole Miller groups of slots: its pairs are copied to slots, the
+// rest of its last group is padding (status "skip"), so no group straddles two aggregates.  One scalar r_j per aggregate.
+//
+// leaves of the digest that binds the scalars: one per pair (pk_i, H_i), then one per aggregate (sig_j, its pair range)
+template <class PkA, class SigA>
+__global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_agg_leaf_digest(size_t np, size_t q, const PkA* __restrict__ pk, const SigA* __restrict__ h,
+                                                         const SigA* __restrict__ sig, const uint64_t* __restrict__ set_off,
+                                                         Digest* __restrict__ out) {
+  const size_t t = BLS_TID();
+  if (t >= np + q) return;
+  Sha256 s;
+  sha256_init(s);
+  if (t < np) {
+    digest_point(s, pk[t]);
+    digest_point(s, h[t]);
+  } else {
+    const size_t j = t - np;
+    digest_point(s, sig[j]);
+    uint8_t b[16];
+    for (int k = 0; k < 8; k++) {
+      b[k] = (uint8_t)(set_off[j] >> (8 * k));
+      b[8 + k] = (uint8_t)(set_off[j + 1] >> (8 * k));
+    }
+    sha256_update(s, b, 16);
+  }
+  Digest d;
+  sha256_final(s, d.b);
+  out[t] = d;
+}
+// slot s <- pair src[s]; src[s] == 0xffffffff: padding or an aggregate decided before the pairing (skipped)
+template <class PkA, class SigA>
+__global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_agg_slots(size_t nslots, const uint32_t* __restrict__ src, const PkA* __restrict__ pk,
+                                                   const SigA* __restrict__ h, PkA* __restrict__ pk_s, SigA* __restrict__ h_s,
+                                                   uint8_t* __restrict__ pre_s) {
+  const size_t s = BLS_TID();
+  if (s >= nslots) return;
+  const uint32_t i = src[s];
+  if (i == 0xffffffffu) {
+    pre_s[s] = PROBE_SKIP;
+    return;
+  }
+  pk_s[s] = pk[i];
+  h_s[s] = h[i];
+  pre_s[s] = ST_OK;
+}
+// k_m6_prep with the scalar of the slot's AGGREGATE: r_{set(i)} = rlc_scalar(root, g_set[i / 6])
+template <class PkA, class HA>
+__global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_m6_prep_sets(size_t n, size_t base, const PkA* __restrict__ pk, const HA* __restrict__ h,
+                                                      const uint8_t* __restrict__ pre, const uint32_t* __restrict__ g_set,
+                                                      const Digest* __restrict__ root, int rbits, M6Arg* __restrict__ args) {
+  size_t c = BLS_TID();
+  if (c >= n) return;
+  const size_t i = base + c;
+  if (pre[i] != ST_OK) return;
+  G1Aff p = m6_g1(pk, h, i);
+  uint32_t sc[RLC_MAX_WORDS];
+  rlc_scalar(sc, root, g_set[i / M6_GROUP], rbits);
+  G1Jac pj;
+  jac_mul_aff_w4(pj, p, sc, rbits / 4);
+  MillerG1 mp;
+  miller_prepare(mp, pj);
+  M6Arg a;
+  const G2Aff q = m6_g2(pk, h, i);
+  m6_make_arg(a, mp, q);
+  args[c] = a;
+}
+// One level of the segmented product: out[j] = prod in[off[j] .. off[j+1]), ranges of at most 16 consecutive nodes of one
+// aggregate.  A thread per output node, or (_w, for levels with few nodes) sixteen lanes per node as in k_reduce_fp12_w.
+__global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_seg_reduce_fp12(size_t n_out, const uint32_t* __restrict__ off, const Fp12* __restrict__ in,
+                                                         Fp12* __restrict__ out) {
+  const size_t j = BLS_TID();
+  if (j >= n_out) return;
+  const uint32_t lo = off[j], hi = off[j + 1];
+  Fp12 acc = in[lo];
+  for (uint32_t m = lo + 1; m < hi; m++) {
+    Fp12 t = in[m];
+    fp12_mul(acc, acc, t);
+  }
+  out[j] = acc;
+}
+__global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_seg_reduce_fp12_w(size_t n_out, const uint32_t* __restrict__ off, const Fp12* __restrict__ in,
+                                                           Fp12* __restrict__ out) {
+  const size_t t = BLS_TID(), j = t >> 4;
+  const int m = (int)(t & 15);
+  Fp12 acc;
+  if (j < n_out && off[j] + m < off[j + 1]) acc = in[off[j] + m]; else fp12_one(acc);
+#pragma unroll 1
+  for (int s = 1; s < 16; s <<= 1) {
+    Fp12 other;
+    words_shfl_xor(other, acc, s);
+    if ((m & (2 * s - 1)) == 0) fp12_mul(acc, acc, other);
+  }
+  if (j < n_out && m == 0) out[j] = acc;
+}
+
 // synthetic data: pk = [k]G, sig = [k]H(frame(msg))
 template <class PkA, class SigA>
 __global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_testdata_sign(size_t n, const uint8_t* scalars, const uint8_t* msgs, const uint64_t* msg_off,

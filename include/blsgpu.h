@@ -64,7 +64,8 @@ typedef struct blsgpu_ctx blsgpu_ctx;
  * blsgpu_sum_points (per-device partial sums of contiguous slices, from 65,536 points per device, then the sum of the partial
  * results) and blsgpu_verify_secure_batch / blsgpu_aggregate_secure_batch (contiguous runs of key sets, balanced by member
  * count); blsgpu_aggregate_verify cuts its pairs over the devices (from 4096 per device) and folds the partial products of
- * Miller values on the first device.  Every other entry point, the *_dev variants and blsgpu_ctx_set_stream use the first device.  One process per
+ * Miller values on the first device; blsgpu_aggregate_verify_batch cuts its aggregates into contiguous runs balanced by pair
+ * count (from 4096 pairs per device), each verified on its own device without a fold.  Every other entry point, the *_dev variants and blsgpu_ctx_set_stream use the first device.  One process per
  * device with blsgpu_miller_partial / blsgpu_final_exp_is_one does the same across processes. */
 int blsgpu_ctx_create(const int* devices, int ndev, blsgpu_ctx** out);
 void blsgpu_ctx_destroy(blsgpu_ctx* ctx);
@@ -133,6 +134,17 @@ int blsgpu_pop_verify_batch(blsgpu_ctx* ctx, int impl_id, int format, size_t n, 
 int blsgpu_aggregate_verify(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t n, const uint8_t* pks,
                             const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* sig, uint8_t* status_out,
                             int64_t index_out[2]);
+/* q x AggregateSignature::verify (reference src/aggregate_signature.rs:230-239 -> sig_core.rs:149-178, sig_basic.rs:41-64 |
+ * sig_aug.rs:27-38 | sig_pop.rs:52-58).  Aggregate j owns pairs set_off[j]..set_off[j+1]-1 of pks / msgs (set_off has q+1
+ * non-decreasing entries, like key_off of blsgpu_verify_secure_batch); msg_off has set_off[q]+1 entries, one message per pair;
+ * sigs holds q aggregate signatures.  status_out[j] and index_out[2j..2j+1] (index_out may be NULL) mean exactly what
+ * blsgpu_aggregate_verify returns for aggregate j alone; indices are positions INSIDE aggregate j.  Duplicate messages
+ * (Basic) are looked for within an aggregate only.  One pipeline and one final exponentiation serve the whole call: every
+ * pair of aggregate j is weighted by one random scalar r_j, and a failing check is descended to the failing aggregates, each
+ * rejected by an exact equation (DESIGN.md section 2). */
+int blsgpu_aggregate_verify_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t q, const uint64_t* set_off,
+                                  const uint8_t* pks, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* sigs,
+                                  uint8_t* status_out, int64_t* index_out);
 
 /* ---- point sums ----------------------------------------------------------------------------------------------
  * Replaces aggregate_signatures / aggregate_public_keys (reference src/traits/sig_core.rs:38-59),

@@ -68,6 +68,9 @@ extern "C" {
     pub fn blsgpu_aggregate_verify(ctx: *mut blsgpu_ctx, impl_id: c_int, scheme: c_int, format: c_int, n: usize,
         pks: *const u8, msgs: *const u8, msg_off: *const u64, sig: *const u8, status_out: *mut u8,
         index_out: *mut i64 /* [2] */) -> c_int;
+    pub fn blsgpu_aggregate_verify_batch(ctx: *mut blsgpu_ctx, impl_id: c_int, scheme: c_int, format: c_int, q: usize,
+        set_off: *const u64, pks: *const u8, msgs: *const u8, msg_off: *const u64, sigs: *const u8, status_out: *mut u8,
+        index_out: *mut i64 /* [2 q] or null */) -> c_int;
     pub fn blsgpu_sum_points(ctx: *mut blsgpu_ctx, group: c_int, format: c_int, n: usize, points: *const u8,
         out: *mut u8, status_out: *mut u8, bad_index_out: *mut i64) -> c_int;
 

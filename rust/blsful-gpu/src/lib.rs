@@ -8,6 +8,7 @@
 //! | [`Engine::verify_batch`] | `Signature::verify` (src/signature.rs:130-138) |
 //! | [`Engine::pop_verify_batch`] | `ProofOfPossession::verify` (src/proof_of_possession.rs:77-81) |
 //! | [`Engine::aggregate_verify`] | `AggregateSignature::verify` (src/aggregate_signature.rs:230-239) |
+//! | [`Engine::aggregate_verify_batch`] | q × `AggregateSignature::verify`, one pipeline per signature scheme present |
 //! | [`Engine::aggregate_signature_from`] / [`Engine::multi_signature_from`] / [`Engine::multi_public_key_from`] | `from_signatures` / `from_public_keys` (aggregate_signature.rs:171-188, multi_signature.rs:147-150, multi_public_key.rs:79-82) |
 //! | [`Engine::verify_secure_batch`] / [`Engine::verify_secure_batch_with_mode`] | `Signature::verify_secure[_with_mode]` (signature.rs:177-197, 256-276) |
 //! | [`Engine::aggregate_secure_batch`] / [`Engine::aggregate_secure_batch_with_mode`] | `aggregate_secure[_with_mode]` (secure_aggregation.rs:159-169, 338-352) |
@@ -369,6 +370,47 @@ impl Engine {
         };
         self.check(rc)?;
         Ok(status_to_result(status, Some((index[0], index[1]))))
+    }
+
+    /// `items[j].0.verify(items[j].1)` for every j, in input order.  One engine call per signature scheme present (the
+    /// C entry point takes one scheme); within a call every aggregate is checked by one pipeline with a single final
+    /// exponentiation, and a rejected aggregate is rejected by its own exact equation.
+    pub fn aggregate_verify_batch<C: GpuImpl, B: AsRef<[u8]>>(
+        &mut self,
+        items: &[(AggregateSignature<C>, &[(PublicKey<C>, B)])],
+    ) -> EngineResult<Vec<BlsResult<()>>> {
+        let parts = |s: &AggregateSignature<C>| match s {
+            AggregateSignature::Basic(p) => (SignatureSchemes::Basic, *p),
+            AggregateSignature::MessageAugmentation(p) => (SignatureSchemes::MessageAugmentation, *p),
+            AggregateSignature::ProofOfPossession(p) => (SignatureSchemes::ProofOfPossession, *p),
+        };
+        let mut out: Vec<Option<BlsResult<()>>> = (0..items.len()).map(|_| None).collect();
+        for scheme in [SignatureSchemes::Basic, SignatureSchemes::MessageAugmentation, SignatureSchemes::ProofOfPossession] {
+            let idx: Vec<usize> = (0..items.len()).filter(|&j| parts(&items[j].0).0 == scheme).collect();
+            if idx.is_empty() {
+                continue;
+            }
+            let q = idx.len();
+            let mut set_off = Vec::with_capacity(q + 1);
+            set_off.push(0u64);
+            for &j in &idx {
+                set_off.push(set_off[set_off.len() - 1] + items[j].1.len() as u64);
+            }
+            let pk_bytes = pack_points(idx.iter().flat_map(|&j| items[j].1.iter().map(|(p, _)| p.0)), C::PK_BYTES);
+            let packed = PackedMessages::from_iter(idx.iter().flat_map(|&j| items[j].1.iter().map(|(_, m)| m.as_ref())));
+            let sig_bytes = pack_points(idx.iter().map(|&j| parts(&items[j].0).1), C::SIG_BYTES);
+            let mut status = vec![0u8; q];
+            let mut index = vec![-1i64; 2 * q];
+            let rc = unsafe {
+                sys::blsgpu_aggregate_verify_batch(self.ctx, C::IMPL_ID, scheme_id(scheme), 1, q, set_off.as_ptr(), pk_bytes.as_ptr(),
+                    packed.bytes.as_ptr(), packed.offsets.as_ptr(), sig_bytes.as_ptr(), status.as_mut_ptr(), index.as_mut_ptr())
+            };
+            self.check(rc)?;
+            for (k, &j) in idx.iter().enumerate() {
+                out[j] = Some(status_to_result(status[k], Some((index[2 * k], index[2 * k + 1]))));
+            }
+        }
+        Ok(out.into_iter().map(|r| r.expect("every scheme variant is covered")).collect())
     }
 
     fn sum_points<P: GroupEncoding>(&mut self, group: c_int, bytes: &[u8], each: usize) -> EngineResult<BlsResult<P>> {

@@ -81,12 +81,24 @@ struct Arena {
   size_t cap = 0, off = 0;
   bool over = false;  // a take ran past the capacity the entry point sized: every later launch is refused (ARENA_OK)
   template <class T>
+  static size_t bytes(size_t count) {
+    return (count * sizeof(T) + 255) & ~size_t(255);
+  }
+  template <class T>
   T* take(size_t count) {
-    size_t bytes = (count * sizeof(T) + 255) & ~size_t(255);
     T* p = reinterpret_cast<T*>(base + off);
-    off += bytes;
+    off += bytes<T>(count);
     if (off > cap) over = true;
     return p;
+  }
+};
+// counts what a sequence of Arena takes occupies, without memory: budgets derived from the takes themselves
+struct ArenaSize {
+  size_t off = 0;
+  template <class T>
+  T* take(size_t count) {
+    off += Arena::bytes<T>(count);
+    return nullptr;
   }
 };
 
@@ -365,7 +377,67 @@ struct Pipe {
   bool root_T_ready = false;   // T = ML(-g, S_root) already computed beside the Miller stage (x_T[0])
   const Fp12* rootF() const { return d_F + lv.back().off; }
   const SigJ* rootS() const { return use_msm ? d_msm_root : use_rlc ? d_S + lv.back().off : d_S; }
+  // `count` probes go in rounds of PROBE_SMALL through the dedicated scratch, or (big) in rounds of as many as line buffer 0
+  // and the point scratch hold
+  bool big_rounds(size_t count) const { return count > PROBE_SMALL && big_items >= 6 * PROBE_SMALL; }
+  size_t round_size(size_t count) const { return big_rounds(count) ? std::min(x_cap, big_items / 6) : PROBE_SMALL; }
 };
+
+// probes per launch of a tree with `leaves` leaves: as many as one bisection level can ask for at once (16 per failing node, at
+// most one node per leaf)
+size_t probe_cap(size_t leaves) { return std::max<size_t>(PROBE_SMALL, std::min<size_t>(leaves, 4096) + 16); }
+// The probe scratch of P for `cap` probes per launch: indices and verdicts, the points and statuses of six pairs per probe,
+// the T values, and the Miller buffers of one small round.  A takes from an Arena, or counts bytes (ArenaSize: probe_scratch_bytes).
+template <class PkA, class SigA, class A>
+void take_probe_scratch(A& a, Pipe<PkA, SigA>& P, size_t cap) {
+  const size_t small = std::min(cap, PROBE_SMALL);
+  P.x_cap = cap;
+  P.d_ok = a.template take<uint8_t>(cap);
+  P.d_idx = a.template take<uint32_t>(cap);
+  P.x_pk = a.template take<PkA>(6 * cap);
+  P.x_h = a.template take<SigA>(6 * cap);
+  P.x_pre = a.template take<uint8_t>(6 * cap);
+  P.x_T = a.template take<Fp12>(cap);
+  P.x_args = a.template take<M6Arg>(6 * small);
+  P.x_lines = a.template take<SLineRec>(6 * small * M6_LINE_RECS);
+}
+template <class PkA, class SigA>
+size_t probe_scratch_bytes(size_t cap) {
+  ArenaSize a;
+  Pipe<PkA, SigA> P;
+  take_probe_scratch(a, P, cap);
+  return a.off;
+}
+// dynamic shared memory of the probe kernels, per device and per call (microseconds): a context per device may run this
+// from several host threads
+template <class PkA, class SigA>
+int set_probe_smem(blsgpu_ctx* ctx) {
+  CK(cudaFuncSetAttribute(k_m6_lines<PkA, SigA>, cudaFuncAttributeMaxDynamicSharedMemorySize, M6_LINES_SMEM));
+  CK(cudaFuncSetAttribute(k_m6_accum, cudaFuncAttributeMaxDynamicSharedMemorySize, M6_ACCUM_SMEM));
+  CK(cudaFuncSetAttribute(k_final6, cudaFuncAttributeMaxDynamicSharedMemorySize, FE6_SMEM));
+  return BLSGPU_OK;
+}
+
+// the levels above `first` of a 16-ary product tree over F and / or sum tree over S (a null tree is skipped); per level the
+// F launch goes first
+template <class J>
+int reduce_levels(blsgpu_ctx* ctx, const std::vector<Level>& lv, size_t first, Fp12* F, J* S) {
+  for (size_t k = first; k + 1 < lv.size(); k++) {
+    if (F) REDUCE_FP12(lv[k].cnt, (const Fp12*)(F + lv[k].off), lv[k + 1].cnt, F + lv[k + 1].off);
+    if (S) REDUCE_JAC(J, lv[k].cnt, (const J*)(S + lv[k].off), lv[k + 1].cnt, S + lv[k + 1].off);
+  }
+  return BLSGPU_OK;
+}
+
+// d_dig[0 .. leaves) holds the leaf digests: the 16-ary SHA-256 tree over them, then d_root = [root, salt of this call]
+int digest_root(blsgpu_ctx* ctx, size_t leaves, Digest* d_dig, Digest* d_root) {
+  const std::vector<Level> ld = make_levels(leaves);
+  for (size_t k = 0; k + 1 < ld.size(); k++)
+    LAUNCH(k_digest_reduce, blocks_for(ld[k + 1].cnt), TPB, ld[k].cnt, d_dig + ld[k].off, ld[k + 1].cnt, d_dig + ld[k + 1].off);
+  CK(cudaMemcpyAsync(d_root, d_dig + ld.back().off, sizeof(Digest), cudaMemcpyDeviceToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(d_root + 1, ctx->salt, 32, cudaMemcpyHostToDevice, ctx->stream));
+  return BLSGPU_OK;
+}
 
 // T[c] = product of the Miller values of probe c's pairs, c < cnt, on `stream`; the scratch batch was filled by k_probe_fill_*
 template <class PkA, class SigA>
@@ -390,23 +462,39 @@ int probe_final(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t cnt, const uint32_t*
   CKR(check_launch(ctx, "k_final6"));
   return BLSGPU_OK;
 }
+// The probes of idx in rounds (P.round_size): a round copies its indices to P.d_idx, fill(cnt) fills the probe batch, then
+// the Miller loops and the final exponentiation against F[idx] (F null: the probes' own pairs only), then after(lo, cnt)
+// consumes the verdicts in P.d_ok; the round ends with a stream synchronisation.
+template <class PkA, class SigA, class Fill, class After>
+int probe_rounds(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, const std::vector<uint32_t>& idx, const Fp12* F, const Fill& fill, const After& after) {
+  const bool big = P.big_rounds(idx.size());
+  const size_t per = P.round_size(idx.size());
+  for (size_t lo = 0; lo < idx.size(); lo += per) {
+    const size_t cnt = std::min(per, idx.size() - lo);
+    CK(cudaMemcpyAsync(P.d_idx, idx.data() + lo, cnt * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CKR(fill(cnt));
+    CKR((probe_miller<PkA, SigA>(ctx, P, ctx->stream, cnt, big ? P.big_args : P.x_args, big ? P.big_lines : P.x_lines)));
+    CKR((probe_final<PkA, SigA>(ctx, P, cnt, F ? P.d_idx : nullptr, F, P.d_ok)));
+    CKR(after(lo, cnt));
+    CK(cudaStreamSynchronize(ctx->stream));
+  }
+  return BLSGPU_OK;
+}
 // node probes over one tree level: res[c] = ( F[cand[c]] * e(-g, S[cand[c]]) == 1 )
 template <class PkA, class SigA>
 int probe_level(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, const std::vector<uint32_t>& cand, const Fp12* F, const typename Pipe<PkA, SigA>::SigJ* S,
                 std::vector<uint8_t>& res) {
   res.resize(cand.size());
-  const bool big = cand.size() > PROBE_SMALL && P.big_items >= 6 * PROBE_SMALL;
-  const size_t per = big ? std::min(P.x_cap, P.big_items / 6) : PROBE_SMALL;
-  for (size_t lo = 0; lo < cand.size(); lo += per) {
-    const size_t cnt = std::min(per, cand.size() - lo);
-    CK(cudaMemcpyAsync(P.d_idx, cand.data() + lo, cnt * 4, cudaMemcpyHostToDevice, ctx->stream));
-    LAUNCH((k_probe_fill_nodes<PkA, SigA>), blocks_for(cnt), TPB, cnt, (const uint32_t*)P.d_idx, S, P.x_pk, P.x_h, P.x_pre);
-    CKR((probe_miller<PkA, SigA>(ctx, P, ctx->stream, cnt, big ? P.big_args : P.x_args, big ? P.big_lines : P.x_lines)));
-    CKR((probe_final<PkA, SigA>(ctx, P, cnt, P.d_idx, F, P.d_ok)));
-    CK(cudaMemcpyAsync(res.data() + lo, P.d_ok, cnt, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-  }
-  return BLSGPU_OK;
+  return probe_rounds(
+      ctx, P, cand, F,
+      [&](size_t cnt) -> int {
+        LAUNCH((k_probe_fill_nodes<PkA, SigA>), blocks_for(cnt), TPB, cnt, (const uint32_t*)P.d_idx, S, P.x_pk, P.x_h, P.x_pre);
+        return BLSGPU_OK;
+      },
+      [&](size_t lo, size_t cnt) -> int {
+        CK(cudaMemcpyAsync(res.data() + lo, P.d_ok, cnt, cudaMemcpyDeviceToHost, ctx->stream));
+        return BLSGPU_OK;
+      });
 }
 
 // The Miller stage over n items: F[g] = prod over the items of group g of ML(r pk, H), after ctx->ev_fork.  prep(stream, cn,
@@ -479,31 +567,14 @@ int pipeline_partials(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t n, const PkA* 
   P.d_Sitem = ctx->arena.take<SigJ>(use_rlc ? n : 1);
   Digest* d_dig = ctx->arena.take<Digest>(levels_total(make_levels(n)) + 2);
   Digest* d_root = P.d_root = d_dig + levels_total(make_levels(n));  // [root, salt]
-  P.d_ok = ctx->arena.take<uint8_t>(std::max<size_t>(n, 16));
-  P.d_idx = ctx->arena.take<uint32_t>(std::max<size_t>(n, 16));
-  // probe scratch (points and statuses for as many probes as one bisection level can ask for at once: 16 per failing
-  // node, at most one node per group; the line records of big levels go through the Miller stage's buffer)
-  P.x_cap = std::max<size_t>(PROBE_SMALL, std::min<size_t>(ng, 4096) + 16);
-  P.x_pk = ctx->arena.take<PkA>(6 * P.x_cap);
-  P.x_h = ctx->arena.take<SigA>(6 * P.x_cap);
-  P.x_pre = ctx->arena.take<uint8_t>(6 * P.x_cap);
-  P.x_T = ctx->arena.take<Fp12>(P.x_cap);
-  P.x_args = ctx->arena.take<M6Arg>(6 * PROBE_SMALL);
-  P.x_lines = ctx->arena.take<SLineRec>(6 * PROBE_SMALL * M6_LINE_RECS);
-  // per device and per call (microseconds): a context per device may run this from several host threads
-  CK(cudaFuncSetAttribute(k_m6_lines<PkA, SigA>, cudaFuncAttributeMaxDynamicSharedMemorySize, M6_LINES_SMEM));
-  CK(cudaFuncSetAttribute(k_m6_accum, cudaFuncAttributeMaxDynamicSharedMemorySize, M6_ACCUM_SMEM));
-  CK(cudaFuncSetAttribute(k_final6, cudaFuncAttributeMaxDynamicSharedMemorySize, FE6_SMEM));
+  take_probe_scratch(ctx->arena, P, probe_cap(ng));  // the line records of big levels go through the Miller stage's buffer
+  CKR((set_probe_smem<PkA, SigA>(ctx)));
 
   const int rbits = P.rbits = use_rlc ? ctx->rlc_bits : 0;
   if (use_rlc) {
     CKR(fresh_salt(ctx));
-    std::vector<Level> ld = make_levels(n);
     LAUNCH((k_leaf_digest<PkA, SigA>), blocks_for(n), TPB, n, d_pk, d_sig, d_h, d_dig);
-    for (size_t k = 0; k + 1 < ld.size(); k++)
-      LAUNCH(k_digest_reduce, blocks_for(ld[k + 1].cnt), TPB, ld[k].cnt, d_dig + ld[k].off, ld[k + 1].cnt, d_dig + ld[k + 1].off);
-    CK(cudaMemcpyAsync(d_root, d_dig + ld.back().off, sizeof(Digest), cudaMemcpyDeviceToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_root + 1, ctx->salt, 32, cudaMemcpyHostToDevice, ctx->stream));
+    CKR(digest_root(ctx, n, d_dig, d_root));
   }
   // S = sum r_i sig_i.  Large batches: bucket multi-scalar multiplication for the total only (the per-group sums the
   // bisection needs are computed if the batch fails) BEFORE the Miller stage, so that its Miller loop T = ML(-g, S) can
@@ -530,8 +601,7 @@ int pipeline_partials(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t n, const PkA* 
       LAUNCH((k_msm_bucket<SigA>), blocks_for(nbuckets), TPB, n, nbuckets, d_sig, c, (const uint32_t*)d_cnt, (const uint32_t*)d_off,
              (const uint32_t*)d_sorted, d_B);
       LAUNCH((k_msm_chunk<SigJ>), blocks_for(nchunks), TPB, nchunks, c, (const SigJ*)d_B, d_V);
-      for (size_t k = 0; k + 1 < lm.size(); k++)
-        REDUCE_JAC(SigJ, lm[k].cnt, (const SigJ*)(d_V + lm[k].off), lm[k + 1].cnt, d_V + lm[k + 1].off);
+      CKR(reduce_levels(ctx, lm, 0, nullptr, d_V));
       P.d_msm_root = d_V + lm.back().off;
       return BLSGPU_OK;
     }();
@@ -559,11 +629,7 @@ int pipeline_partials(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t n, const PkA* 
     LAUNCH((k_group_sum<SigJ>), blocks_for(ng), TPB, n, (const SigJ*)P.d_Sitem, ng, d_S);
   }
   stage_mark(ctx, BLSGPU_STAGE_REDUCE);
-  for (size_t k = 0; k + 1 < lv.size(); k++) {
-    REDUCE_FP12(lv[k].cnt, (const Fp12*)(d_F + lv[k].off), lv[k + 1].cnt, d_F + lv[k + 1].off);
-    if (use_rlc && !use_msm)
-      REDUCE_JAC(SigJ, lv[k].cnt, (const SigJ*)(d_S + lv[k].off), lv[k + 1].cnt, d_S + lv[k + 1].off);
-  }
+  CKR(reduce_levels(ctx, lv, 0, d_F, use_rlc && !use_msm ? d_S : nullptr));
   if (!use_rlc) LAUNCH((k_reduce_aff<SigA>), 1, 32, (size_t)1, d_sig, (size_t)1, d_S);  // S = the single aggregate signature
   return BLSGPU_OK;
 }
@@ -595,8 +661,7 @@ int pipeline_check(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, bool* ok_out) {
 template <class PkA, class SigA, class BeforeLeaves>
 int descend_tree(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, std::vector<uint32_t>& bad, const BeforeLeaves& before_leaves) {
   const std::vector<Level>& lv = P.lv;
-  const size_t one_round = P.big_items >= 6 * PROBE_SMALL ? std::min(P.x_cap, P.big_items / 6) : PROBE_SMALL;  // what probe_level takes at once
-  const size_t BISECT_FANOUT = std::min<size_t>(1024, one_round);
+  const size_t BISECT_FANOUT = std::min<size_t>(1024, P.round_size(SIZE_MAX));  // at most one round of probe_level
   auto children = [&](const std::vector<uint32_t>& nodes, size_t level) {  // nodes at `level` -> their children at level - 1
     std::vector<uint32_t> out;
     const size_t cn = lv[level].cnt;
@@ -640,8 +705,7 @@ int pipeline_bisect(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P) {
   if (P.use_msm && !by_nodes) {
     LAUNCH((k_scale_sig<SigA>), blocks_for(n), TPB, n, P.d_sig, P.d_status, P.d_root, P.rbits, P.d_Sitem);
     LAUNCH((k_group_sum<SigJ>), blocks_for(ng), TPB, n, (const SigJ*)P.d_Sitem, ng, P.d_S);
-    for (size_t k = 0; k + 1 < lv.size(); k++)
-      REDUCE_JAC(SigJ, lv[k].cnt, (const SigJ*)(P.d_S + lv[k].off), lv[k + 1].cnt, P.d_S + lv[k + 1].off);
+    CKR(reduce_levels(ctx, lv, 0, nullptr, P.d_S));
   }
   if (by_nodes) {
     const size_t n1 = lv[1].cnt, nblocks = node_msm_blocks(ctx, n1);
@@ -649,8 +713,7 @@ int pipeline_bisect(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P) {
     SigJ* d_W = ctx->arena.take<SigJ>(n1 * 32);
     LAUNCH((k_node_msm<SigA>), (unsigned)nblocks, 128, n, n1, ng, P.d_sig, (const uint8_t*)P.d_status, (const RlcScalar*)P.d_r, d_buckets, d_W);
     LAUNCH((k_node_combine<SigJ>), blocks_for(n1), TPB, n1, (const SigJ*)d_W, P.d_S + lv[1].off);
-    for (size_t k = 1; k + 1 < lv.size(); k++)
-      REDUCE_JAC(SigJ, lv[k].cnt, (const SigJ*)(P.d_S + lv[k].off), lv[k + 1].cnt, P.d_S + lv[k + 1].off);
+    CKR(reduce_levels(ctx, lv, 1, nullptr, P.d_S));
   }
   std::vector<uint32_t> bad;
   CKR((descend_tree<PkA, SigA>(ctx, P, bad, [&](const std::vector<uint32_t>& cand) -> int {
@@ -678,44 +741,38 @@ int pipeline_bisect(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P) {
       size_t i = (size_t)gidx * M6_GROUP + m;
       if (i < n) items.push_back((uint32_t)i);
     }
-  const bool big = items.size() > PROBE_SMALL && P.big_items >= 6 * PROBE_SMALL;
-  const size_t per = big ? std::min(P.x_cap, P.big_items / 6) : PROBE_SMALL;
-  for (size_t lo = 0; lo < items.size(); lo += per) {
-    const size_t cnt = std::min(per, items.size() - lo);
-    CK(cudaMemcpyAsync(P.d_idx, items.data() + lo, cnt * 4, cudaMemcpyHostToDevice, ctx->stream));
-    LAUNCH((k_probe_fill_leaves<PkA, SigA>), blocks_for(cnt), TPB, cnt, (const uint32_t*)P.d_idx, P.d_pk, P.d_h, P.d_sig,
-           (const uint8_t*)P.d_status, P.x_pk, P.x_h, P.x_pre);
-    CKR((probe_miller<PkA, SigA>(ctx, P, ctx->stream, cnt, big ? P.big_args : P.x_args, big ? P.big_lines : P.x_lines)));
-    CKR((probe_final<PkA, SigA>(ctx, P, cnt, nullptr, nullptr, P.d_ok)));
-    LAUNCH(k_mark_invalid, blocks_for(cnt), TPB, cnt, (const uint32_t*)P.d_idx, (const uint8_t*)P.d_ok, P.d_status);
-    CK(cudaStreamSynchronize(ctx->stream));
-  }
-  return BLSGPU_OK;
+  return probe_rounds(
+      ctx, P, items, nullptr,
+      [&](size_t cnt) -> int {
+        LAUNCH((k_probe_fill_leaves<PkA, SigA>), blocks_for(cnt), TPB, cnt, (const uint32_t*)P.d_idx, P.d_pk, P.d_h, P.d_sig,
+               (const uint8_t*)P.d_status, P.x_pk, P.x_h, P.x_pre);
+        return BLSGPU_OK;
+      },
+      [&](size_t, size_t cnt) -> int {
+        LAUNCH(k_mark_invalid, blocks_for(cnt), TPB, cnt, (const uint32_t*)P.d_idx, (const uint8_t*)P.d_ok, P.d_status);
+        return BLSGPU_OK;
+      });
 }
 
+// the slice's verdict on its own: root check, bisection if it fails; the call's last stage ends here
 template <class PkA, class SigA>
-int run_pairing_pipeline(blsgpu_ctx* ctx, size_t n, const PkA* d_pk, const SigA* d_sig, const SigA* d_h, uint8_t* d_status,
-                         bool use_rlc, int* agg_ok) {
-  Pipe<PkA, SigA> P;
-  CKR((pipeline_partials<PkA, SigA>(ctx, P, n, d_pk, d_sig, d_h, d_status, use_rlc)));
+int check_and_bisect(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P) {
   bool ok = false;
   CKR((pipeline_check<PkA, SigA>(ctx, P, &ok)));
-  if (!use_rlc) *agg_ok = ok;
-  else if (!ok) CKR((pipeline_bisect<PkA, SigA>(ctx, P)));
+  if (!ok) CKR((pipeline_bisect<PkA, SigA>(ctx, P)));
   stage_mark(ctx, BLSGPU_STAGE_COUNT);
   return BLSGPU_OK;
 }
 
-// device scratch of run_pairing_pipeline for n items, without the Miller line buffers
+// device scratch of pipeline_partials for n items, without the Miller line buffers
 template <class PkA, class SigA>
 size_t pipeline_other_bytes(size_t n) {
   typedef typename PtInfo<SigA>::Jac SigJ;
   size_t total = levels_total(make_levels(std::max<size_t>(n, 1)));
   size_t gtotal = levels_total(make_levels((std::max<size_t>(n, 1) + M6_GROUP - 1) / M6_GROUP));
-  const size_t x_cap = std::max<size_t>(PROBE_SMALL, std::min<size_t>((n + M6_GROUP - 1) / M6_GROUP, 4096) + 16);
   return gtotal * (sizeof(Fp12) + sizeof(SigJ)) + n * (sizeof(SigJ) + sizeof(Fp12) + sizeof(SigJ)) + total * sizeof(Digest) +
          n * (16 + 4 * 32) + ((size_t)32 << 16) * (12 + 2 * sizeof(SigJ)) + (1 << 20) + (n + 64) * 8 + 16 * 256 + 4096 +
-         x_cap * (6 * (sizeof(PkA) + sizeof(SigA) + 1) + sizeof(Fp12)) + 6 * PROBE_SMALL * M6_ITEM_BYTES + 16 * 256 +
+         probe_scratch_bytes<PkA, SigA>(probe_cap((n + M6_GROUP - 1) / M6_GROUP)) +
          // failure path of the bucket route: window sums of the level-1 nodes, bucket scratch of 592 x 4 warps at most, item / group lists
          (n >= MSM_MIN_ITEMS ? (n / 96 + 2) * 32 * sizeof(SigJ) + std::min<size_t>(n / 384 + 1, 592) * 128 * NODE_BUCKETS * sizeof(SigJ) + n * 5 + 8 * 256 : 0);
 }
@@ -786,11 +843,7 @@ int verify_points(blsgpu_ctx* ctx, int msg_mode, const DstParam& dst, size_t n, 
   typedef typename ImplT<IMPL>::SigAff SigA;
   Pipe<PkA, SigA> P;
   CKR((verify_points_partials<IMPL>(ctx, P, msg_mode, dst, n, d_pk, d_sig, d_stpk, d_stsig, d_msgs, d_moff, d_status_out)));
-  bool ok = false;
-  CKR((pipeline_check<PkA, SigA>(ctx, P, &ok)));
-  if (!ok) CKR((pipeline_bisect<PkA, SigA>(ctx, P)));
-  stage_mark(ctx, BLSGPU_STAGE_COUNT);
-  return BLSGPU_OK;
+  return check_and_bisect(ctx, P);
 }
 
 // verify over device-resident compressed inputs.  msg_mode: 0 msg, 1 pk||msg, 2 pk bytes (PoP).
@@ -814,16 +867,10 @@ int verify_dev_partials(blsgpu_ctx* ctx, Pipe<typename ImplT<IMPL>::PkAff, typen
 }
 template <int IMPL>
 int verify_dev(blsgpu_ctx* ctx, int msg_mode, const DstParam& dst, int format, size_t n, const uint8_t* d_pks, const uint8_t* d_sigs,
-               const uint8_t* d_msgs, const uint64_t* d_moff, uint8_t* d_status_out, size_t arena_reserved) {
-  typedef typename ImplT<IMPL>::PkAff PkA;
-  typedef typename ImplT<IMPL>::SigAff SigA;
-  (void)arena_reserved;
-  Pipe<PkA, SigA> P;
+               const uint8_t* d_msgs, const uint64_t* d_moff, uint8_t* d_status_out) {
+  Pipe<typename ImplT<IMPL>::PkAff, typename ImplT<IMPL>::SigAff> P;
   CKR((verify_dev_partials<IMPL>(ctx, P, msg_mode, dst, format, n, d_pks, d_sigs, d_msgs, d_moff, d_status_out)));
-  bool ok = false;
-  CKR((pipeline_check<PkA, SigA>(ctx, P, &ok)));
-  if (!ok) CKR((pipeline_bisect<PkA, SigA>(ctx, P)));
-  stage_mark(ctx, BLSGPU_STAGE_COUNT);
+  CKR(check_and_bisect(ctx, P));
   stage_collect(ctx);
   return BLSGPU_OK;
 }
@@ -832,19 +879,24 @@ int verify_dev(blsgpu_ctx* ctx, int msg_mode, const DstParam& dst, int format, s
 // d_F[k], d_S[k] on this context's device: is  prod F_j * e(-g, sum S_j)  == 1 ?   One product/sum launch, one cooperative
 // probe, one six-lane final exponentiation - the "host multiplies the partials and runs a single final exponentiation" step
 // of the north star, executed on a GPU because the engine has no CPU arithmetic.
-int ensure_fold_scratch(blsgpu_ctx* ctx, size_t bytes) {
-  if (ctx->fold_cap >= bytes) return BLSGPU_OK;
-  if (ctx->fold_scratch) CK(cudaFree(ctx->fold_scratch));
-  ctx->fold_scratch = nullptr;
-  ctx->fold_cap = 0;
-  CK(cudaMalloc(&ctx->fold_scratch, bytes));
-  ctx->fold_cap = bytes;
+// A over the fold scratch of at least `bytes` (a small device buffer apart from the arena, regrown between calls)
+int fold_arena(blsgpu_ctx* ctx, size_t bytes, Arena& A) {
+  if (ctx->fold_cap < bytes) {
+    if (ctx->fold_scratch) CK(cudaFree(ctx->fold_scratch));
+    ctx->fold_scratch = nullptr;
+    ctx->fold_cap = 0;
+    CK(cudaMalloc(&ctx->fold_scratch, bytes));
+    ctx->fold_cap = bytes;
+  }
+  A = Arena();
+  A.base = ctx->fold_scratch;
+  A.cap = ctx->fold_cap;
   return BLSGPU_OK;
 }
 template <class PkA, class SigA>
 size_t fold_bytes(size_t k) {
   typedef typename PtInfo<SigA>::Jac SigJ;
-  return (k + 2) * (sizeof(Fp12) + sizeof(SigJ) + sizeof(SigA) + PtInfo<SigA>::LEN + 600) + 6 * (sizeof(PkA) + sizeof(SigA) + 1 + M6_ITEM_BYTES) +
+  return (k + 2) * (sizeof(Fp12) + sizeof(SigJ) + sizeof(SigA) + PtInfo<SigA>::LEN + 600) + probe_scratch_bytes<PkA, SigA>(1) +
          2 * sizeof(Fp12) + 64 * 256;
 }
 template <class PkA, class SigA>
@@ -853,21 +905,12 @@ int fold_check(blsgpu_ctx* ctx, Arena& A, size_t k, const Fp12* d_F, const typen
   Pipe<PkA, SigA> P;  // only its probe scratch is used
   Fp12* d_Froot = A.take<Fp12>(1);
   SigJ* d_Sroot = A.take<SigJ>(1);
-  P.x_cap = 1;
-  P.x_pk = A.take<PkA>(6);
-  P.x_h = A.take<SigA>(6);
-  P.x_pre = A.take<uint8_t>(6);
-  P.x_T = A.take<Fp12>(1);
-  P.x_args = A.take<M6Arg>(6);
-  P.x_lines = A.take<SLineRec>(6 * M6_LINE_RECS);
-  P.d_ok = A.take<uint8_t>(16);
+  take_probe_scratch(A, P, 1);
   if (A.over) {
     ctx->err = "internal: fold scratch sized too small";
     return BLSGPU_E_ALLOC;
   }
-  CK(cudaFuncSetAttribute(k_m6_lines<PkA, SigA>, cudaFuncAttributeMaxDynamicSharedMemorySize, M6_LINES_SMEM));
-  CK(cudaFuncSetAttribute(k_m6_accum, cudaFuncAttributeMaxDynamicSharedMemorySize, M6_ACCUM_SMEM));
-  CK(cudaFuncSetAttribute(k_final6, cudaFuncAttributeMaxDynamicSharedMemorySize, FE6_SMEM));
+  CKR((set_probe_smem<PkA, SigA>(ctx)));
   if (k > 16) {
     ctx->err = "fold: at most 16 partial results";
     return BLSGPU_E_ARG;
@@ -882,6 +925,21 @@ int fold_check(blsgpu_ctx* ctx, Arena& A, size_t k, const Fp12* d_F, const typen
   CK(cudaStreamSynchronize(ctx->stream));
   *ok_out = ok != 0;
   return BLSGPU_OK;
+}
+// the partial results of the slices in P (the roots of their trees, on device d for P[d]) meet on the first device
+template <class PkA, class SigA>
+int fold_roots(blsgpu_ctx* ctx, const std::vector<const Pipe<PkA, SigA>*>& P, bool* ok_out) {
+  typedef typename PtInfo<SigA>::Jac SigJ;
+  const size_t ndev = P.size();
+  Arena A;
+  CKR(fold_arena(ctx, fold_bytes<PkA, SigA>(ndev), A));
+  Fp12* d_Fk = A.take<Fp12>(ndev);
+  SigJ* d_Sk = A.take<SigJ>(ndev);
+  for (size_t d = 0; d < ndev; d++) {
+    CK(cudaMemcpyPeerAsync(d_Fk + d, ctx->devices[0], P[d]->rootF(), ctx->devices[d], sizeof(Fp12), ctx->stream));
+    CK(cudaMemcpyPeerAsync(d_Sk + d, ctx->devices[0], P[d]->rootS(), ctx->devices[d], sizeof(SigJ), ctx->stream));
+  }
+  return fold_check<PkA, SigA>(ctx, A, ndev, d_Fk, d_Sk, ok_out);
 }
 
 // what verify_dev takes from the arena before the pipeline's own scratch
@@ -913,6 +971,24 @@ bool offsets_ok(const uint64_t* off, size_t n) {
 
 bool args_ok(int impl_id, int scheme, int format) {
   return (impl_id == 1 || impl_id == 2) && scheme >= 0 && scheme <= 2 && (format == 0 || format == 1);
+}
+// f(std::integral_constant<int, IMPL>) for impl_id 2 (Bls12381G2Impl) or 1 (Bls12381G1Impl): the template instance of the impl
+template <class F>
+int with_impl(int impl_id, const F& f) {
+  return impl_id == 2 ? f(std::integral_constant<int, 2>()) : f(std::integral_constant<int, 1>());
+}
+
+// off[lo .. hi] rebased to off[lo]: the offsets of a run of records as the run's own
+std::vector<uint64_t> rebased(const uint64_t* off, size_t lo, size_t hi) {
+  std::vector<uint64_t> r(hi - lo + 1);
+  for (size_t i = lo; i <= hi; i++) r[i - lo] = off[i] - off[lo];
+  return r;
+}
+// key_off of q key sets: non-decreasing, at most 2^32 - 16 keys in all
+bool key_offsets_ok(const uint64_t* key_off, size_t q) {
+  for (size_t j = 0; j < q; j++)
+    if (key_off[j + 1] < key_off[j] || key_off[q] > 0xfffffff0ull) return false;
+  return true;
 }
 
 template <class T>
@@ -1091,12 +1167,10 @@ int blsgpu_verify_batch_dev(blsgpu_ctx* ctx, int impl_id, int scheme, int format
   DstParam dst;
   make_dst(dst, impl_id, scheme, false);
   int mode = scheme == 1 ? 1 : 0;
-  if (impl_id == 2) {
-    CKR(ensure_verify_arena<2>(ctx, n, 0));
-    return verify_dev<2>(ctx, mode, dst, format, n, pks_dev, sigs_dev, msgs_dev, msg_off_dev, status_out_dev, 0);
-  }
-  CKR(ensure_verify_arena<1>(ctx, n, 0));
-  return verify_dev<1>(ctx, mode, dst, format, n, pks_dev, sigs_dev, msgs_dev, msg_off_dev, status_out_dev, 0);
+  return with_impl(impl_id, [&](auto I) {
+    CKR(ensure_verify_arena<I>(ctx, n, 0));
+    return verify_dev<I>(ctx, mode, dst, format, n, pks_dev, sigs_dev, msgs_dev, msg_off_dev, status_out_dev);
+  });
 }
 
 namespace {
@@ -1114,13 +1188,11 @@ int host_partials(blsgpu_ctx* ctx, Pipe<typename ImplT<IMPL>::PkAff, typename Im
   CKR(upload(ctx, d_pks, pks, n * pk_len));
   CKR(upload(ctx, d_sigs, sigs, n * sig_len));
   CKR(upload(ctx, d_msgs, msg_off ? msgs + msg_off[0] : msgs, msg_bytes));
-  std::vector<uint64_t> off;  // rebased to the slice's first message (all zero without messages: PoP)
   if (msg_off && msg_off[0] == 0) {
     CKR(upload(ctx, d_off, msg_off, n + 1));  // the usual case: the caller's offsets go up as they are (no 8n-byte host copy)
   } else {
-    off.assign(n + 1, 0);
-    if (msg_off)
-      for (size_t i = 0; i <= n; i++) off[i] = msg_off[i] - msg_off[0];
+    // rebased to the slice's first message (all zero without messages: PoP)
+    const std::vector<uint64_t> off = msg_off ? rebased(msg_off, 0, n) : std::vector<uint64_t>(n + 1, 0);
     CKR(upload(ctx, d_off, off.data(), n + 1));
   }
   uint8_t* d_st = ctx->arena.take<uint8_t>(n);
@@ -1134,15 +1206,11 @@ int host_partials(blsgpu_ctx* ctx, Pipe<typename ImplT<IMPL>::PkAff, typename Im
 template <int IMPL>
 int host_finish(blsgpu_ctx* ctx, Pipe<typename ImplT<IMPL>::PkAff, typename ImplT<IMPL>::SigAff>& P, bool batch_ok, const uint8_t* d_st, size_t n,
                 uint8_t* status_out) {
-  typedef typename ImplT<IMPL>::PkAff PkA;
-  typedef typename ImplT<IMPL>::SigAff SigA;
   CKR(set_device(ctx));
-  if (!batch_ok) {
-    bool ok = false;
-    CKR((pipeline_check<PkA, SigA>(ctx, P, &ok)));
-    if (!ok) CKR((pipeline_bisect<PkA, SigA>(ctx, P)));
-  }
-  stage_mark(ctx, BLSGPU_STAGE_COUNT);
+  if (batch_ok)
+    stage_mark(ctx, BLSGPU_STAGE_COUNT);
+  else
+    CKR(check_and_bisect(ctx, P));
   CK(cudaMemcpyAsync(status_out, d_st, n, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   stage_collect(ctx);
@@ -1158,6 +1226,48 @@ int verify_host_one(blsgpu_ctx* ctx, int msg_mode, const DstParam& dst, int form
   return host_finish<IMPL>(ctx, P, false, d_st, n, status_out);
 }
 
+// A context on several devices: independent work (point sums of slices, key sets, quorums) goes to the devices in contiguous
+// runs, one host thread per device on the device's own child context - the same sharding blsgpu_verify_batch does, minus the
+// fold (nothing is shared between the runs).  cut[d] .. cut[d + 1] is device d's run; f(device context, d) returns a BLSGPU_* code.
+int run_on_devices(blsgpu_ctx* ctx, const std::function<int(blsgpu_ctx*, size_t)>& f) {
+  const size_t ndev = 1 + ctx->peers.size();
+  std::vector<int> rc(ndev, BLSGPU_OK);
+  auto body = [&](size_t d) {
+    blsgpu_ctx* c = d == 0 ? ctx : ctx->peers[d - 1];
+    rc[d] = set_device(c);
+    if (rc[d] == BLSGPU_OK) rc[d] = f(c, d);
+  };
+  std::vector<std::thread> workers;
+  for (size_t d = 1; d < ndev; d++) workers.emplace_back(body, d);
+  body(0);
+  for (std::thread& w : workers) w.join();
+  for (size_t d = 0; d < ndev; d++)
+    if (rc[d] != BLSGPU_OK) {
+      if (d) ctx->err = "device " + std::to_string(ctx->devices[d]) + ": " + ctx->peers[d - 1]->err;
+      return rc[d];
+    }
+  return set_device(ctx);
+}
+// cut points of `sets` sets with cumulative weights off[0..sets] into ndev runs of about equal weight
+std::vector<size_t> balanced_cuts(size_t sets, const uint64_t* off, size_t ndev) {
+  std::vector<size_t> cut(ndev + 1, sets);
+  cut[0] = 0;
+  const uint64_t total = off[sets] - off[0];
+  size_t j = 0;
+  for (size_t d = 1; d < ndev; d++) {
+    const uint64_t want = off[0] + total * d / ndev;
+    while (j < sets && off[j] < want) j++;
+    cut[d] = j;
+  }
+  return cut;
+}
+// sets 0 .. sets-1 cut into contiguous runs over the devices, balanced by the cumulative weights off[0 .. sets]:
+// run(device context, lo, hi) handles sets lo .. hi-1; a device whose run is empty does nothing
+int run_cut(blsgpu_ctx* ctx, size_t sets, const uint64_t* off, const std::function<int(blsgpu_ctx*, size_t, size_t)>& run) {
+  const std::vector<size_t> cut = balanced_cuts(sets, off, 1 + ctx->peers.size());
+  return run_on_devices(ctx, [&](blsgpu_ctx* c, size_t d) { return cut[d] == cut[d + 1] ? (int)BLSGPU_OK : run(c, cut[d], cut[d + 1]); });
+}
+
 // A context created on several devices cuts a host-buffer batch into contiguous slices, one per device, each driven by its
 // own host thread (SURVEY 8e).  Every device folds its slice into ONE partial product of Miller values and ONE partial sum
 // of r_i sig_i; the partial results meet on the first device, which multiplies / adds them and runs a single Miller loop
@@ -1170,59 +1280,34 @@ int verify_host_fold(blsgpu_ctx* ctx, int msg_mode, const DstParam& dst, int for
                      const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
   typedef typename ImplT<IMPL>::PkAff PkA;
   typedef typename ImplT<IMPL>::SigAff SigA;
-  typedef typename PtInfo<SigA>::Jac SigJ;
   const size_t ndev = 1 + ctx->peers.size();
   const size_t pk_len = IMPL == 2 ? 48 : 96, sig_len = IMPL == 2 ? 96 : 48;
   std::vector<Pipe<PkA, SigA>> P(ndev);
   std::vector<uint8_t*> d_st(ndev, nullptr);
-  std::vector<int> rc(ndev, BLSGPU_OK);
-  auto dev_ctx = [&](size_t d) { return d == 0 ? ctx : ctx->peers[d - 1]; };
   auto lo = [&](size_t d) { return n * d / ndev; };
-  auto run_all = [&](const std::function<void(size_t)>& f) {
-    std::vector<std::thread> workers;
-    for (size_t d = 1; d < ndev; d++) workers.emplace_back(f, d);
-    f(0);
-    for (std::thread& w : workers) w.join();
-    for (size_t d = 0; d < ndev; d++)
-      if (rc[d] != BLSGPU_OK) {
-        if (d) ctx->err = "device " + std::to_string(ctx->devices[d]) + ": " + ctx->peers[d - 1]->err;
-        return rc[d];
-      }
-    return (int)BLSGPU_OK;
-  };
-  CKR(run_all([&](size_t d) {
+  CKR(run_on_devices(ctx, [&](blsgpu_ctx* c, size_t d) {
     const size_t s = lo(d), e = lo(d + 1);
-    rc[d] = host_partials<IMPL>(dev_ctx(d), P[d], msg_mode, dst, format, e - s, pks + s * pk_len, sigs + s * sig_len, msgs,
-                                msg_off ? msg_off + s : nullptr, &d_st[d]);
+    return host_partials<IMPL>(c, P[d], msg_mode, dst, format, e - s, pks + s * pk_len, sigs + s * sig_len, msgs, msg_off ? msg_off + s : nullptr,
+                               &d_st[d]);
   }));
-  // the partial results meet on the first device
-  CKR(set_device(ctx));
-  CKR(ensure_fold_scratch(ctx, fold_bytes<PkA, SigA>(ndev)));
-  Arena A;
-  A.base = ctx->fold_scratch;
-  A.cap = ctx->fold_cap;
-  Fp12* d_Fk = A.take<Fp12>(ndev);
-  SigJ* d_Sk = A.take<SigJ>(ndev);
-  for (size_t d = 0; d < ndev; d++) {
-    CK(cudaMemcpyPeerAsync(d_Fk + d, ctx->devices[0], P[d].rootF(), ctx->devices[d], sizeof(Fp12), ctx->stream));
-    CK(cudaMemcpyPeerAsync(d_Sk + d, ctx->devices[0], P[d].rootS(), ctx->devices[d], sizeof(SigJ), ctx->stream));
-  }
+  std::vector<const Pipe<PkA, SigA>*> roots;
+  for (const Pipe<PkA, SigA>& p : P) roots.push_back(&p);
   bool ok = false;
-  CKR((fold_check<PkA, SigA>(ctx, A, ndev, d_Fk, d_Sk, &ok)));
-  return run_all([&](size_t d) {
+  CKR((fold_roots<PkA, SigA>(ctx, roots, &ok)));
+  return run_on_devices(ctx, [&](blsgpu_ctx* c, size_t d) {
     const size_t s = lo(d), e = lo(d + 1);
-    rc[d] = host_finish<IMPL>(dev_ctx(d), P[d], ok, d_st[d], e - s, status_out + s);
+    return host_finish<IMPL>(c, P[d], ok, d_st[d], e - s, status_out + s);
   });
 }
 
 int verify_host_common(blsgpu_ctx* ctx, int impl_id, int msg_mode, const DstParam& dst, int format, size_t n, const uint8_t* pks,
                        const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
   const size_t ndev = 1 + ctx->peers.size();
-  if (ndev == 1 || n < ndev * SHARD_MIN_ITEMS)
-    return impl_id == 2 ? verify_host_one<2>(ctx, msg_mode, dst, format, n, pks, sigs, msgs, msg_off, status_out)
-                        : verify_host_one<1>(ctx, msg_mode, dst, format, n, pks, sigs, msgs, msg_off, status_out);
-  return impl_id == 2 ? verify_host_fold<2>(ctx, msg_mode, dst, format, n, pks, sigs, msgs, msg_off, status_out)
-                      : verify_host_fold<1>(ctx, msg_mode, dst, format, n, pks, sigs, msgs, msg_off, status_out);
+  const bool fold = ndev > 1 && n >= ndev * SHARD_MIN_ITEMS;
+  return with_impl(impl_id, [&](auto I) {
+    return fold ? verify_host_fold<I>(ctx, msg_mode, dst, format, n, pks, sigs, msgs, msg_off, status_out)
+                : verify_host_one<I>(ctx, msg_mode, dst, format, n, pks, sigs, msgs, msg_off, status_out);
+  });
 }
 
 template <int IMPL>
@@ -1259,10 +1344,8 @@ int fold_bytes_impl(blsgpu_ctx* ctx, size_t k, const uint8_t* gts, const uint8_t
   typedef typename ImplT<IMPL>::SigAff SigA;
   typedef typename PtInfo<SigA>::Jac SigJ;
   const size_t Ls = PtInfo<SigA>::LEN;
-  CKR(ensure_fold_scratch(ctx, fold_bytes<PkA, SigA>(k)));
   Arena A;
-  A.base = ctx->fold_scratch;
-  A.cap = ctx->fold_cap;
+  CKR(fold_arena(ctx, fold_bytes<PkA, SigA>(k), A));
   uint8_t* d_gt = A.take<uint8_t>(576 * k);
   uint8_t* d_sb = A.take<uint8_t>(Ls * k);
   Fp12* d_Fk = A.take<Fp12>(k);
@@ -1315,8 +1398,7 @@ int blsgpu_miller_partial(blsgpu_ctx* ctx, int impl_id, int scheme, int format, 
   DstParam dst;
   make_dst(dst, impl_id, scheme, false);
   const int mode = scheme == 1 ? 1 : 0;
-  return impl_id == 2 ? miller_partial_impl<2>(ctx, mode, dst, format, n, pks, sigs, msgs, msg_off, gt_out, sum_out)
-                      : miller_partial_impl<1>(ctx, mode, dst, format, n, pks, sigs, msgs, msg_off, gt_out, sum_out);
+  return with_impl(impl_id, [&](auto I) { return miller_partial_impl<I>(ctx, mode, dst, format, n, pks, sigs, msgs, msg_off, gt_out, sum_out); });
 }
 
 int blsgpu_final_exp_is_one(blsgpu_ctx* ctx, int impl_id, size_t k, const uint8_t* partial_gts, const uint8_t* partial_sums, int* is_one_out) {
@@ -1327,8 +1409,7 @@ int blsgpu_final_exp_is_one(blsgpu_ctx* ctx, int impl_id, size_t k, const uint8_
     return BLSGPU_E_ARG;
   }
   CKR(set_device(ctx));
-  return impl_id == 2 ? fold_bytes_impl<2>(ctx, k, partial_gts, partial_sums, is_one_out)
-                      : fold_bytes_impl<1>(ctx, k, partial_gts, partial_sums, is_one_out);
+  return with_impl(impl_id, [&](auto I) { return fold_bytes_impl<I>(ctx, k, partial_gts, partial_sums, is_one_out); });
 }
 
 int blsgpu_partial_finish(blsgpu_ctx* ctx, int batch_ok, uint8_t* status_out) {
@@ -1376,42 +1457,6 @@ int blsgpu_pop_verify_batch(blsgpu_ctx* ctx, int impl_id, int format, size_t n, 
   return verify_host_common(ctx, impl_id, 2, dst, format, n, pks, sigs, nullptr, nullptr, status_out);
 }
 
-// ---------------------------------------------------------------------------------------------------------------------
-// A context on several devices: independent work (point sums of slices, key sets, quorums) goes to the devices in contiguous
-// runs, one host thread per device on the device's own child context - the same sharding blsgpu_verify_batch does, minus the
-// fold (nothing is shared between the runs).  cut[d] .. cut[d + 1] is device d's run; f(device context, d) returns a BLSGPU_* code.
-static int run_on_devices(blsgpu_ctx* ctx, const std::function<int(blsgpu_ctx*, size_t)>& f) {
-  const size_t ndev = 1 + ctx->peers.size();
-  std::vector<int> rc(ndev, BLSGPU_OK);
-  auto body = [&](size_t d) {
-    blsgpu_ctx* c = d == 0 ? ctx : ctx->peers[d - 1];
-    rc[d] = set_device(c);
-    if (rc[d] == BLSGPU_OK) rc[d] = f(c, d);
-  };
-  std::vector<std::thread> workers;
-  for (size_t d = 1; d < ndev; d++) workers.emplace_back(body, d);
-  body(0);
-  for (std::thread& w : workers) w.join();
-  for (size_t d = 0; d < ndev; d++)
-    if (rc[d] != BLSGPU_OK) {
-      if (d) ctx->err = "device " + std::to_string(ctx->devices[d]) + ": " + ctx->peers[d - 1]->err;
-      return rc[d];
-    }
-  return set_device(ctx);
-}
-// cut points of `sets` sets with cumulative weights off[0..sets] into ndev runs of about equal weight
-static std::vector<size_t> balanced_cuts(size_t sets, const uint64_t* off, size_t ndev) {
-  std::vector<size_t> cut(ndev + 1, sets);
-  cut[0] = 0;
-  const uint64_t total = off[sets] - off[0];
-  size_t j = 0;
-  for (size_t d = 1; d < ndev; d++) {
-    const uint64_t want = off[0] + total * d / ndev;
-    while (j < sets && off[j] < want) j++;
-    cut[d] = j;
-  }
-  return cut;
-}
 // AggregateSignature::verify in phases, so that a context on several devices can cut the pairs over its devices (SURVEY 8e,
 // cfg 4): (1) every device decodes its slice of the keys (the first one also the signature), (2) the host applies the
 // reference's checks in the reference's order over the whole input, (3) every device hashes its messages and folds its pairs
@@ -1554,7 +1599,6 @@ static int aggregate_verify_multi(blsgpu_ctx* ctx, int scheme, int format, size_
                                   const uint64_t* msg_off, const uint8_t* sig, uint8_t* status_out, int64_t index_out[2]) {
   typedef typename ImplT<IMPL>::PkAff PkA;
   typedef typename ImplT<IMPL>::SigAff SigA;
-  typedef typename PtInfo<SigA>::Jac SigJ;
   const size_t ndev = 1 + ctx->peers.size(), pk_len = PtInfo<PkA>::LEN;
   std::vector<AggSlice<IMPL>> S(ndev);
   std::vector<uint8_t> st(n + 1);
@@ -1566,8 +1610,7 @@ static int aggregate_verify_multi(blsgpu_ctx* ctx, int scheme, int format, size_
   std::vector<uint32_t> inf0(lo(1) + 1, 0);
   CKR(run_on_devices(ctx, [&](blsgpu_ctx* c, size_t d) {
     const size_t s0 = lo(d), cnt = lo(d + 1) - s0;
-    off[d].resize(cnt + 1);
-    for (size_t i = 0; i <= cnt; i++) off[d][i] = msg_off[s0 + i] - msg_off[s0];
+    off[d] = rebased(msg_off, s0, s0 + cnt);
     return agg_decode<IMPL>(c, S[d], format, cnt, pks + s0 * pk_len, msgs + msg_off[s0], off[d].data(), d == 0 ? sig : nullptr,
                             d == 0 ? st0.data() : st.data() + s0, d == 0 ? inf0.data() : inf.data() + s0);
   }));
@@ -1585,18 +1628,10 @@ static int aggregate_verify_multi(blsgpu_ctx* ctx, int scheme, int format, size_
     }
     return (int)BLSGPU_OK;
   }));
-  CKR(ensure_fold_scratch(ctx, fold_bytes<PkA, SigA>(ndev)));
-  Arena A;
-  A.base = ctx->fold_scratch;
-  A.cap = ctx->fold_cap;
-  Fp12* d_Fk = A.take<Fp12>(ndev);
-  SigJ* d_Sk = A.take<SigJ>(ndev);
-  for (size_t d = 0; d < ndev; d++) {
-    CK(cudaMemcpyPeerAsync(d_Fk + d, ctx->devices[0], S[d].P.rootF(), ctx->devices[d], sizeof(Fp12), ctx->stream));
-    CK(cudaMemcpyPeerAsync(d_Sk + d, ctx->devices[0], S[d].P.rootS(), ctx->devices[d], sizeof(SigJ), ctx->stream));
-  }
+  std::vector<const Pipe<PkA, SigA>*> roots;
+  for (const AggSlice<IMPL>& slice : S) roots.push_back(&slice.P);
   bool ok = false;
-  CKR((fold_check<PkA, SigA>(ctx, A, ndev, d_Fk, d_Sk, &ok)));
+  CKR((fold_roots<PkA, SigA>(ctx, roots, &ok)));
   *status_out = ok ? BLSGPU_ST_OK : BLSGPU_ST_INVALID_SIGNATURE;
   return BLSGPU_OK;
 }
@@ -1613,11 +1648,11 @@ int blsgpu_aggregate_verify(blsgpu_ctx* ctx, int impl_id, int scheme, int format
   }
   CHECK_OFFSETS(msg_off, n, "blsgpu_aggregate_verify");
   CKR(set_device(ctx));
-  if (!ctx->peers.empty() && n >= (1 + ctx->peers.size()) * SHARD_MIN_ITEMS)
-    return impl_id == 2 ? aggregate_verify_multi<2>(ctx, scheme, format, n, pks, msgs, msg_off, sig, status_out, index_out)
-                        : aggregate_verify_multi<1>(ctx, scheme, format, n, pks, msgs, msg_off, sig, status_out, index_out);
-  return impl_id == 2 ? aggregate_verify_impl<2>(ctx, scheme, format, n, pks, msgs, msg_off, sig, status_out, index_out)
-                      : aggregate_verify_impl<1>(ctx, scheme, format, n, pks, msgs, msg_off, sig, status_out, index_out);
+  const bool multi = !ctx->peers.empty() && n >= (1 + ctx->peers.size()) * SHARD_MIN_ITEMS;
+  return with_impl(impl_id, [&](auto I) {
+    return multi ? aggregate_verify_multi<I>(ctx, scheme, format, n, pks, msgs, msg_off, sig, status_out, index_out)
+                 : aggregate_verify_impl<I>(ctx, scheme, format, n, pks, msgs, msg_off, sig, status_out, index_out);
+  });
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -1667,11 +1702,10 @@ static int aggregate_batch_impl(blsgpu_ctx* ctx, int scheme, int format, size_t 
   Pipe<PkA, SigA> P;
   P.lv = make_levels(q);
   const size_t qtotal = levels_total(P.lv), ndig = levels_total(make_levels(np + q));
-  P.x_cap = std::max<size_t>(PROBE_SMALL, std::min<size_t>(q, 4096) + 16);
   size_t head = np * (Lp + sizeof(PkA) + sizeof(SigA) + 2) + msg_bytes + (np + 1) * 8 + q * (Ls + sizeof(SigA) + 2) + (q + 1) * 8 +
                 np * sizeof(SigJ) + (ndig + 2) * sizeof(Digest) + nslots * (sizeof(PkA) + sizeof(SigA) + 1 + 4) + ng * 4 +
-                seg_off.size() * 4 + seg_total * sizeof(Fp12) + qtotal * (sizeof(Fp12) + sizeof(SigJ)) + P.x_cap * 5 +
-                P.x_cap * (6 * (sizeof(PkA) + sizeof(SigA) + 1) + sizeof(Fp12)) + 6 * PROBE_SMALL * M6_ITEM_BYTES + 40 * 256;
+                seg_off.size() * 4 + seg_total * sizeof(Fp12) + qtotal * (sizeof(Fp12) + sizeof(SigJ)) +
+                probe_scratch_bytes<PkA, SigA>(probe_cap(q)) + 40 * 256;
   CKR((ensure_pipeline_arena<PkA, SigA>(ctx, nslots, head)));
   stage_reset(ctx);
   uint8_t *d_pkb, *d_sigb, *d_msgs;
@@ -1743,15 +1777,9 @@ static int aggregate_batch_impl(blsgpu_ctx* ctx, int scheme, int format, size_t 
   Digest* d_dig = ctx->arena.take<Digest>(ndig + 2);
   Digest* d_root = d_dig + ndig;  // [root, salt]
   CKR(fresh_salt(ctx));
-  {
-    const std::vector<Level> ld = make_levels(np + q);
-    LAUNCH((k_agg_leaf_digest<PkA, SigA>), blocks_for(np + q), TPB, np, q, (const PkA*)d_pk, (const SigA*)d_h, (const SigA*)d_sig,
-           (const uint64_t*)d_soff, d_dig);
-    for (size_t k = 0; k + 1 < ld.size(); k++)
-      LAUNCH(k_digest_reduce, blocks_for(ld[k + 1].cnt), TPB, ld[k].cnt, d_dig + ld[k].off, ld[k + 1].cnt, d_dig + ld[k + 1].off);
-    CK(cudaMemcpyAsync(d_root, d_dig + ld.back().off, sizeof(Digest), cudaMemcpyDeviceToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_root + 1, ctx->salt, 32, cudaMemcpyHostToDevice, ctx->stream));
-  }
+  LAUNCH((k_agg_leaf_digest<PkA, SigA>), blocks_for(np + q), TPB, np, q, (const PkA*)d_pk, (const SigA*)d_h, (const SigA*)d_sig,
+         (const uint64_t*)d_soff, d_dig);
+  CKR(digest_root(ctx, np + q, d_dig, d_root));
   PkA* d_pks = ctx->arena.take<PkA>(nslots);
   SigA* d_hs = ctx->arena.take<SigA>(nslots);
   uint8_t* d_pres = ctx->arena.take<uint8_t>(nslots);
@@ -1768,18 +1796,9 @@ static int aggregate_batch_impl(blsgpu_ctx* ctx, int scheme, int format, size_t 
   P.d_root = d_root;
   P.d_F = ctx->arena.take<Fp12>(qtotal);
   P.d_S = ctx->arena.take<SigJ>(qtotal);
-  P.d_ok = ctx->arena.take<uint8_t>(P.x_cap);
-  P.d_idx = ctx->arena.take<uint32_t>(P.x_cap);
-  P.x_pk = ctx->arena.take<PkA>(6 * P.x_cap);
-  P.x_h = ctx->arena.take<SigA>(6 * P.x_cap);
-  P.x_pre = ctx->arena.take<uint8_t>(6 * P.x_cap);
-  P.x_T = ctx->arena.take<Fp12>(P.x_cap);
-  P.x_args = ctx->arena.take<M6Arg>(6 * PROBE_SMALL);
-  P.x_lines = ctx->arena.take<SLineRec>(6 * PROBE_SMALL * M6_LINE_RECS);
+  take_probe_scratch(ctx->arena, P, probe_cap(q));
   Fp12* d_Fseg = ctx->arena.take<Fp12>(std::max<size_t>(seg_total, 1));
-  CK(cudaFuncSetAttribute(k_m6_lines<PkA, SigA>, cudaFuncAttributeMaxDynamicSharedMemorySize, M6_LINES_SMEM));
-  CK(cudaFuncSetAttribute(k_m6_accum, cudaFuncAttributeMaxDynamicSharedMemorySize, M6_ACCUM_SMEM));
-  CK(cudaFuncSetAttribute(k_final6, cudaFuncAttributeMaxDynamicSharedMemorySize, FE6_SMEM));
+  CKR((set_probe_smem<PkA, SigA>(ctx)));
   stage_mark(ctx, BLSGPU_STAGE_SCALE_SIG);
   LAUNCH((k_scale_sig<SigA>), blocks_for(q), TPB, q, (const SigA*)d_sig, (const uint8_t*)d_agg_pre, (const Digest*)d_root, rbits, P.d_S);
   CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
@@ -1807,11 +1826,7 @@ static int aggregate_batch_impl(blsgpu_ctx* ctx, int scheme, int format, size_t 
       out_off += n_out;
     }
   }
-  const std::vector<Level>& lv = P.lv;
-  for (size_t k = 0; k + 1 < lv.size(); k++) {
-    REDUCE_FP12(lv[k].cnt, (const Fp12*)(P.d_F + lv[k].off), lv[k + 1].cnt, P.d_F + lv[k + 1].off);
-    REDUCE_JAC(SigJ, lv[k].cnt, (const SigJ*)(P.d_S + lv[k].off), lv[k + 1].cnt, P.d_S + lv[k + 1].off);
-  }
+  CKR(reduce_levels(ctx, P.lv, 0, P.d_F, P.d_S));
   bool ok = false;
   CKR((pipeline_check<PkA, SigA>(ctx, P, &ok)));
   for (size_t j = 0; j < q; j++)
@@ -1860,21 +1875,17 @@ int blsgpu_aggregate_verify_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int 
   // aggregates lo .. hi-1 on context c, with their pair and message offsets rebased to 0
   auto run = [&](blsgpu_ctx* c, size_t lo, size_t hi) -> int {
     const size_t a = (size_t)set_off[lo], b = (size_t)set_off[hi];
-    std::vector<uint64_t> so(hi - lo + 1), mo(b - a + 1);
-    for (size_t j = lo; j <= hi; j++) so[j - lo] = set_off[j] - a;
-    for (size_t i = a; i <= b; i++) mo[i - a] = msg_off[i] - msg_off[a];
+    const std::vector<uint64_t> so = rebased(set_off, lo, hi), mo = rebased(msg_off, a, b);
     const uint8_t* pk = pks ? pks + a * pk_len : nullptr;
     const uint8_t* ms = msgs ? msgs + msg_off[a] : nullptr;
-    return impl_id == 2 ? aggregate_batch_impl<2>(c, scheme, format, hi - lo, so.data(), pk, ms, mo.data(), sigs + lo * sig_len, status_out + lo,
-                                                  index_out + 2 * lo)
-                        : aggregate_batch_impl<1>(c, scheme, format, hi - lo, so.data(), pk, ms, mo.data(), sigs + lo * sig_len, status_out + lo,
-                                                  index_out + 2 * lo);
+    return with_impl(impl_id, [&](auto I) {
+      return aggregate_batch_impl<I>(c, scheme, format, hi - lo, so.data(), pk, ms, mo.data(), sigs + lo * sig_len, status_out + lo, index_out + 2 * lo);
+    });
   };
   const size_t ndev = 1 + ctx->peers.size();
   if (ndev == 1 || np < ndev * SHARD_MIN_ITEMS) return run(ctx, 0, q);
   // aggregates are independent: contiguous runs per device, balanced by pair count, nothing to fold
-  const std::vector<size_t> cut = balanced_cuts(q, set_off, ndev);
-  return run_on_devices(ctx, [&](blsgpu_ctx* c, size_t d) { return cut[d] == cut[d + 1] ? (int)BLSGPU_OK : run(c, cut[d], cut[d + 1]); });
+  return run_cut(ctx, q, set_off, run);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -1907,17 +1918,11 @@ static int sum_points_impl(blsgpu_ctx* ctx, int format, size_t n, const uint8_t*
       }
   }
   // level 1 from the affine leaves, then Jacobian levels
-  size_t n1 = n ? (n + 15) / 16 : 1;
+  const size_t n1 = n ? (n + 15) / 16 : 1;
   LAUNCH((k_reduce_aff<A>), blocks_for(n1), TPB, n, (const A*)d_pts, n1, d_tree);
-  size_t cur = n1;
-  J* src = d_tree;
-  while (cur > 1) {
-    size_t nxt = (cur + 15) / 16;
-    REDUCE_JAC(J, cur, (const J*)src, nxt, src + cur);
-    src += cur;
-    cur = nxt;
-  }
-  LAUNCH((k_to_affine<A>), 1, 32, (size_t)1, (const J*)src, d_res);
+  const std::vector<Level> lj = make_levels(n1);
+  CKR(reduce_levels(ctx, lj, 0, nullptr, d_tree));
+  LAUNCH((k_to_affine<A>), 1, 32, (size_t)1, (const J*)(d_tree + lj.back().off), d_res);
   LAUNCH((k_encode<A>), 1, 32, (size_t)1, (const A*)d_res, format, d_out);
   CK(cudaMemcpyAsync(out, d_out, L, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
@@ -2081,8 +2086,7 @@ int blsgpu_pairing_product_is_one(blsgpu_ctx* ctx, size_t n, const uint8_t* g1_p
       return BLSGPU_E_ARG;
     }
   LAUNCH(k_miller_pairs, blocks_for(n), TPB, n, (const G1Aff*)d_p, (const G2Aff*)d_q, d_F);
-  for (size_t k = 0; k + 1 < lv.size(); k++)
-    REDUCE_FP12(lv[k].cnt, (const Fp12*)(d_F + lv[k].off), lv[k + 1].cnt, d_F + lv[k + 1].off);
+  CKR(reduce_levels(ctx, lv, 0, d_F, (PtInfo<G1Aff>::Jac*)nullptr));
   LAUNCH(k_final_is_one, 1, 32, (const Fp12*)(d_F + lv.back().off), d_ok);
   uint8_t ok = 0;
   CK(cudaMemcpyAsync(&ok, d_ok, 1, cudaMemcpyDeviceToHost, ctx->stream));
@@ -2116,12 +2120,11 @@ int blsgpu_testdata_sign(blsgpu_ctx* ctx, int impl_id, int scheme, size_t n, con
   DstParam dst;
   make_dst(dst, impl_id, pop_proof ? 2 : scheme, pop_proof);
   int mode = pop_proof ? 2 : scheme == 1 ? 1 : 0;
-  if (impl_id == 2)
-    LAUNCH((k_testdata_sign<G1Aff, G2Aff>), blocks_for(n), TPB, n, (const uint8_t*)d_k, (const uint8_t*)d_m, (const uint64_t*)d_off, mode, dst,
-           d_pk, d_sig);
-  else
-    LAUNCH((k_testdata_sign<G2Aff, G1Aff>), blocks_for(n), TPB, n, (const uint8_t*)d_k, (const uint8_t*)d_m, (const uint64_t*)d_off, mode, dst,
-           d_pk, d_sig);
+  CKR(with_impl(impl_id, [&](auto I) {
+    LAUNCH((k_testdata_sign<typename ImplT<I>::PkAff, typename ImplT<I>::SigAff>), blocks_for(n), TPB, n, (const uint8_t*)d_k, (const uint8_t*)d_m,
+           (const uint64_t*)d_off, mode, dst, d_pk, d_sig);
+    return BLSGPU_OK;
+  }));
   CK(cudaMemcpyAsync(out_pks, d_pk, n * pk_len, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaMemcpyAsync(out_sigs, d_sig, n * sig_len, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
@@ -2372,31 +2375,22 @@ int blsgpu_verify_secure_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int for
     return BLSGPU_E_ARG;
   }
   if (q == 0) return BLSGPU_OK;
-  for (size_t j = 0; j < q; j++)
-    if (key_off[j + 1] < key_off[j] || key_off[q] > 0xfffffff0ull) {
-      ctx->err = "blsgpu_verify_secure_batch: key_off must be non-decreasing and below 2^32";
-      return BLSGPU_E_ARG;
-    }
+  if (!key_offsets_ok(key_off, q)) {
+    ctx->err = "blsgpu_verify_secure_batch: key_off must be non-decreasing and below 2^32";
+    return BLSGPU_E_ARG;
+  }
   CHECK_OFFSETS(msg_off, q, "blsgpu_verify_secure_batch");
   CKR(set_device(ctx));
   auto one = [&](blsgpu_ctx* c, size_t cnt, const uint64_t* ko, const uint8_t* pk, const uint8_t* sg, const uint8_t* ms, const uint64_t* mo,
                  uint8_t* st) {
-    return impl_id == 2 ? verify_secure_impl<2>(c, scheme, format, cnt, ko, pk, sg, ms, mo, st)
-                        : verify_secure_impl<1>(c, scheme, format, cnt, ko, pk, sg, ms, mo, st);
+    return with_impl(impl_id, [&](auto I) { return verify_secure_impl<I>(c, scheme, format, cnt, ko, pk, sg, ms, mo, st); });
   };
   const size_t ndev = 1 + ctx->peers.size();
   if (ndev == 1 || q < 2 * ndev || key_off[q] - key_off[0] < SHARD_MIN_ITEMS * ndev) return one(ctx, q, key_off, pks, sigs, msgs, msg_off, status_out);
   // quorums are independent (SURVEY 8e, cfg 5): contiguous runs of quorums per device, balanced by member count
   const size_t pk_len = impl_id == 2 ? 48 : 96, sig_len = impl_id == 2 ? 96 : 48;
-  const std::vector<size_t> cut = balanced_cuts(q, key_off, ndev);
-  return run_on_devices(ctx, [&](blsgpu_ctx* c, size_t d) {
-    const size_t lo = cut[d], hi = cut[d + 1];
-    if (hi == lo) return (int)BLSGPU_OK;
-    std::vector<uint64_t> ko(hi - lo + 1), mo(hi - lo + 1);
-    for (size_t j = lo; j <= hi; j++) {
-      ko[j - lo] = key_off[j] - key_off[lo];
-      mo[j - lo] = msg_off[j] - msg_off[lo];
-    }
+  return run_cut(ctx, q, key_off, [&](blsgpu_ctx* c, size_t lo, size_t hi) {
+    const std::vector<uint64_t> ko = rebased(key_off, lo, hi), mo = rebased(msg_off, lo, hi);
     return one(c, hi - lo, ko.data(), pks ? pks + key_off[lo] * pk_len : nullptr, sigs + lo * sig_len, msgs ? msgs + msg_off[lo] : nullptr,
                mo.data(), status_out + lo);
   });
@@ -2412,24 +2406,19 @@ int blsgpu_aggregate_secure_batch(blsgpu_ctx* ctx, int impl_id, int format, size
     return BLSGPU_E_ARG;
   }
   if (q == 0) return BLSGPU_OK;
-  for (size_t j = 0; j < q; j++)
-    if (key_off[j + 1] < key_off[j] || key_off[q] > 0xfffffff0ull) {
-      ctx->err = "blsgpu_aggregate_secure_batch: key_off must be non-decreasing and below 2^32";
-      return BLSGPU_E_ARG;
-    }
+  if (!key_offsets_ok(key_off, q)) {
+    ctx->err = "blsgpu_aggregate_secure_batch: key_off must be non-decreasing and below 2^32";
+    return BLSGPU_E_ARG;
+  }
   CKR(set_device(ctx));
   auto one = [&](blsgpu_ctx* c, size_t cnt, const uint64_t* ko, const uint8_t* pk, const uint8_t* ms, uint8_t* o, uint8_t* st) {
-    return impl_id == 2 ? aggregate_secure_impl<2>(c, format, cnt, ko, pk, ms, o, st) : aggregate_secure_impl<1>(c, format, cnt, ko, pk, ms, o, st);
+    return with_impl(impl_id, [&](auto I) { return aggregate_secure_impl<I>(c, format, cnt, ko, pk, ms, o, st); });
   };
   const size_t ndev = 1 + ctx->peers.size();
   if (ndev == 1 || q < 2 * ndev || key_off[q] - key_off[0] < SHARD_MIN_ITEMS * ndev) return one(ctx, q, key_off, pks, member_sigs, out_sigs, status_out);
   const size_t pk_len = impl_id == 2 ? 48 : 96, sig_len = impl_id == 2 ? 96 : 48;
-  const std::vector<size_t> cut = balanced_cuts(q, key_off, ndev);
-  return run_on_devices(ctx, [&](blsgpu_ctx* c, size_t d) {
-    const size_t lo = cut[d], hi = cut[d + 1];
-    if (hi == lo) return (int)BLSGPU_OK;
-    std::vector<uint64_t> ko(hi - lo + 1);
-    for (size_t j = lo; j <= hi; j++) ko[j - lo] = key_off[j] - key_off[lo];
+  return run_cut(ctx, q, key_off, [&](blsgpu_ctx* c, size_t lo, size_t hi) {
+    const std::vector<uint64_t> ko = rebased(key_off, lo, hi);
     return one(c, hi - lo, ko.data(), pks + key_off[lo] * pk_len, member_sigs + key_off[lo] * sig_len, out_sigs + lo * sig_len, status_out + lo);
   });
 }
@@ -2533,7 +2522,8 @@ int blsgpu_combine_shares_batch(blsgpu_ctx* ctx, int group, size_t q, const uint
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// Wire-format front end: tagged signatures, schemes mixed in one call.  The host only regroups bytes by tag.
+// Wire-format front end: tagged signatures, schemes mixed in one call.  Fixed-size records: blsgpu_verify_batch_records in
+// tagged mode does the rest.
 int blsgpu_verify_batch_wire(blsgpu_ctx* ctx, int impl_id, size_t n, const uint8_t* pks, const uint8_t* tagged_sigs, const uint8_t* msgs,
                              const uint64_t* msg_off, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_verify_batch_wire");
@@ -2543,27 +2533,13 @@ int blsgpu_verify_batch_wire(blsgpu_ctx* ctx, int impl_id, size_t n, const uint8
     return BLSGPU_E_ARG;
   }
   CHECK_OFFSETS(msg_off, n, "blsgpu_verify_batch_wire");
-  const size_t pk_len = impl_id == 2 ? 48 : 96, sig_len = impl_id == 2 ? 96 : 48, rec = sig_len + 1;
-  for (int scheme = 0; scheme < 3; scheme++) {
-    std::vector<size_t> idx;
-    for (size_t i = 0; i < n; i++)
-      if (tagged_sigs[i * rec] == (uint8_t)scheme) idx.push_back(i);
-    if (idx.empty()) continue;
-    std::vector<uint8_t> p(idx.size() * pk_len), g(idx.size() * sig_len), m, st(idx.size());
-    std::vector<uint64_t> off(idx.size() + 1, 0);
-    for (size_t k = 0; k < idx.size(); k++) {
-      const size_t i = idx[k];
-      memcpy(&p[k * pk_len], pks + i * pk_len, pk_len);
-      memcpy(&g[k * sig_len], tagged_sigs + i * rec + 1, sig_len);
-      m.insert(m.end(), msgs + msg_off[i], msgs + msg_off[i + 1]);
-      off[k + 1] = m.size();
-    }
-    CKR(blsgpu_verify_batch(ctx, impl_id, scheme, 1, idx.size(), p.data(), g.data(), m.data(), off.data(), st.data()));
-    for (size_t k = 0; k < idx.size(); k++) status_out[idx[k]] = st[k];
+  const size_t pk_len = impl_id == 2 ? 48 : 96, rec = (impl_id == 2 ? 96 : 48) + 1;
+  std::vector<uint64_t> pk_off(n + 1), sig_off(n + 1);
+  for (size_t i = 0; i <= n; i++) {
+    pk_off[i] = i * pk_len;
+    sig_off[i] = i * rec;
   }
-  for (size_t i = 0; i < n; i++)
-    if (tagged_sigs[i * rec] > 2) status_out[i] = BLSGPU_ST_DESERIALIZE;
-  return BLSGPU_OK;
+  return blsgpu_verify_batch_records(ctx, impl_id, 1, -1, n, pks, pk_off.data(), tagged_sigs, sig_off.data(), msgs, msg_off, status_out);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -2791,8 +2767,7 @@ int blsgpu_pok_verify_batch(blsgpu_ctx* ctx, int impl_id, int scheme, size_t n, 
   if (n == 0) return BLSGPU_OK;
   CHECK_OFFSETS(msg_off, n, "blsgpu_pok_verify_batch");
   CKR(set_device(ctx));
-  return impl_id == 2 ? pok_verify_impl<2>(ctx, scheme, n, commitments, proofs, pks, challenges32, msgs, msg_off, status_out)
-                      : pok_verify_impl<1>(ctx, scheme, n, commitments, proofs, pks, challenges32, msgs, msg_off, status_out);
+  return with_impl(impl_id, [&](auto I) { return pok_verify_impl<I>(ctx, scheme, n, commitments, proofs, pks, challenges32, msgs, msg_off, status_out); });
 }
 
 int blsgpu_signcrypt_verify_share_batch(blsgpu_ctx* ctx, int impl_id, int scheme, size_t n, const uint8_t* shares, const uint8_t* pk_shares,
@@ -2807,8 +2782,9 @@ int blsgpu_signcrypt_verify_share_batch(blsgpu_ctx* ctx, int impl_id, int scheme
   if (n == 0) return BLSGPU_OK;
   CHECK_OFFSETS(v_off, n, "blsgpu_signcrypt_verify_share_batch");
   CKR(set_device(ctx));
-  return impl_id == 2 ? signcrypt_share_impl<2>(ctx, scheme, n, shares, pk_shares, u_points, w_points, v_bytes, v_off, ok_out, status_out)
-                      : signcrypt_share_impl<1>(ctx, scheme, n, shares, pk_shares, u_points, w_points, v_bytes, v_off, ok_out, status_out);
+  return with_impl(impl_id, [&](auto I) {
+    return signcrypt_share_impl<I>(ctx, scheme, n, shares, pk_shares, u_points, w_points, v_bytes, v_off, ok_out, status_out);
+  });
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -2829,6 +2805,10 @@ int blsgpu_verify_batch_records(blsgpu_ctx* ctx, int impl_id, int format, int sc
   CHECK_OFFSETS(pk_off, n, "blsgpu_verify_batch_records");
   CHECK_OFFSETS(sig_off, n, "blsgpu_verify_batch_records");
   CHECK_OFFSETS(msg_off, n, "blsgpu_verify_batch_records");
+  if ((!pk_bytes && pk_off[n] > pk_off[0]) || (!sig_bytes && sig_off[n] > sig_off[0]) || (!msgs && msg_off[n] > msg_off[0])) {
+    ctx->err = "blsgpu_verify_batch_records: pk_bytes, sig_bytes or msgs is null";
+    return BLSGPU_E_ARG;
+  }
   const size_t pk_len = impl_id == 2 ? 48 : 96, sig_len = impl_id == 2 ? 96 : 48;
   // InvalidLength (public_key.rs:159-164, signature.rs:236-241) and the serde_bare tag (signature.rs:120-126) per record;
   // well-formed records are regrouped by scheme and go through blsgpu_verify_batch in `format`

@@ -111,6 +111,7 @@ def load_library() -> ctypes.CDLL:
         "blsgpu_ctx_set_stream": (c.c_int, [vp, vp]),
         "blsgpu_verify_batch": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u8p, u8p, u8p, u64p, u8p]),
         "blsgpu_verify_batch_dev": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u8p, u8p, u8p, u64p, u8p]),
+        "blsgpu_verify_batch_grouped": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u8p, u8p, vp, c.c_size_t, u8p, u64p, u8p]),
         "blsgpu_miller_partial": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u8p, u8p, u8p, u64p, u8p, u8p]),
         "blsgpu_final_exp_is_one": (c.c_int, [vp, c.c_int, c.c_size_t, u8p, u8p, c.POINTER(c.c_int)]),
         "blsgpu_partial_finish": (c.c_int, [vp, c.c_int, u8p]),
@@ -151,7 +152,7 @@ def load_library() -> ctypes.CDLL:
 EXPORTED_SYMBOLS = [
     "blsgpu_ctx_create", "blsgpu_ctx_destroy", "blsgpu_last_error", "blsgpu_ctx_set_rlc_salt", "blsgpu_ctx_set_rlc_bits",
     "blsgpu_ctx_set_stream",
-    "blsgpu_verify_batch",
+    "blsgpu_verify_batch", "blsgpu_verify_batch_grouped",
     "blsgpu_miller_partial", "blsgpu_final_exp_is_one", "blsgpu_partial_finish",
     "blsgpu_verify_batch_dev", "blsgpu_pop_verify_batch", "blsgpu_aggregate_verify", "blsgpu_aggregate_verify_batch", "blsgpu_sum_points",
     "blsgpu_verify_secure_batch", "blsgpu_aggregate_secure_batch", "blsgpu_hash_to_curve_batch", "blsgpu_recode_points",
@@ -299,6 +300,30 @@ class Engine:
         rc = self._lib.blsgpu_verify_batch(self._ctx, impl_id, scheme, fmt, n, _ptr(pk), _ptr(sg), _ptr(data), _ptr(off),
                                            _ptr(status))
         self._check(rc, "blsgpu_verify_batch")
+        return status
+
+    def verify_batch_grouped(self, impl_id: int, scheme: int, pks, sigs, msg_idx, msgs: Sequence[bytes],
+                             fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """verify_batch where item i signs msgs[msg_idx[i]]: each message is hashed once and items of one message share
+        their Miller loops.  The statuses equal verify_batch's on the same items with their messages written out."""
+        pk = _pack_points(pks, pk_len(impl_id), "public key")
+        sg = _pack_points(sigs, sig_len(impl_id), "signature")
+        idx = np.ascontiguousarray(msg_idx, dtype=np.uint32).reshape(-1)
+        n = pk.size // pk_len(impl_id)
+        if sg.size // sig_len(impl_id) != n or idx.size != n:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        data, off = pack_messages(msgs)
+        return self.verify_batch_grouped_packed(impl_id, scheme, pk, sg, idx, data, off, fmt)
+
+    def verify_batch_grouped_packed(self, impl_id, scheme, pk: np.ndarray, sg: np.ndarray, msg_idx: np.ndarray, data: np.ndarray,
+                                    off: np.ndarray, fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """Flat-buffer form: msg_idx uint32[n], the q messages as data / off (q + 1 offsets)."""
+        msg_idx = np.ascontiguousarray(msg_idx, dtype=np.uint32).reshape(-1)
+        n = msg_idx.size
+        status = np.empty(n, dtype=np.uint8)
+        rc = self._lib.blsgpu_verify_batch_grouped(self._ctx, impl_id, scheme, fmt, n, _ptr(pk), _ptr(sg), _ptr(msg_idx), off.size - 1,
+                                                   _ptr(data), _ptr(off), _ptr(status))
+        self._check(rc, "blsgpu_verify_batch_grouped")
         return status
 
     def verify_batch_dev(self, impl_id, scheme, n, pk_ptr: int, sig_ptr: int, msg_ptr: int, off_ptr: int, status_ptr: int,

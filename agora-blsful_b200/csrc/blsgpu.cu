@@ -548,6 +548,61 @@ int miller_stage(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t n, const PkA* d_pk,
   return BLSGPU_OK;
 }
 
+// The bucket multi-scalar multiplication S = sum r_i sig_i over n items, r_i = rlc_scalar(root, i) (0 for an item whose
+// status is not OK): its window plan, and its takes from an Arena (or an ArenaSize: msm_bytes)
+struct MsmPlan {
+  int c, nwin;
+  size_t nbuckets, nchunks;
+  std::vector<Level> lm;  // the tree over the chunk sums
+  MsmPlan(size_t n, int rbits) : c(msm_window_bits(n, rbits)), nwin((rbits + c - 1) / c) {
+    nbuckets = ((size_t)1 << c) * nwin;
+    nchunks = nbuckets / MSM_CHUNK;
+    lm = make_levels(nchunks);
+  }
+};
+template <class SigJ, class A>
+void take_msm(A& a, size_t n, const MsmPlan& m, RlcScalar*& d_r, uint32_t*& d_cnt, uint32_t*& d_sorted, SigJ*& d_B, SigJ*& d_V) {
+  d_r = a.template take<RlcScalar>(n);
+  d_cnt = a.template take<uint32_t>(3 * m.nbuckets);  // histograms, offsets, cursors
+  d_sorted = a.template take<uint32_t>((size_t)m.nwin * n);
+  d_B = a.template take<SigJ>(m.nbuckets);
+  d_V = a.template take<SigJ>(levels_total(m.lm));
+}
+template <class SigJ>
+size_t msm_bytes(size_t n, int rbits) {
+  ArenaSize a;
+  RlcScalar* r;
+  uint32_t *cnt, *sorted;
+  SigJ *B, *V;
+  take_msm(a, n, MsmPlan(n, rbits), r, cnt, sorted, B, V);
+  return a.off;
+}
+// *r_out = the scalars (kept for the failure path and the key side of blsgpu_verify_batch_grouped), *sum_out = S
+template <class SigA>
+int msm_sum(blsgpu_ctx* ctx, size_t n, const SigA* d_sig, const uint8_t* d_status, const Digest* d_root, int rbits, RlcScalar** r_out,
+            typename PtInfo<SigA>::Jac** sum_out) {
+  typedef typename PtInfo<SigA>::Jac SigJ;
+  const MsmPlan m(n, rbits);
+  const int c = m.c, nwin = m.nwin;
+  const size_t nbuckets = m.nbuckets, nchunks = m.nchunks;
+  RlcScalar* d_r;
+  uint32_t *d_cnt, *d_sorted;
+  SigJ *d_B, *d_V;
+  take_msm(ctx->arena, n, m, d_r, d_cnt, d_sorted, d_B, d_V);
+  uint32_t *d_off = d_cnt + nbuckets, *d_cur = d_off + nbuckets;
+  CK(cudaMemsetAsync(d_cnt, 0, nbuckets * sizeof(uint32_t), ctx->stream));
+  LAUNCH(k_msm_count, blocks_for(n), TPB, n, (const uint8_t*)d_status, (const Digest*)d_root, rbits, c, nwin, d_r, d_cnt);
+  LAUNCH(k_msm_scan, (unsigned)nwin, 1024, c, (const uint32_t*)d_cnt, d_off, d_cur);
+  LAUNCH(k_msm_scatter, blocks_for(n), TPB, n, (const RlcScalar*)d_r, c, nwin, (const uint32_t*)d_off, d_cur, d_sorted);
+  LAUNCH((k_msm_bucket<SigA>), blocks_for(nbuckets), TPB, n, nbuckets, d_sig, c, (const uint32_t*)d_cnt, (const uint32_t*)d_off,
+         (const uint32_t*)d_sorted, d_B);
+  LAUNCH((k_msm_chunk<SigJ>), blocks_for(nchunks), TPB, nchunks, c, (const SigJ*)d_B, d_V);
+  CKR(reduce_levels(ctx, m.lm, 0, nullptr, d_V));
+  *r_out = d_r;
+  *sum_out = d_V + m.lm.back().off;
+  return BLSGPU_OK;
+}
+
 template <class PkA, class SigA>
 int pipeline_partials(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t n, const PkA* d_pk, const SigA* d_sig, const SigA* d_h, uint8_t* d_status,
                       bool use_rlc) {
@@ -582,31 +637,7 @@ int pipeline_partials(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t n, const PkA* 
   // (Running the bucket kernels themselves beside the Miller stage was measured: they evict Miller blocks, +70 ms at 1M.)
   stage_mark(ctx, BLSGPU_STAGE_SCALE_SIG);
   const bool use_msm = P.use_msm = use_rlc && n >= MSM_MIN_ITEMS;
-  if (use_msm) {
-    int rc = [&]() -> int {
-      const int c = msm_window_bits(n, rbits);
-      const int nwin = (rbits + c - 1) / c;
-      const size_t nb = (size_t)1 << c, nbuckets = nb * nwin, nchunks = nbuckets / MSM_CHUNK;
-      RlcScalar* d_r = P.d_r = ctx->arena.take<RlcScalar>(n);
-      uint32_t* d_cnt = ctx->arena.take<uint32_t>(3 * nbuckets);
-      uint32_t *d_off = d_cnt + nbuckets, *d_cur = d_off + nbuckets;
-      uint32_t* d_sorted = ctx->arena.take<uint32_t>((size_t)nwin * n);
-      SigJ* d_B = ctx->arena.take<SigJ>(nbuckets);
-      std::vector<Level> lm = make_levels(nchunks);
-      SigJ* d_V = ctx->arena.take<SigJ>(levels_total(lm));
-      CK(cudaMemsetAsync(d_cnt, 0, nbuckets * sizeof(uint32_t), ctx->stream));
-      LAUNCH(k_msm_count, blocks_for(n), TPB, n, (const uint8_t*)d_status, (const Digest*)d_root, rbits, c, nwin, d_r, d_cnt);
-      LAUNCH(k_msm_scan, (unsigned)nwin, 1024, c, (const uint32_t*)d_cnt, d_off, d_cur);
-      LAUNCH(k_msm_scatter, blocks_for(n), TPB, n, (const RlcScalar*)d_r, c, nwin, (const uint32_t*)d_off, d_cur, d_sorted);
-      LAUNCH((k_msm_bucket<SigA>), blocks_for(nbuckets), TPB, n, nbuckets, d_sig, c, (const uint32_t*)d_cnt, (const uint32_t*)d_off,
-             (const uint32_t*)d_sorted, d_B);
-      LAUNCH((k_msm_chunk<SigJ>), blocks_for(nchunks), TPB, nchunks, c, (const SigJ*)d_B, d_V);
-      CKR(reduce_levels(ctx, lm, 0, nullptr, d_V));
-      P.d_msm_root = d_V + lm.back().off;
-      return BLSGPU_OK;
-    }();
-    CKR(rc);
-  }
+  if (use_msm) CKR((msm_sum<SigA>(ctx, n, d_sig, d_status, d_root, rbits, &P.d_r, &P.d_msm_root)));
   CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
   P.root_T_ready = false;
   if (use_msm) {
@@ -779,12 +810,10 @@ size_t pipeline_other_bytes(size_t n) {
 size_t m6_line_bytes(size_t n, size_t chunk) {
   return (n > chunk ? 2 : 1) * std::max<size_t>(std::min(std::max<size_t>(n, 1), chunk), 6 * PROBE_SMALL) * M6_ITEM_BYTES;
 }
-// Plans the pass size of the Miller kernels for this call and sizes the arena: `head_bytes` is what the entry point takes
-// from the arena besides the pipeline's own scratch.  If the allocation fails the pass size is halved (more passes) until
-// it fits or reaches the minimum.
-template <class PkA, class SigA>
-int ensure_pipeline_arena(blsgpu_ctx* ctx, size_t n, size_t head_bytes) {
-  const size_t other = head_bytes + pipeline_other_bytes<PkA, SigA>(n);
+// Plans the pass size of the Miller kernels for a call over n Miller items and sizes the arena: `other` is everything the
+// call takes from the arena besides the Miller line buffers.  If the allocation fails the pass size is halved (more passes)
+// until it fits or reaches the minimum.
+int ensure_miller_arena(blsgpu_ctx* ctx, size_t n, size_t other) {
   plan_m6_chunk(ctx, n, other);
   for (;;) {
     const int r = ensure_arena(ctx, other + m6_line_bytes(n, ctx->m6_chunk));
@@ -792,6 +821,11 @@ int ensure_pipeline_arena(blsgpu_ctx* ctx, size_t n, size_t head_bytes) {
     (void)cudaGetLastError();
     ctx->m6_chunk = std::max(M6_CHUNK_MIN, std::min(ctx->m6_chunk, n) / 2 / 120 * 120);
   }
+}
+// the same for the pipeline over n items: `head_bytes` is what the entry point takes besides the pipeline's own scratch
+template <class PkA, class SigA>
+int ensure_pipeline_arena(blsgpu_ctx* ctx, size_t n, size_t head_bytes) {
+  return ensure_miller_arena(ctx, n, head_bytes + pipeline_other_bytes<PkA, SigA>(n));
 }
 
 // compressed bytes -> affine points + per-item status: decompression (square root), then the subgroup check
@@ -1886,6 +1920,315 @@ int blsgpu_aggregate_verify_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int 
   if (ndev == 1 || np < ndev * SHARD_MIN_ITEMS) return run(ctx, 0, q);
   // aggregates are independent: contiguous runs per device, balanced by pair count, nothing to fold
   return run_cut(ctx, q, set_off, run);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// n x Signature::verify where many items share a message.  The batch equation of blsgpu_verify_batch regroups by bilinearity:
+//   prod_i e(r_i pk_i, H(m_i)) = prod_l e(P_l, H_l),   P_l = sum_{i in leaf l} r_i pk_i
+// so the q messages are hashed once each and the Miller stage runs once per LEAF (at most GROUPED_LEAF items of one message)
+// instead of once per item.  The scalars are blsgpu_verify_batch's (rlc_scalar(root, i), item order), the root binds every
+// pk, signature, message hash and message index.  A failing check descends the tree of Miller groups of leaves, probes the
+// leaves of the failing groups, and decides every item of a failing leaf by its own exact equation (DESIGN.md section 2).
+#ifndef BLSGPU_GROUPED_LEAF
+#define BLSGPU_GROUPED_LEAF 96
+#endif
+namespace {
+constexpr uint32_t GROUPED_LEAF = BLSGPU_GROUPED_LEAF;  // items per leaf at most (DESIGN.md section 6: the measured trade)
+constexpr uint32_t LEAF_MSM_MIN = 16;  // leaves with fewer items take k_leaf_scale: 32 lanes of buckets do not pay below this
+template <class PkA, class SigA>
+struct Grouped {
+  typedef typename PtInfo<PkA>::Jac PkJ;
+  typedef typename PtInfo<SigA>::Jac SigJ;
+  size_t n = 0, q = 0, nl = 0, nbig = 0, nsmall = 0, msg_bytes = 0, blocks = 1;
+  uint8_t *pkb, *sigb, *msgs, *mpre, *stpk, *stsig, *status, *lpre;
+  uint64_t* moff;
+  uint32_t *midx, *order, *big, *small;  // big / small: the leaves of k_leaf_msm / k_leaf_scale
+  GLeaf* leaves;
+  PkA* pk;
+  SigA *sig, *hq, *hl;  // hq: per message, hl: per leaf
+  Digest* dig;          // leaf digests, their tree, [root, salt]
+  RlcScalar* r;         // the scalars of the per-item route (the bucket route's come from msm_sum)
+  SigJ* s_item;         // per-item route: r_i sig_i and the tree over them
+  PkJ *p_jac, *p_buckets, *p_W;
+  PkA* p_aff;
+  SigJ *s_jac, *s_buckets, *s_W;  // failure path: S_l per leaf
+  SigA* s_aff;
+  Pipe<PkA, SigA> P;  // the tree over the Miller groups of leaves
+};
+// every take of the grouped pipeline but the bucket MSM's (msm_sum) and the Miller line buffers (miller_stage)
+template <class PkA, class SigA, class A>
+void take_grouped(A& a, Grouped<PkA, SigA>& G) {
+  typedef typename Grouped<PkA, SigA>::PkJ PkJ;
+  typedef typename Grouped<PkA, SigA>::SigJ SigJ;
+  const size_t n = G.n, nl = G.nl, ng = (nl + M6_GROUP - 1) / M6_GROUP, ndig = levels_total(make_levels(n));
+  G.pkb = a.template take<uint8_t>(n * PtInfo<PkA>::LEN);
+  G.sigb = a.template take<uint8_t>(n * PtInfo<SigA>::LEN);
+  G.msgs = a.template take<uint8_t>(std::max<size_t>(G.msg_bytes, 1));
+  G.moff = a.template take<uint64_t>(G.q + 1);
+  G.mpre = a.template take<uint8_t>(G.q);
+  G.midx = a.template take<uint32_t>(n);
+  G.order = a.template take<uint32_t>(n);
+  G.leaves = a.template take<GLeaf>(nl);
+  G.big = a.template take<uint32_t>(std::max<size_t>(G.nbig, 1));
+  G.small = a.template take<uint32_t>(std::max<size_t>(G.nsmall, 1));
+  G.pk = a.template take<PkA>(n);
+  G.sig = a.template take<SigA>(n);
+  G.stpk = a.template take<uint8_t>(n);
+  G.stsig = a.template take<uint8_t>(n);
+  G.status = a.template take<uint8_t>(n);
+  G.hq = a.template take<SigA>(G.q);
+  G.dig = a.template take<Digest>(ndig + 2);
+  if (n < MSM_MIN_ITEMS) {
+    G.r = a.template take<RlcScalar>(n);
+    G.s_item = a.template take<SigJ>(ndig);
+  }
+  G.p_jac = a.template take<PkJ>(nl);
+  G.p_aff = a.template take<PkA>(nl);
+  G.hl = a.template take<SigA>(nl);
+  G.lpre = a.template take<uint8_t>(nl);
+  G.p_buckets = a.template take<PkJ>(G.nbig ? G.blocks * 128 * LEAF_BUCKETS : 1);
+  G.p_W = a.template take<PkJ>(G.nbig * 32 + 1);
+  G.s_jac = a.template take<SigJ>(nl);
+  G.s_aff = a.template take<SigA>(nl);
+  G.s_buckets = a.template take<SigJ>(G.nbig ? G.blocks * 128 * LEAF_BUCKETS : 1);
+  G.s_W = a.template take<SigJ>(G.nbig * 32 + 1);
+  const size_t gtotal = levels_total(make_levels(ng));
+  G.P.d_F = a.template take<Fp12>(gtotal);
+  G.P.d_S = a.template take<SigJ>(gtotal);
+  take_probe_scratch(a, G.P, probe_cap(ng));
+}
+// the grouped pipeline's device scratch without the Miller line buffers: its takes, the bucket MSM's, and the Jacobian
+// scratch hash_points holds for the q hashes
+template <class PkA, class SigA>
+size_t grouped_bytes(Grouped<PkA, SigA> G, int rbits) {
+  ArenaSize a;
+  take_grouped(a, G);
+  return a.off + (G.n >= MSM_MIN_ITEMS ? msm_bytes<typename Grouped<PkA, SigA>::SigJ>(G.n, rbits) : 0) +
+         Arena::bytes<typename Grouped<PkA, SigA>::SigJ>(G.q) + 4 * 256;
+}
+// sum_{i in l} r_i * pts[i] into out[l] for every leaf: the bucket kernel for the big leaves, per-item scaling for the small
+template <class A, class G>
+int leaf_sums(blsgpu_ctx* ctx, const G& g, const A* pts, const RlcScalar* d_r, int rbits, typename PtInfo<A>::Jac* buckets,
+              typename PtInfo<A>::Jac* W, typename PtInfo<A>::Jac* out) {
+  typedef typename PtInfo<A>::Jac J;
+  if (g.nbig) {
+    LAUNCH((k_leaf_msm<A>), (unsigned)g.blocks, 128, g.nbig, (const uint32_t*)g.big, (const GLeaf*)g.leaves, (const uint32_t*)g.order, pts, d_r,
+           rbits, buckets, W);
+    LAUNCH((k_leaf_combine<J>), blocks_for(g.nbig), TPB, g.nbig, (const uint32_t*)g.big, rbits, (const J*)W, out);
+  }
+  if (g.nsmall)
+    LAUNCH((k_leaf_scale<A>), blocks_for(g.nsmall), TPB, g.nsmall, (const uint32_t*)g.small, (const GLeaf*)g.leaves, (const uint32_t*)g.order, pts,
+           d_r, rbits, out);
+  return BLSGPU_OK;
+}
+
+template <int IMPL>
+int verify_grouped_impl(blsgpu_ctx* ctx, int scheme, int format, size_t n, const uint8_t* pks, const uint8_t* sigs, const uint32_t* msg_idx,
+                        size_t q, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
+  typedef typename ImplT<IMPL>::PkAff PkA;
+  typedef typename ImplT<IMPL>::SigAff SigA;
+  typedef typename PtInfo<PkA>::Jac PkJ;
+  typedef typename PtInfo<SigA>::Jac SigJ;
+  // group: counting sort of the items by message, then every message's run cut into leaves
+  std::vector<uint32_t> order(n), start(q + 1, 0);
+  for (size_t i = 0; i < n; i++) start[msg_idx[i] + 1]++;
+  for (size_t j = 0; j < q; j++) start[j + 1] += start[j];
+  {
+    std::vector<uint32_t> cur(start.begin(), start.end() - 1);
+    for (size_t i = 0; i < n; i++) order[cur[msg_idx[i]]++] = (uint32_t)i;
+  }
+  std::vector<GLeaf> leaves;
+  std::vector<uint32_t> big, small;
+  std::vector<uint8_t> mpre(q, PROBE_SKIP);  // a message no item signs is not hashed
+  for (size_t j = 0; j < q; j++)
+    for (uint32_t f = start[j]; f < start[j + 1]; f += GROUPED_LEAF) {
+      const uint32_t cnt = std::min(GROUPED_LEAF, start[j + 1] - f);
+      (cnt >= LEAF_MSM_MIN ? big : small).push_back((uint32_t)leaves.size());
+      leaves.push_back({f, cnt, (uint32_t)j});
+      mpre[j] = BLSGPU_ST_OK;
+    }
+  Grouped<PkA, SigA> G;
+  G.n = n;
+  G.q = q;
+  G.nl = leaves.size();
+  G.nbig = big.size();
+  G.nsmall = small.size();
+  G.msg_bytes = (size_t)(msg_off[q] - msg_off[0]);
+  G.blocks = node_msm_blocks(ctx, G.nbig);
+  const int rbits = ctx->rlc_bits;
+  CKR(ensure_miller_arena(ctx, G.nl, grouped_bytes(G, rbits)));
+  take_grouped(ctx->arena, G);
+  ARENA_OK();
+  Pipe<PkA, SigA>& P = G.P;
+  stage_reset(ctx);
+  const std::vector<uint64_t> moff = rebased(msg_off, 0, q);
+  CK(cudaMemcpyAsync(G.pkb, pks, n * PtInfo<PkA>::LEN, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(G.sigb, sigs, n * PtInfo<SigA>::LEN, cudaMemcpyHostToDevice, ctx->stream));
+  if (G.msg_bytes) CK(cudaMemcpyAsync(G.msgs, msgs + msg_off[0], G.msg_bytes, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(G.moff, moff.data(), (q + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(G.mpre, mpre.data(), q, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(G.midx, msg_idx, n * 4, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(G.order, order.data(), n * 4, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(G.leaves, leaves.data(), G.nl * sizeof(GLeaf), cudaMemcpyHostToDevice, ctx->stream));
+  if (G.nbig) CK(cudaMemcpyAsync(G.big, big.data(), G.nbig * 4, cudaMemcpyHostToDevice, ctx->stream));
+  if (G.nsmall) CK(cudaMemcpyAsync(G.small, small.data(), G.nsmall * 4, cudaMemcpyHostToDevice, ctx->stream));
+  // decode, per-item statuses (item order throughout)
+  stage_mark(ctx, BLSGPU_STAGE_DECODE_PK);
+  CKR((decode_points<PkA>(ctx, n, (const uint8_t*)G.pkb, format, G.pk, G.stpk, BLSGPU_KERNEL_DECODE_PK)));
+  stage_mark(ctx, BLSGPU_STAGE_DECODE_SIG);
+  CKR((decode_points<SigA>(ctx, n, (const uint8_t*)G.sigb, format, G.sig, G.stsig, BLSGPU_KERNEL_DECODE_SIG)));
+  LAUNCH((k_prestatus<PkA, SigA>), blocks_for(n), TPB, n, (const uint8_t*)G.stpk, (const uint8_t*)G.stsig, (const PkA*)G.pk, (const SigA*)G.sig,
+         G.status);
+  // one hash per message, then the scalars of blsgpu_verify_batch
+  stage_mark(ctx, BLSGPU_STAGE_HASH);
+  DstParam dst;
+  make_dst(dst, IMPL, scheme, false);
+  CKR((hash_points<SigA, PkA>(ctx, q, (const uint8_t*)G.msgs, (const uint64_t*)G.moff, 0, (const PkA*)nullptr, (const uint8_t*)G.mpre, dst, G.hq)));
+  CKR(fresh_salt(ctx));
+  const size_t ndig = levels_total(make_levels(n));
+  Digest* d_root = G.dig + ndig;
+  LAUNCH((k_grouped_leaf_digest<PkA, SigA>), blocks_for(n), TPB, n, (const PkA*)G.pk, (const SigA*)G.sig, (const SigA*)G.hq, (const uint32_t*)G.midx,
+         G.dig);
+  CKR(digest_root(ctx, n, G.dig, d_root));
+  // the signature side: S = sum r_i sig_i (the bucket method, or per-item scaling and a tree for small batches)
+  stage_mark(ctx, BLSGPU_STAGE_SCALE_SIG);
+  RlcScalar* d_r = nullptr;
+  SigJ* d_S = nullptr;
+  if (n >= MSM_MIN_ITEMS) {
+    CKR((msm_sum<SigA>(ctx, n, G.sig, G.status, d_root, rbits, &d_r, &d_S)));
+  } else {
+    d_r = G.r;
+    const std::vector<Level> lvn = make_levels(n);
+    LAUNCH(k_msm_count, blocks_for(n), TPB, n, (const uint8_t*)G.status, (const Digest*)d_root, rbits, 0, 0, d_r, (uint32_t*)nullptr);
+    LAUNCH((k_scale_sig<SigA>), blocks_for(n), TPB, n, (const SigA*)G.sig, (const uint8_t*)G.status, (const Digest*)d_root, rbits, G.s_item);
+    CKR(reduce_levels(ctx, lvn, 0, nullptr, G.s_item));
+    d_S = G.s_item + lvn.back().off;
+  }
+  // the key side: P_l = sum_{i in l} r_i pk_i, affine, with H of the leaf's message
+  stage_mark(ctx, BLSGPU_STAGE_MILLER);
+  CKR((leaf_sums<PkA>(ctx, G, (const PkA*)G.pk, (const RlcScalar*)d_r, rbits, G.p_buckets, G.p_W, G.p_jac)));
+  LAUNCH((k_to_affine_batch<PkA>), blocks_for((G.nl + TO_AFFINE_BATCH - 1) / TO_AFFINE_BATCH), TPB, G.nl, (const PkJ*)G.p_jac, G.p_aff);
+  LAUNCH((k_leaf_gather<PkA, SigA>), blocks_for(G.nl), TPB, G.nl, (const GLeaf*)G.leaves, (const PkA*)G.p_aff, (const SigA*)G.hq, G.hl, G.lpre);
+  // the tree over Miller groups of six leaves; its root is checked against S
+  const size_t ng = (G.nl + M6_GROUP - 1) / M6_GROUP;
+  P.n = G.nl;
+  P.ng = ng;
+  P.lv = make_levels(ng);
+  P.use_rlc = true;
+  P.use_msm = true;  // rootS() = the total S
+  P.rbits = rbits;
+  P.d_pk = G.p_aff;
+  P.d_sig = G.s_aff;
+  P.d_h = G.hl;
+  P.d_status = G.lpre;
+  P.d_root = d_root;
+  P.d_msm_root = d_S;
+  CKR((set_probe_smem<PkA, SigA>(ctx)));
+  CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
+  // T = ML(-g, S) on the aux stream, beside the Miller stage
+  CK(cudaStreamWaitEvent(ctx->aux, ctx->ev_fork, 0));
+  ARENA_OK();
+  k_probe_fill_nodes<PkA, SigA><<<1, TPB, 0, ctx->aux>>>((size_t)1, (const uint32_t*)nullptr, (const SigJ*)d_S, P.x_pk, P.x_h, P.x_pre);
+  CKR(check_launch(ctx, "k_probe_fill_nodes"));
+  CKR((probe_miller<PkA, SigA>(ctx, P, ctx->aux, 1, P.x_args, P.x_lines)));
+  CK(cudaEventRecord(ctx->ev_aux, ctx->aux));
+  P.root_T_ready = true;
+  // the leaves are weighted already: the stock prep with rbits = 0
+  CKR((miller_stage<PkA, SigA>(ctx, P, G.nl, G.p_aff, G.hl, G.lpre, P.d_F, [&](cudaStream_t s, size_t cn, size_t base, M6Arg* args) {
+    k_m6_prep<PkA, SigA><<<blocks_for(cn), TPB, 0, s>>>(cn, base, (const PkA*)G.p_aff, (const SigA*)G.hl, (const uint8_t*)G.lpre, (const Digest*)nullptr,
+                                                        0, args);
+  })));
+  CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_aux, 0));
+  stage_mark(ctx, BLSGPU_STAGE_REDUCE);
+  CKR(reduce_levels(ctx, P.lv, 0, P.d_F, (SigJ*)nullptr));
+  bool ok = false;
+  CKR((pipeline_check<PkA, SigA>(ctx, P, &ok)));
+  if (!ok) {
+    // S_l per leaf (the same kernels over the signatures), summed per Miller group and up the tree
+    CKR((leaf_sums<SigA>(ctx, G, (const SigA*)G.sig, (const RlcScalar*)d_r, rbits, G.s_buckets, G.s_W, G.s_jac)));
+    LAUNCH((k_group_sum<SigJ>), blocks_for(ng), TPB, G.nl, (const SigJ*)G.s_jac, ng, P.d_S);
+    CKR(reduce_levels(ctx, P.lv, 0, (Fp12*)nullptr, P.d_S));
+    LAUNCH((k_to_affine_batch<SigA>), blocks_for((G.nl + TO_AFFINE_BATCH - 1) / TO_AFFINE_BATCH), TPB, G.nl, (const SigJ*)G.s_jac, G.s_aff);
+    std::vector<uint32_t> bad;
+    CKR((descend_tree<PkA, SigA>(ctx, P, bad, [](const std::vector<uint32_t>&) { return (int)BLSGPU_OK; })));
+    // the leaves of the failing groups: e(P_l, H_l) e(-g, S_l) == 1 ?
+    std::vector<uint32_t> cand;
+    for (uint32_t g : bad)
+      for (int m = 0; m < M6_GROUP; m++)
+        if ((size_t)g * M6_GROUP + m < G.nl) cand.push_back(g * M6_GROUP + m);
+    std::vector<uint8_t> res(cand.size());
+    CKR(probe_rounds(
+        ctx, P, cand, nullptr,
+        [&](size_t cnt) -> int {
+          LAUNCH((k_probe_fill_leaves<PkA, SigA>), blocks_for(cnt), TPB, cnt, (const uint32_t*)P.d_idx, (const PkA*)G.p_aff, (const SigA*)G.hl,
+                 (const SigA*)G.s_aff, (const uint8_t*)G.lpre, P.x_pk, P.x_h, P.x_pre);
+          return BLSGPU_OK;
+        },
+        [&](size_t lo, size_t cnt) -> int {
+          CK(cudaMemcpyAsync(res.data() + lo, P.d_ok, cnt, cudaMemcpyDeviceToHost, ctx->stream));
+          return BLSGPU_OK;
+        }));
+    // every item of a failing leaf is decided by its own exact equation e(pk_i, H(m_i)) e(-g, sig_i) == 1
+    std::vector<uint32_t> items;
+    for (size_t c = 0; c < cand.size(); c++)
+      if (!res[c])
+        for (uint32_t t = 0; t < leaves[cand[c]].count; t++) items.push_back(order[leaves[cand[c]].first + t]);
+    CKR(probe_rounds(
+        ctx, P, items, nullptr,
+        [&](size_t cnt) -> int {
+          LAUNCH((k_probe_fill_grouped<PkA, SigA>), blocks_for(cnt), TPB, cnt, (const uint32_t*)P.d_idx, (const PkA*)G.pk, (const uint32_t*)G.midx,
+                 (const SigA*)G.hq, (const SigA*)G.sig, (const uint8_t*)G.status, P.x_pk, P.x_h, P.x_pre);
+          return BLSGPU_OK;
+        },
+        [&](size_t, size_t cnt) -> int {
+          LAUNCH(k_mark_invalid, blocks_for(cnt), TPB, cnt, (const uint32_t*)P.d_idx, (const uint8_t*)P.d_ok, G.status);
+          return BLSGPU_OK;
+        }));
+  }
+  stage_mark(ctx, BLSGPU_STAGE_COUNT);
+  CK(cudaMemcpyAsync(status_out, G.status, n, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  stage_collect(ctx);
+  return BLSGPU_OK;
+}
+}  // namespace
+
+int blsgpu_verify_batch_grouped(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t n, const uint8_t* pks, const uint8_t* sigs,
+                                const uint32_t* msg_idx, size_t q, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
+  NVTX_RANGE("blsgpu_verify_batch_grouped");
+  if (!ctx) return BLSGPU_E_ARG;
+  if (!args_ok(impl_id, scheme, format) || (n && (!pks || !sigs || !msg_idx || !msg_off || !status_out))) {
+    ctx->err = "blsgpu_verify_batch_grouped: bad arguments";
+    return BLSGPU_E_ARG;
+  }
+  if (n == 0) return BLSGPU_OK;
+  if (n > 0xfffffff0ull) {
+    ctx->err = "blsgpu_verify_batch_grouped: at most 2^32 - 16 items per call";
+    return BLSGPU_E_ARG;
+  }
+  CHECK_OFFSETS(msg_off, q, "blsgpu_verify_batch_grouped");
+  if (msg_off[q] > msg_off[0] && !msgs) {
+    ctx->err = "blsgpu_verify_batch_grouped: msgs is null";
+    return BLSGPU_E_ARG;
+  }
+  for (size_t i = 0; i < n; i++)
+    if (msg_idx[i] >= q) {
+      ctx->err = "blsgpu_verify_batch_grouped: msg_idx[" + std::to_string(i) + "] is not below q";
+      return BLSGPU_E_ARG;
+    }
+  CKR(set_device(ctx));
+  if (scheme == 1) {
+    // MessageAugmentation hashes pk || msg: no two items share a hash.  Per-item messages through blsgpu_verify_batch's pipeline.
+    std::vector<uint64_t> off(n + 1, 0);
+    for (size_t i = 0; i < n; i++) off[i + 1] = off[i] + (msg_off[msg_idx[i] + 1] - msg_off[msg_idx[i]]);
+    std::vector<uint8_t> data(std::max<uint64_t>(off[n], 1));
+    for (size_t i = 0; i < n; i++)
+      if (off[i + 1] > off[i]) memcpy(data.data() + off[i], msgs + msg_off[msg_idx[i]], (size_t)(off[i + 1] - off[i]));
+    DstParam dst;
+    make_dst(dst, impl_id, scheme, false);
+    return with_impl(impl_id, [&](auto I) { return verify_host_one<I>(ctx, 1, dst, format, n, pks, sigs, data.data(), off.data(), status_out); });
+  }
+  return with_impl(impl_id, [&](auto I) { return verify_grouped_impl<I>(ctx, scheme, format, n, pks, sigs, msg_idx, q, msgs, msg_off, status_out); });
 }
 
 // ---------------------------------------------------------------------------------------------------------------------

@@ -101,6 +101,15 @@ int blsgpu_verify_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int format, si
 int blsgpu_verify_batch_dev(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t n, const uint8_t* pks_dev,
                             const uint8_t* sigs_dev, const uint8_t* msgs_dev, const uint64_t* msg_off_dev,
                             uint8_t* status_out_dev);
+/* n x Signature::verify(&pk_i, msg_{msg_idx[i]}) where many items share a message (reference: the same chain as
+ * blsgpu_verify_batch).  q messages: message j = msgs[msg_off[j] .. msg_off[j+1]); item i signs message msg_idx[i] < q
+ * (items need not be sorted, a message may have any number of items, including none).  status_out[i] is exactly what
+ * blsgpu_verify_batch returns for item i with its own copy of the message.  Basic and ProofOfPossession hash each message
+ * once and run one Miller loop per run of up to 96 items of one message; MessageAugmentation hashes pk || msg, so it runs
+ * blsgpu_verify_batch's pipeline on per-item messages.  msg_idx[i] >= q, at most 2^32 - 16 items.  First device only. */
+int blsgpu_verify_batch_grouped(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t n, const uint8_t* pks,
+                                const uint8_t* sigs, const uint32_t* msg_idx, size_t q, const uint8_t* msgs,
+                                const uint64_t* msg_off, uint8_t* status_out);
 
 /* ---- one batch cut over several GPUs / processes (SURVEY.md section 8e) ---------------------------------------------------
  * The random-linear-combination check of a batch factors over slices: every slice folds into ONE partial product of

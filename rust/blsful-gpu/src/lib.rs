@@ -323,6 +323,60 @@ impl Engine {
         Ok(status)
     }
 
+    /// `sigs[i].verify(&pks[i], msgs[msg_idx[i]])` for every i, where many items share a message: each message is
+    /// hashed once and the items of one message share their Miller loops.  The results equal [`Engine::verify_batch`]'s
+    /// on the same items with their messages written out; the scheme rule is the same (a signature of another scheme
+    /// than the first gets `InvalidSignatureScheme`).
+    pub fn verify_batch_grouped<C: GpuImpl, B: AsRef<[u8]>>(
+        &mut self,
+        pks: &[PublicKey<C>],
+        sigs: &[Signature<C>],
+        msg_idx: &[u32],
+        msgs: &[B],
+    ) -> EngineResult<Vec<BlsResult<()>>> {
+        let n = sigs.len();
+        if pks.len() != n || msg_idx.len() != n {
+            return Err(EngineError { code: sys::BLSGPU_E_ARG, message: "verify_batch_grouped: slice lengths differ".into() });
+        }
+        if n == 0 {
+            return Ok(Vec::new());
+        }
+        let scheme = signature_scheme(&sigs[0]);
+        let pk_bytes = pack_points(pks.iter().map(|p| p.0), C::PK_BYTES);
+        let sig_bytes = pack_points(sigs.iter().map(|s| *s.as_raw_value()), C::SIG_BYTES);
+        let packed = PackedMessages::from_iter(msgs.iter());
+        let status = self.verify_batch_grouped_bytes::<C>(scheme, SerializationFormat::Modern, &pk_bytes, &sig_bytes, msg_idx, &packed)?;
+        Ok(status
+            .iter()
+            .zip(sigs)
+            .map(|(&st, s)| if signature_scheme(s) != scheme { Err(BlsError::InvalidSignatureScheme) } else { status_to_result(st, None) })
+            .collect())
+    }
+
+    /// The zero-copy form of [`Engine::verify_batch_grouped`]: points already serialised (`format` says how), one status
+    /// byte per item.
+    pub fn verify_batch_grouped_bytes<C: GpuImpl>(
+        &mut self,
+        scheme: SignatureSchemes,
+        format: SerializationFormat,
+        pks: &[u8],
+        sigs: &[u8],
+        msg_idx: &[u32],
+        msgs: &PackedMessages,
+    ) -> EngineResult<Vec<u8>> {
+        let n = msg_idx.len();
+        if pks.len() != n * C::PK_BYTES || sigs.len() != n * C::SIG_BYTES {
+            return Err(EngineError { code: sys::BLSGPU_E_ARG, message: "verify_batch_grouped_bytes: buffer sizes do not match n".into() });
+        }
+        let mut status = vec![0u8; n];
+        let rc = unsafe {
+            sys::blsgpu_verify_batch_grouped(self.ctx, C::IMPL_ID, scheme_id(scheme), format_id(format), n, pks.as_ptr(), sigs.as_ptr(),
+                msg_idx.as_ptr(), msgs.len(), msgs.bytes.as_ptr(), msgs.offsets.as_ptr(), status.as_mut_ptr())
+        };
+        self.check(rc)?;
+        Ok(status)
+    }
+
     /// `pops[i].verify(pks[i])` for every i.
     pub fn pop_verify_batch<C: GpuImpl>(
         &mut self,

@@ -5,6 +5,7 @@ crate would gain (INTEGRATION.md) are mirrored here in Python over the same C AB
 argument meaning and error behaviour:
 
   Signature::verify            -> verify_batch            (reference src/signature.rs:130-138)
+                               -> verify_batch_keyed      (keys decoded once into a KeySet, named by index)
   ProofOfPossession::verify    -> pop_verify_batch        (src/proof_of_possession.rs:77-81)
   AggregateSignature::verify   -> aggregate_verify        (src/aggregate_signature.rs:230-239)
                                -> aggregate_verify_batch_status (q aggregates in one call)
@@ -112,6 +113,10 @@ def load_library() -> ctypes.CDLL:
         "blsgpu_verify_batch": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u8p, u8p, u8p, u64p, u8p]),
         "blsgpu_verify_batch_dev": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u8p, u8p, u8p, u64p, u8p]),
         "blsgpu_verify_batch_grouped": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u8p, u8p, vp, c.c_size_t, u8p, u64p, u8p]),
+        "blsgpu_keyset_create": (c.c_int, [vp, c.c_int, c.c_int, c.c_size_t, u8p, u8p, c.POINTER(c.c_uint64)]),
+        "blsgpu_keyset_destroy": (c.c_int, [vp, c.c_uint64]),
+        "blsgpu_verify_batch_keyed": (c.c_int, [vp, c.c_uint64, c.c_int, c.c_int, c.c_size_t, vp, u8p, u8p, u64p, u8p]),
+        "blsgpu_verify_batch_grouped_keyed": (c.c_int, [vp, c.c_uint64, c.c_int, c.c_int, c.c_size_t, vp, u8p, vp, c.c_size_t, u8p, u64p, u8p]),
         "blsgpu_miller_partial": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u8p, u8p, u8p, u64p, u8p, u8p]),
         "blsgpu_final_exp_is_one": (c.c_int, [vp, c.c_int, c.c_size_t, u8p, u8p, c.POINTER(c.c_int)]),
         "blsgpu_partial_finish": (c.c_int, [vp, c.c_int, u8p]),
@@ -153,6 +158,7 @@ EXPORTED_SYMBOLS = [
     "blsgpu_ctx_create", "blsgpu_ctx_destroy", "blsgpu_last_error", "blsgpu_ctx_set_rlc_salt", "blsgpu_ctx_set_rlc_bits",
     "blsgpu_ctx_set_stream",
     "blsgpu_verify_batch", "blsgpu_verify_batch_grouped",
+    "blsgpu_keyset_create", "blsgpu_keyset_destroy", "blsgpu_verify_batch_keyed", "blsgpu_verify_batch_grouped_keyed",
     "blsgpu_miller_partial", "blsgpu_final_exp_is_one", "blsgpu_partial_finish",
     "blsgpu_verify_batch_dev", "blsgpu_pop_verify_batch", "blsgpu_aggregate_verify", "blsgpu_aggregate_verify_batch", "blsgpu_sum_points",
     "blsgpu_verify_secure_batch", "blsgpu_aggregate_secure_batch", "blsgpu_hash_to_curve_batch", "blsgpu_recode_points",
@@ -236,6 +242,27 @@ def _pack_points(points, length: int, what: str) -> np.ndarray:
         if len(p) != length:
             raise BlsError(ST_INVALID_LENGTH, f"{what}: expected {length} bytes, got {len(p)}")
     return np.frombuffer(b"".join(bytes(p) for p in points), dtype=np.uint8)
+
+
+class KeySet:
+    """Public keys of one impl decoded once on the engine's first device (blsgpu_keyset_create), named by index in
+    Engine.verify_batch_keyed / verify_batch_grouped_keyed.  status[i]: ST_OK, ST_DESERIALIZE or ST_LEGACY_FORMAT for key i
+    (a key that failed to decode stays in the set and gives its items that status).  The engine owns the device memory:
+    close() frees it, and so does Engine.close()."""
+
+    def __init__(self, engine: "Engine", impl_id: int, ident: int, status: np.ndarray):
+        self._engine = engine
+        self.impl_id = impl_id
+        self.id = ident
+        self.status = status
+
+    def __len__(self) -> int:
+        return self.status.size
+
+    def close(self) -> None:
+        if self.id and getattr(self._engine, "_ctx", None):
+            self._engine._check(self._engine._lib.blsgpu_keyset_destroy(self._engine._ctx, self.id), "blsgpu_keyset_destroy")
+        self.id = 0
 
 
 class Engine:
@@ -324,6 +351,66 @@ class Engine:
         rc = self._lib.blsgpu_verify_batch_grouped(self._ctx, impl_id, scheme, fmt, n, _ptr(pk), _ptr(sg), _ptr(msg_idx), off.size - 1,
                                                    _ptr(data), _ptr(off), _ptr(status))
         self._check(rc, "blsgpu_verify_batch_grouped")
+        return status
+
+    # ---- key sets: public keys decoded once, verify calls that name them by index -----------------------------------
+    def key_set(self, impl_id: int, pks, fmt: int = SerializationFormat.Modern) -> KeySet:
+        """Decodes and subgroup-checks the keys once; they stay in device memory until KeySet.close() or Engine.close()."""
+        pk = _pack_points(pks, pk_len(impl_id), "public key")
+        n = pk.size // pk_len(impl_id)
+        status = np.zeros(n, dtype=np.uint8)
+        ident = ctypes.c_uint64(0)
+        self._check(self._lib.blsgpu_keyset_create(self._ctx, impl_id, fmt, n, _ptr(pk), _ptr(status), ctypes.byref(ident)),
+                    "blsgpu_keyset_create")
+        return KeySet(self, impl_id, ident.value, status)
+
+    def verify_batch_keyed(self, keys: KeySet, scheme: int, key_idx, sigs, msgs: Sequence[bytes],
+                           fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """verify_batch with pks[i] = key key_idx[i] of `keys` (fmt is the signatures' format)."""
+        sg = _pack_points(sigs, sig_len(keys.impl_id), "signature")
+        idx = np.ascontiguousarray(key_idx, dtype=np.uint32).reshape(-1)
+        if sg.size // sig_len(keys.impl_id) != idx.size or len(msgs) != idx.size:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        data, off = pack_messages(msgs)
+        return self.verify_batch_keyed_packed(keys, scheme, idx, sg, data, off, fmt)
+
+    def verify_batch_keyed_packed(self, keys: KeySet, scheme: int, key_idx: np.ndarray, sg: np.ndarray, data: np.ndarray, off: np.ndarray,
+                                  fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """Flat-buffer form: key_idx uint32[n], sg n signatures, the n messages as data / off (n + 1 offsets)."""
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32).reshape(-1)
+        n = off.size - 1
+        if key_idx.size != n:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        status = np.empty(n, dtype=np.uint8)
+        rc = self._lib.blsgpu_verify_batch_keyed(self._ctx, keys.id, scheme, fmt, n, _ptr(key_idx), _ptr(sg), _ptr(data), _ptr(off),
+                                                 _ptr(status))
+        self._check(rc, "blsgpu_verify_batch_keyed")
+        return status
+
+    def verify_batch_grouped_keyed(self, keys: KeySet, scheme: int, key_idx, sigs, msg_idx, msgs: Sequence[bytes],
+                                   fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """verify_batch_grouped with pks[i] = key key_idx[i] of `keys` (fmt is the signatures' format)."""
+        sg = _pack_points(sigs, sig_len(keys.impl_id), "signature")
+        kidx = np.ascontiguousarray(key_idx, dtype=np.uint32).reshape(-1)
+        midx = np.ascontiguousarray(msg_idx, dtype=np.uint32).reshape(-1)
+        n = kidx.size
+        if sg.size // sig_len(keys.impl_id) != n or midx.size != n:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        data, off = pack_messages(msgs)
+        return self.verify_batch_grouped_keyed_packed(keys, scheme, kidx, sg, midx, data, off, fmt)
+
+    def verify_batch_grouped_keyed_packed(self, keys: KeySet, scheme: int, key_idx: np.ndarray, sg: np.ndarray, msg_idx: np.ndarray,
+                                          data: np.ndarray, off: np.ndarray, fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """Flat-buffer form: key_idx and msg_idx uint32[n], sg n signatures, the q messages as data / off (q + 1 offsets)."""
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32).reshape(-1)
+        msg_idx = np.ascontiguousarray(msg_idx, dtype=np.uint32).reshape(-1)
+        n = msg_idx.size
+        if key_idx.size != n:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        status = np.empty(n, dtype=np.uint8)
+        rc = self._lib.blsgpu_verify_batch_grouped_keyed(self._ctx, keys.id, scheme, fmt, n, _ptr(key_idx), _ptr(sg), _ptr(msg_idx),
+                                                         off.size - 1, _ptr(data), _ptr(off), _ptr(status))
+        self._check(rc, "blsgpu_verify_batch_grouped_keyed")
         return status
 
     def verify_batch_dev(self, impl_id, scheme, n, pk_ptr: int, sig_ptr: int, msg_ptr: int, off_ptr: int, status_ptr: int,

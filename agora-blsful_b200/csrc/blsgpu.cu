@@ -6,6 +6,7 @@
 #include <sys/random.h>
 
 #include <algorithm>
+#include <atomic>
 #include <functional>
 #include <cstdio>
 #include <cstdlib>
@@ -114,9 +115,19 @@ struct PendingSlice {
   virtual int finish(blsgpu_ctx* ctx, bool batch_ok, uint8_t* status_out) = 0;
 };
 
+// public keys decoded once (blsgpu_keyset_create): n affine points of the impl's key group and their decode statuses, in a
+// device allocation of their own on the first device (apart from the arena, so that regrowing the arena keeps them)
+struct KeySet {
+  int impl_id = 0;
+  size_t n = 0;
+  void* pts = nullptr;
+  uint8_t* st = nullptr;
+};
+
 struct blsgpu_ctx {
   std::vector<int> devices;
   std::unique_ptr<PendingSlice> pending;  // invalidated by every call that re-plans the arena
+  std::unordered_map<uint64_t, KeySet> keysets;  // by id: ids come from a process-wide counter and are never reused
   uint8_t* fold_scratch = nullptr;        // small device buffer of the fold (blsgpu_final_exp_is_one), apart from the arena
   size_t fold_cap = 0;
   std::vector<blsgpu_ctx*> peers;  // one single-device context per further device (devices[1..]); see verify_host_common
@@ -836,6 +847,24 @@ int decode_points(blsgpu_ctx* ctx, size_t n, const uint8_t* d_in, int format, A*
   return BLSGPU_OK;
 }
 
+// The public keys of a verify call: n compressed keys in the call's format (`bytes`), or, for the keyed entry points, the
+// index of every item's key (`idx`) in a key set decoded once (`set`).  Host pointers until the call uploads them.
+struct Keys {
+  const uint8_t* bytes = nullptr;
+  const KeySet* set = nullptr;
+  const uint32_t* idx = nullptr;
+  Keys(const uint8_t* b = nullptr) : bytes(b) {}
+  Keys(const KeySet* s, const uint32_t* i) : set(s), idx(i) {}
+};
+// the key step of a verify call, the one step where keyed and unkeyed calls differ: d_pk / d_st of the n items, by decoding
+// their bytes or by gathering them from the key set (no decode or subgroup check)
+template <class PkA>
+int load_keys(blsgpu_ctx* ctx, size_t n, const Keys& d_keys, int format, PkA* d_pk, uint8_t* d_st) {
+  if (!d_keys.set) return decode_points<PkA>(ctx, n, d_keys.bytes, format, d_pk, d_st, BLSGPU_KERNEL_DECODE_PK);
+  LAUNCH((k_gather_keys<PkA>), blocks_for(n), TPB, n, d_keys.idx, (const PkA*)d_keys.set->pts, (const uint8_t*)d_keys.set->st, d_pk, d_st);
+  return BLSGPU_OK;
+}
+
 // hash_to_curve of n framed messages into affine points: k_hash leaves Jacobian points in scratch that is handed back to
 // the arena at once (later takes on the same stream may reuse it), k_to_affine_batch normalises them 16 per inversion
 template <class HA, class PkA>
@@ -880,11 +909,11 @@ int verify_points(blsgpu_ctx* ctx, int msg_mode, const DstParam& dst, size_t n, 
   return check_and_bisect(ctx, P);
 }
 
-// verify over device-resident compressed inputs.  msg_mode: 0 msg, 1 pk||msg, 2 pk bytes (PoP).
-// verify_dev_partials stops after the slice's partial results (its product of Miller values and sum of r_i sig_i).
+// verify over device-resident inputs: compressed signatures, keys as bytes or key-set indices.  msg_mode: 0 msg, 1 pk||msg,
+// 2 pk bytes (PoP).  verify_dev_partials stops after the slice's partial results (its product of Miller values and sum of r_i sig_i).
 template <int IMPL>
 int verify_dev_partials(blsgpu_ctx* ctx, Pipe<typename ImplT<IMPL>::PkAff, typename ImplT<IMPL>::SigAff>& P, int msg_mode, const DstParam& dst,
-                        int format, size_t n, const uint8_t* d_pks, const uint8_t* d_sigs, const uint8_t* d_msgs, const uint64_t* d_moff,
+                        int format, size_t n, const Keys& d_keys, const uint8_t* d_sigs, const uint8_t* d_msgs, const uint64_t* d_moff,
                         uint8_t* d_status_out) {
   typedef typename ImplT<IMPL>::PkAff PkA;
   typedef typename ImplT<IMPL>::SigAff SigA;
@@ -894,7 +923,7 @@ int verify_dev_partials(blsgpu_ctx* ctx, Pipe<typename ImplT<IMPL>::PkAff, typen
   uint8_t* d_stsig = ctx->arena.take<uint8_t>(n);
   stage_reset(ctx);
   stage_mark(ctx, BLSGPU_STAGE_DECODE_PK);
-  CKR((decode_points<PkA>(ctx, n, d_pks, format, d_pk, d_stpk, BLSGPU_KERNEL_DECODE_PK)));
+  CKR((load_keys<PkA>(ctx, n, d_keys, format, d_pk, d_stpk)));
   stage_mark(ctx, BLSGPU_STAGE_DECODE_SIG);
   CKR((decode_points<SigA>(ctx, n, d_sigs, format, d_sig, d_stsig, BLSGPU_KERNEL_DECODE_SIG)));
   return verify_points_partials<IMPL>(ctx, P, msg_mode, dst, n, d_pk, d_sig, d_stpk, d_stsig, d_msgs, d_moff, d_status_out);
@@ -1032,6 +1061,21 @@ int upload(blsgpu_ctx* ctx, T*& d, const T* h, size_t count) {
   if (count) CK(cudaMemcpyAsync(d, h, count * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
   return BLSGPU_OK;
 }
+// the keys of a call on the device: its compressed key bytes, or its key indices, uploaded to the arena
+template <class PkA>
+int upload_keys(blsgpu_ctx* ctx, size_t n, const Keys& keys, Keys& d_keys) {
+  d_keys = keys;
+  if (keys.set) {
+    uint32_t* d_idx;
+    CKR(upload(ctx, d_idx, keys.idx, n));
+    d_keys.idx = d_idx;
+  } else {
+    uint8_t* d_pks;
+    CKR(upload(ctx, d_pks, keys.bytes, n * PtInfo<PkA>::LEN));
+    d_keys.bytes = d_pks;
+  }
+  return BLSGPU_OK;
+}
 
 int set_device(blsgpu_ctx* ctx) {
   CK(cudaSetDevice(ctx->devices[0]));
@@ -1123,6 +1167,10 @@ void blsgpu_ctx_destroy(blsgpu_ctx* ctx) {
   for (blsgpu_ctx* peer : ctx->peers) blsgpu_ctx_destroy(peer);
   cudaSetDevice(ctx->devices[0]);
   ctx->pending.reset();
+  for (const auto& ks : ctx->keysets) {
+    cudaFree(ks.second.pts);
+    cudaFree(ks.second.st);
+  }
   if (ctx->arena.base) cudaFree(ctx->arena.base);
   if (ctx->fold_scratch) cudaFree(ctx->fold_scratch);
   for (int i = 0; i <= BLSGPU_STAGE_COUNT; i++) cudaEventDestroy(ctx->ev[i]);
@@ -1211,15 +1259,16 @@ namespace {
 // host buffers of one slice -> its partial results (state in P, statuses so far in *d_st_out); the stream is synchronised
 template <int IMPL>
 int host_partials(blsgpu_ctx* ctx, Pipe<typename ImplT<IMPL>::PkAff, typename ImplT<IMPL>::SigAff>& P, int msg_mode, const DstParam& dst, int format,
-                  size_t n, const uint8_t* pks, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off, uint8_t** d_st_out) {
+                  size_t n, const Keys& keys, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off, uint8_t** d_st_out) {
   CKR(set_device(ctx));
   const size_t pk_len = IMPL == 2 ? 48 : 96, sig_len = IMPL == 2 ? 96 : 48;
   size_t msg_bytes = msg_off ? (size_t)(msg_off[n] - msg_off[0]) : 0;
-  size_t in_bytes = n * (pk_len + sig_len + 1) + msg_bytes + (n + 1) * 8 + 16 * 256 + 8192;
+  size_t in_bytes = n * (pk_len + sig_len + 1) + msg_bytes + (n + 1) * 8 + 16 * 256 + 8192;  // key bytes or (fewer) key indices
   CKR(ensure_verify_arena<IMPL>(ctx, n, in_bytes));
-  uint8_t *d_pks, *d_sigs, *d_msgs;
+  uint8_t *d_sigs, *d_msgs;
   uint64_t* d_off;
-  CKR(upload(ctx, d_pks, pks, n * pk_len));
+  Keys d_keys;
+  CKR(upload_keys<typename ImplT<IMPL>::PkAff>(ctx, n, keys, d_keys));
   CKR(upload(ctx, d_sigs, sigs, n * sig_len));
   CKR(upload(ctx, d_msgs, msg_off ? msgs + msg_off[0] : msgs, msg_bytes));
   if (msg_off && msg_off[0] == 0) {
@@ -1231,7 +1280,7 @@ int host_partials(blsgpu_ctx* ctx, Pipe<typename ImplT<IMPL>::PkAff, typename Im
   }
   uint8_t* d_st = ctx->arena.take<uint8_t>(n);
   *d_st_out = d_st;
-  CKR((verify_dev_partials<IMPL>(ctx, P, msg_mode, dst, format, n, d_pks, d_sigs, d_msgs, d_off, d_st)));
+  CKR((verify_dev_partials<IMPL>(ctx, P, msg_mode, dst, format, n, d_keys, d_sigs, d_msgs, d_off, d_st)));
   CK(cudaStreamSynchronize(ctx->stream));
   return BLSGPU_OK;
 }
@@ -1252,11 +1301,11 @@ int host_finish(blsgpu_ctx* ctx, Pipe<typename ImplT<IMPL>::PkAff, typename Impl
 }
 
 template <int IMPL>
-int verify_host_one(blsgpu_ctx* ctx, int msg_mode, const DstParam& dst, int format, size_t n, const uint8_t* pks, const uint8_t* sigs,
+int verify_host_one(blsgpu_ctx* ctx, int msg_mode, const DstParam& dst, int format, size_t n, const Keys& keys, const uint8_t* sigs,
                     const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
   Pipe<typename ImplT<IMPL>::PkAff, typename ImplT<IMPL>::SigAff> P;
   uint8_t* d_st = nullptr;
-  CKR((host_partials<IMPL>(ctx, P, msg_mode, dst, format, n, pks, sigs, msgs, msg_off, &d_st)));
+  CKR((host_partials<IMPL>(ctx, P, msg_mode, dst, format, n, keys, sigs, msgs, msg_off, &d_st)));
   return host_finish<IMPL>(ctx, P, false, d_st, n, status_out);
 }
 
@@ -1940,7 +1989,9 @@ struct Grouped {
   typedef typename PtInfo<PkA>::Jac PkJ;
   typedef typename PtInfo<SigA>::Jac SigJ;
   size_t n = 0, q = 0, nl = 0, nbig = 0, nsmall = 0, msg_bytes = 0, blocks = 1;
+  bool keyed = false;  // the keys come from a key set: key indices instead of key bytes
   uint8_t *pkb, *sigb, *msgs, *mpre, *stpk, *stsig, *status, *lpre;
+  uint32_t* kidx;
   uint64_t* moff;
   uint32_t *midx, *order, *big, *small;  // big / small: the leaves of k_leaf_msm / k_leaf_scale
   GLeaf* leaves;
@@ -1961,7 +2012,10 @@ void take_grouped(A& a, Grouped<PkA, SigA>& G) {
   typedef typename Grouped<PkA, SigA>::PkJ PkJ;
   typedef typename Grouped<PkA, SigA>::SigJ SigJ;
   const size_t n = G.n, nl = G.nl, ng = (nl + M6_GROUP - 1) / M6_GROUP, ndig = levels_total(make_levels(n));
-  G.pkb = a.template take<uint8_t>(n * PtInfo<PkA>::LEN);
+  if (G.keyed)
+    G.kidx = a.template take<uint32_t>(n);
+  else
+    G.pkb = a.template take<uint8_t>(n * PtInfo<PkA>::LEN);
   G.sigb = a.template take<uint8_t>(n * PtInfo<SigA>::LEN);
   G.msgs = a.template take<uint8_t>(std::max<size_t>(G.msg_bytes, 1));
   G.moff = a.template take<uint64_t>(G.q + 1);
@@ -2023,7 +2077,7 @@ int leaf_sums(blsgpu_ctx* ctx, const G& g, const A* pts, const RlcScalar* d_r, i
 }
 
 template <int IMPL>
-int verify_grouped_impl(blsgpu_ctx* ctx, int scheme, int format, size_t n, const uint8_t* pks, const uint8_t* sigs, const uint32_t* msg_idx,
+int verify_grouped_impl(blsgpu_ctx* ctx, int scheme, int format, size_t n, const Keys& keys, const uint8_t* sigs, const uint32_t* msg_idx,
                         size_t q, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
   typedef typename ImplT<IMPL>::PkAff PkA;
   typedef typename ImplT<IMPL>::SigAff SigA;
@@ -2050,6 +2104,7 @@ int verify_grouped_impl(blsgpu_ctx* ctx, int scheme, int format, size_t n, const
   Grouped<PkA, SigA> G;
   G.n = n;
   G.q = q;
+  G.keyed = keys.set != nullptr;
   G.nl = leaves.size();
   G.nbig = big.size();
   G.nsmall = small.size();
@@ -2062,7 +2117,14 @@ int verify_grouped_impl(blsgpu_ctx* ctx, int scheme, int format, size_t n, const
   Pipe<PkA, SigA>& P = G.P;
   stage_reset(ctx);
   const std::vector<uint64_t> moff = rebased(msg_off, 0, q);
-  CK(cudaMemcpyAsync(G.pkb, pks, n * PtInfo<PkA>::LEN, cudaMemcpyHostToDevice, ctx->stream));
+  Keys d_keys = keys;
+  if (G.keyed) {
+    CK(cudaMemcpyAsync(G.kidx, keys.idx, n * 4, cudaMemcpyHostToDevice, ctx->stream));
+    d_keys.idx = G.kidx;
+  } else {
+    CK(cudaMemcpyAsync(G.pkb, keys.bytes, n * PtInfo<PkA>::LEN, cudaMemcpyHostToDevice, ctx->stream));
+    d_keys.bytes = G.pkb;
+  }
   CK(cudaMemcpyAsync(G.sigb, sigs, n * PtInfo<SigA>::LEN, cudaMemcpyHostToDevice, ctx->stream));
   if (G.msg_bytes) CK(cudaMemcpyAsync(G.msgs, msgs + msg_off[0], G.msg_bytes, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(G.moff, moff.data(), (q + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
@@ -2074,7 +2136,7 @@ int verify_grouped_impl(blsgpu_ctx* ctx, int scheme, int format, size_t n, const
   if (G.nsmall) CK(cudaMemcpyAsync(G.small, small.data(), G.nsmall * 4, cudaMemcpyHostToDevice, ctx->stream));
   // decode, per-item statuses (item order throughout)
   stage_mark(ctx, BLSGPU_STAGE_DECODE_PK);
-  CKR((decode_points<PkA>(ctx, n, (const uint8_t*)G.pkb, format, G.pk, G.stpk, BLSGPU_KERNEL_DECODE_PK)));
+  CKR((load_keys<PkA>(ctx, n, d_keys, format, G.pk, G.stpk)));
   stage_mark(ctx, BLSGPU_STAGE_DECODE_SIG);
   CKR((decode_points<SigA>(ctx, n, (const uint8_t*)G.sigb, format, G.sig, G.stsig, BLSGPU_KERNEL_DECODE_SIG)));
   LAUNCH((k_prestatus<PkA, SigA>), blocks_for(n), TPB, n, (const uint8_t*)G.stpk, (const uint8_t*)G.stsig, (const PkA*)G.pk, (const SigA*)G.sig,
@@ -2191,31 +2253,49 @@ int verify_grouped_impl(blsgpu_ctx* ctx, int scheme, int format, size_t n, const
   stage_collect(ctx);
   return BLSGPU_OK;
 }
-}  // namespace
 
-int blsgpu_verify_batch_grouped(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t n, const uint8_t* pks, const uint8_t* sigs,
-                                const uint32_t* msg_idx, size_t q, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
-  NVTX_RANGE("blsgpu_verify_batch_grouped");
-  if (!ctx) return BLSGPU_E_ARG;
-  if (!args_ok(impl_id, scheme, format) || (n && (!pks || !sigs || !msg_idx || !msg_off || !status_out))) {
-    ctx->err = "blsgpu_verify_batch_grouped: bad arguments";
+// the key set `id` of this context, or nullptr with the error set (an id that was destroyed, never issued, or is another context's)
+const KeySet* find_keyset(blsgpu_ctx* ctx, uint64_t id, const char* what) {
+  const auto it = ctx->keysets.find(id);
+  if (it != ctx->keysets.end()) return &it->second;
+  ctx->err = std::string(what) + ": key set " + std::to_string(id) + " is not held by this context";
+  return nullptr;
+}
+// keyed calls: every item names a key of the set
+bool key_idx_ok(blsgpu_ctx* ctx, const char* what, const Keys& keys, size_t n) {
+  if (!keys.set) return true;
+  for (size_t i = 0; i < n; i++)
+    if (keys.idx[i] >= keys.set->n) {
+      ctx->err = std::string(what) + ": key_idx[" + std::to_string(i) + "] is not below the key set's size " + std::to_string(keys.set->n);
+      return false;
+    }
+  return true;
+}
+
+// blsgpu_verify_batch_grouped and its keyed form: the argument checks, then the grouped pipeline, or for MessageAugmentation
+// blsgpu_verify_batch's pipeline on per-item messages
+int verify_grouped_common(blsgpu_ctx* ctx, const char* what, int impl_id, int scheme, int format, size_t n, const Keys& keys, const uint8_t* sigs,
+                          const uint32_t* msg_idx, size_t q, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
+  if (!args_ok(impl_id, scheme, format) || (n && (!(keys.set ? (const void*)keys.idx : (const void*)keys.bytes) || !sigs || !msg_idx || !msg_off || !status_out))) {
+    ctx->err = std::string(what) + ": bad arguments";
     return BLSGPU_E_ARG;
   }
   if (n == 0) return BLSGPU_OK;
   if (n > 0xfffffff0ull) {
-    ctx->err = "blsgpu_verify_batch_grouped: at most 2^32 - 16 items per call";
+    ctx->err = std::string(what) + ": at most 2^32 - 16 items per call";
     return BLSGPU_E_ARG;
   }
-  CHECK_OFFSETS(msg_off, q, "blsgpu_verify_batch_grouped");
+  CHECK_OFFSETS(msg_off, q, what);
   if (msg_off[q] > msg_off[0] && !msgs) {
-    ctx->err = "blsgpu_verify_batch_grouped: msgs is null";
+    ctx->err = std::string(what) + ": msgs is null";
     return BLSGPU_E_ARG;
   }
   for (size_t i = 0; i < n; i++)
     if (msg_idx[i] >= q) {
-      ctx->err = "blsgpu_verify_batch_grouped: msg_idx[" + std::to_string(i) + "] is not below q";
+      ctx->err = std::string(what) + ": msg_idx[" + std::to_string(i) + "] is not below q";
       return BLSGPU_E_ARG;
     }
+  if (!key_idx_ok(ctx, what, keys, n)) return BLSGPU_E_ARG;
   CKR(set_device(ctx));
   if (scheme == 1) {
     // MessageAugmentation hashes pk || msg: no two items share a hash.  Per-item messages through blsgpu_verify_batch's pipeline.
@@ -2226,9 +2306,118 @@ int blsgpu_verify_batch_grouped(blsgpu_ctx* ctx, int impl_id, int scheme, int fo
       if (off[i + 1] > off[i]) memcpy(data.data() + off[i], msgs + msg_off[msg_idx[i]], (size_t)(off[i + 1] - off[i]));
     DstParam dst;
     make_dst(dst, impl_id, scheme, false);
-    return with_impl(impl_id, [&](auto I) { return verify_host_one<I>(ctx, 1, dst, format, n, pks, sigs, data.data(), off.data(), status_out); });
+    return with_impl(impl_id, [&](auto I) { return verify_host_one<I>(ctx, 1, dst, format, n, keys, sigs, data.data(), off.data(), status_out); });
   }
-  return with_impl(impl_id, [&](auto I) { return verify_grouped_impl<I>(ctx, scheme, format, n, pks, sigs, msg_idx, q, msgs, msg_off, status_out); });
+  return with_impl(impl_id, [&](auto I) { return verify_grouped_impl<I>(ctx, scheme, format, n, keys, sigs, msg_idx, q, msgs, msg_off, status_out); });
+}
+
+// n compressed keys -> a key set of this context: decoded and subgroup-checked once into a device allocation of its own
+template <class PkA>
+int keyset_create_impl(blsgpu_ctx* ctx, int impl_id, int format, size_t n, const uint8_t* pks, uint8_t* status_out, uint64_t* keyset_out) {
+  static std::atomic<uint64_t> next_id{1};
+  KeySet s;
+  s.impl_id = impl_id;
+  s.n = n;
+  uint8_t* d_bytes = nullptr;
+  const int r = [&]() -> int {
+    CK(cudaMalloc(&s.pts, std::max<size_t>(n, 1) * sizeof(PkA)));
+    CK(cudaMalloc(&s.st, std::max<size_t>(n, 1)));
+    if (n) {
+      CK(cudaMalloc(&d_bytes, n * PtInfo<PkA>::LEN));
+      CK(cudaMemcpyAsync(d_bytes, pks, n * PtInfo<PkA>::LEN, cudaMemcpyHostToDevice, ctx->stream));
+      CKR((decode_points<PkA>(ctx, n, (const uint8_t*)d_bytes, format, (PkA*)s.pts, s.st)));
+      if (status_out) CK(cudaMemcpyAsync(status_out, s.st, n, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    CK(cudaStreamSynchronize(ctx->stream));
+    return BLSGPU_OK;
+  }();
+  cudaFree(d_bytes);
+  if (r != BLSGPU_OK) {  // no set is created
+    cudaFree(s.pts);
+    cudaFree(s.st);
+    (void)cudaGetLastError();
+    return r;
+  }
+  const uint64_t id = next_id.fetch_add(1);
+  ctx->keysets[id] = s;
+  *keyset_out = id;
+  return BLSGPU_OK;
+}
+}  // namespace
+
+int blsgpu_verify_batch_grouped(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t n, const uint8_t* pks, const uint8_t* sigs,
+                                const uint32_t* msg_idx, size_t q, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
+  NVTX_RANGE("blsgpu_verify_batch_grouped");
+  if (!ctx) return BLSGPU_E_ARG;
+  return verify_grouped_common(ctx, "blsgpu_verify_batch_grouped", impl_id, scheme, format, n, pks, sigs, msg_idx, q, msgs, msg_off, status_out);
+}
+
+// ---- key sets -----------------------------------------------------------------------------------------------------------
+int blsgpu_keyset_create(blsgpu_ctx* ctx, int impl_id, int format, size_t n, const uint8_t* pks, uint8_t* status_out, uint64_t* keyset_out) {
+  NVTX_RANGE("blsgpu_keyset_create");
+  if (!ctx) return BLSGPU_E_ARG;
+  if ((impl_id != 1 && impl_id != 2) || (format != 0 && format != 1) || !keyset_out || (n && !pks)) {
+    ctx->err = "blsgpu_keyset_create: bad arguments";
+    return BLSGPU_E_ARG;
+  }
+  if (n > 0xfffffff0ull) {
+    ctx->err = "blsgpu_keyset_create: at most 2^32 - 16 keys per set";
+    return BLSGPU_E_ARG;
+  }
+  CKR(set_device(ctx));
+  CKR(ensure_arena(ctx, 0));  // takes nothing from the arena: ends a pending slice like any other call
+  return with_impl(impl_id, [&](auto I) { return keyset_create_impl<typename ImplT<I>::PkAff>(ctx, impl_id, format, n, pks, status_out, keyset_out); });
+}
+
+int blsgpu_keyset_destroy(blsgpu_ctx* ctx, uint64_t keyset) {
+  NVTX_RANGE("blsgpu_keyset_destroy");
+  if (!ctx) return BLSGPU_E_ARG;
+  const KeySet* s = find_keyset(ctx, keyset, "blsgpu_keyset_destroy");
+  if (!s) return BLSGPU_E_ARG;
+  ctx->pending.reset();
+  CKR(set_device(ctx));
+  const cudaError_t e1 = cudaFree(s->pts), e2 = cudaFree(s->st);  // cudaFree waits for the work that may still read the set
+  ctx->keysets.erase(keyset);
+  CK(e1 != cudaSuccess ? e1 : e2);
+  return BLSGPU_OK;
+}
+
+int blsgpu_verify_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t n, const uint32_t* key_idx, const uint8_t* sigs,
+                              const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
+  NVTX_RANGE("blsgpu_verify_batch_keyed");
+  if (!ctx) return BLSGPU_E_ARG;
+  const char* what = "blsgpu_verify_batch_keyed";
+  const KeySet* set = find_keyset(ctx, keyset, what);
+  if (!set) return BLSGPU_E_ARG;
+  if (!args_ok(set->impl_id, scheme, format) || (n && (!key_idx || !sigs || !msg_off || !status_out))) {
+    ctx->err = "blsgpu_verify_batch_keyed: bad arguments";
+    return BLSGPU_E_ARG;
+  }
+  if (n == 0) return BLSGPU_OK;
+  if (n > 0xfffffff0ull) {
+    ctx->err = "blsgpu_verify_batch_keyed: at most 2^32 - 16 items per call";
+    return BLSGPU_E_ARG;
+  }
+  CHECK_OFFSETS(msg_off, n, what);
+  if (msg_off[n] > msg_off[0] && !msgs) {
+    ctx->err = "blsgpu_verify_batch_keyed: msgs is null";
+    return BLSGPU_E_ARG;
+  }
+  const Keys keys(set, key_idx);
+  if (!key_idx_ok(ctx, what, keys, n)) return BLSGPU_E_ARG;
+  DstParam dst;
+  make_dst(dst, set->impl_id, scheme, false);
+  return with_impl(set->impl_id, [&](auto I) { return verify_host_one<I>(ctx, scheme == 1 ? 1 : 0, dst, format, n, keys, sigs, msgs, msg_off, status_out); });
+}
+
+int blsgpu_verify_batch_grouped_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t n, const uint32_t* key_idx, const uint8_t* sigs,
+                                      const uint32_t* msg_idx, size_t q, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
+  NVTX_RANGE("blsgpu_verify_batch_grouped_keyed");
+  if (!ctx) return BLSGPU_E_ARG;
+  const char* what = "blsgpu_verify_batch_grouped_keyed";
+  const KeySet* set = find_keyset(ctx, keyset, what);
+  if (!set) return BLSGPU_E_ARG;
+  return verify_grouped_common(ctx, what, set->impl_id, scheme, format, n, Keys(set, key_idx), sigs, msg_idx, q, msgs, msg_off, status_out);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------

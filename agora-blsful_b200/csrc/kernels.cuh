@@ -180,6 +180,18 @@ __global__ void __launch_bounds__(128, SplitBlocks<A>::value) k_subgroup_check(s
   st[i] = ST_DESERIALIZE;
 }
 
+// keyed verification: item i takes the decoded point and the decode status of key key_idx[i] of a key set that k_decode and
+// k_subgroup_check filled once (a key that failed to decode is the identity there, as k_decode leaves it for the item)
+template <class A>
+__global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_gather_keys(size_t n, const uint32_t* __restrict__ key_idx, const A* __restrict__ set_pts,
+                                                     const uint8_t* __restrict__ set_st, A* __restrict__ out, uint8_t* __restrict__ st) {
+  size_t i = BLS_TID();
+  if (i >= n) return;
+  const uint32_t k = key_idx[i];
+  out[i] = set_pts[k];
+  st[i] = set_st[k];
+}
+
 // affine points -> compressed bytes in `format`
 template <class A>
 __global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_encode(size_t n, const A* __restrict__ in, int format, uint8_t* __restrict__ out) {

@@ -65,7 +65,8 @@ typedef struct blsgpu_ctx blsgpu_ctx;
  * results) and blsgpu_verify_secure_batch / blsgpu_aggregate_secure_batch (contiguous runs of key sets, balanced by member
  * count); blsgpu_aggregate_verify cuts its pairs over the devices (from 4096 per device) and folds the partial products of
  * Miller values on the first device; blsgpu_aggregate_verify_batch cuts its aggregates into contiguous runs balanced by pair
- * count (from 4096 pairs per device), each verified on its own device without a fold.  Every other entry point, the *_dev variants and blsgpu_ctx_set_stream use the first device.  One process per
+ * count (from 4096 pairs per device), each verified on its own device without a fold.  Every other entry point (among them
+ * blsgpu_verify_batch_grouped, the key sets and the keyed verify calls), the *_dev variants and blsgpu_ctx_set_stream use the first device.  One process per
  * device with blsgpu_miller_partial / blsgpu_final_exp_is_one does the same across processes. */
 int blsgpu_ctx_create(const int* devices, int ndev, blsgpu_ctx** out);
 void blsgpu_ctx_destroy(blsgpu_ctx* ctx);
@@ -110,6 +111,30 @@ int blsgpu_verify_batch_dev(blsgpu_ctx* ctx, int impl_id, int scheme, int format
 int blsgpu_verify_batch_grouped(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t n, const uint8_t* pks,
                                 const uint8_t* sigs, const uint32_t* msg_idx, size_t q, const uint8_t* msgs,
                                 const uint64_t* msg_off, uint8_t* status_out);
+
+/* ---- key sets: public keys decoded once, named by index ---------------------------------------------------------------
+ * The reference parses and checks a PublicKey<C> once (src/public_key.rs:55-75); the calls above decode every key again
+ * on every call.  A key set holds keys that barely change between calls (a validator set, a masternode list, the signers of
+ * a quorum) decoded and subgroup-checked once, in device memory the context owns apart from its per-call scratch: 145 bytes
+ * per key of impl_id 2 (G1 keys), 273 bytes per key of impl_id 1 (G2 keys).  First device only.
+ *
+ * Decode n public keys of impl_id (compressed, in `format`) once and keep them on the context's first device.
+ * status_out[i] (may be NULL): BLSGPU_ST_OK, DESERIALIZE or LEGACY_FORMAT for key i.  Keys that fail to decode stay in
+ * the set, so that items naming them get exactly the status blsgpu_verify_batch gives for those bytes.
+ * *keyset_out: a non-zero id, unique in the process (never reused).  n = 0 makes an empty set; at most 2^32 - 16 keys.
+ * Synchronises before returning; on BLSGPU_E_ALLOC or BLSGPU_E_CUDA no set is created.  An id this context does not hold
+ * (destroyed, or another context's) is BLSGPU_E_ARG in every call below.  blsgpu_ctx_destroy frees the sets still alive. */
+int blsgpu_keyset_create(blsgpu_ctx* ctx, int impl_id, int format, size_t n, const uint8_t* pks, uint8_t* status_out,
+                         uint64_t* keyset_out);
+int blsgpu_keyset_destroy(blsgpu_ctx* ctx, uint64_t keyset);
+/* blsgpu_verify_batch with pks[i] = the bytes key key_idx[i] of the set was created from; `format` is that of sigs only.
+ * key_idx[i] at or above the set's size is BLSGPU_E_ARG.  No key is decoded: the keys are gathered from the set. */
+int blsgpu_verify_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t n, const uint32_t* key_idx,
+                              const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out);
+/* blsgpu_verify_batch_grouped with pks[i] = the bytes of key key_idx[i] */
+int blsgpu_verify_batch_grouped_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t n,
+                                      const uint32_t* key_idx, const uint8_t* sigs, const uint32_t* msg_idx, size_t q,
+                                      const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out);
 
 /* ---- one batch cut over several GPUs / processes (SURVEY.md section 8e) ---------------------------------------------------
  * The random-linear-combination check of a batch factors over slices: every slice folds into ONE partial product of

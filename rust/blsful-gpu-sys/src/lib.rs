@@ -53,6 +53,17 @@ extern "C" {
     pub fn blsgpu_verify_batch_grouped(ctx: *mut blsgpu_ctx, impl_id: c_int, scheme: c_int, format: c_int, n: usize,
         pks: *const u8, sigs: *const u8, msg_idx: *const u32, q: usize, msgs: *const u8, msg_off: *const u64,
         status_out: *mut u8) -> c_int;
+
+    // ---- key sets: public keys decoded once, verify calls that name them by index ------------------------------------
+    pub fn blsgpu_keyset_create(ctx: *mut blsgpu_ctx, impl_id: c_int, format: c_int, n: usize, pks: *const u8,
+        status_out: *mut u8 /* [n] or null */, keyset_out: *mut u64) -> c_int;
+    pub fn blsgpu_keyset_destroy(ctx: *mut blsgpu_ctx, keyset: u64) -> c_int;
+    pub fn blsgpu_verify_batch_keyed(ctx: *mut blsgpu_ctx, keyset: u64, scheme: c_int, format: c_int, n: usize,
+        key_idx: *const u32, sigs: *const u8, msgs: *const u8, msg_off: *const u64, status_out: *mut u8) -> c_int;
+    pub fn blsgpu_verify_batch_grouped_keyed(ctx: *mut blsgpu_ctx, keyset: u64, scheme: c_int, format: c_int, n: usize,
+        key_idx: *const u32, sigs: *const u8, msg_idx: *const u32, q: usize, msgs: *const u8, msg_off: *const u64,
+        status_out: *mut u8) -> c_int;
+
     pub fn blsgpu_verify_batch_dev(ctx: *mut blsgpu_ctx, impl_id: c_int, scheme: c_int, format: c_int, n: usize,
         pks_dev: *const u8, sigs_dev: *const u8, msgs_dev: *const u8, msg_off_dev: *const u64,
         status_out_dev: *mut u8) -> c_int;

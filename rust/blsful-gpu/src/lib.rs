@@ -6,6 +6,7 @@
 //! | here | n × (or q ×) the blsful call |
 //! |---|---|
 //! | [`Engine::verify_batch`] | `Signature::verify` (src/signature.rs:130-138) |
+//! | [`Engine::verify_batch_keyed`] / [`Engine::verify_batch_grouped_keyed`] | `Signature::verify` against keys decoded once into a [`KeySet`] |
 //! | [`Engine::pop_verify_batch`] | `ProofOfPossession::verify` (src/proof_of_possession.rs:77-81) |
 //! | [`Engine::aggregate_verify`] | `AggregateSignature::verify` (src/aggregate_signature.rs:230-239) |
 //! | [`Engine::aggregate_verify_batch`] | q × `AggregateSignature::verify`, one pipeline per signature scheme present |
@@ -28,6 +29,7 @@
 
 use std::ffi::CStr;
 use std::fmt;
+use std::marker::PhantomData;
 use std::os::raw::c_int;
 use std::ptr;
 
@@ -198,6 +200,26 @@ pub struct Partial {
     pub gt: [u8; 576],
     /// Random-linear-combination sum of the slice's signatures, compressed (signature group).
     pub sig_sum: Vec<u8>,
+}
+
+/// Public keys decoded once into device memory of the [`Engine`] that made them ([`Engine::key_set`]), named by index
+/// in [`Engine::verify_batch_keyed`] and [`Engine::verify_batch_grouped_keyed`].  Only the engine's id of the set is held
+/// here: [`Engine::drop_key_set`] frees the memory, and so does dropping the engine.  Used with another engine, or after
+/// it was freed, the id is an `EngineError` (`BLSGPU_E_ARG`), never undefined behaviour.
+pub struct KeySet<C: GpuImpl> {
+    id: u64,
+    len: usize,
+    _impl: PhantomData<C>,
+}
+
+impl<C: GpuImpl> KeySet<C> {
+    pub fn len(&self) -> usize {
+        self.len
+    }
+
+    pub fn is_empty(&self) -> bool {
+        self.len == 0
+    }
 }
 
 /// RAII owner of a `blsgpu_ctx` (one per thread; a context is not thread-safe, different contexts are independent).
@@ -371,6 +393,139 @@ impl Engine {
         let mut status = vec![0u8; n];
         let rc = unsafe {
             sys::blsgpu_verify_batch_grouped(self.ctx, C::IMPL_ID, scheme_id(scheme), format_id(format), n, pks.as_ptr(), sigs.as_ptr(),
+                msg_idx.as_ptr(), msgs.len(), msgs.bytes.as_ptr(), msgs.offsets.as_ptr(), status.as_mut_ptr())
+        };
+        self.check(rc)?;
+        Ok(status)
+    }
+
+    // ---------------------------------------------------------------------------------------------------------
+    // Key sets: public keys decoded once on the device, verify calls that name them by index
+    // ---------------------------------------------------------------------------------------------------------
+
+    /// Decodes and subgroup-checks `pks` once into device memory this engine owns (first device).  For key sets that
+    /// barely change between calls (a validator set, a masternode list, the signers of a quorum): the keyed calls then
+    /// send a 4-byte index per item instead of the key and skip its decode.
+    pub fn key_set<C: GpuImpl>(&mut self, pks: &[PublicKey<C>]) -> EngineResult<KeySet<C>> {
+        let bytes = pack_points(pks.iter().map(|p| p.0), C::PK_BYTES);
+        Ok(self.key_set_bytes::<C>(SerializationFormat::Modern, &bytes)?.0)
+    }
+
+    /// The byte form of [`Engine::key_set`]: keys serialised in `format`, with one status per key (`BLSGPU_ST_OK`,
+    /// `DESERIALIZE` or `LEGACY_FORMAT`).  A key that fails to decode stays in the set; items that name it get that status.
+    pub fn key_set_bytes<C: GpuImpl>(&mut self, format: SerializationFormat, pks: &[u8]) -> EngineResult<(KeySet<C>, Vec<u8>)> {
+        if pks.len() % C::PK_BYTES != 0 {
+            return Err(EngineError { code: sys::BLSGPU_E_ARG, message: "key_set_bytes: not a whole number of keys".into() });
+        }
+        let n = pks.len() / C::PK_BYTES;
+        let mut status = vec![0u8; n];
+        let mut id = 0u64;
+        let rc = unsafe { sys::blsgpu_keyset_create(self.ctx, C::IMPL_ID, format_id(format), n, pks.as_ptr(), status.as_mut_ptr(), &mut id) };
+        self.check(rc)?;
+        Ok((KeySet { id, len: n, _impl: PhantomData }, status))
+    }
+
+    /// Frees the device memory of a key set now (dropping the engine frees every set it still holds).
+    pub fn drop_key_set<C: GpuImpl>(&mut self, keys: KeySet<C>) -> EngineResult<()> {
+        let rc = unsafe { sys::blsgpu_keyset_destroy(self.ctx, keys.id) };
+        self.check(rc)
+    }
+
+    /// [`Engine::verify_batch`] with `pks[i]` = key `key_idx[i]` of `keys`.  An index at or past the end of the set is an
+    /// `EngineError` (`BLSGPU_E_ARG`), as is a set of another engine.
+    pub fn verify_batch_keyed<C: GpuImpl, B: AsRef<[u8]>>(
+        &mut self,
+        keys: &KeySet<C>,
+        key_idx: &[u32],
+        sigs: &[Signature<C>],
+        msgs: &[B],
+    ) -> EngineResult<Vec<BlsResult<()>>> {
+        let n = sigs.len();
+        if key_idx.len() != n || msgs.len() != n {
+            return Err(EngineError { code: sys::BLSGPU_E_ARG, message: "verify_batch_keyed: slice lengths differ".into() });
+        }
+        if n == 0 {
+            return Ok(Vec::new());
+        }
+        let scheme = signature_scheme(&sigs[0]);
+        let sig_bytes = pack_points(sigs.iter().map(|s| *s.as_raw_value()), C::SIG_BYTES);
+        let packed = PackedMessages::from_iter(msgs.iter());
+        let status = self.verify_batch_keyed_bytes(keys, scheme, SerializationFormat::Modern, key_idx, &sig_bytes, &packed)?;
+        Ok(status
+            .iter()
+            .zip(sigs)
+            .map(|(&st, s)| if signature_scheme(s) != scheme { Err(BlsError::InvalidSignatureScheme) } else { status_to_result(st, None) })
+            .collect())
+    }
+
+    /// The zero-copy form of [`Engine::verify_batch_keyed`]: signatures already serialised in `format`.
+    pub fn verify_batch_keyed_bytes<C: GpuImpl>(
+        &mut self,
+        keys: &KeySet<C>,
+        scheme: SignatureSchemes,
+        format: SerializationFormat,
+        key_idx: &[u32],
+        sigs: &[u8],
+        msgs: &PackedMessages,
+    ) -> EngineResult<Vec<u8>> {
+        let n = msgs.len();
+        if key_idx.len() != n || sigs.len() != n * C::SIG_BYTES {
+            return Err(EngineError { code: sys::BLSGPU_E_ARG, message: "verify_batch_keyed_bytes: buffer sizes do not match n".into() });
+        }
+        let mut status = vec![0u8; n];
+        let rc = unsafe {
+            sys::blsgpu_verify_batch_keyed(self.ctx, keys.id, scheme_id(scheme), format_id(format), n, key_idx.as_ptr(), sigs.as_ptr(),
+                msgs.bytes.as_ptr(), msgs.offsets.as_ptr(), status.as_mut_ptr())
+        };
+        self.check(rc)?;
+        Ok(status)
+    }
+
+    /// [`Engine::verify_batch_grouped`] with `pks[i]` = key `key_idx[i]` of `keys`.
+    pub fn verify_batch_grouped_keyed<C: GpuImpl, B: AsRef<[u8]>>(
+        &mut self,
+        keys: &KeySet<C>,
+        key_idx: &[u32],
+        sigs: &[Signature<C>],
+        msg_idx: &[u32],
+        msgs: &[B],
+    ) -> EngineResult<Vec<BlsResult<()>>> {
+        let n = sigs.len();
+        if key_idx.len() != n || msg_idx.len() != n {
+            return Err(EngineError { code: sys::BLSGPU_E_ARG, message: "verify_batch_grouped_keyed: slice lengths differ".into() });
+        }
+        if n == 0 {
+            return Ok(Vec::new());
+        }
+        let scheme = signature_scheme(&sigs[0]);
+        let sig_bytes = pack_points(sigs.iter().map(|s| *s.as_raw_value()), C::SIG_BYTES);
+        let packed = PackedMessages::from_iter(msgs.iter());
+        let status = self.verify_batch_grouped_keyed_bytes(keys, scheme, SerializationFormat::Modern, key_idx, &sig_bytes, msg_idx, &packed)?;
+        Ok(status
+            .iter()
+            .zip(sigs)
+            .map(|(&st, s)| if signature_scheme(s) != scheme { Err(BlsError::InvalidSignatureScheme) } else { status_to_result(st, None) })
+            .collect())
+    }
+
+    /// The zero-copy form of [`Engine::verify_batch_grouped_keyed`]: signatures already serialised in `format`.
+    pub fn verify_batch_grouped_keyed_bytes<C: GpuImpl>(
+        &mut self,
+        keys: &KeySet<C>,
+        scheme: SignatureSchemes,
+        format: SerializationFormat,
+        key_idx: &[u32],
+        sigs: &[u8],
+        msg_idx: &[u32],
+        msgs: &PackedMessages,
+    ) -> EngineResult<Vec<u8>> {
+        let n = msg_idx.len();
+        if key_idx.len() != n || sigs.len() != n * C::SIG_BYTES {
+            return Err(EngineError { code: sys::BLSGPU_E_ARG, message: "verify_batch_grouped_keyed_bytes: buffer sizes do not match n".into() });
+        }
+        let mut status = vec![0u8; n];
+        let rc = unsafe {
+            sys::blsgpu_verify_batch_grouped_keyed(self.ctx, keys.id, scheme_id(scheme), format_id(format), n, key_idx.as_ptr(), sigs.as_ptr(),
                 msg_idx.as_ptr(), msgs.len(), msgs.bytes.as_ptr(), msgs.offsets.as_ptr(), status.as_mut_ptr())
         };
         self.check(rc)?;

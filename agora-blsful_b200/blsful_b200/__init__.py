@@ -13,6 +13,8 @@ argument meaning and error behaviour:
                                -> sum_signatures / sum_public_keys (src/multi_signature.rs:80-107, multi_public_key.rs:79-83)
   Signature::verify_secure[_with_mode] -> verify_secure_batch   (src/signature.rs:177-197,256-276)
   aggregate_secure[_with_mode] -> aggregate_secure_batch  (src/secure_aggregation.rs:159-169,338-352)
+                               -> verify_secure_batch_keyed / aggregate_secure_batch_keyed (members named by index
+                                  into a KeySet)
 
 There is no CPU fallback: importing works anywhere, but creating an Engine without the CUDA library or a GPU raises.
 """
@@ -126,6 +128,8 @@ def load_library() -> ctypes.CDLL:
         "blsgpu_sum_points": (c.c_int, [vp, c.c_int, c.c_int, c.c_size_t, u8p, u8p, u8p, i64p]),
         "blsgpu_verify_secure_batch": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u64p, u8p, u8p, u8p, u64p, u8p]),
         "blsgpu_aggregate_secure_batch": (c.c_int, [vp, c.c_int, c.c_int, c.c_size_t, u64p, u8p, u8p, u8p, u8p]),
+        "blsgpu_verify_secure_batch_keyed": (c.c_int, [vp, c.c_uint64, c.c_int, c.c_int, c.c_size_t, u64p, vp, u8p, u8p, u64p, u8p]),
+        "blsgpu_aggregate_secure_batch_keyed": (c.c_int, [vp, c.c_uint64, c.c_int, c.c_size_t, u64p, vp, u8p, u8p, u8p]),
         "blsgpu_hash_to_curve_batch": (c.c_int, [vp, c.c_int, c.c_size_t, u8p, u64p, u8p, c.c_size_t, u8p]),
         "blsgpu_recode_points": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u8p, u8p, u8p]),
         "blsgpu_fp_mul_batch": (c.c_int, [vp, c.c_int, c.c_size_t, u8p, u8p, u8p]),
@@ -161,7 +165,8 @@ EXPORTED_SYMBOLS = [
     "blsgpu_keyset_create", "blsgpu_keyset_destroy", "blsgpu_verify_batch_keyed", "blsgpu_verify_batch_grouped_keyed",
     "blsgpu_miller_partial", "blsgpu_final_exp_is_one", "blsgpu_partial_finish",
     "blsgpu_verify_batch_dev", "blsgpu_pop_verify_batch", "blsgpu_aggregate_verify", "blsgpu_aggregate_verify_batch", "blsgpu_sum_points",
-    "blsgpu_verify_secure_batch", "blsgpu_aggregate_secure_batch", "blsgpu_hash_to_curve_batch", "blsgpu_recode_points",
+    "blsgpu_verify_secure_batch", "blsgpu_aggregate_secure_batch",
+    "blsgpu_verify_secure_batch_keyed", "blsgpu_aggregate_secure_batch_keyed", "blsgpu_hash_to_curve_batch", "blsgpu_recode_points",
     "blsgpu_fp_mul_batch", "blsgpu_pairing_product_is_one", "blsgpu_testdata_sign", "blsgpu_imad_peak",
     "blsgpu_combine_shares_batch", "blsgpu_verify_batch_wire", "blsgpu_pairing_check_batch",
     "blsgpu_signcrypt_valid_batch", "blsgpu_signcrypt_verify_share_batch", "blsgpu_pok_verify_batch", "blsgpu_verify_batch_records", "blsgpu_selftest", "blsgpu_plan_msm", "blsgpu_plan_shards", "blsgpu_verify_share_batch", "blsgpu_last_stage_ms", "blsgpu_last_kernel_ms", "blsgpu_launch_count",
@@ -584,6 +589,67 @@ class Engine:
         status = np.empty(q, dtype=np.uint8)
         rc = self._lib.blsgpu_aggregate_secure_batch(self._ctx, impl_id, fmt, q, _ptr(koff), _ptr(pk), _ptr(sg), _ptr(out), _ptr(status))
         self._check(rc, "blsgpu_aggregate_secure_batch")
+        return status, out
+
+    def verify_secure_batch_keyed(self, keys: KeySet, scheme: int, key_idx_sets: Sequence[Sequence[int]], sigs, msgs: Sequence[bytes],
+                                  fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """verify_secure_batch with quorum j's keys = keys of `keys` at key_idx_sets[j], encoded in fmt."""
+        q = len(key_idx_sets)
+        koff = np.zeros(q + 1, dtype=np.uint64)
+        if q:
+            koff[1:] = np.cumsum([len(k) for k in key_idx_sets], dtype=np.uint64)
+        idx = np.array([k for ks in key_idx_sets for k in ks], dtype=np.uint32)
+        sg = _pack_points(sigs, sig_len(keys.impl_id), "signature")
+        if sg.size // sig_len(keys.impl_id) != q or len(msgs) != q:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        data, off = pack_messages(msgs)
+        return self.verify_secure_batch_keyed_packed(keys, scheme, koff, idx, sg, data, off, fmt)
+
+    def verify_secure_batch_keyed_packed(self, keys: KeySet, scheme: int, koff: np.ndarray, key_idx: np.ndarray, sg: np.ndarray,
+                                         data: np.ndarray, off: np.ndarray, fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """Flat-buffer form: koff[q + 1] member offsets, key_idx uint32[koff[q]], sg q signatures, the q messages as data / off."""
+        koff = np.ascontiguousarray(koff, dtype=np.uint64).reshape(-1)
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32).reshape(-1)
+        q = koff.size - 1
+        if key_idx.size != (int(koff[-1]) if q else 0) or off.size - 1 != q:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        status = np.empty(q, dtype=np.uint8)
+        rc = self._lib.blsgpu_verify_secure_batch_keyed(self._ctx, keys.id, scheme, fmt, q, _ptr(koff), _ptr(key_idx), _ptr(sg), _ptr(data),
+                                                        _ptr(off), _ptr(status))
+        self._check(rc, "blsgpu_verify_secure_batch_keyed")
+        return status
+
+    def aggregate_secure_batch_keyed(self, keys: KeySet, key_idx_sets: Sequence[Sequence[int]], sig_sets: Sequence[Sequence[bytes]],
+                                     fmt: int = SerializationFormat.Modern) -> Tuple[np.ndarray, List[bytes]]:
+        """aggregate_secure_batch with quorum j's keys = keys of `keys` at key_idx_sets[j], encoded in fmt."""
+        q = len(key_idx_sets)
+        if len(sig_sets) != q or any(len(k) != len(s) for k, s in zip(key_idx_sets, sig_sets)):
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        koff = np.zeros(q + 1, dtype=np.uint64)
+        if q:
+            koff[1:] = np.cumsum([len(k) for k in key_idx_sets], dtype=np.uint64)
+        idx = np.array([k for ks in key_idx_sets for k in ks], dtype=np.uint32)
+        sg = _pack_points([s for ss in sig_sets for s in ss], sig_len(keys.impl_id), "signature")
+        status, out = self.aggregate_secure_batch_keyed_packed(keys, koff, idx, sg, fmt)
+        L = sig_len(keys.impl_id)
+        return status, [out[j * L:(j + 1) * L].tobytes() for j in range(q)]
+
+    def aggregate_secure_batch_keyed_packed(self, keys: KeySet, koff: np.ndarray, key_idx: np.ndarray, sg: np.ndarray,
+                                            fmt: int = SerializationFormat.Modern) -> Tuple[np.ndarray, np.ndarray]:
+        """Flat-buffer form: koff[q + 1] member offsets, key_idx uint32[koff[q]], sg one signature per member; returns
+        (status[q], q signatures flat)."""
+        koff = np.ascontiguousarray(koff, dtype=np.uint64).reshape(-1)
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32).reshape(-1)
+        sg = _pack_points(sg, sig_len(keys.impl_id), "signature")
+        q = koff.size - 1
+        m = int(koff[-1]) if q else 0
+        if key_idx.size != m or sg.size // sig_len(keys.impl_id) != m:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        out = np.zeros(q * sig_len(keys.impl_id), dtype=np.uint8)
+        status = np.empty(q, dtype=np.uint8)
+        rc = self._lib.blsgpu_aggregate_secure_batch_keyed(self._ctx, keys.id, fmt, q, _ptr(koff), _ptr(key_idx), _ptr(sg), _ptr(out),
+                                                           _ptr(status))
+        self._check(rc, "blsgpu_aggregate_secure_batch_keyed")
         return status, out
 
     def recode_points_packed(self, group: int, pts: np.ndarray, fmt_in: int, fmt_out: int) -> np.ndarray:

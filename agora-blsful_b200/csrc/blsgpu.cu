@@ -117,12 +117,29 @@ struct PendingSlice {
 
 // public keys decoded once (blsgpu_keyset_create): n affine points of the impl's key group and their decode statuses, in a
 // device allocation of their own on the first device (apart from the arena, so that regrowing the arena keeps them)
+// The secure view of a key set in one format (ensure_secure_view, built by the first keyed secure call in that format):
+// every key re-encoded in the format, and its dense rank in memcmp order of those encodings (equal bytes, equal rank).
+struct SecureView {
+  uint8_t* enc = nullptr;            // device, n encodings
+  uint32_t* rank = nullptr;          // device, n ranks
+  std::vector<uint32_t> host_rank;  // the same ranks, for quorums the host plans
+};
 struct KeySet {
   int impl_id = 0;
   size_t n = 0;
   void* pts = nullptr;
   uint8_t* st = nullptr;
+  SecureView view[2];  // by format
 };
+// every device allocation of a key set (cudaFree waits for the work that may still read it); the first error
+static cudaError_t free_keyset(const KeySet& s) {
+  cudaError_t e = cudaSuccess;
+  for (void* p : {s.pts, (void*)s.st, (void*)s.view[0].enc, (void*)s.view[0].rank, (void*)s.view[1].enc, (void*)s.view[1].rank}) {
+    const cudaError_t r = cudaFree(p);
+    if (e == cudaSuccess) e = r;
+  }
+  return e;
+}
 
 struct blsgpu_ctx {
   std::vector<int> devices;
@@ -1167,10 +1184,7 @@ void blsgpu_ctx_destroy(blsgpu_ctx* ctx) {
   for (blsgpu_ctx* peer : ctx->peers) blsgpu_ctx_destroy(peer);
   cudaSetDevice(ctx->devices[0]);
   ctx->pending.reset();
-  for (const auto& ks : ctx->keysets) {
-    cudaFree(ks.second.pts);
-    cudaFree(ks.second.st);
-  }
+  for (const auto& ks : ctx->keysets) free_keyset(ks.second);
   if (ctx->arena.base) cudaFree(ctx->arena.base);
   if (ctx->fold_scratch) cudaFree(ctx->fold_scratch);
   for (int i = 0; i <= BLSGPU_STAGE_COUNT; i++) cudaEventDestroy(ctx->ev[i]);
@@ -2255,7 +2269,7 @@ int verify_grouped_impl(blsgpu_ctx* ctx, int scheme, int format, size_t n, const
 }
 
 // the key set `id` of this context, or nullptr with the error set (an id that was destroyed, never issued, or is another context's)
-const KeySet* find_keyset(blsgpu_ctx* ctx, uint64_t id, const char* what) {
+KeySet* find_keyset(blsgpu_ctx* ctx, uint64_t id, const char* what) {
   const auto it = ctx->keysets.find(id);
   if (it != ctx->keysets.end()) return &it->second;
   ctx->err = std::string(what) + ": key set " + std::to_string(id) + " is not held by this context";
@@ -2376,9 +2390,9 @@ int blsgpu_keyset_destroy(blsgpu_ctx* ctx, uint64_t keyset) {
   if (!s) return BLSGPU_E_ARG;
   ctx->pending.reset();
   CKR(set_device(ctx));
-  const cudaError_t e1 = cudaFree(s->pts), e2 = cudaFree(s->st);  // cudaFree waits for the work that may still read the set
+  const cudaError_t e = free_keyset(*s);
   ctx->keysets.erase(keyset);
-  CK(e1 != cudaSuccess ? e1 : e2);
+  CK(e);
   return BLSGPU_OK;
 }
 
@@ -2744,71 +2758,175 @@ SecurePlan make_secure_plan(size_t q, const uint64_t* key_off, const uint8_t* pk
 
 // device part shared by verify and aggregate: out_sum[j] = sum_i t_i * points[src(i)] ; zero_out[m] flags t_m == 0.
 // One bucket multi-scalar multiplication per key set: a warp per set, a lane per 8-bit window (kernels.cuh k_secure_msm).
+// The plan is on the device: d_ord indexes d_key_bytes, d_src indexes d_points.
 template <class A>
-int secure_weighted_sums(blsgpu_ctx* ctx, const SecurePlan& pl, const uint64_t* key_off, const uint8_t* d_key_bytes, int key_len, const std::vector<uint32_t>& src,
-                         const A* d_points, typename PtInfo<A>::Jac* d_sum, uint8_t* d_zero) {
+int secure_weighted_sums(blsgpu_ctx* ctx, size_t q, size_t M, const uint64_t* d_koff, const uint32_t* d_ord, const uint32_t* d_set,
+                         const uint32_t* d_pos, const uint8_t* d_key_bytes, int key_len, const uint32_t* d_src, const A* d_points,
+                         typename PtInfo<A>::Jac* d_sum, uint8_t* d_zero) {
   typedef typename PtInfo<A>::Jac J;
-  uint32_t *d_ord, *d_set, *d_pos, *d_src;
-  uint64_t* d_koff;
-  CKR(upload(ctx, d_koff, key_off, pl.q + 1));
-  CKR(upload(ctx, d_ord, pl.ord.data(), pl.M));
-  CKR(upload(ctx, d_set, pl.set_of.data(), pl.M));
-  CKR(upload(ctx, d_pos, pl.pos.data(), pl.M));
-  CKR(upload(ctx, d_src, src.data(), pl.M));
-  Digest* d_base = ctx->arena.take<Digest>(pl.q);
-  int8_t* d_digits = ctx->arena.take<int8_t>(std::max<size_t>(pl.M, 1) * SECURE_WINDOWS);
-  const size_t nblocks = secure_msm_blocks(ctx, pl.q);
+  Digest* d_base = ctx->arena.take<Digest>(q);
+  int8_t* d_digits = ctx->arena.take<int8_t>(std::max<size_t>(M, 1) * SECURE_WINDOWS);
+  const size_t nblocks = secure_msm_blocks(ctx, q);
   J* d_buckets = ctx->arena.take<J>(nblocks * 128 * SECURE_BUCKETS);
-  J* d_W = ctx->arena.take<J>(pl.q * SECURE_WINDOWS);
-  LAUNCH(k_secure_base, blocks_for(pl.q), TPB, pl.q, (const uint64_t*)d_koff, (const uint32_t*)d_ord, d_key_bytes, key_len, d_base);
-  if (pl.M)
-    LAUNCH(k_secure_digits, blocks_for(pl.M), TPB, pl.M, (const uint32_t*)d_set, (const uint32_t*)d_pos, (const Digest*)d_base, d_digits, d_zero);
-  LAUNCH((k_secure_msm<A>), (unsigned)nblocks, 128, pl.q, (const uint64_t*)d_koff, (const uint32_t*)d_src, (const int8_t*)d_digits, d_points,
-         d_buckets, d_W);
-  LAUNCH((k_secure_combine<J>), blocks_for(pl.q), TPB, pl.q, (const J*)d_W, d_sum);
+  J* d_W = ctx->arena.take<J>(q * SECURE_WINDOWS);
+  LAUNCH(k_secure_base, blocks_for(q), TPB, q, d_koff, d_ord, d_key_bytes, key_len, d_base);
+  if (M) LAUNCH(k_secure_digits, blocks_for(M), TPB, M, d_set, d_pos, (const Digest*)d_base, d_digits, d_zero);
+  LAUNCH((k_secure_msm<A>), (unsigned)nblocks, 128, q, d_koff, d_src, (const int8_t*)d_digits, d_points, d_buckets, d_W);
+  LAUNCH((k_secure_combine<J>), blocks_for(q), TPB, q, (const J*)d_W, d_sum);
   return BLSGPU_OK;
 }
 
-size_t secure_plan_bytes(const blsgpu_ctx* ctx, const SecurePlan& pl, size_t jac_size) {
-  return (pl.q + 1) * 8 + pl.M * (16 + SECURE_WINDOWS) + pl.q * 32 + secure_msm_blocks(ctx, pl.q) * 128 * SECURE_BUCKETS * jac_size +
-         (pl.q * SECURE_WINDOWS + 2) * jac_size + 24 * 256;
+size_t secure_plan_bytes(const blsgpu_ctx* ctx, size_t q, size_t M, size_t jac_size) {
+  return (q + 1) * 8 + M * (16 + SECURE_WINDOWS) + q * 32 + secure_msm_blocks(ctx, q) * 128 * SECURE_BUCKETS * jac_size +
+         (q * SECURE_WINDOWS + 2) * jac_size + 24 * 256;
+}
+
+// Quorums of at most this many members are planned by k_secure_plan_keyed in shared memory (8 bytes per member, so 32 KB:
+// within the default limit of dynamic shared memory, 10x Dash's largest quorum of 400); larger ones by make_secure_plan on
+// the host, over 4-byte big-endian ranks.
+constexpr uint32_t SECURE_PLAN_CAP = 4096;
+
+// A secure call's keys on the device, as the key step (secure_keys) leaves them: the plan (koff, and per sorted member
+// ord = the index of its key in key_bytes and pts, set, pos, and first = the member index of the first equal key), the
+// keys' encodings in the call's format and their decoded points, and the key statuses: per member (st_per_member) or
+// already reduced to each quorum's first bad key.
+template <class PkA>
+struct SecureKeys {
+  const uint64_t* koff = nullptr;
+  const uint32_t *ord = nullptr, *set = nullptr, *pos = nullptr, *first = nullptr;
+  const uint8_t* key_bytes = nullptr;
+  const PkA* pts = nullptr;
+  const uint8_t* st = nullptr;
+  bool st_per_member = false;
+  std::vector<SecurePlan> host_plans;  // host-side plans whose uploads may still be in flight
+};
+
+// The key step of a secure call, the one step where keyed and unkeyed calls differ.  Unkeyed: upload the members' key
+// bytes, decode them, plan on the host by those bytes (make_secure_plan) and upload the plan.  Keyed: upload key_idx, plan
+// on the device by the set's secure view in `format` (k_secure_plan_keyed; make_secure_plan over the ranks for quorums
+// above SECURE_PLAN_CAP), and take the keys' encodings and points from the view and the set.  with_first: the plan's
+// `first` is needed (aggregate).
+template <class PkA>
+int secure_keys(blsgpu_ctx* ctx, int format, size_t q, const uint64_t* key_off, const Keys& keys, bool with_first, SecureKeys<PkA>& K) {
+  const size_t M = (size_t)key_off[q], Lp = PtInfo<PkA>::LEN;
+  uint64_t* d_koff;
+  if (!keys.set) {
+    K.host_plans.push_back(make_secure_plan(q, key_off, keys.bytes, Lp));
+    const SecurePlan& pl = K.host_plans.back();
+    uint8_t* d_pkb;
+    CKR(upload(ctx, d_pkb, keys.bytes, M * Lp));
+    PkA* d_pk = ctx->arena.take<PkA>(std::max<size_t>(M, 1));
+    uint8_t* d_stpk = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
+    if (M) CKR((decode_points<PkA>(ctx, M, (const uint8_t*)d_pkb, format, d_pk, d_stpk)));
+    uint32_t *d_ord, *d_set, *d_pos, *d_first = nullptr;
+    CKR(upload(ctx, d_koff, key_off, q + 1));
+    CKR(upload(ctx, d_ord, pl.ord.data(), M));
+    CKR(upload(ctx, d_set, pl.set_of.data(), M));
+    CKR(upload(ctx, d_pos, pl.pos.data(), M));
+    if (with_first) CKR(upload(ctx, d_first, pl.first.data(), M));
+    K.koff = d_koff;
+    K.ord = d_ord;
+    K.set = d_set;
+    K.pos = d_pos;
+    K.first = d_first;
+    K.key_bytes = d_pkb;
+    K.pts = d_pk;
+    K.st = d_stpk;
+    K.st_per_member = true;
+    return BLSGPU_OK;
+  }
+  const SecureView& v = keys.set->view[format];
+  uint32_t* d_kidx;
+  CKR(upload(ctx, d_koff, key_off, q + 1));
+  CKR(upload(ctx, d_kidx, keys.idx, M));
+  uint32_t* d_ord = ctx->arena.take<uint32_t>(std::max<size_t>(M, 1));
+  uint32_t* d_set = ctx->arena.take<uint32_t>(std::max<size_t>(M, 1));
+  uint32_t* d_pos = ctx->arena.take<uint32_t>(std::max<size_t>(M, 1));
+  uint32_t* d_first = ctx->arena.take<uint32_t>(std::max<size_t>(M, 1));
+  uint8_t* d_keyst = ctx->arena.take<uint8_t>(q);
+  uint32_t slots = 1;
+  for (size_t j = 0; j < q; j++) {
+    const uint64_t cnt = key_off[j + 1] - key_off[j];
+    while (cnt <= SECURE_PLAN_CAP && slots < cnt) slots <<= 1;
+  }
+  ARENA_OK();
+  k_secure_plan_keyed<<<(unsigned)q, 256, slots * sizeof(unsigned long long), ctx->stream>>>(q, d_koff, d_kidx, v.rank, keys.set->st, slots, d_ord,
+                                                                                             d_set, d_pos, d_first, d_keyst);
+  CKR(check_launch(ctx, "k_secure_plan_keyed"));
+  for (size_t j = 0; j < q; j++) {
+    const size_t lo = (size_t)key_off[j], cnt = (size_t)(key_off[j + 1] - lo);
+    if (cnt <= SECURE_PLAN_CAP) continue;
+    std::vector<uint8_t> be(cnt * 4);
+    for (size_t p = 0; p < cnt; p++) {
+      const uint32_t r = v.host_rank[keys.idx[lo + p]];
+      for (int b = 0; b < 4; b++) be[p * 4 + b] = (uint8_t)(r >> (24 - 8 * b));
+    }
+    const uint64_t one[2] = {0, cnt};
+    K.host_plans.push_back(make_secure_plan(1, one, be.data(), 4));
+    SecurePlan& pl = K.host_plans.back();
+    for (size_t i = 0; i < cnt; i++) {  // to the call's indices: set indices in ord, member indices in first
+      pl.ord[i] = keys.idx[lo + pl.ord[i]];
+      pl.set_of[i] = (uint32_t)j;
+      pl.first[i] += (uint32_t)lo;
+    }
+    CK(cudaMemcpyAsync(d_ord + lo, pl.ord.data(), cnt * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_set + lo, pl.set_of.data(), cnt * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_pos + lo, pl.pos.data(), cnt * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_first + lo, pl.first.data(), cnt * 4, cudaMemcpyHostToDevice, ctx->stream));
+  }
+  K.koff = d_koff;
+  K.ord = d_ord;
+  K.set = d_set;
+  K.pos = d_pos;
+  K.first = d_first;
+  K.key_bytes = v.enc;
+  K.pts = (const PkA*)keys.set->pts;
+  K.st = d_keyst;
+  K.st_per_member = false;
+  return BLSGPU_OK;
+}
+// quorum j's key status (its first bad key in member order) from the statuses secure_keys left, downloaded to `st`
+template <class PkA>
+uint8_t secure_key_status(const SecureKeys<PkA>& K, const std::vector<uint8_t>& st, const uint64_t* key_off, size_t j) {
+  if (!K.st_per_member) return st[j];
+  uint8_t s = BLSGPU_ST_OK;
+  for (size_t i = (size_t)key_off[j]; i < (size_t)key_off[j + 1] && s == BLSGPU_ST_OK; i++) s = st[i];
+  return s;
 }
 
 template <int IMPL>
-int verify_secure_impl(blsgpu_ctx* ctx, int scheme, int format, size_t q, const uint64_t* key_off, const uint8_t* pks, const uint8_t* sigs,
+int verify_secure_impl(blsgpu_ctx* ctx, int scheme, int format, size_t q, const uint64_t* key_off, const Keys& keys, const uint8_t* sigs,
                        const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
   typedef typename ImplT<IMPL>::PkAff PkA;
   typedef typename ImplT<IMPL>::SigAff SigA;
   typedef typename ImplT<IMPL>::PkJac PkJ;
   const size_t Lp = PtInfo<PkA>::LEN, Ls = PtInfo<SigA>::LEN;
-  SecurePlan pl = make_secure_plan(q, key_off, pks, Lp);
-  const size_t M = pl.M, msg_bytes = (size_t)msg_off[q];
+  const size_t M = (size_t)key_off[q], msg_bytes = (size_t)msg_off[q];
   size_t head = M * (Lp + sizeof(PkA) + 2) + q * (Ls + 2 * sizeof(SigA) + sizeof(PkA) + sizeof(PkJ) + 8) + msg_bytes + (q + 1) * 8 +
-                secure_plan_bytes(ctx, pl, sizeof(PkJ)) + 32 * 256;
+                secure_plan_bytes(ctx, q, M, sizeof(PkJ)) + 32 * 256;
   CKR(ensure_verify_arena<IMPL>(ctx, q, head));
   stage_reset(ctx);
-  uint8_t *d_pkb, *d_sigb, *d_msgs;
+  SecureKeys<PkA> K;
+  CKR((secure_keys<PkA>(ctx, format, q, key_off, keys, false, K)));
+  uint8_t *d_sigb, *d_msgs;
   uint64_t* d_moff;
-  CKR(upload(ctx, d_pkb, pks, M * Lp));
   CKR(upload(ctx, d_sigb, sigs, q * Ls));
   CKR(upload(ctx, d_msgs, msgs, msg_bytes));
   CKR(upload(ctx, d_moff, msg_off, q + 1));
-  PkA* d_pk = ctx->arena.take<PkA>(std::max<size_t>(M, 1));
   SigA* d_sig = ctx->arena.take<SigA>(q);
-  uint8_t* d_stpk = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
   uint8_t* d_stsig = ctx->arena.take<uint8_t>(q);
   uint8_t* d_zero = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
   PkJ* d_sum = ctx->arena.take<PkJ>(q);
   PkA* d_agg = ctx->arena.take<PkA>(q);
   uint8_t* d_setst = ctx->arena.take<uint8_t>(q);
   uint8_t* d_status = ctx->arena.take<uint8_t>(q);
-  if (M) CKR((decode_points<PkA>(ctx, M, (const uint8_t*)d_pkb, format, d_pk, d_stpk)));
   CKR((decode_points<SigA>(ctx, q, (const uint8_t*)d_sigb, format, d_sig, d_stsig)));
-  CKR((secure_weighted_sums<PkA>(ctx, pl, key_off, d_pkb, (int)Lp, pl.ord, d_pk, d_sum, d_zero)));
+  CKR((secure_weighted_sums<PkA>(ctx, q, M, K.koff, K.ord, K.set, K.pos, K.key_bytes, (int)Lp, K.ord, K.pts, d_sum, d_zero)));
   LAUNCH((k_to_affine<PkA>), blocks_for(q), TPB, q, (const PkJ*)d_sum, d_agg);
-  std::vector<uint8_t> stpk(M), stsig(q), zero(M);
+  const size_t nst = K.st_per_member ? M : q;
+  std::vector<uint8_t> stpk(nst), stsig(q), zero(M);
   std::vector<uint32_t> siginf(q);
-  if (M) CK(cudaMemcpyAsync(stpk.data(), d_stpk, M, cudaMemcpyDeviceToHost, ctx->stream));
+  if (nst) CK(cudaMemcpyAsync(stpk.data(), K.st, nst, cudaMemcpyDeviceToHost, ctx->stream));
   if (M) CK(cudaMemcpyAsync(zero.data(), d_zero, M, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaMemcpyAsync(stsig.data(), d_stsig, q, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaMemcpy2DAsync(siginf.data(), 4, reinterpret_cast<const uint8_t*>(d_sig) + offsetof(SigA, inf), sizeof(SigA), 4, q,
@@ -2819,8 +2937,7 @@ int verify_secure_impl(blsgpu_ctx* ctx, int scheme, int format, size_t q, const 
   std::vector<uint8_t> pre(q, BLSGPU_ST_OK);
   for (size_t j = 0; j < q; j++) {
     size_t lo = (size_t)key_off[j], hi = (size_t)key_off[j + 1];
-    uint8_t s = BLSGPU_ST_OK;
-    for (size_t i = lo; i < hi && s == BLSGPU_ST_OK; i++) s = stpk[i];
+    uint8_t s = secure_key_status(K, stpk, key_off, j);
     if (s == BLSGPU_ST_OK) s = stsig[j];
     if (s == BLSGPU_ST_OK && lo == hi) s = siginf[j] ? 0xff : BLSGPU_ST_INVALID_SIGNATURE;  // 0xff: "OK, nothing to check"
     if (s == BLSGPU_ST_OK)
@@ -2843,39 +2960,35 @@ int verify_secure_impl(blsgpu_ctx* ctx, int scheme, int format, size_t q, const 
 }
 
 template <int IMPL>
-int aggregate_secure_impl(blsgpu_ctx* ctx, int format, size_t q, const uint64_t* key_off, const uint8_t* pks, const uint8_t* member_sigs,
+int aggregate_secure_impl(blsgpu_ctx* ctx, int format, size_t q, const uint64_t* key_off, const Keys& keys, const uint8_t* member_sigs,
                           uint8_t* out_sigs, uint8_t* status_out) {
   typedef typename ImplT<IMPL>::PkAff PkA;
   typedef typename ImplT<IMPL>::SigAff SigA;
   typedef typename ImplT<IMPL>::SigJac SigJ;
   const size_t Lp = PtInfo<PkA>::LEN, Ls = PtInfo<SigA>::LEN;
-  SecurePlan pl = make_secure_plan(q, key_off, pks, Lp);
-  const size_t M = pl.M;
+  const size_t M = (size_t)key_off[q];
   size_t need = M * (Lp + Ls + sizeof(PkA) + sizeof(SigA) + 3) + q * (Ls + sizeof(SigA) + sizeof(SigJ) + 8) +
-                secure_plan_bytes(ctx, pl, sizeof(SigJ)) + 32 * 256;
+                secure_plan_bytes(ctx, q, M, sizeof(SigJ)) + 32 * 256;
   CKR(ensure_arena(ctx, need));
-  uint8_t *d_pkb, *d_sigb;
-  CKR(upload(ctx, d_pkb, pks, M * Lp));
+  SecureKeys<PkA> K;
+  CKR((secure_keys<PkA>(ctx, format, q, key_off, keys, true, K)));
+  uint8_t* d_sigb;
   CKR(upload(ctx, d_sigb, member_sigs, M * Ls));
-  PkA* d_pk = ctx->arena.take<PkA>(std::max<size_t>(M, 1));
   SigA* d_sig = ctx->arena.take<SigA>(std::max<size_t>(M, 1));
-  uint8_t* d_stpk = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
   uint8_t* d_stsig = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
   uint8_t* d_zero = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
   SigJ* d_sum = ctx->arena.take<SigJ>(q);
   SigA* d_agg = ctx->arena.take<SigA>(q);
   uint8_t* d_out = ctx->arena.take<uint8_t>(q * Ls);
-  if (M) {
-    CKR((decode_points<PkA>(ctx, M, (const uint8_t*)d_pkb, format, d_pk, d_stpk)));
-    CKR((decode_points<SigA>(ctx, M, (const uint8_t*)d_sigb, format, d_sig, d_stsig)));
-  }
+  if (M) CKR((decode_points<SigA>(ctx, M, (const uint8_t*)d_sigb, format, d_sig, d_stsig)));
   // sum_i t_i * sig[first original index whose key bytes equal sorted key i]   (secure_aggregation.rs:138-153)
-  CKR((secure_weighted_sums<SigA>(ctx, pl, key_off, d_pkb, (int)Lp, pl.first, d_sig, d_sum, d_zero)));
+  CKR((secure_weighted_sums<SigA>(ctx, q, M, K.koff, K.ord, K.set, K.pos, K.key_bytes, (int)Lp, K.first, d_sig, d_sum, d_zero)));
   LAUNCH((k_to_affine<SigA>), blocks_for(q), TPB, q, (const SigJ*)d_sum, d_agg);
   LAUNCH((k_encode<SigA>), blocks_for(q), TPB, q, (const SigA*)d_agg, format, d_out);
-  std::vector<uint8_t> stpk(M), stsig(M), zero(M);
+  const size_t nst = K.st_per_member ? M : q;
+  std::vector<uint8_t> stpk(nst), stsig(M), zero(M);
+  if (nst) CK(cudaMemcpyAsync(stpk.data(), K.st, nst, cudaMemcpyDeviceToHost, ctx->stream));
   if (M) {
-    CK(cudaMemcpyAsync(stpk.data(), d_stpk, M, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(stsig.data(), d_stsig, M, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(zero.data(), d_zero, M, cudaMemcpyDeviceToHost, ctx->stream));
   }
@@ -2883,8 +2996,7 @@ int aggregate_secure_impl(blsgpu_ctx* ctx, int format, size_t q, const uint64_t*
   CK(cudaStreamSynchronize(ctx->stream));
   for (size_t j = 0; j < q; j++) {
     size_t lo = (size_t)key_off[j], hi = (size_t)key_off[j + 1];
-    uint8_t s = BLSGPU_ST_OK;
-    for (size_t i = lo; i < hi && s == BLSGPU_ST_OK; i++) s = stpk[i];
+    uint8_t s = secure_key_status(K, stpk, key_off, j);
     for (size_t i = lo; i < hi && s == BLSGPU_ST_OK; i++) s = stsig[i];
     if (s == BLSGPU_ST_OK)
       for (size_t i = lo; i < hi; i++)
@@ -2892,6 +3004,77 @@ int aggregate_secure_impl(blsgpu_ctx* ctx, int format, size_t q, const uint64_t*
     status_out[j] = s;
     if (s != BLSGPU_ST_OK) memset(out_sigs + j * Ls, 0, Ls);
   }
+  return BLSGPU_OK;
+}
+
+// The secure view of key set s in `format` (SecureView), built once: k_encode of every key, the encodings downloaded and
+// ranked on the host, the ranks uploaded.  Device allocations of its own, like the set; freed with the set.
+template <class PkA>
+int ensure_secure_view(blsgpu_ctx* ctx, KeySet& s, int format) {
+  SecureView& v = s.view[format];
+  if (v.enc) return BLSGPU_OK;
+  const size_t n = s.n, L = PtInfo<PkA>::LEN;
+  SecureView nv;
+  nv.host_rank.resize(n);
+  const int r = [&]() -> int {
+    CK(cudaMalloc(&nv.enc, std::max<size_t>(n, 1) * L));
+    CK(cudaMalloc(&nv.rank, std::max<size_t>(n, 1) * 4));
+    if (n) {
+      std::vector<uint8_t> enc(n * L);
+      LAUNCH((k_encode<PkA>), blocks_for(n), TPB, n, (const PkA*)s.pts, format, nv.enc);
+      CK(cudaMemcpyAsync(enc.data(), nv.enc, n * L, cudaMemcpyDeviceToHost, ctx->stream));
+      CK(cudaStreamSynchronize(ctx->stream));
+      // sort by the first 8 bytes, then by all of them: memcmp order
+      std::vector<std::pair<uint64_t, uint32_t>> o(n);
+      for (size_t i = 0; i < n; i++) {
+        uint64_t pre = 0;
+        for (int b = 0; b < 8; b++) pre = (pre << 8) | enc[i * L + b];
+        o[i] = {pre, (uint32_t)i};
+      }
+      std::sort(o.begin(), o.end(), [&](const std::pair<uint64_t, uint32_t>& a, const std::pair<uint64_t, uint32_t>& b) {
+        if (a.first != b.first) return a.first < b.first;
+        return memcmp(&enc[(size_t)a.second * L], &enc[(size_t)b.second * L], L) < 0;
+      });
+      uint32_t rk = 0;
+      for (size_t i = 0; i < n; i++) {
+        if (i && (o[i].first != o[i - 1].first || memcmp(&enc[(size_t)o[i].second * L], &enc[(size_t)o[i - 1].second * L], L) != 0)) rk++;
+        nv.host_rank[o[i].second] = rk;
+      }
+      CK(cudaMemcpyAsync(nv.rank, nv.host_rank.data(), n * 4, cudaMemcpyHostToDevice, ctx->stream));
+      CK(cudaStreamSynchronize(ctx->stream));
+    }
+    return BLSGPU_OK;
+  }();
+  if (r != BLSGPU_OK) {  // no view is kept
+    cudaFree(nv.enc);
+    cudaFree(nv.rank);
+    (void)cudaGetLastError();
+    return r;
+  }
+  v = std::move(nv);
+  return BLSGPU_OK;
+}
+
+// the argument checks of both keyed secure calls (those of the unkeyed calls, on the set's impl, plus the set id and every
+// key index), then the set's secure view in `format`.  *ko: key_off rebased to 0, *idx: key_idx from the first member.
+int secure_keyed_args(blsgpu_ctx* ctx, const char* what, uint64_t keyset, int scheme, int format, size_t q, const uint64_t* key_off,
+                      const uint32_t* key_idx, bool args_present, KeySet** set_out, std::vector<uint64_t>* ko, const uint32_t** idx) {
+  KeySet* set = find_keyset(ctx, keyset, what);
+  if (!set) return BLSGPU_E_ARG;
+  if (!args_ok(set->impl_id, scheme, format) || (q && (!key_off || !args_present)) || (q && key_off[q] > key_off[0] && !key_idx) ||
+      (set->impl_id == 1 && format == 0)) {
+    ctx->err = std::string(what) + ": bad arguments (Legacy mode exists only for Bls12381G2Impl)";
+    return BLSGPU_E_ARG;
+  }
+  if (q == 0) return BLSGPU_OK;
+  if (!key_offsets_ok(key_off, q)) {
+    ctx->err = std::string(what) + ": key_off must be non-decreasing and below 2^32";
+    return BLSGPU_E_ARG;
+  }
+  *ko = rebased(key_off, 0, q);
+  *idx = key_idx ? key_idx + key_off[0] : nullptr;
+  if (!key_idx_ok(ctx, what, Keys(set, *idx), (size_t)(*ko)[q])) return BLSGPU_E_ARG;
+  *set_out = set;
   return BLSGPU_OK;
 }
 
@@ -2952,6 +3135,45 @@ int blsgpu_aggregate_secure_batch(blsgpu_ctx* ctx, int impl_id, int format, size
   return run_cut(ctx, q, key_off, [&](blsgpu_ctx* c, size_t lo, size_t hi) {
     const std::vector<uint64_t> ko = rebased(key_off, lo, hi);
     return one(c, hi - lo, ko.data(), pks + key_off[lo] * pk_len, member_sigs + key_off[lo] * sig_len, out_sigs + lo * sig_len, status_out + lo);
+  });
+}
+
+int blsgpu_verify_secure_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t q, const uint64_t* key_off,
+                                     const uint32_t* key_idx, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off,
+                                     uint8_t* status_out) {
+  NVTX_RANGE("blsgpu_verify_secure_batch_keyed");
+  if (!ctx) return BLSGPU_E_ARG;
+  const char* what = "blsgpu_verify_secure_batch_keyed";
+  KeySet* set = nullptr;
+  std::vector<uint64_t> ko;
+  const uint32_t* idx = nullptr;
+  CKR(secure_keyed_args(ctx, what, keyset, scheme, format, q, key_off, key_idx, sigs && msg_off && status_out, &set, &ko, &idx));
+  if (q == 0) return BLSGPU_OK;
+  CHECK_OFFSETS(msg_off, q, what);
+  CKR(set_device(ctx));
+  return with_impl(set->impl_id, [&](auto I) {
+    CKR((ensure_secure_view<typename ImplT<I>::PkAff>(ctx, *set, format)));
+    return verify_secure_impl<I>(ctx, scheme, format, q, ko.data(), Keys(set, idx), sigs, msgs, msg_off, status_out);
+  });
+}
+
+int blsgpu_aggregate_secure_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int format, size_t q, const uint64_t* key_off,
+                                        const uint32_t* key_idx, const uint8_t* member_sigs, uint8_t* out_sigs, uint8_t* status_out) {
+  NVTX_RANGE("blsgpu_aggregate_secure_batch_keyed");
+  if (!ctx) return BLSGPU_E_ARG;
+  const char* what = "blsgpu_aggregate_secure_batch_keyed";
+  KeySet* set = nullptr;
+  std::vector<uint64_t> ko;
+  const uint32_t* idx = nullptr;
+  CKR(secure_keyed_args(ctx, what, keyset, 0, format, q, key_off, key_idx, out_sigs && status_out && (!key_off || key_off[q] == key_off[0] || member_sigs),
+                        &set, &ko, &idx));
+  if (q == 0) return BLSGPU_OK;
+  CKR(set_device(ctx));
+  return with_impl(set->impl_id, [&](auto I) {
+    CKR((ensure_secure_view<typename ImplT<I>::PkAff>(ctx, *set, format)));
+    const size_t Ls = PtInfo<typename ImplT<I>::SigAff>::LEN;
+    return aggregate_secure_impl<I>(ctx, format, q, ko.data(), Keys(set, idx), member_sigs ? member_sigs + key_off[0] * Ls : nullptr, out_sigs,
+                                    status_out);
   });
 }
 

@@ -1097,6 +1097,67 @@ __global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_secure_combine(size_t q
   }
   out[set] = acc;
 }
+// keyed secure aggregation: the plan make_secure_plan (blsgpu.cu) builds on the host, built per quorum on the device from
+// the dense byte-order ranks of a key set's secure view.  One block per quorum j with members key_idx[lo..hi):
+//   keyst[j]  the set status of its first bad key in member order (ST_OK if none), for every quorum;
+//   and for quorums of at most `slots` members (the host plans the others): (rank, member position) sorted in shared
+//   memory, ties by position = the reference's stable sort on the byte strings.  Sorted member i (lo <= i < hi) gets
+//   ord[i] = its key's SET index, set_of[i] = j, pos[i] = i - lo, first[i] = the member index of the first member of its
+//   equal-rank run (the first match of duplicate keys, secure_aggregation.rs:140-147).
+// slots: a power of two, the dynamic shared memory is slots 64-bit words.
+__global__ void __launch_bounds__(256) k_secure_plan_keyed(size_t q, const uint64_t* __restrict__ key_off, const uint32_t* __restrict__ key_idx,
+                                                           const uint32_t* __restrict__ rank, const uint8_t* __restrict__ set_st, uint32_t slots,
+                                                           uint32_t* __restrict__ ord, uint32_t* __restrict__ set_of, uint32_t* __restrict__ pos,
+                                                           uint32_t* __restrict__ first, uint8_t* __restrict__ keyst) {
+  extern __shared__ unsigned long long srt[];
+  __shared__ uint32_t bad;
+  const size_t j = blockIdx.x;
+  if (j >= q) return;
+  const uint64_t lo = key_off[j];
+  const uint32_t cnt = (uint32_t)(key_off[j + 1] - lo);
+  if (threadIdx.x == 0) bad = 0xffffffffu;
+  __syncthreads();
+  for (uint32_t p = threadIdx.x; p < cnt; p += blockDim.x)
+    if (set_st[key_idx[lo + p]] != ST_OK) atomicMin(&bad, p);
+  __syncthreads();
+  if (threadIdx.x == 0) keyst[j] = bad == 0xffffffffu ? (uint8_t)ST_OK : set_st[key_idx[lo + bad]];
+  if (cnt > slots) return;
+  uint32_t N = 1;
+  while (N < cnt) N <<= 1;
+  for (uint32_t t = threadIdx.x; t < N; t += blockDim.x)  // ranks are below 2^32 - 16: the padding sorts last
+    srt[t] = t < cnt ? ((unsigned long long)rank[key_idx[lo + t]] << 32) | t : ~0ull;
+  __syncthreads();
+  for (uint32_t k = 2; k <= N; k <<= 1)  // bitonic sort, ascending
+    for (uint32_t h = k >> 1; h > 0; h >>= 1) {
+      for (uint32_t t = threadIdx.x; t < N; t += blockDim.x) {
+        const uint32_t u = t ^ h;
+        if (u > t) {
+          const unsigned long long a = srt[t], b = srt[u];
+          if ((a > b) == ((t & k) == 0)) {
+            srt[t] = b;
+            srt[u] = a;
+          }
+        }
+      }
+      __syncthreads();
+    }
+  for (uint32_t t = threadIdx.x; t < cnt; t += blockDim.x) {
+    const unsigned long long v = srt[t];
+    const uint32_t r = (uint32_t)(v >> 32);
+    uint32_t a = 0, b = t;  // the start of t's equal-rank run: the lowest member position of that rank
+    while (a < b) {
+      const uint32_t m = (a + b) >> 1;
+      if ((uint32_t)(srt[m] >> 32) < r)
+        a = m + 1;
+      else
+        b = m;
+    }
+    ord[lo + t] = key_idx[lo + (uint32_t)v];
+    set_of[lo + t] = (uint32_t)j;
+    pos[lo + t] = t;
+    first[lo + t] = (uint32_t)lo + (uint32_t)srt[a];
+  }
+}
 
 // ---- threshold-share combination (vsss-rs `combine` behind Signature::from_shares / PublicKey::from_shares) ------------
 // identifiers: 32 big-endian bytes -> raw words; flag 1: >= r (DeserializationError), 2: zero (VsssError)

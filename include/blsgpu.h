@@ -66,7 +66,8 @@ typedef struct blsgpu_ctx blsgpu_ctx;
  * count); blsgpu_aggregate_verify cuts its pairs over the devices (from 4096 per device) and folds the partial products of
  * Miller values on the first device; blsgpu_aggregate_verify_batch cuts its aggregates into contiguous runs balanced by pair
  * count (from 4096 pairs per device), each verified on its own device without a fold.  Every other entry point (among them
- * blsgpu_verify_batch_grouped, the key sets and the keyed verify calls), the *_dev variants and blsgpu_ctx_set_stream use the first device.  One process per
+ * blsgpu_verify_batch_grouped, the key sets, the keyed verify calls and the keyed secure calls), the *_dev variants and
+ * blsgpu_ctx_set_stream use the first device.  One process per
  * device with blsgpu_miller_partial / blsgpu_final_exp_is_one does the same across processes. */
 int blsgpu_ctx_create(const int* devices, int ndev, blsgpu_ctx** out);
 void blsgpu_ctx_destroy(blsgpu_ctx* ctx);
@@ -204,6 +205,25 @@ int blsgpu_verify_secure_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int for
  * signature of the FIRST equal key, as the reference's `position` lookup does (:140-147). */
 int blsgpu_aggregate_secure_batch(blsgpu_ctx* ctx, int impl_id, int format, size_t q, const uint64_t* key_off,
                                   const uint8_t* pks, const uint8_t* member_sigs, uint8_t* out_sigs, uint8_t* status_out);
+
+/* Keyed secure aggregation: quorum j's members are key_idx[key_off[j] .. key_off[j+1]), each an index into a key set
+ * (blsgpu_keyset_create); impl_id is the set's.  Each call is the unkeyed call above with pks[i] = key key_idx[i] of the
+ * set encoded in the call's `format`, as the reference's *_with_mode on already-parsed keys: when `format` is the set's,
+ * those are the bytes the set was created from, and every status and output byte equals the unkeyed call's on them.  A set
+ * may be used in either format.  A key that failed to decode at creation gives its quorum the status it was created with
+ * (the first bad key in member order decides).  The argument rules are the unkeyed calls'; an id this context does not hold
+ * and a key_idx entry at or above the set's size are BLSGPU_E_ARG.  No key is decoded, and no member's key bytes cross the
+ * bus: the call uploads key_off and key_idx (4 bytes per member) and sorts the quorums on the device.
+ * Secure view: the first keyed secure call in a format builds, once per set and format, every key's encoding in that format
+ * and its rank in byte order: 52 bytes per key of impl_id 2 and 100 of impl_id 1 on the device, 4 per key on the host.  The
+ * build encodes on the device and sorts on the host (once, O(n log n) for n keys); the view lives until the set is
+ * destroyed.  First device only. */
+int blsgpu_verify_secure_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t q,
+                                     const uint64_t* key_off, const uint32_t* key_idx, const uint8_t* sigs,
+                                     const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out);
+int blsgpu_aggregate_secure_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int format, size_t q, const uint64_t* key_off,
+                                        const uint32_t* key_idx, const uint8_t* member_sigs, uint8_t* out_sigs,
+                                        uint8_t* status_out);
 
 /* ---- building blocks (parity tests, metrics) ------------------------------------------------------------------ */
 /* hash_to_point (reference src/traits/hash_to_point.rs:6-12, src/impls/g2.rs:15-17, src/impls/g1.rs:17-19):

@@ -94,6 +94,11 @@ extern "C" {
         status_out: *mut u8) -> c_int;
     pub fn blsgpu_aggregate_secure_batch(ctx: *mut blsgpu_ctx, impl_id: c_int, format: c_int, q: usize,
         key_off: *const u64, pks: *const u8, member_sigs: *const u8, out_sigs: *mut u8, status_out: *mut u8) -> c_int;
+    pub fn blsgpu_verify_secure_batch_keyed(ctx: *mut blsgpu_ctx, keyset: u64, scheme: c_int, format: c_int, q: usize,
+        key_off: *const u64, key_idx: *const u32, sigs: *const u8, msgs: *const u8, msg_off: *const u64,
+        status_out: *mut u8) -> c_int;
+    pub fn blsgpu_aggregate_secure_batch_keyed(ctx: *mut blsgpu_ctx, keyset: u64, format: c_int, q: usize,
+        key_off: *const u64, key_idx: *const u32, member_sigs: *const u8, out_sigs: *mut u8, status_out: *mut u8) -> c_int;
 
     // ---- threshold shares -----------------------------------------------------------------------------------------------
     /// shares: records of 32 + 48|96 bytes = `Vec::<u8>::from(&InnerPointShareG1|G2)` (reference src/lib.rs:150-157)

@@ -7,6 +7,7 @@
 //! |---|---|
 //! | [`Engine::verify_batch`] | `Signature::verify` (src/signature.rs:130-138) |
 //! | [`Engine::verify_batch_keyed`] / [`Engine::verify_batch_grouped_keyed`] | `Signature::verify` against keys decoded once into a [`KeySet`] |
+//! | [`Engine::verify_secure_batch_keyed_with_mode`] / [`Engine::aggregate_secure_batch_keyed_with_mode`] | `verify_secure_with_mode` / `aggregate_secure_with_mode` over quorum members named by index into a [`KeySet`] |
 //! | [`Engine::pop_verify_batch`] | `ProofOfPossession::verify` (src/proof_of_possession.rs:77-81) |
 //! | [`Engine::aggregate_verify`] | `AggregateSignature::verify` (src/aggregate_signature.rs:230-239) |
 //! | [`Engine::aggregate_verify_batch`] | q × `AggregateSignature::verify`, one pipeline per signature scheme present |
@@ -203,7 +204,8 @@ pub struct Partial {
 }
 
 /// Public keys decoded once into device memory of the [`Engine`] that made them ([`Engine::key_set`]), named by index
-/// in [`Engine::verify_batch_keyed`] and [`Engine::verify_batch_grouped_keyed`].  Only the engine's id of the set is held
+/// in [`Engine::verify_batch_keyed`], [`Engine::verify_batch_grouped_keyed`] and the keyed secure calls
+/// ([`Engine::verify_secure_batch_keyed_with_mode`], [`Engine::aggregate_secure_batch_keyed_with_mode`]).  Only the engine's id of the set is held
 /// here: [`Engine::drop_key_set`] frees the memory, and so does dropping the engine.  Used with another engine, or after
 /// it was freed, the id is an `EngineError` (`BLSGPU_E_ARG`), never undefined behaviour.
 pub struct KeySet<C: GpuImpl> {
@@ -220,6 +222,17 @@ impl<C: GpuImpl> KeySet<C> {
     pub fn is_empty(&self) -> bool {
         self.len == 0
     }
+}
+
+/// Member offsets and flat key indices of quorums named by index into a key set.
+fn pack_index_sets(sets: &[&[u32]]) -> (Vec<u64>, Vec<u32>) {
+    let mut off = vec![0u64];
+    let mut idx = Vec::new();
+    for set in sets {
+        idx.extend_from_slice(set);
+        off.push(idx.len() as u64);
+    }
+    (off, idx)
 }
 
 /// RAII owner of a `blsgpu_ctx` (one per thread; a context is not thread-safe, different contexts are independent).
@@ -759,6 +772,84 @@ impl Engine {
         let mut status = vec![0u8; q];
         let rc = unsafe {
             sys::blsgpu_aggregate_secure_batch(self.ctx, C::IMPL_ID, format_id(format), q, key_off.as_ptr(), pk_bytes.as_ptr(),
+                member.as_ptr(), out.as_mut_ptr(), status.as_mut_ptr())
+        };
+        self.check(rc)?;
+        let out = self.recode_back::<C>(C::SIG_GROUP, out, C::SIG_BYTES, format)?;
+        Ok((0..q)
+            .map(|j| {
+                if mismatched[j] {
+                    return Err(BlsError::InvalidInputs("Mismatched array lengths".to_string()));
+                }
+                status_to_result(status[j], None)?;
+                unpack_point(&out[j * C::SIG_BYTES..(j + 1) * C::SIG_BYTES])
+                    .ok_or_else(|| BlsError::DeserializationError("engine returned an invalid point".into()))
+            })
+            .collect())
+    }
+
+    /// [`Engine::verify_secure_batch_with_mode`] with quorum j's keys = the keys of `keys` at `key_idx_sets[j]`.  The set
+    /// may have been made in either format; its keys are hashed in `format`'s byte form.  An index at or past the end of the
+    /// set is an `EngineError` (`BLSGPU_E_ARG`), as is a set of another engine.
+    pub fn verify_secure_batch_keyed_with_mode<C: GpuImpl, B: AsRef<[u8]>>(
+        &mut self,
+        keys: &KeySet<C>,
+        key_idx_sets: &[&[u32]],
+        sigs: &[Signature<C>],
+        msgs: &[B],
+        format: SerializationFormat,
+    ) -> EngineResult<Vec<BlsResult<()>>> {
+        let q = key_idx_sets.len();
+        if sigs.len() != q || msgs.len() != q {
+            return Err(EngineError { code: sys::BLSGPU_E_ARG, message: "verify_secure_batch_keyed: slice lengths differ".into() });
+        }
+        if q == 0 {
+            return Ok(Vec::new());
+        }
+        let scheme = signature_scheme(&sigs[0]);
+        let (key_off, key_idx) = pack_index_sets(key_idx_sets);
+        let sig_bytes = self.recode::<C>(C::SIG_GROUP, pack_points(sigs.iter().map(|s| *s.as_raw_value()), C::SIG_BYTES), C::SIG_BYTES, format)?;
+        let packed = PackedMessages::from_iter(msgs.iter());
+        let mut status = vec![0u8; q];
+        let rc = unsafe {
+            sys::blsgpu_verify_secure_batch_keyed(self.ctx, keys.id, scheme_id(scheme), format_id(format), q, key_off.as_ptr(),
+                key_idx.as_ptr(), sig_bytes.as_ptr(), packed.bytes.as_ptr(), packed.offsets.as_ptr(), status.as_mut_ptr())
+        };
+        self.check(rc)?;
+        Ok(status
+            .iter()
+            .zip(sigs)
+            .map(|(&st, s)| if signature_scheme(s) != scheme { Err(BlsError::InvalidSignatureScheme) } else { status_to_result(st, None) })
+            .collect())
+    }
+
+    /// [`Engine::aggregate_secure_batch_with_mode`] with quorum j's keys = the keys of `keys` at `key_idx_sets[j]`.
+    pub fn aggregate_secure_batch_keyed_with_mode<C: GpuImpl>(
+        &mut self,
+        keys: &KeySet<C>,
+        key_idx_sets: &[&[u32]],
+        sig_sets: &[&[<C as Pairing>::Signature]],
+        format: SerializationFormat,
+    ) -> EngineResult<Vec<BlsResult<<C as Pairing>::Signature>>> {
+        let q = key_idx_sets.len();
+        if sig_sets.len() != q {
+            return Err(EngineError { code: sys::BLSGPU_E_ARG, message: "aggregate_secure_batch_keyed: slice lengths differ".into() });
+        }
+        // as in aggregate_secure_batch_with_mode: a quorum whose two lists differ in length is sent empty and reported here
+        let mismatched: Vec<bool> = key_idx_sets.iter().zip(sig_sets).map(|(k, s)| k.len() != s.len()).collect();
+        let sets: Vec<&[u32]> = key_idx_sets.iter().zip(&mismatched).map(|(k, &m)| if m { &k[..0] } else { *k }).collect();
+        let (key_off, key_idx) = pack_index_sets(&sets);
+        let mut member = Vec::new();
+        for (s, &m) in sig_sets.iter().zip(&mismatched) {
+            if !m {
+                member.extend_from_slice(&pack_points(s.iter().copied(), C::SIG_BYTES));
+            }
+        }
+        let member = self.recode::<C>(C::SIG_GROUP, member, C::SIG_BYTES, format)?;
+        let mut out = vec![0u8; q * C::SIG_BYTES];
+        let mut status = vec![0u8; q];
+        let rc = unsafe {
+            sys::blsgpu_aggregate_secure_batch_keyed(self.ctx, keys.id, format_id(format), q, key_off.as_ptr(), key_idx.as_ptr(),
                 member.as_ptr(), out.as_mut_ptr(), status.as_mut_ptr())
         };
         self.check(rc)?;

@@ -15,6 +15,9 @@ argument meaning and error behaviour:
   aggregate_secure[_with_mode] -> aggregate_secure_batch  (src/secure_aggregation.rs:159-169,338-352)
                                -> verify_secure_batch_keyed / aggregate_secure_batch_keyed (members named by index
                                   into a KeySet)
+  MultiSignature::verify(&MultiPublicKey::from_public_keys(..), msg)
+                               -> verify_multisig_batch / verify_multisig_batch_keyed (src/multi_signature.rs:127-135)
+                               -> sum_points_batch (many from_signatures / from_public_keys sums in one call)
 
 There is no CPU fallback: importing works anywhere, but creating an Engine without the CUDA library or a GPU raises.
 """
@@ -130,6 +133,9 @@ def load_library() -> ctypes.CDLL:
         "blsgpu_aggregate_secure_batch": (c.c_int, [vp, c.c_int, c.c_int, c.c_size_t, u64p, u8p, u8p, u8p, u8p]),
         "blsgpu_verify_secure_batch_keyed": (c.c_int, [vp, c.c_uint64, c.c_int, c.c_int, c.c_size_t, u64p, vp, u8p, u8p, u64p, u8p]),
         "blsgpu_aggregate_secure_batch_keyed": (c.c_int, [vp, c.c_uint64, c.c_int, c.c_size_t, u64p, vp, u8p, u8p, u8p]),
+        "blsgpu_verify_multisig_batch": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u64p, u8p, u8p, u8p, u64p, u8p]),
+        "blsgpu_verify_multisig_batch_keyed": (c.c_int, [vp, c.c_uint64, c.c_int, c.c_int, c.c_size_t, u64p, vp, u8p, u8p, u64p, u8p]),
+        "blsgpu_sum_points_batch": (c.c_int, [vp, c.c_int, c.c_int, c.c_size_t, u64p, u8p, u8p, u8p, i64p]),
         "blsgpu_hash_to_curve_batch": (c.c_int, [vp, c.c_int, c.c_size_t, u8p, u64p, u8p, c.c_size_t, u8p]),
         "blsgpu_recode_points": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u8p, u8p, u8p]),
         "blsgpu_fp_mul_batch": (c.c_int, [vp, c.c_int, c.c_size_t, u8p, u8p, u8p]),
@@ -166,7 +172,8 @@ EXPORTED_SYMBOLS = [
     "blsgpu_miller_partial", "blsgpu_final_exp_is_one", "blsgpu_partial_finish",
     "blsgpu_verify_batch_dev", "blsgpu_pop_verify_batch", "blsgpu_aggregate_verify", "blsgpu_aggregate_verify_batch", "blsgpu_sum_points",
     "blsgpu_verify_secure_batch", "blsgpu_aggregate_secure_batch",
-    "blsgpu_verify_secure_batch_keyed", "blsgpu_aggregate_secure_batch_keyed", "blsgpu_hash_to_curve_batch", "blsgpu_recode_points",
+    "blsgpu_verify_secure_batch_keyed", "blsgpu_aggregate_secure_batch_keyed",
+    "blsgpu_verify_multisig_batch", "blsgpu_verify_multisig_batch_keyed", "blsgpu_sum_points_batch", "blsgpu_hash_to_curve_batch", "blsgpu_recode_points",
     "blsgpu_fp_mul_batch", "blsgpu_pairing_product_is_one", "blsgpu_testdata_sign", "blsgpu_imad_peak",
     "blsgpu_combine_shares_batch", "blsgpu_verify_batch_wire", "blsgpu_pairing_check_batch",
     "blsgpu_signcrypt_valid_batch", "blsgpu_signcrypt_verify_share_batch", "blsgpu_pok_verify_batch", "blsgpu_verify_batch_records", "blsgpu_selftest", "blsgpu_plan_msm", "blsgpu_plan_shards", "blsgpu_verify_share_batch", "blsgpu_last_stage_ms", "blsgpu_last_kernel_ms", "blsgpu_launch_count",
@@ -651,6 +658,94 @@ class Engine:
                                                            _ptr(status))
         self._check(rc, "blsgpu_aggregate_secure_batch_keyed")
         return status, out
+
+    # ---- multi-signatures over signer subsets ----------------------------------------------------------------------------
+    def verify_multisig_batch(self, impl_id: int, scheme: int, key_sets: Sequence[Sequence[bytes]], sigs, msgs: Sequence[bytes],
+                              fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """status[j] == 0  <=>  MultiSignature::verify(&MultiPublicKey::from_public_keys(key_sets[j]), msgs[j]).is_ok()
+        (multi_signature.rs:127-135); otherwise the reference's error for sum_points then verify."""
+        q = len(key_sets)
+        koff = np.zeros(q + 1, dtype=np.uint64)
+        if q:
+            koff[1:] = np.cumsum([len(k) for k in key_sets], dtype=np.uint64)
+        pk = _pack_points([k for ks in key_sets for k in ks], pk_len(impl_id), "public key")
+        sg = _pack_points(sigs, sig_len(impl_id), "signature")
+        if sg.size // sig_len(impl_id) != q or len(msgs) != q:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        data, off = pack_messages(msgs)
+        return self.verify_multisig_batch_packed(impl_id, scheme, koff, pk, sg, data, off, fmt)
+
+    def verify_multisig_batch_packed(self, impl_id: int, scheme: int, koff: np.ndarray, pk: np.ndarray, sg: np.ndarray, data: np.ndarray,
+                                     off: np.ndarray, fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """Flat-buffer form: koff[q + 1] key offsets, pk koff[q] keys, sg q signatures, the q messages as data / off."""
+        koff = np.ascontiguousarray(koff, dtype=np.uint64).reshape(-1)
+        q = koff.size - 1
+        pk, sg = _pack_points(pk, pk_len(impl_id), "public key"), _pack_points(sg, sig_len(impl_id), "signature")
+        if pk.size != (int(koff[-1]) if q else 0) * pk_len(impl_id) or sg.size != q * sig_len(impl_id) or off.size - 1 != q:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        status = np.empty(q, dtype=np.uint8)
+        rc = self._lib.blsgpu_verify_multisig_batch(self._ctx, impl_id, scheme, fmt, q, _ptr(koff), _ptr(pk), _ptr(sg), _ptr(data), _ptr(off),
+                                                    _ptr(status))
+        self._check(rc, "blsgpu_verify_multisig_batch")
+        return status
+
+    def verify_multisig_batch_keyed(self, keys: KeySet, scheme: int, key_idx_sets: Sequence[Sequence[int]], sigs, msgs: Sequence[bytes],
+                                    fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """verify_multisig_batch with set j's keys = keys of `keys` at key_idx_sets[j] (fmt is the signatures' format)."""
+        q = len(key_idx_sets)
+        koff = np.zeros(q + 1, dtype=np.uint64)
+        if q:
+            koff[1:] = np.cumsum([len(k) for k in key_idx_sets], dtype=np.uint64)
+        idx = np.array([k for ks in key_idx_sets for k in ks], dtype=np.uint32)
+        sg = _pack_points(sigs, sig_len(keys.impl_id), "signature")
+        if sg.size // sig_len(keys.impl_id) != q or len(msgs) != q:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        data, off = pack_messages(msgs)
+        return self.verify_multisig_batch_keyed_packed(keys, scheme, koff, idx, sg, data, off, fmt)
+
+    def verify_multisig_batch_keyed_packed(self, keys: KeySet, scheme: int, koff: np.ndarray, key_idx: np.ndarray, sg: np.ndarray,
+                                           data: np.ndarray, off: np.ndarray, fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """Flat-buffer form: koff[q + 1] member offsets, key_idx uint32[koff[q]], sg q signatures, the q messages as data / off."""
+        koff = np.ascontiguousarray(koff, dtype=np.uint64).reshape(-1)
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32).reshape(-1)
+        q = koff.size - 1
+        sg = _pack_points(sg, sig_len(keys.impl_id), "signature")
+        if key_idx.size != (int(koff[-1]) if q else 0) or sg.size != q * sig_len(keys.impl_id) or off.size - 1 != q:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        status = np.empty(q, dtype=np.uint8)
+        rc = self._lib.blsgpu_verify_multisig_batch_keyed(self._ctx, keys.id, scheme, fmt, q, _ptr(koff), _ptr(key_idx), _ptr(sg), _ptr(data),
+                                                          _ptr(off), _ptr(status))
+        self._check(rc, "blsgpu_verify_multisig_batch_keyed")
+        return status
+
+    def sum_points_batch(self, group: int, point_sets: Sequence[Sequence[bytes]],
+                         fmt: int = SerializationFormat.Modern) -> Tuple[np.ndarray, np.ndarray, List[bytes]]:
+        """q x sum_points in one call: (status[q], bad_index[q] counted inside each set, q compressed sums; zeroed where a
+        set fails)."""
+        q = len(point_sets)
+        length = 48 if group == 1 else 96
+        soff = np.zeros(q + 1, dtype=np.uint64)
+        if q:
+            soff[1:] = np.cumsum([len(s) for s in point_sets], dtype=np.uint64)
+        pts = _pack_points([p for ps in point_sets for p in ps], length, "point")
+        status, bad, out = self.sum_points_batch_packed(group, soff, pts, fmt)
+        return status, bad, [out[j * length:(j + 1) * length].tobytes() for j in range(q)]
+
+    def sum_points_batch_packed(self, group: int, set_off: np.ndarray, pts: np.ndarray,
+                                fmt: int = SerializationFormat.Modern) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """Flat-buffer form: set_off[q + 1] point offsets, pts set_off[q] points; returns (status, bad_index, q sums flat)."""
+        length = 48 if group == 1 else 96
+        set_off = np.ascontiguousarray(set_off, dtype=np.uint64).reshape(-1)
+        q = set_off.size - 1
+        pts = _pack_points(pts, length, "point")
+        if pts.size != (int(set_off[-1]) if q else 0) * length:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        out = np.zeros(q * length, dtype=np.uint8)
+        status = np.empty(q, dtype=np.uint8)
+        bad = np.full(q, -1, dtype=np.int64)
+        rc = self._lib.blsgpu_sum_points_batch(self._ctx, group, fmt, q, _ptr(set_off), _ptr(pts), _ptr(out), _ptr(status), _ptr(bad))
+        self._check(rc, "blsgpu_sum_points_batch")
+        return status, bad, out
 
     def recode_points_packed(self, group: int, pts: np.ndarray, fmt_in: int, fmt_out: int) -> np.ndarray:
         L = 48 if group == 1 else 96

@@ -362,6 +362,42 @@ std::vector<Level> make_levels(size_t n) {
 }
 size_t levels_total(const std::vector<Level>& lv) { return lv.back().off + lv.back().cnt; }
 
+// A segmented 16-ary reduction over segments of cnt[j] >= 1 nodes: levels of ranges of at most 16 consecutive nodes of one
+// segment, until one node per segment.  n[k]: the nodes of level k (n[0]: every segment's nodes, in segment order); off: the
+// n[k] + 1 range offsets of every level k >= 1, concatenated.
+struct SegLevels {
+  std::vector<uint32_t> off;
+  std::vector<size_t> n;
+  size_t below_top() const {  // the nodes of every level but the last (the last is one node per segment)
+    size_t t = 0;
+    for (size_t k = 0; k + 1 < n.size(); k++) t += n[k];
+    return t;
+  }
+};
+SegLevels seg_levels(std::vector<size_t> cnt) {
+  SegLevels s;
+  const size_t q = cnt.size();
+  size_t total = 0;
+  for (size_t c : cnt) total += c;
+  s.n.push_back(total);
+  while (s.n.back() > q) {
+    uint32_t in = 0;
+    size_t outs = 0;
+    s.off.push_back(0);
+    for (size_t j = 0; j < q; j++) {
+      const size_t o = (cnt[j] + 15) / 16;
+      for (size_t k = 0; k < o; k++) {
+        in += (uint32_t)std::min<size_t>(16, cnt[j] - 16 * k);
+        s.off.push_back(in);
+      }
+      cnt[j] = o;
+      outs += o;
+    }
+    s.n.push_back(outs);
+  }
+  return s;
+}
+
 // -----------------------------------------------------------------------------------------------------------------
 // The batch pipeline on decoded points.  PkA/SigA are the affine types of the impl.
 //   pre[i]   : status before pairing work (non-OK items are excluded from the batch equation)
@@ -453,6 +489,37 @@ int reduce_levels(blsgpu_ctx* ctx, const std::vector<Level>& lv, size_t first, F
   for (size_t k = first; k + 1 < lv.size(); k++) {
     if (F) REDUCE_FP12(lv[k].cnt, (const Fp12*)(F + lv[k].off), lv[k + 1].cnt, F + lv[k + 1].off);
     if (S) REDUCE_JAC(J, lv[k].cnt, (const J*)(S + lv[k].off), lv[k + 1].cnt, S + lv[k + 1].off);
+  }
+  return BLSGPU_OK;
+}
+
+// the levels of a segmented reduction (seg_levels; d_off = its offsets on the device): level 0 in nodes[0 .. n[0]), the
+// levels between in nodes after it, the last level (one node per segment) in top.  A level of few nodes takes the
+// sixteen-lanes-per-node kernel, as REDUCE_FP12 / REDUCE_JAC do.
+int seg_reduce(blsgpu_ctx* ctx, size_t n_out, const uint32_t* off, const Fp12* in, Fp12* out) {
+  if (n_out <= REDUCE_WIDE_MAX)
+    LAUNCH(k_seg_reduce_fp12_w, blocks_for(n_out * 16), TPB, n_out, off, in, out);
+  else
+    LAUNCH(k_seg_reduce_fp12, blocks_for(n_out), TPB, n_out, off, in, out);
+  return BLSGPU_OK;
+}
+template <class J>
+int seg_reduce(blsgpu_ctx* ctx, size_t n_out, const uint32_t* off, const J* in, J* out) {
+  if (n_out <= REDUCE_WIDE_MAX)
+    LAUNCH((k_seg_reduce_jac_w<J>), blocks_for(n_out * 16), TPB, n_out, off, in, out);
+  else
+    LAUNCH((k_seg_reduce_jac<J>), blocks_for(n_out), TPB, n_out, off, in, out);
+  return BLSGPU_OK;
+}
+template <class T>
+int seg_reduce_levels(blsgpu_ctx* ctx, const SegLevels& s, const uint32_t* d_off, T* nodes, T* top) {
+  size_t in_off = 0, out_off = s.n[0], o = 0;
+  for (size_t k = 1; k < s.n.size(); k++) {
+    const size_t n_out = s.n[k];
+    CKR(seg_reduce(ctx, n_out, d_off + o, (const T*)(nodes + in_off), k + 1 == s.n.size() ? top : nodes + out_off));
+    o += n_out + 1;
+    in_off = out_off;
+    out_off += n_out;
   }
   return BLSGPU_OK;
 }
@@ -1773,29 +1840,11 @@ static int aggregate_batch_impl(blsgpu_ctx* ctx, int scheme, int format, size_t 
   for (size_t j = 0; j < q; j++) g_first[j + 1] = g_first[j] + std::max<size_t>(1, (size_t)(set_off[j + 1] - set_off[j] + M6_GROUP - 1) / M6_GROUP);
   const size_t ng = g_first[q], nslots = ng * M6_GROUP;
   // the segmented product: levels of ranges of <= 16 consecutive nodes of one aggregate, until one node per aggregate
-  std::vector<uint32_t> seg_off;       // every level's n_out + 1 range offsets, concatenated
-  std::vector<size_t> seg_n{ng};       // nodes per level (level 0: the groups)
-  {
-    std::vector<size_t> cnt(q);
-    for (size_t j = 0; j < q; j++) cnt[j] = g_first[j + 1] - g_first[j];
-    while (seg_n.back() > q) {
-      uint32_t in = 0;
-      size_t outs = 0;
-      seg_off.push_back(0);
-      for (size_t j = 0; j < q; j++) {
-        const size_t o = (cnt[j] + 15) / 16;
-        for (size_t k = 0; k < o; k++) {
-          in += (uint32_t)std::min<size_t>(16, cnt[j] - 16 * k);
-          seg_off.push_back(in);
-        }
-        cnt[j] = o;
-        outs += o;
-      }
-      seg_n.push_back(outs);
-    }
-  }
-  size_t seg_total = 0;
-  for (size_t k = 0; k + 1 < seg_n.size(); k++) seg_total += seg_n[k];  // every level but the last (which is the set tree's)
+  std::vector<size_t> cnt(q);
+  for (size_t j = 0; j < q; j++) cnt[j] = g_first[j + 1] - g_first[j];
+  const SegLevels seg = seg_levels(std::move(cnt));
+  const std::vector<uint32_t>& seg_off = seg.off;
+  const size_t seg_total = seg.below_top();  // the last level is the set tree's leaves
   Pipe<PkA, SigA> P;
   P.lv = make_levels(q);
   const size_t qtotal = levels_total(P.lv), ndig = levels_total(make_levels(np + q));
@@ -1901,28 +1950,14 @@ static int aggregate_batch_impl(blsgpu_ctx* ctx, int scheme, int format, size_t 
   CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
   P.root_T_ready = false;
   stage_mark(ctx, BLSGPU_STAGE_MILLER);
-  const bool segmented = seg_n.size() > 1;  // some aggregate spans more than one group
+  const bool segmented = seg.n.size() > 1;  // some aggregate spans more than one group
   CKR((miller_stage<PkA, SigA>(ctx, P, nslots, d_pks, d_hs, d_pres, segmented ? d_Fseg : P.d_F,
                                [&](cudaStream_t s, size_t cn, size_t base, M6Arg* args) {
                                  k_m6_prep_sets<PkA, SigA><<<blocks_for(cn), TPB, 0, s>>>(cn, base, d_pks, d_hs, (const uint8_t*)d_pres,
                                                                                           (const uint32_t*)d_gset, (const Digest*)d_root, rbits, args);
                                })));
   stage_mark(ctx, BLSGPU_STAGE_REDUCE);
-  {
-    size_t in_off = 0, out_off = seg_n[0], o = 0;
-    for (size_t k = 1; k < seg_n.size(); k++) {
-      const size_t n_out = seg_n[k];
-      const Fp12* in = d_Fseg + in_off;
-      Fp12* out = k + 1 == seg_n.size() ? P.d_F : d_Fseg + out_off;
-      if (n_out <= REDUCE_WIDE_MAX)
-        LAUNCH(k_seg_reduce_fp12_w, blocks_for(n_out * 16), TPB, n_out, (const uint32_t*)(d_segoff + o), in, out);
-      else
-        LAUNCH(k_seg_reduce_fp12, blocks_for(n_out), TPB, n_out, (const uint32_t*)(d_segoff + o), in, out);
-      o += n_out + 1;
-      in_off = out_off;
-      out_off += n_out;
-    }
-  }
+  CKR(seg_reduce_levels<Fp12>(ctx, seg, d_segoff, d_Fseg, P.d_F));
   CKR(reduce_levels(ctx, P.lv, 0, P.d_F, P.d_S));
   bool ok = false;
   CKR((pipeline_check<PkA, SigA>(ctx, P, &ok)));
@@ -3175,6 +3210,229 @@ int blsgpu_aggregate_secure_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int fo
     return aggregate_secure_impl<I>(ctx, format, q, ko.data(), Keys(set, idx), member_sigs ? member_sigs + key_off[0] * Ls : nullptr, out_sigs,
                                     status_out);
   });
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Multi-signatures over signer subsets, and point sums of many sets: MultiSignature::verify(MultiPublicKey of set j, msg_j)
+// is core_verify against the SUM of set j's keys, so the q key sums are formed on the device (a segmented sum balanced by
+// member count) and the q (sum, signature, message) triples go through verify_points like any batch of q signatures.
+namespace {
+
+// The segmented sum of q point sets, set j = members off[j] .. off[j+1]-1 (off rebased to 0): chunks of at most 16 members of
+// one set for k_seg_sum_gather (an empty set has one chunk without members, so that every set has a node), then the levels of
+// seg_levels over each set's chunks.  A set of 2^20 members is 65,536 chunks next to one chunk per set of 3: the threads
+// of every launch do about equal work however skewed the set sizes are.
+struct SegSumPlan {
+  size_t q;
+  std::vector<uint32_t> coff, cset;  // chunk c: members coff[c] .. coff[c+1]-1 of set cset[c]
+  SegLevels lv;
+  SegSumPlan(size_t q_, const uint64_t* off) : q(q_) {
+    std::vector<size_t> cnt(q);
+    coff.push_back(0);
+    for (size_t j = 0; j < q; j++) {
+      const uint64_t lo = off[j], hi = off[j + 1];
+      cnt[j] = 0;
+      for (uint64_t m = lo; m < hi || cnt[j] == 0; m += 16, cnt[j]++) {
+        coff.push_back((uint32_t)std::min<uint64_t>(m + 16, hi));
+        cset.push_back((uint32_t)j);
+      }
+    }
+    lv = seg_levels(std::move(cnt));
+  }
+  size_t nchunks() const { return cset.size(); }
+  template <class J>
+  size_t bytes() const {
+    return Arena::bytes<uint32_t>(coff.size()) + Arena::bytes<uint32_t>(cset.size()) + Arena::bytes<uint32_t>(std::max<size_t>(lv.off.size(), 1)) +
+           Arena::bytes<J>(std::max<size_t>(lv.below_top(), 1)) + Arena::bytes<unsigned long long>(q) + Arena::bytes<J>(q);
+  }
+};
+
+// sum[j] = the sum of set j's points (the identity for an empty set), first_bad[j] = (member << 8 | status) of its first
+// member that failed to decode or ~0 (kernels.cuh k_seg_sum_gather).  Member m's point is d_pts[d_idx[m]], or d_pts[m] when
+// d_idx is null; likewise its status in d_st.
+template <class A>
+int seg_point_sums(blsgpu_ctx* ctx, const SegSumPlan& pl, const uint32_t* d_idx, const A* d_pts, const uint8_t* d_st,
+                   typename PtInfo<A>::Jac** sum_out, unsigned long long** first_bad_out) {
+  typedef typename PtInfo<A>::Jac J;
+  uint32_t *d_coff, *d_cset, *d_segoff;
+  CKR(upload(ctx, d_coff, pl.coff.data(), pl.coff.size()));
+  CKR(upload(ctx, d_cset, pl.cset.data(), pl.cset.size()));
+  CKR(upload(ctx, d_segoff, pl.lv.off.data(), pl.lv.off.size()));
+  J* d_nodes = ctx->arena.take<J>(std::max<size_t>(pl.lv.below_top(), 1));
+  unsigned long long* d_bad = ctx->arena.take<unsigned long long>(pl.q);
+  J* d_sum = ctx->arena.take<J>(pl.q);
+  ARENA_OK();
+  CK(cudaMemsetAsync(d_bad, 0xff, pl.q * sizeof(unsigned long long), ctx->stream));
+  const bool levels = pl.lv.n.size() > 1;  // some set has more than one chunk
+  LAUNCH((k_seg_sum_gather<A>), blocks_for(pl.nchunks()), TPB, pl.nchunks(), (const uint32_t*)d_coff, (const uint32_t*)d_cset, d_idx, d_pts, d_st,
+         levels ? d_nodes : d_sum, d_bad);
+  if (levels) CKR(seg_reduce_levels<J>(ctx, pl.lv, d_segoff, d_nodes, d_sum));
+  *sum_out = d_sum;
+  *first_bad_out = d_bad;
+  return BLSGPU_OK;
+}
+
+// q x MultiSignature::verify: the key step (upload and decode the members' keys, or their indices into a key set), the
+// segmented key sums, then verify_points on (sum_j, sig_j, msg_j).  Key offsets start at 0 (the entry points rebase them).
+// The per-set status before any pairing work is k_prestatus's over (first bad key of the set, signature decode status,
+// signature identity, sum identity): the reference's order for sum_points followed by verify.
+template <int IMPL>
+int verify_multisig_impl(blsgpu_ctx* ctx, int scheme, int format, size_t q, const uint64_t* key_off, const Keys& keys, const uint8_t* sigs,
+                         const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
+  typedef typename ImplT<IMPL>::PkAff PkA;
+  typedef typename ImplT<IMPL>::SigAff SigA;
+  typedef typename ImplT<IMPL>::PkJac PkJ;
+  const size_t Lp = PtInfo<PkA>::LEN, Ls = PtInfo<SigA>::LEN;
+  const size_t M = (size_t)key_off[q], msg_bytes = (size_t)msg_off[q];
+  const SegSumPlan pl(q, key_off);
+  const size_t head = (keys.set ? M * 4 : M * (Lp + sizeof(PkA) + 1)) + pl.bytes<PkJ>() + q * (Ls + sizeof(SigA) + sizeof(PkA) + 3) + msg_bytes +
+                      (q + 1) * 8 + 16 * 256;
+  CKR(ensure_verify_arena<IMPL>(ctx, q, head));
+  stage_reset(ctx);
+  stage_mark(ctx, BLSGPU_STAGE_DECODE_PK);  // the key side: decode (unkeyed calls) and the segmented sums
+  Keys d_keys;
+  CKR(upload_keys<PkA>(ctx, M, keys, d_keys));
+  const PkA* d_pts = keys.set ? (const PkA*)keys.set->pts : nullptr;
+  const uint8_t* d_st = keys.set ? (const uint8_t*)keys.set->st : nullptr;
+  if (!keys.set) {
+    PkA* d_pk = ctx->arena.take<PkA>(std::max<size_t>(M, 1));
+    uint8_t* d_stpk = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
+    if (M) CKR((decode_points<PkA>(ctx, M, d_keys.bytes, format, d_pk, d_stpk, BLSGPU_KERNEL_DECODE_PK)));
+    d_pts = d_pk;
+    d_st = d_stpk;
+  }
+  PkJ* d_sum;
+  unsigned long long* d_bad;
+  CKR((seg_point_sums<PkA>(ctx, pl, keys.set ? d_keys.idx : nullptr, d_pts, d_st, &d_sum, &d_bad)));
+  PkA* d_agg = ctx->arena.take<PkA>(q);
+  uint8_t* d_setst = ctx->arena.take<uint8_t>(q);
+  LAUNCH((k_to_affine_batch<PkA>), blocks_for((q + TO_AFFINE_BATCH - 1) / TO_AFFINE_BATCH), TPB, q, (const PkJ*)d_sum, d_agg);
+  LAUNCH(k_seg_first_bad_status, blocks_for(q), TPB, q, (const unsigned long long*)d_bad, d_setst);
+  stage_mark(ctx, BLSGPU_STAGE_DECODE_SIG);
+  uint8_t *d_sigb, *d_msgs;
+  uint64_t* d_moff;
+  CKR(upload(ctx, d_sigb, sigs, q * Ls));
+  CKR(upload(ctx, d_msgs, msgs, msg_bytes));
+  CKR(upload(ctx, d_moff, msg_off, q + 1));
+  SigA* d_sig = ctx->arena.take<SigA>(q);
+  uint8_t* d_stsig = ctx->arena.take<uint8_t>(q);
+  uint8_t* d_status = ctx->arena.take<uint8_t>(q);
+  CKR((decode_points<SigA>(ctx, q, (const uint8_t*)d_sigb, format, d_sig, d_stsig, BLSGPU_KERNEL_DECODE_SIG)));
+  DstParam dst;
+  make_dst(dst, IMPL, scheme, false);
+  // MessageAugmentation hashes the multi key || msg (sig_aug.rs:20-24 on the MultiPublicKey's bytes)
+  CKR((verify_points<IMPL>(ctx, scheme == 1 ? 1 : 0, dst, q, d_agg, d_sig, d_setst, d_stsig, d_msgs, d_moff, d_status)));
+  CK(cudaMemcpyAsync(status_out, d_status, q, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  stage_collect(ctx);
+  return BLSGPU_OK;
+}
+
+// q x blsgpu_sum_points in one pass: decode, segmented sums, encode; per set the first bad element, counted inside the set
+template <class A>
+int sum_points_batch_impl(blsgpu_ctx* ctx, int format, size_t q, const uint64_t* set_off, const uint8_t* points, uint8_t* out,
+                          uint8_t* status_out, int64_t* bad_index_out) {
+  typedef typename PtInfo<A>::Jac J;
+  const size_t L = PtInfo<A>::LEN, M = (size_t)set_off[q];
+  const SegSumPlan pl(q, set_off);
+  CKR(ensure_arena(ctx, M * (L + sizeof(A) + 1) + pl.bytes<J>() + q * (sizeof(A) + L) + 16 * 256));
+  uint8_t* d_in;
+  CKR(upload(ctx, d_in, points, M * L));
+  A* d_pts = ctx->arena.take<A>(std::max<size_t>(M, 1));
+  uint8_t* d_st = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
+  ARENA_OK();
+  if (M) CKR((decode_points<A>(ctx, M, (const uint8_t*)d_in, format, d_pts, d_st)));
+  J* d_sum;
+  unsigned long long* d_bad;
+  CKR((seg_point_sums<A>(ctx, pl, nullptr, d_pts, d_st, &d_sum, &d_bad)));
+  A* d_res = ctx->arena.take<A>(q);
+  uint8_t* d_out = ctx->arena.take<uint8_t>(q * L);
+  LAUNCH((k_to_affine_batch<A>), blocks_for((q + TO_AFFINE_BATCH - 1) / TO_AFFINE_BATCH), TPB, q, (const J*)d_sum, d_res);
+  LAUNCH((k_encode<A>), blocks_for(q), TPB, q, (const A*)d_res, format, d_out);
+  std::vector<unsigned long long> bad(q);
+  CK(cudaMemcpyAsync(out, d_out, q * L, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(bad.data(), d_bad, q * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  for (size_t j = 0; j < q; j++) {
+    if (bad[j] == ~0ull) {
+      status_out[j] = BLSGPU_ST_OK;
+      if (bad_index_out) bad_index_out[j] = -1;
+      continue;
+    }
+    status_out[j] = (uint8_t)(bad[j] & 0xff);
+    if (bad_index_out) bad_index_out[j] = (int64_t)((bad[j] >> 8) - set_off[j]);
+    memset(out + j * L, 0, L);
+  }
+  return BLSGPU_OK;
+}
+
+// the argument checks of both multi-signature calls (the secure calls' rules; both formats for both impls, as
+// blsgpu_verify_batch), then the pipeline with key_off rebased to 0 and the keys from the first member on
+int verify_multisig_common(blsgpu_ctx* ctx, const char* what, int impl_id, int scheme, int format, size_t q, const uint64_t* key_off, Keys keys,
+                           const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
+  const void* members = keys.set ? (const void*)keys.idx : (const void*)keys.bytes;
+  if (!args_ok(impl_id, scheme, format) || (q && (!key_off || !sigs || !msg_off || !status_out)) || (q && key_off[q] > key_off[0] && !members)) {
+    ctx->err = std::string(what) + ": bad arguments";
+    return BLSGPU_E_ARG;
+  }
+  if (q == 0) return BLSGPU_OK;
+  if (!key_offsets_ok(key_off, q)) {
+    ctx->err = std::string(what) + ": key_off must be non-decreasing and below 2^32";
+    return BLSGPU_E_ARG;
+  }
+  CHECK_OFFSETS(msg_off, q, what);
+  if (msg_off[q] > msg_off[0] && !msgs) {
+    ctx->err = std::string(what) + ": msgs is null";
+    return BLSGPU_E_ARG;
+  }
+  const std::vector<uint64_t> ko = rebased(key_off, 0, q);
+  if (keys.set && keys.idx) keys.idx += key_off[0];
+  if (!keys.set && keys.bytes) keys.bytes += key_off[0] * (impl_id == 2 ? 48 : 96);
+  if (!key_idx_ok(ctx, what, keys, (size_t)ko[q])) return BLSGPU_E_ARG;
+  CKR(set_device(ctx));
+  return with_impl(impl_id, [&](auto I) { return verify_multisig_impl<I>(ctx, scheme, format, q, ko.data(), keys, sigs, msgs, msg_off, status_out); });
+}
+
+}  // namespace
+
+int blsgpu_verify_multisig_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t q, const uint64_t* key_off, const uint8_t* pks,
+                                 const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
+  NVTX_RANGE("blsgpu_verify_multisig_batch");
+  if (!ctx) return BLSGPU_E_ARG;
+  return verify_multisig_common(ctx, "blsgpu_verify_multisig_batch", impl_id, scheme, format, q, key_off, Keys(pks), sigs, msgs, msg_off, status_out);
+}
+
+int blsgpu_verify_multisig_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t q, const uint64_t* key_off,
+                                       const uint32_t* key_idx, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off,
+                                       uint8_t* status_out) {
+  NVTX_RANGE("blsgpu_verify_multisig_batch_keyed");
+  if (!ctx) return BLSGPU_E_ARG;
+  const char* what = "blsgpu_verify_multisig_batch_keyed";
+  const KeySet* set = find_keyset(ctx, keyset, what);
+  if (!set) return BLSGPU_E_ARG;
+  return verify_multisig_common(ctx, what, set->impl_id, scheme, format, q, key_off, Keys(set, key_idx), sigs, msgs, msg_off, status_out);
+}
+
+int blsgpu_sum_points_batch(blsgpu_ctx* ctx, int group, int format, size_t q, const uint64_t* set_off, const uint8_t* points, uint8_t* out,
+                            uint8_t* status_out, int64_t* bad_index_out) {
+  NVTX_RANGE("blsgpu_sum_points_batch");
+  if (!ctx) return BLSGPU_E_ARG;
+  const char* what = "blsgpu_sum_points_batch";
+  if ((group != 1 && group != 2) || (format != 0 && format != 1) || (q && (!set_off || !out || !status_out)) ||
+      (q && set_off[q] > set_off[0] && !points)) {
+    ctx->err = std::string(what) + ": bad arguments";
+    return BLSGPU_E_ARG;
+  }
+  if (q == 0) return BLSGPU_OK;
+  if (!key_offsets_ok(set_off, q)) {
+    ctx->err = std::string(what) + ": set_off must be non-decreasing and below 2^32";
+    return BLSGPU_E_ARG;
+  }
+  const std::vector<uint64_t> so = rebased(set_off, 0, q);
+  const uint8_t* pts = points ? points + set_off[0] * (group == 1 ? 48 : 96) : nullptr;
+  CKR(set_device(ctx));
+  return group == 1 ? sum_points_batch_impl<G1Aff>(ctx, format, q, so.data(), pts, out, status_out, bad_index_out)
+                    : sum_points_batch_impl<G2Aff>(ctx, format, q, so.data(), pts, out, status_out, bad_index_out);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------

@@ -1510,6 +1510,70 @@ __global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_seg_reduce_fp12_w(size_
   if (j < n_out && m == 0) out[j] = acc;
 }
 
+// ---- segmented point sums (blsgpu_verify_multisig_batch[_keyed], blsgpu_sum_points_batch) --------------------------------------
+// The first level: a thread per CHUNK of at most 16 consecutive members of one set (members coff[c] .. coff[c+1]-1 of set
+// cset[c]; a chunk of an empty set has none and gives the identity).  Member m's point is pts[idx[m]] (members named by index
+// into a key set) or pts[m] (idx null: points decoded in member order); a point that failed to decode is the identity there
+// (k_decode / k_subgroup_check), so it adds nothing.  The same pass finds each set's first member whose status is not OK:
+// first_bad[set] = min over such members of (m << 8 | status), ~0 where there is none.
+template <class A>
+__global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_seg_sum_gather(size_t nchunks, const uint32_t* __restrict__ coff,
+                                                        const uint32_t* __restrict__ cset, const uint32_t* __restrict__ idx,
+                                                        const A* __restrict__ pts, const uint8_t* __restrict__ st,
+                                                        typename PtInfo<A>::Jac* __restrict__ out, unsigned long long* __restrict__ first_bad) {
+  const size_t c = BLS_TID();
+  if (c >= nchunks) return;
+  const uint32_t lo = coff[c], hi = coff[c + 1];
+  typename PtInfo<A>::Jac acc;
+  jac_set_inf(acc);
+  unsigned long long bad = ~0ull;
+  for (uint32_t m = lo; m < hi; m++) {
+    const uint32_t k = idx ? idx[m] : m;
+    const uint8_t s = st[k];
+    if (s != ST_OK && bad == ~0ull) bad = ((unsigned long long)m << 8) | s;
+    A p = pts[k];
+    jac_add_mixed(acc, acc, p);
+  }
+  out[c] = acc;
+  if (bad != ~0ull) atomicMin(first_bad + cset[c], bad);
+}
+// per set: the status of its first member that failed to decode (k_seg_sum_gather), or OK
+__global__ void k_seg_first_bad_status(size_t q, const unsigned long long* __restrict__ first_bad, uint8_t* __restrict__ st) {
+  const size_t j = BLS_TID();
+  if (j >= q) return;
+  const unsigned long long b = first_bad[j];
+  st[j] = b == ~0ull ? (uint8_t)ST_OK : (uint8_t)(b & 0xff);
+}
+// One level of the segmented sum: out[j] = sum in[off[j] .. off[j+1]), the Jacobian twins of k_seg_reduce_fp12 / _w.
+template <class J>
+__global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_seg_reduce_jac(size_t n_out, const uint32_t* __restrict__ off, const J* __restrict__ in,
+                                                        J* __restrict__ out) {
+  const size_t j = BLS_TID();
+  if (j >= n_out) return;
+  const uint32_t lo = off[j], hi = off[j + 1];
+  J acc = in[lo];
+  for (uint32_t m = lo + 1; m < hi; m++) {
+    J t = in[m];
+    jac_add(acc, acc, t);
+  }
+  out[j] = acc;
+}
+template <class J>
+__global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_seg_reduce_jac_w(size_t n_out, const uint32_t* __restrict__ off, const J* __restrict__ in,
+                                                          J* __restrict__ out) {
+  const size_t t = BLS_TID(), j = t >> 4;
+  const int m = (int)(t & 15);
+  J acc;
+  if (j < n_out && off[j] + m < off[j + 1]) acc = in[off[j] + m]; else jac_set_inf(acc);
+#pragma unroll 1
+  for (int s = 1; s < 16; s <<= 1) {
+    J other;
+    words_shfl_xor(other, acc, s);
+    if ((m & (2 * s - 1)) == 0) jac_add(acc, acc, other);
+  }
+  if (j < n_out && m == 0) out[j] = acc;
+}
+
 // ---- signatures over shared messages (blsgpu_verify_batch_grouped) --------------------------------------------------------
 // The host counting-sorts the items by message (order[]) and cuts every message's run into LEAVES of at most
 // GROUPED_LEAF consecutive entries of order[].  The Miller stage runs over the leaves: ML(P_l, H_l) with

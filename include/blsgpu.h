@@ -66,8 +66,8 @@ typedef struct blsgpu_ctx blsgpu_ctx;
  * count); blsgpu_aggregate_verify cuts its pairs over the devices (from 4096 per device) and folds the partial products of
  * Miller values on the first device; blsgpu_aggregate_verify_batch cuts its aggregates into contiguous runs balanced by pair
  * count (from 4096 pairs per device), each verified on its own device without a fold.  Every other entry point (among them
- * blsgpu_verify_batch_grouped, the key sets, the keyed verify calls and the keyed secure calls), the *_dev variants and
- * blsgpu_ctx_set_stream use the first device.  One process per
+ * blsgpu_verify_batch_grouped, the key sets, the keyed verify calls, the keyed secure calls, blsgpu_verify_multisig_batch[_keyed]
+ * and blsgpu_sum_points_batch), the *_dev variants and blsgpu_ctx_set_stream use the first device.  One process per
  * device with blsgpu_miller_partial / blsgpu_final_exp_is_one does the same across processes. */
 int blsgpu_ctx_create(const int* devices, int ndev, blsgpu_ctx** out);
 void blsgpu_ctx_destroy(blsgpu_ctx* ctx);
@@ -225,6 +225,36 @@ int blsgpu_aggregate_secure_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int fo
                                         const uint32_t* key_idx, const uint8_t* member_sigs, uint8_t* out_sigs,
                                         uint8_t* status_out);
 
+/* ---- multi-signatures over signer subsets ------------------------------------------------------------------------
+ * q x MultiSignature::verify(MultiPublicKey::from_public_keys(keys of set j), msg_j)  (reference src/multi_signature.rs:127-135,
+ * src/multi_public_key.rs:79-83, src/traits/pk_multi.rs:7-13 -> core_verify sig_core.rs:120-146).  Set j owns keys
+ * key_off[j] .. key_off[j+1]-1 of pks (key_off: q+1 non-decreasing entries below 2^32, as blsgpu_verify_secure_batch); one
+ * signature and one message per set.
+ * status_out[j] is exactly blsgpu_sum_points(pk group, format, keys of set j) followed by blsgpu_verify_batch(impl, scheme,
+ * format, [that sum], [sig_j], [msg_j]): the first key of the set (in member order) that fails to decode, else the
+ * signature's decode error, else SIG_IDENTITY, else PK_IDENTITY when the sum is the identity (an empty set, P and -P, only
+ * identity keys), else OK or INVALID_SIGNATURE.  Identity keys add nothing; a key named twice counts twice.
+ * MessageAugmentation hashes the compressed multi key || msg.  Both formats for both impls, as blsgpu_verify_batch.
+ * The key sums are one segmented sum on the device, balanced by member count (chunks of 16 members of one set, then levels
+ * of ranges of 16 partial sums), recorded as BLSGPU_STAGE_DECODE_PK together with the keys' decode; the q (sum, signature,
+ * message) triples then take blsgpu_verify_batch's pipeline (one random-linear-combination check, bisection on failure).
+ * At most 2^32 - 16 members per call; q = 0 is OK.  First device only. */
+int blsgpu_verify_multisig_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t q, const uint64_t* key_off,
+                                 const uint8_t* pks, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off,
+                                 uint8_t* status_out);
+/* the same with set j's keys = keys key_idx[key_off[j] .. key_off[j+1]) of a key set; `format` is that of sigs only.  An id
+ * this context does not hold and a key_idx entry at or above the set's size are BLSGPU_E_ARG; a key that failed to decode
+ * at creation gives its set the status it was created with.  No key is decoded: 4 bytes per member cross the bus. */
+int blsgpu_verify_multisig_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t q,
+                                       const uint64_t* key_off, const uint32_t* key_idx, const uint8_t* sigs,
+                                       const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out);
+/* q x blsgpu_sum_points: set j = points set_off[j] .. set_off[j+1]-1; out: q compressed sums in `format` (zeroed for a
+ * failing set); status_out[j] / bad_index_out[j] (may be NULL): what blsgpu_sum_points returns for set j alone, the index
+ * counted inside set j.  MultiSignature::from_signatures / MultiPublicKey::from_public_keys / aggregate_signatures for many
+ * sets (the binding applies from_signatures' scheme rules).  The same segmented sum as above.  First device only. */
+int blsgpu_sum_points_batch(blsgpu_ctx* ctx, int group, int format, size_t q, const uint64_t* set_off, const uint8_t* points,
+                            uint8_t* out, uint8_t* status_out, int64_t* bad_index_out);
+
 /* ---- building blocks (parity tests, metrics) ------------------------------------------------------------------ */
 /* hash_to_point (reference src/traits/hash_to_point.rs:6-12, src/impls/g2.rs:15-17, src/impls/g1.rs:17-19):
  * out = compressed Modern points, group 2 -> 96 B each (G2Impl signatures), group 1 -> 48 B each. */
@@ -345,7 +375,7 @@ int blsgpu_plan_shards(size_t sets, const uint64_t* set_off, int ndev, uint64_t*
 
 /* ---- metrics ---------------------------------------------------------------------------------------------------
  * Per-stage device times (CUDA events on the engine's stream) of the LAST verify call on the first device. */
-#define BLSGPU_STAGE_DECODE_PK 0
+#define BLSGPU_STAGE_DECODE_PK 0 /* blsgpu_verify_multisig_batch[_keyed]: the keys' decode and their segmented sums */
 #define BLSGPU_STAGE_DECODE_SIG 1
 #define BLSGPU_STAGE_HASH 2
 #define BLSGPU_STAGE_SCALE_SIG 3 /* sum r_i sig_i (bucket multi-scalar multiplication) */

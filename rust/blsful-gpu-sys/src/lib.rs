@@ -100,6 +100,16 @@ extern "C" {
     pub fn blsgpu_aggregate_secure_batch_keyed(ctx: *mut blsgpu_ctx, keyset: u64, format: c_int, q: usize,
         key_off: *const u64, key_idx: *const u32, member_sigs: *const u8, out_sigs: *mut u8, status_out: *mut u8) -> c_int;
 
+    // ---- multi-signatures over signer subsets ------------------------------------------------------------------------------
+    pub fn blsgpu_verify_multisig_batch(ctx: *mut blsgpu_ctx, impl_id: c_int, scheme: c_int, format: c_int, q: usize,
+        key_off: *const u64, pks: *const u8, sigs: *const u8, msgs: *const u8, msg_off: *const u64,
+        status_out: *mut u8) -> c_int;
+    pub fn blsgpu_verify_multisig_batch_keyed(ctx: *mut blsgpu_ctx, keyset: u64, scheme: c_int, format: c_int, q: usize,
+        key_off: *const u64, key_idx: *const u32, sigs: *const u8, msgs: *const u8, msg_off: *const u64,
+        status_out: *mut u8) -> c_int;
+    pub fn blsgpu_sum_points_batch(ctx: *mut blsgpu_ctx, group: c_int, format: c_int, q: usize, set_off: *const u64,
+        points: *const u8, out: *mut u8, status_out: *mut u8, bad_index_out: *mut i64 /* [q] or null */) -> c_int;
+
     // ---- threshold shares -----------------------------------------------------------------------------------------------
     /// shares: records of 32 + 48|96 bytes = `Vec::<u8>::from(&InnerPointShareG1|G2)` (reference src/lib.rs:150-157)
     pub fn blsgpu_combine_shares_batch(ctx: *mut blsgpu_ctx, group: c_int, q: usize, share_off: *const u64,

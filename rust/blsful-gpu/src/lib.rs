@@ -12,6 +12,8 @@
 //! | [`Engine::aggregate_verify`] | `AggregateSignature::verify` (src/aggregate_signature.rs:230-239) |
 //! | [`Engine::aggregate_verify_batch`] | q × `AggregateSignature::verify`, one pipeline per signature scheme present |
 //! | [`Engine::aggregate_signature_from`] / [`Engine::multi_signature_from`] / [`Engine::multi_public_key_from`] | `from_signatures` / `from_public_keys` (aggregate_signature.rs:171-188, multi_signature.rs:147-150, multi_public_key.rs:79-82) |
+//! | [`Engine::multi_public_keys_from`] / [`Engine::multi_signatures_from`] | q × `from_public_keys` / `MultiSignature::from_signatures` in one call |
+//! | [`Engine::multi_signature_verify_batch_with_mode`] / [`Engine::multi_signature_verify_batch_keyed_with_mode`] | q × `MultiSignature::verify` (multi_signature.rs:127-135) against the sum of each set's keys, given as keys or as indices into a [`KeySet`] |
 //! | [`Engine::verify_secure_batch`] / [`Engine::verify_secure_batch_with_mode`] | `Signature::verify_secure[_with_mode]` (signature.rs:177-197, 256-276) |
 //! | [`Engine::aggregate_secure_batch`] / [`Engine::aggregate_secure_batch_with_mode`] | `aggregate_secure[_with_mode]` (secure_aggregation.rs:159-169, 338-352) |
 //! | [`Engine::signatures_from_shares`] / [`Engine::public_keys_from_shares`] | `Signature::from_shares` / `PublicKey::from_shares` (signature.rs:151-165, public_key.rs:128-143) |
@@ -233,6 +235,15 @@ fn pack_index_sets(sets: &[&[u32]]) -> (Vec<u64>, Vec<u32>) {
         off.push(idx.len() as u64);
     }
     (off, idx)
+}
+
+// cumulative offsets of sets of the given sizes (q + 1 entries)
+fn set_offsets<I: IntoIterator<Item = usize>>(sizes: I) -> Vec<u64> {
+    let mut off = vec![0u64];
+    for s in sizes {
+        off.push(off[off.len() - 1] + s as u64);
+    }
+    off
 }
 
 /// RAII owner of a `blsgpu_ctx` (one per thread; a context is not thread-safe, different contexts are independent).
@@ -687,6 +698,152 @@ impl Engine {
     pub fn multi_public_key_from<C: GpuImpl>(&mut self, keys: &[PublicKey<C>]) -> EngineResult<BlsResult<MultiPublicKey<C>>> {
         let bytes = pack_points(keys.iter().map(|p| p.0), C::PK_BYTES);
         Ok(self.sum_points::<<C as Pairing>::PublicKey>(C::PK_GROUP, &bytes, C::PK_BYTES)?.map(MultiPublicKey))
+    }
+
+    /// q point sums in one engine call (`blsgpu_sum_points_batch`): set j's result is what `sum_points` gives for it alone.
+    fn sum_points_batch<P: GroupEncoding>(&mut self, group: c_int, set_off: &[u64], bytes: &[u8], each: usize) -> EngineResult<Vec<BlsResult<P>>> {
+        let q = set_off.len() - 1;
+        let mut out = vec![0u8; q * each];
+        let mut status = vec![0u8; q];
+        let mut bad = vec![-1i64; q];
+        let rc = unsafe {
+            sys::blsgpu_sum_points_batch(self.ctx, group, 1, q, set_off.as_ptr(), bytes.as_ptr(), out.as_mut_ptr(), status.as_mut_ptr(),
+                bad.as_mut_ptr())
+        };
+        self.check(rc)?;
+        Ok((0..q)
+            .map(|j| {
+                status_to_result(status[j], Some((bad[j], -1)))?;
+                unpack_point::<P>(&out[j * each..(j + 1) * each])
+                    .ok_or_else(|| BlsError::DeserializationError("engine returned an invalid point".into()))
+            })
+            .collect())
+    }
+
+    /// `MultiPublicKey::from_public_keys(key_sets[j])` for every j, in one engine call.
+    pub fn multi_public_keys_from<C: GpuImpl>(&mut self, key_sets: &[&[PublicKey<C>]]) -> EngineResult<Vec<BlsResult<MultiPublicKey<C>>>> {
+        let set_off = set_offsets(key_sets.iter().map(|s| s.len()));
+        let bytes = pack_points(key_sets.iter().flat_map(|s| s.iter().map(|p| p.0)), C::PK_BYTES);
+        Ok(self.sum_points_batch::<<C as Pairing>::PublicKey>(C::PK_GROUP, &set_off, &bytes, C::PK_BYTES)?
+            .into_iter()
+            .map(|r| r.map(MultiPublicKey))
+            .collect())
+    }
+
+    /// `MultiSignature::from_signatures(sig_sets[j])` for every j, in one engine call; each set keeps
+    /// [`Engine::multi_signature_from`]'s rules (at least two signatures, one scheme, no MessageAugmentation after the first).
+    pub fn multi_signatures_from<C: GpuImpl>(&mut self, sig_sets: &[&[Signature<C>]]) -> EngineResult<Vec<BlsResult<MultiSignature<C>>>> {
+        let rule = |sigs: &[Signature<C>]| -> BlsResult<SignatureSchemes> {
+            if sigs.len() < 2 {
+                return Err(BlsError::InvalidSignature);
+            }
+            let scheme = signature_scheme(&sigs[0]);
+            if sigs[1..].iter().any(|s| signature_scheme(s) != scheme || matches!(s, Signature::MessageAugmentation(_))) {
+                return Err(BlsError::InvalidSignatureScheme);
+            }
+            Ok(scheme)
+        };
+        let decided: Vec<BlsResult<SignatureSchemes>> = sig_sets.iter().map(|s| rule(*s)).collect();
+        // a set the rules refuse is sent empty and reported here
+        let set_off = set_offsets(sig_sets.iter().zip(&decided).map(|(s, d)| if d.is_ok() { s.len() } else { 0 }));
+        let bytes = pack_points(sig_sets.iter().zip(&decided).filter(|(_, d)| d.is_ok()).flat_map(|(s, _)| s.iter().map(|x| *x.as_raw_value())),
+            C::SIG_BYTES);
+        let sums = self.sum_points_batch::<<C as Pairing>::Signature>(C::SIG_GROUP, &set_off, &bytes, C::SIG_BYTES)?;
+        Ok(decided
+            .into_iter()
+            .zip(sums)
+            .map(|(d, s)| {
+                let (scheme, p) = (d?, s?);
+                Ok(match scheme {
+                    SignatureSchemes::Basic => MultiSignature::Basic(p),
+                    SignatureSchemes::MessageAugmentation => MultiSignature::MessageAugmentation(p),
+                    SignatureSchemes::ProofOfPossession => MultiSignature::ProofOfPossession(p),
+                })
+            })
+            .collect())
+    }
+
+    // ---------------------------------------------------------------------------------------------------------
+    // multi-signatures over signer subsets: q (MultiSignature, signer set, message) per call
+    // ---------------------------------------------------------------------------------------------------------
+
+    /// `sigs[j].verify(&MultiPublicKey::from_public_keys(key_sets[j]), msgs[j])` for every j, in input order
+    /// (`src/multi_signature.rs:127-135`).  One engine call per signature scheme present; the key sums are formed on the
+    /// device.  `format` is the encoding the points cross the bus in.
+    pub fn multi_signature_verify_batch_with_mode<C: GpuImpl, B: AsRef<[u8]>>(
+        &mut self,
+        sigs: &[MultiSignature<C>],
+        key_sets: &[&[PublicKey<C>]],
+        msgs: &[B],
+        format: SerializationFormat,
+    ) -> EngineResult<Vec<BlsResult<()>>> {
+        if key_sets.len() != sigs.len() || msgs.len() != sigs.len() {
+            return Err(EngineError { code: sys::BLSGPU_E_ARG, message: "multi_signature_verify_batch: slice lengths differ".into() });
+        }
+        self.multisig_by_scheme(sigs, format, |eng, idx, scheme, sig_bytes, packed, status| {
+            let sets: Vec<&[PublicKey<C>]> = idx.iter().map(|&j| key_sets[j]).collect();
+            let (key_off, pk_bytes) = eng.pack_key_sets::<C>(&sets, format)?;
+            let rc = unsafe {
+                sys::blsgpu_verify_multisig_batch(eng.ctx, C::IMPL_ID, scheme_id(scheme), format_id(format), idx.len(), key_off.as_ptr(),
+                    pk_bytes.as_ptr(), sig_bytes.as_ptr(), packed.bytes.as_ptr(), packed.offsets.as_ptr(), status.as_mut_ptr())
+            };
+            eng.check(rc)
+        }, msgs)
+    }
+
+    /// [`Engine::multi_signature_verify_batch_with_mode`] with set j's keys = the keys of `keys` at `key_idx_sets[j]`.  An
+    /// index at or past the end of the set is an `EngineError` (`BLSGPU_E_ARG`), as is a set of another engine.
+    pub fn multi_signature_verify_batch_keyed_with_mode<C: GpuImpl, B: AsRef<[u8]>>(
+        &mut self,
+        keys: &KeySet<C>,
+        key_idx_sets: &[&[u32]],
+        sigs: &[MultiSignature<C>],
+        msgs: &[B],
+        format: SerializationFormat,
+    ) -> EngineResult<Vec<BlsResult<()>>> {
+        if key_idx_sets.len() != sigs.len() || msgs.len() != sigs.len() {
+            return Err(EngineError { code: sys::BLSGPU_E_ARG, message: "multi_signature_verify_batch_keyed: slice lengths differ".into() });
+        }
+        self.multisig_by_scheme(sigs, format, |eng, idx, scheme, sig_bytes, packed, status| {
+            let sets: Vec<&[u32]> = idx.iter().map(|&j| key_idx_sets[j]).collect();
+            let (key_off, key_idx) = pack_index_sets(&sets);
+            let rc = unsafe {
+                sys::blsgpu_verify_multisig_batch_keyed(eng.ctx, keys.id, scheme_id(scheme), format_id(format), idx.len(), key_off.as_ptr(),
+                    key_idx.as_ptr(), sig_bytes.as_ptr(), packed.bytes.as_ptr(), packed.offsets.as_ptr(), status.as_mut_ptr())
+            };
+            eng.check(rc)
+        }, msgs)
+    }
+
+    // the multi-signatures of each scheme present (input positions idx), their signatures in `format` and messages, through
+    // call(engine, idx, scheme, signature bytes, messages, statuses); the results in input order
+    fn multisig_by_scheme<C: GpuImpl, B: AsRef<[u8]>>(
+        &mut self,
+        sigs: &[MultiSignature<C>],
+        format: SerializationFormat,
+        call: impl Fn(&mut Self, &[usize], SignatureSchemes, &[u8], &PackedMessages, &mut [u8]) -> EngineResult<()>,
+        msgs: &[B],
+    ) -> EngineResult<Vec<BlsResult<()>>> {
+        let parts = |s: &MultiSignature<C>| match s {
+            MultiSignature::Basic(p) => (SignatureSchemes::Basic, *p),
+            MultiSignature::MessageAugmentation(p) => (SignatureSchemes::MessageAugmentation, *p),
+            MultiSignature::ProofOfPossession(p) => (SignatureSchemes::ProofOfPossession, *p),
+        };
+        let mut out: Vec<Option<BlsResult<()>>> = (0..sigs.len()).map(|_| None).collect();
+        for scheme in [SignatureSchemes::Basic, SignatureSchemes::MessageAugmentation, SignatureSchemes::ProofOfPossession] {
+            let idx: Vec<usize> = (0..sigs.len()).filter(|&j| parts(&sigs[j]).0 == scheme).collect();
+            if idx.is_empty() {
+                continue;
+            }
+            let sig_bytes = self.recode::<C>(C::SIG_GROUP, pack_points(idx.iter().map(|&j| parts(&sigs[j]).1), C::SIG_BYTES), C::SIG_BYTES, format)?;
+            let packed = PackedMessages::from_iter(idx.iter().map(|&j| msgs[j].as_ref()));
+            let mut status = vec![0u8; idx.len()];
+            call(self, &idx, scheme, &sig_bytes, &packed, &mut status)?;
+            for (k, &j) in idx.iter().enumerate() {
+                out[j] = Some(status_to_result(status[k], None));
+            }
+        }
+        Ok(out.into_iter().map(|r| r.expect("every scheme variant is covered")).collect())
     }
 
     // ---------------------------------------------------------------------------------------------------------

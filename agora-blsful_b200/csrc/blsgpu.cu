@@ -935,10 +935,10 @@ int decode_points(blsgpu_ctx* ctx, size_t n, const uint8_t* d_in, int format, A*
 // index of every item's key (`idx`) in a key set decoded once (`set`).  Host pointers until the call uploads them.
 struct Keys {
   const uint8_t* bytes = nullptr;
-  const KeySet* set = nullptr;
+  KeySet* set = nullptr;
   const uint32_t* idx = nullptr;
   Keys(const uint8_t* b = nullptr) : bytes(b) {}
-  Keys(const KeySet* s, const uint32_t* i) : set(s), idx(i) {}
+  Keys(KeySet* s, const uint32_t* i) : set(s), idx(i) {}
 };
 // the key step of a verify call, the one step where keyed and unkeyed calls differ: d_pk / d_st of the n items, by decoding
 // their bytes or by gathering them from the key set (no decode or subgroup check)
@@ -1101,21 +1101,6 @@ int ensure_verify_arena(blsgpu_ctx* ctx, size_t n, size_t head_bytes) {
   return ensure_pipeline_arena<typename ImplT<IMPL>::PkAff, typename ImplT<IMPL>::SigAff>(ctx, n, head_bytes + verify_head_bytes<IMPL>(n));
 }
 
-// host offset arrays: n + 1 non-decreasing entries, every record shorter than 2^32 bytes (the kernels keep lengths in 32 bits)
-bool offsets_ok(const uint64_t* off, size_t n) {
-  if (!off) return false;
-  for (size_t i = 0; i < n; i++)
-    if (off[i + 1] < off[i] || off[i + 1] - off[i] > 0xffffffffull) return false;
-  return true;
-}
-#define CHECK_OFFSETS(off, n, what)                                                                    \
-  do {                                                                                                 \
-    if (!offsets_ok((off), (n))) {                                                                     \
-      ctx->err = std::string(what) + ": offsets must be non-decreasing with records below 2^32 bytes"; \
-      return BLSGPU_E_ARG;                                                                             \
-    }                                                                                                  \
-  } while (0)
-
 bool args_ok(int impl_id, int scheme, int format) {
   return (impl_id == 1 || impl_id == 2) && scheme >= 0 && scheme <= 2 && (format == 0 || format == 1);
 }
@@ -1124,6 +1109,15 @@ template <class F>
 int with_impl(int impl_id, const F& f) {
   return impl_id == 2 ? f(std::integral_constant<int, 2>()) : f(std::integral_constant<int, 1>());
 }
+// f(PointType<A>) for group 1 (G1 points) or 2 (G2 points): the affine point type of the group
+template <class A>
+struct PointType {
+  typedef A type;
+};
+template <class F>
+int with_group(int group, const F& f) {
+  return group == 1 ? f(PointType<G1Aff>()) : f(PointType<G2Aff>());
+}
 
 // off[lo .. hi] rebased to off[lo]: the offsets of a run of records as the run's own
 std::vector<uint64_t> rebased(const uint64_t* off, size_t lo, size_t hi) {
@@ -1131,11 +1125,68 @@ std::vector<uint64_t> rebased(const uint64_t* off, size_t lo, size_t hi) {
   for (size_t i = lo; i <= hi; i++) r[i - lo] = off[i] - off[lo];
   return r;
 }
-// key_off of q key sets: non-decreasing, at most 2^32 - 16 keys in all
-bool key_offsets_ok(const uint64_t* key_off, size_t q) {
-  for (size_t j = 0; j < q; j++)
-    if (key_off[j + 1] < key_off[j] || key_off[q] > 0xfffffff0ull) return false;
-  return true;
+
+// ---- the argument rules of the entry points (include/blsgpu.h, "Arguments").  Each check returns a BLSGPU_* code and
+// names the entry point (`what`) in ctx->err.
+constexpr uint64_t MEMBERS_CAP = 0xfffffff0ull;  // items / members of a call that counts them in 32 bits (2^32 - 16)
+constexpr uint64_t NO_CAP = ~0ull;
+
+int arg_error(blsgpu_ctx* ctx, const char* what, const std::string& why) {
+  ctx->err = std::string(what) + ": " + why;
+  return BLSGPU_E_ARG;
+}
+// a buffer of `count` elements may be null only when it holds none
+int check_buffer(blsgpu_ctx* ctx, const char* what, const char* name, const void* buf, uint64_t count) {
+  return buf || count == 0 ? (int)BLSGPU_OK : arg_error(ctx, what, std::string(name) + " is null");
+}
+// n + 1 offsets: non-decreasing, every record below 2^32 (the kernels keep lengths and counts in 32 bits)
+int check_offsets(blsgpu_ctx* ctx, const char* what, const char* name, const uint64_t* off, size_t n) {
+  CKR(check_buffer(ctx, what, name, off, 1));
+  for (size_t i = 0; i < n; i++)
+    if (off[i + 1] < off[i] || off[i + 1] - off[i] > 0xffffffffull)
+      return arg_error(ctx, what, std::string(name) + ": offsets must be non-decreasing with records below 2^32");
+  return BLSGPU_OK;
+}
+// ragged records buf / off[0..n]: the offsets' rule, and buf non-null when the records span bytes
+int check_records(blsgpu_ctx* ctx, const char* what, const char* buf_name, const uint8_t* buf, const char* off_name, const uint64_t* off,
+                  size_t n) {
+  CKR(check_offsets(ctx, what, off_name, off, n));
+  return check_buffer(ctx, what, buf_name, buf, off[n] - off[0]);
+}
+// q sets of members (key_off, set_off, share_off, pair_off): the offsets' rule and at most `cap` members in all.
+// off0 = the offsets rebased to 0; the caller shifts its member buffers by off[0] members once.
+int check_sets(blsgpu_ctx* ctx, const char* what, const char* name, const uint64_t* off, size_t q, uint64_t cap, std::vector<uint64_t>& off0) {
+  CKR(check_buffer(ctx, what, name, off, 1));
+  off0.resize(q + 1);
+  off0[0] = 0;
+  for (size_t j = 0; j < q; j++) {
+    if (off[j + 1] < off[j] || off[j + 1] - off[j] > 0xffffffffull)
+      return arg_error(ctx, what, std::string(name) + ": offsets must be non-decreasing with sets below 2^32 members");
+    off0[j + 1] = off[j + 1] - off[0];
+  }
+  return off0[q] > cap ? arg_error(ctx, what, "at most 2^32 - 16 members per call") : (int)BLSGPU_OK;
+}
+// the key set `id` of this context (an id that was destroyed, never issued, or is another context's is refused)
+int find_keyset(blsgpu_ctx* ctx, const char* what, uint64_t id, KeySet*& set) {
+  const auto it = ctx->keysets.find(id);
+  if (it == ctx->keysets.end()) return arg_error(ctx, what, "key set " + std::to_string(id) + " is not held by this context");
+  set = &it->second;
+  return BLSGPU_OK;
+}
+// the keys of `count` members from member `first` on: the call's key bytes, or indices into a key set (at most 2^32 - 16,
+// each below the set's size).  keys comes back shifted to `first`.
+int check_keys(blsgpu_ctx* ctx, const char* what, int impl_id, Keys& keys, uint64_t first, uint64_t count) {
+  if (!keys.set) {
+    if (keys.bytes) keys.bytes += first * (impl_id == 2 ? 48 : 96);
+    return check_buffer(ctx, what, "pks", keys.bytes, count);
+  }
+  if (keys.idx) keys.idx += first;
+  CKR(check_buffer(ctx, what, "key_idx", keys.idx, count));
+  if (count > MEMBERS_CAP) return arg_error(ctx, what, "at most 2^32 - 16 members per call");
+  for (uint64_t i = 0; i < count; i++)
+    if (keys.idx[i] >= keys.set->n)
+      return arg_error(ctx, what, "key_idx[" + std::to_string(i) + "] is not below the key set's size " + std::to_string(keys.set->n));
+  return BLSGPU_OK;
 }
 
 template <class T>
@@ -1144,6 +1195,14 @@ int upload(blsgpu_ctx* ctx, T*& d, const T* h, size_t count) {
   ARENA_OK();
   if (count) CK(cudaMemcpyAsync(d, h, count * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
   return BLSGPU_OK;
+}
+// checked ragged records on the device as records from byte 0: the bytes off[0] .. off[n] and the offsets rebased to 0 (the
+// caller's offsets go up as they are when they start at 0: no host copy)
+int upload_records(blsgpu_ctx* ctx, const uint8_t* buf, const uint64_t* off, size_t n, uint8_t*& d_buf, uint64_t*& d_off) {
+  CKR(upload(ctx, d_buf, off[n] > off[0] ? buf + off[0] : buf, (size_t)(off[n] - off[0])));
+  if (off[0] == 0) return upload(ctx, d_off, off, n + 1);
+  const std::vector<uint64_t> r = rebased(off, 0, n);
+  return upload(ctx, d_off, r.data(), n + 1);
 }
 // the keys of a call on the device: its compressed key bytes, or its key indices, uploaded to the arena
 template <class PkA>
@@ -1321,10 +1380,7 @@ int blsgpu_verify_batch_dev(blsgpu_ctx* ctx, int impl_id, int scheme, int format
                             const uint8_t* sigs_dev, const uint8_t* msgs_dev, const uint64_t* msg_off_dev, uint8_t* status_out_dev) {
   NVTX_RANGE("blsgpu_verify_batch_dev");
   if (!ctx) return BLSGPU_E_ARG;
-  if (!args_ok(impl_id, scheme, format) || (n && (!pks_dev || !sigs_dev || !msg_off_dev || !status_out_dev))) {
-    ctx->err = "blsgpu_verify_batch_dev: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if (!args_ok(impl_id, scheme, format) || (n && (!pks_dev || !sigs_dev || !msg_off_dev || !status_out_dev))) return arg_error(ctx, __func__, "bad arguments");
   if (n == 0) return BLSGPU_OK;
   CKR(set_device(ctx));
   DstParam dst;
@@ -1351,14 +1407,8 @@ int host_partials(blsgpu_ctx* ctx, Pipe<typename ImplT<IMPL>::PkAff, typename Im
   Keys d_keys;
   CKR(upload_keys<typename ImplT<IMPL>::PkAff>(ctx, n, keys, d_keys));
   CKR(upload(ctx, d_sigs, sigs, n * sig_len));
-  CKR(upload(ctx, d_msgs, msg_off ? msgs + msg_off[0] : msgs, msg_bytes));
-  if (msg_off && msg_off[0] == 0) {
-    CKR(upload(ctx, d_off, msg_off, n + 1));  // the usual case: the caller's offsets go up as they are (no 8n-byte host copy)
-  } else {
-    // rebased to the slice's first message (all zero without messages: PoP)
-    const std::vector<uint64_t> off = msg_off ? rebased(msg_off, 0, n) : std::vector<uint64_t>(n + 1, 0);
-    CKR(upload(ctx, d_off, off.data(), n + 1));
-  }
+  const std::vector<uint64_t> no_msgs(msg_off ? 0 : n + 1, 0);  // PoP: every message empty
+  CKR(upload_records(ctx, msgs, msg_off ? msg_off : no_msgs.data(), n, d_msgs, d_off));
   uint8_t* d_st = ctx->arena.take<uint8_t>(n);
   *d_st_out = d_st;
   CKR((verify_dev_partials<IMPL>(ctx, P, msg_mode, dst, format, n, d_keys, d_sigs, d_msgs, d_off, d_st)));
@@ -1474,6 +1524,20 @@ int verify_host_common(blsgpu_ctx* ctx, int impl_id, int msg_mode, const DstPara
   });
 }
 
+// blsgpu_verify_batch and its keyed form (which stays on the first device)
+int verify_batch_common(blsgpu_ctx* ctx, const char* what, int impl_id, int scheme, int format, size_t n, Keys keys, const uint8_t* sigs,
+                        const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
+  if (!args_ok(impl_id, scheme, format) || (n && (!sigs || !status_out))) return arg_error(ctx, what, "bad arguments");
+  if (n == 0) return BLSGPU_OK;
+  CKR(check_keys(ctx, what, impl_id, keys, 0, n));
+  CKR(check_records(ctx, what, "msgs", msgs, "msg_off", msg_off, n));
+  DstParam dst;
+  make_dst(dst, impl_id, scheme, false);
+  const int mode = scheme == 1 ? 1 : 0;
+  if (!keys.set) return verify_host_common(ctx, impl_id, mode, dst, format, n, keys.bytes, sigs, msgs, msg_off, status_out);
+  return with_impl(impl_id, [&](auto I) { return verify_host_one<I>(ctx, mode, dst, format, n, keys, sigs, msgs, msg_off, status_out); });
+}
+
 template <int IMPL>
 struct PendingImpl : PendingSlice {
   Pipe<typename ImplT<IMPL>::PkAff, typename ImplT<IMPL>::SigAff> P;
@@ -1503,7 +1567,7 @@ int miller_partial_impl(blsgpu_ctx* ctx, int msg_mode, const DstParam& dst, int 
   return BLSGPU_OK;
 }
 template <int IMPL>
-int fold_bytes_impl(blsgpu_ctx* ctx, size_t k, const uint8_t* gts, const uint8_t* sums, int* ok_out) {
+int fold_bytes_impl(blsgpu_ctx* ctx, const char* what, size_t k, const uint8_t* gts, const uint8_t* sums, int* ok_out) {
   typedef typename ImplT<IMPL>::PkAff PkA;
   typedef typename ImplT<IMPL>::SigAff SigA;
   typedef typename PtInfo<SigA>::Jac SigJ;
@@ -1530,10 +1594,7 @@ int fold_bytes_impl(blsgpu_ctx* ctx, size_t k, const uint8_t* gts, const uint8_t
   CK(cudaMemcpyAsync(flag.data(), d_flag, 2 * k, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   for (uint8_t f : flag)
-    if (f) {
-      ctx->err = "blsgpu_final_exp_is_one: a partial result is not a canonical field element / group element";
-      return BLSGPU_E_ARG;
-    }
+    if (f) return arg_error(ctx, what, "a partial result is not a canonical field element / group element");
   bool ok = false;
   CKR((fold_check<PkA, SigA>(ctx, A, k, d_Fk, d_Sk, &ok)));
   *ok_out = ok ? 1 : 0;
@@ -1545,10 +1606,7 @@ int blsgpu_miller_partial(blsgpu_ctx* ctx, int impl_id, int scheme, int format, 
                           const uint8_t* msgs, const uint64_t* msg_off, uint8_t gt_out[576], uint8_t* sum_out) {
   NVTX_RANGE("blsgpu_miller_partial");
   if (!ctx) return BLSGPU_E_ARG;
-  if (!args_ok(impl_id, scheme, format) || !gt_out || !sum_out || (n && (!pks || !sigs || !msg_off))) {
-    ctx->err = "blsgpu_miller_partial: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if (!args_ok(impl_id, scheme, format) || !gt_out || !sum_out || (n && (!pks || !sigs))) return arg_error(ctx, __func__, "bad arguments");
   const size_t Ls = impl_id == 2 ? 96 : 48;
   if (n == 0) {  // the empty slice: (1, O)
     ctx->pending.reset();
@@ -1558,7 +1616,7 @@ int blsgpu_miller_partial(blsgpu_ctx* ctx, int impl_id, int scheme, int format, 
     sum_out[0] = 0xc0;
     return BLSGPU_OK;
   }
-  CHECK_OFFSETS(msg_off, n, "blsgpu_miller_partial");
+  CKR(check_records(ctx, __func__, "msgs", msgs, "msg_off", msg_off, n));
   DstParam dst;
   make_dst(dst, impl_id, scheme, false);
   const int mode = scheme == 1 ? 1 : 0;
@@ -1568,22 +1626,17 @@ int blsgpu_miller_partial(blsgpu_ctx* ctx, int impl_id, int scheme, int format, 
 int blsgpu_final_exp_is_one(blsgpu_ctx* ctx, int impl_id, size_t k, const uint8_t* partial_gts, const uint8_t* partial_sums, int* is_one_out) {
   NVTX_RANGE("blsgpu_final_exp_is_one");
   if (!ctx) return BLSGPU_E_ARG;
-  if ((impl_id != 1 && impl_id != 2) || k == 0 || k > 16 || !partial_gts || !partial_sums || !is_one_out) {
-    ctx->err = "blsgpu_final_exp_is_one: bad arguments (1 to 16 partial results)";
-    return BLSGPU_E_ARG;
-  }
+  if ((impl_id != 1 && impl_id != 2) || k == 0 || k > 16 || !partial_gts || !partial_sums || !is_one_out)
+    return arg_error(ctx, __func__, "bad arguments (1 to 16 partial results)");
   CKR(set_device(ctx));
-  return with_impl(impl_id, [&](auto I) { return fold_bytes_impl<I>(ctx, k, partial_gts, partial_sums, is_one_out); });
+  return with_impl(impl_id, [&](auto I) { return fold_bytes_impl<I>(ctx, __func__, k, partial_gts, partial_sums, is_one_out); });
 }
 
 int blsgpu_partial_finish(blsgpu_ctx* ctx, int batch_ok, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_partial_finish");
   if (!ctx) return BLSGPU_E_ARG;
   if (!ctx->pending) return BLSGPU_OK;  // an empty slice, or nothing pending
-  if (!status_out) {
-    ctx->err = "blsgpu_partial_finish: status_out is null";
-    return BLSGPU_E_ARG;
-  }
+  if (!status_out) return arg_error(ctx, __func__, "status_out is null");
   std::unique_ptr<PendingSlice> p = std::move(ctx->pending);
   return p->finish(ctx, batch_ok != 0, status_out);
 }
@@ -1592,29 +1645,14 @@ int blsgpu_verify_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int format, si
                         const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_verify_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  if (!args_ok(impl_id, scheme, format) || (n && (!pks || !sigs || !msg_off || !status_out))) {
-    ctx->err = "blsgpu_verify_batch: bad arguments";
-    return BLSGPU_E_ARG;
-  }
-  if (n == 0) return BLSGPU_OK;
-  CHECK_OFFSETS(msg_off, n, "blsgpu_verify_batch");
-  if (msg_off[n] > msg_off[0] && !msgs) {
-    ctx->err = "blsgpu_verify_batch: msgs is null";
-    return BLSGPU_E_ARG;
-  }
-  DstParam dst;
-  make_dst(dst, impl_id, scheme, false);
-  return verify_host_common(ctx, impl_id, scheme == 1 ? 1 : 0, dst, format, n, pks, sigs, msgs, msg_off, status_out);
+  return verify_batch_common(ctx, __func__, impl_id, scheme, format, n, pks, sigs, msgs, msg_off, status_out);
 }
 
 int blsgpu_pop_verify_batch(blsgpu_ctx* ctx, int impl_id, int format, size_t n, const uint8_t* pks, const uint8_t* sigs,
                             uint8_t* status_out) {
   NVTX_RANGE("blsgpu_pop_verify_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  if (!args_ok(impl_id, 2, format) || (n && (!pks || !sigs || !status_out))) {
-    ctx->err = "blsgpu_pop_verify_batch: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if (!args_ok(impl_id, 2, format) || (n && (!pks || !sigs || !status_out))) return arg_error(ctx, __func__, "bad arguments");
   if (n == 0) return BLSGPU_OK;
   DstParam dst;
   make_dst(dst, impl_id, 2, true);
@@ -1639,7 +1677,6 @@ struct AggSlice {
 };
 // (1) st_out[n] and inf_out[n] get the slice's decode statuses and identity flags; with `sig` also st_out[n] / inf_out[n]
 // (the signature's); without it the slice's signature slot holds the identity (it adds nothing to the fold).
-// msg_off is the slice's own (starting at 0).
 template <int IMPL>
 static int agg_decode(blsgpu_ctx* ctx, AggSlice<IMPL>& S, int format, size_t n, const uint8_t* pks, const uint8_t* msgs, const uint64_t* msg_off,
                       const uint8_t* sig, uint8_t* st_out, uint32_t* inf_out) {
@@ -1647,14 +1684,13 @@ static int agg_decode(blsgpu_ctx* ctx, AggSlice<IMPL>& S, int format, size_t n, 
   typedef typename ImplT<IMPL>::SigAff SigA;
   const size_t pk_len = PtInfo<PkA>::LEN, sig_len = PtInfo<SigA>::LEN;
   S.n = n;
-  size_t msg_bytes = (size_t)msg_off[n];
+  size_t msg_bytes = (size_t)(msg_off[n] - msg_off[0]);
   size_t head = n * (pk_len + sizeof(PkA) + sizeof(SigA) + 2) + msg_bytes + (n + 1) * 8 + sig_len + sizeof(SigA) + 16 * 256 +
                 std::max<size_t>(n, 1) * sizeof(typename PtInfo<SigA>::Jac);
   CKR((ensure_pipeline_arena<PkA, SigA>(ctx, std::max<size_t>(n, 1), head)));
   uint8_t *d_pks, *d_sigb;
   CKR(upload(ctx, d_pks, pks, n * pk_len));
-  CKR(upload(ctx, S.d_msgs, msgs, msg_bytes));
-  CKR(upload(ctx, S.d_off, msg_off, n + 1));
+  CKR(upload_records(ctx, msgs, msg_off, n, S.d_msgs, S.d_off));
   d_sigb = ctx->arena.take<uint8_t>(sig_len);
   S.d_pk = ctx->arena.take<PkA>(std::max<size_t>(n, 1));
   S.d_sig = ctx->arena.take<SigA>(1);
@@ -1767,15 +1803,13 @@ static int aggregate_verify_multi(blsgpu_ctx* ctx, int scheme, int format, size_
   std::vector<AggSlice<IMPL>> S(ndev);
   std::vector<uint8_t> st(n + 1);
   std::vector<uint32_t> inf(n + 1, 0);
-  std::vector<std::vector<uint64_t>> off(ndev);
   auto lo = [&](size_t d) { return n * d / ndev; };
   // the signature's status and identity flag come back at the END of slice 0's arrays: stage them, then move them to [n]
   std::vector<uint8_t> st0(lo(1) + 1);
   std::vector<uint32_t> inf0(lo(1) + 1, 0);
   CKR(run_on_devices(ctx, [&](blsgpu_ctx* c, size_t d) {
     const size_t s0 = lo(d), cnt = lo(d + 1) - s0;
-    off[d] = rebased(msg_off, s0, s0 + cnt);
-    return agg_decode<IMPL>(c, S[d], format, cnt, pks + s0 * pk_len, msgs + msg_off[s0], off[d].data(), d == 0 ? sig : nullptr,
+    return agg_decode<IMPL>(c, S[d], format, cnt, pks + s0 * pk_len, msgs, msg_off + s0, d == 0 ? sig : nullptr,
                             d == 0 ? st0.data() : st.data() + s0, d == 0 ? inf0.data() : inf.data() + s0);
   }));
   std::copy(st0.begin(), st0.end() - 1, st.begin());
@@ -1806,11 +1840,8 @@ int blsgpu_aggregate_verify(blsgpu_ctx* ctx, int impl_id, int scheme, int format
   if (!ctx) return BLSGPU_E_ARG;
   int64_t dummy[2];
   if (!index_out) index_out = dummy;
-  if (!args_ok(impl_id, scheme, format) || !sig || !status_out || !msg_off || (n && !pks)) {
-    ctx->err = "blsgpu_aggregate_verify: bad arguments";
-    return BLSGPU_E_ARG;
-  }
-  CHECK_OFFSETS(msg_off, n, "blsgpu_aggregate_verify");
+  if (!args_ok(impl_id, scheme, format) || !sig || !status_out || (n && !pks)) return arg_error(ctx, __func__, "bad arguments");
+  CKR(check_records(ctx, __func__, "msgs", msgs, "msg_off", msg_off, n));
   CKR(set_device(ctx));
   const bool multi = !ctx->peers.empty() && n >= (1 + ctx->peers.size()) * SHARD_MIN_ITEMS;
   return with_impl(impl_id, [&](auto I) {
@@ -1981,22 +2012,16 @@ int blsgpu_aggregate_verify_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int 
                                   const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* sigs, uint8_t* status_out, int64_t* index_out) {
   NVTX_RANGE("blsgpu_aggregate_verify_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  if (!args_ok(impl_id, scheme, format) || (q && (!set_off || !msg_off || !sigs || !status_out))) {
-    ctx->err = "blsgpu_aggregate_verify_batch: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if (!args_ok(impl_id, scheme, format) || (q && (!sigs || !status_out))) return arg_error(ctx, __func__, "bad arguments");
   if (q == 0) return BLSGPU_OK;
-  CHECK_OFFSETS(set_off, q, "blsgpu_aggregate_verify_batch (set_off)");
-  const size_t p0 = (size_t)set_off[0], np = (size_t)set_off[q] - p0;
-  if (np > 0xfffffff0ull) {
-    ctx->err = "blsgpu_aggregate_verify_batch: at most 2^32 - 16 pairs per call";
-    return BLSGPU_E_ARG;
-  }
-  CHECK_OFFSETS(msg_off + p0, np, "blsgpu_aggregate_verify_batch (msg_off)");
-  if ((np && !pks) || (msg_off[p0 + np] > msg_off[p0] && !msgs)) {
-    ctx->err = "blsgpu_aggregate_verify_batch: pks or msgs is null";
-    return BLSGPU_E_ARG;
-  }
+  std::vector<uint64_t> so;
+  CKR(check_sets(ctx, __func__, "set_off", set_off, q, MEMBERS_CAP, so));
+  const size_t np = (size_t)so[q];
+  Keys keys(pks);
+  CKR(check_keys(ctx, __func__, impl_id, keys, set_off[0], np));
+  CKR(check_buffer(ctx, __func__, "msg_off", msg_off, 1));
+  msg_off += set_off[0];  // one message per pair
+  CKR(check_records(ctx, __func__, "msgs", msgs, "msg_off", msg_off, np));
   CKR(set_device(ctx));
   std::vector<int64_t> idx_scratch;
   if (!index_out) {
@@ -2006,18 +2031,18 @@ int blsgpu_aggregate_verify_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int 
   const size_t pk_len = impl_id == 2 ? 48 : 96, sig_len = impl_id == 2 ? 96 : 48;
   // aggregates lo .. hi-1 on context c, with their pair and message offsets rebased to 0
   auto run = [&](blsgpu_ctx* c, size_t lo, size_t hi) -> int {
-    const size_t a = (size_t)set_off[lo], b = (size_t)set_off[hi];
-    const std::vector<uint64_t> so = rebased(set_off, lo, hi), mo = rebased(msg_off, a, b);
-    const uint8_t* pk = pks ? pks + a * pk_len : nullptr;
+    const size_t a = (size_t)so[lo], b = (size_t)so[hi];
+    const std::vector<uint64_t> s = rebased(so.data(), lo, hi), mo = rebased(msg_off, a, b);
+    const uint8_t* pk = keys.bytes ? keys.bytes + a * pk_len : nullptr;
     const uint8_t* ms = msgs ? msgs + msg_off[a] : nullptr;
     return with_impl(impl_id, [&](auto I) {
-      return aggregate_batch_impl<I>(c, scheme, format, hi - lo, so.data(), pk, ms, mo.data(), sigs + lo * sig_len, status_out + lo, index_out + 2 * lo);
+      return aggregate_batch_impl<I>(c, scheme, format, hi - lo, s.data(), pk, ms, mo.data(), sigs + lo * sig_len, status_out + lo, index_out + 2 * lo);
     });
   };
   const size_t ndev = 1 + ctx->peers.size();
   if (ndev == 1 || np < ndev * SHARD_MIN_ITEMS) return run(ctx, 0, q);
   // aggregates are independent: contiguous runs per device, balanced by pair count, nothing to fold
-  return run_cut(ctx, q, set_off, run);
+  return run_cut(ctx, q, so.data(), run);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -2303,48 +2328,17 @@ int verify_grouped_impl(blsgpu_ctx* ctx, int scheme, int format, size_t n, const
   return BLSGPU_OK;
 }
 
-// the key set `id` of this context, or nullptr with the error set (an id that was destroyed, never issued, or is another context's)
-KeySet* find_keyset(blsgpu_ctx* ctx, uint64_t id, const char* what) {
-  const auto it = ctx->keysets.find(id);
-  if (it != ctx->keysets.end()) return &it->second;
-  ctx->err = std::string(what) + ": key set " + std::to_string(id) + " is not held by this context";
-  return nullptr;
-}
-// keyed calls: every item names a key of the set
-bool key_idx_ok(blsgpu_ctx* ctx, const char* what, const Keys& keys, size_t n) {
-  if (!keys.set) return true;
-  for (size_t i = 0; i < n; i++)
-    if (keys.idx[i] >= keys.set->n) {
-      ctx->err = std::string(what) + ": key_idx[" + std::to_string(i) + "] is not below the key set's size " + std::to_string(keys.set->n);
-      return false;
-    }
-  return true;
-}
-
 // blsgpu_verify_batch_grouped and its keyed form: the argument checks, then the grouped pipeline, or for MessageAugmentation
 // blsgpu_verify_batch's pipeline on per-item messages
-int verify_grouped_common(blsgpu_ctx* ctx, const char* what, int impl_id, int scheme, int format, size_t n, const Keys& keys, const uint8_t* sigs,
+int verify_grouped_common(blsgpu_ctx* ctx, const char* what, int impl_id, int scheme, int format, size_t n, Keys keys, const uint8_t* sigs,
                           const uint32_t* msg_idx, size_t q, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
-  if (!args_ok(impl_id, scheme, format) || (n && (!(keys.set ? (const void*)keys.idx : (const void*)keys.bytes) || !sigs || !msg_idx || !msg_off || !status_out))) {
-    ctx->err = std::string(what) + ": bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if (!args_ok(impl_id, scheme, format) || (n && (!sigs || !msg_idx || !status_out))) return arg_error(ctx, what, "bad arguments");
   if (n == 0) return BLSGPU_OK;
-  if (n > 0xfffffff0ull) {
-    ctx->err = std::string(what) + ": at most 2^32 - 16 items per call";
-    return BLSGPU_E_ARG;
-  }
-  CHECK_OFFSETS(msg_off, q, what);
-  if (msg_off[q] > msg_off[0] && !msgs) {
-    ctx->err = std::string(what) + ": msgs is null";
-    return BLSGPU_E_ARG;
-  }
+  if (n > MEMBERS_CAP) return arg_error(ctx, what, "at most 2^32 - 16 items per call");
+  CKR(check_keys(ctx, what, impl_id, keys, 0, n));
+  CKR(check_records(ctx, what, "msgs", msgs, "msg_off", msg_off, q));
   for (size_t i = 0; i < n; i++)
-    if (msg_idx[i] >= q) {
-      ctx->err = std::string(what) + ": msg_idx[" + std::to_string(i) + "] is not below q";
-      return BLSGPU_E_ARG;
-    }
-  if (!key_idx_ok(ctx, what, keys, n)) return BLSGPU_E_ARG;
+    if (msg_idx[i] >= q) return arg_error(ctx, what, "msg_idx[" + std::to_string(i) + "] is not below q");
   CKR(set_device(ctx));
   if (scheme == 1) {
     // MessageAugmentation hashes pk || msg: no two items share a hash.  Per-item messages through blsgpu_verify_batch's pipeline.
@@ -2398,21 +2392,16 @@ int blsgpu_verify_batch_grouped(blsgpu_ctx* ctx, int impl_id, int scheme, int fo
                                 const uint32_t* msg_idx, size_t q, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_verify_batch_grouped");
   if (!ctx) return BLSGPU_E_ARG;
-  return verify_grouped_common(ctx, "blsgpu_verify_batch_grouped", impl_id, scheme, format, n, pks, sigs, msg_idx, q, msgs, msg_off, status_out);
+  return verify_grouped_common(ctx, __func__, impl_id, scheme, format, n, pks, sigs, msg_idx, q, msgs, msg_off, status_out);
 }
 
 // ---- key sets -----------------------------------------------------------------------------------------------------------
 int blsgpu_keyset_create(blsgpu_ctx* ctx, int impl_id, int format, size_t n, const uint8_t* pks, uint8_t* status_out, uint64_t* keyset_out) {
   NVTX_RANGE("blsgpu_keyset_create");
   if (!ctx) return BLSGPU_E_ARG;
-  if ((impl_id != 1 && impl_id != 2) || (format != 0 && format != 1) || !keyset_out || (n && !pks)) {
-    ctx->err = "blsgpu_keyset_create: bad arguments";
-    return BLSGPU_E_ARG;
-  }
-  if (n > 0xfffffff0ull) {
-    ctx->err = "blsgpu_keyset_create: at most 2^32 - 16 keys per set";
-    return BLSGPU_E_ARG;
-  }
+  if ((impl_id != 1 && impl_id != 2) || (format != 0 && format != 1) || !keyset_out) return arg_error(ctx, __func__, "bad arguments");
+  CKR(check_buffer(ctx, __func__, "pks", pks, n));
+  if (n > MEMBERS_CAP) return arg_error(ctx, __func__, "at most 2^32 - 16 keys per set");
   CKR(set_device(ctx));
   CKR(ensure_arena(ctx, 0));  // takes nothing from the arena: ends a pending slice like any other call
   return with_impl(impl_id, [&](auto I) { return keyset_create_impl<typename ImplT<I>::PkAff>(ctx, impl_id, format, n, pks, status_out, keyset_out); });
@@ -2421,8 +2410,8 @@ int blsgpu_keyset_create(blsgpu_ctx* ctx, int impl_id, int format, size_t n, con
 int blsgpu_keyset_destroy(blsgpu_ctx* ctx, uint64_t keyset) {
   NVTX_RANGE("blsgpu_keyset_destroy");
   if (!ctx) return BLSGPU_E_ARG;
-  const KeySet* s = find_keyset(ctx, keyset, "blsgpu_keyset_destroy");
-  if (!s) return BLSGPU_E_ARG;
+  KeySet* s = nullptr;
+  CKR(find_keyset(ctx, __func__, keyset, s));
   ctx->pending.reset();
   CKR(set_device(ctx));
   const cudaError_t e = free_keyset(*s);
@@ -2435,38 +2424,18 @@ int blsgpu_verify_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int 
                               const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_verify_batch_keyed");
   if (!ctx) return BLSGPU_E_ARG;
-  const char* what = "blsgpu_verify_batch_keyed";
-  const KeySet* set = find_keyset(ctx, keyset, what);
-  if (!set) return BLSGPU_E_ARG;
-  if (!args_ok(set->impl_id, scheme, format) || (n && (!key_idx || !sigs || !msg_off || !status_out))) {
-    ctx->err = "blsgpu_verify_batch_keyed: bad arguments";
-    return BLSGPU_E_ARG;
-  }
-  if (n == 0) return BLSGPU_OK;
-  if (n > 0xfffffff0ull) {
-    ctx->err = "blsgpu_verify_batch_keyed: at most 2^32 - 16 items per call";
-    return BLSGPU_E_ARG;
-  }
-  CHECK_OFFSETS(msg_off, n, what);
-  if (msg_off[n] > msg_off[0] && !msgs) {
-    ctx->err = "blsgpu_verify_batch_keyed: msgs is null";
-    return BLSGPU_E_ARG;
-  }
-  const Keys keys(set, key_idx);
-  if (!key_idx_ok(ctx, what, keys, n)) return BLSGPU_E_ARG;
-  DstParam dst;
-  make_dst(dst, set->impl_id, scheme, false);
-  return with_impl(set->impl_id, [&](auto I) { return verify_host_one<I>(ctx, scheme == 1 ? 1 : 0, dst, format, n, keys, sigs, msgs, msg_off, status_out); });
+  KeySet* set = nullptr;
+  CKR(find_keyset(ctx, __func__, keyset, set));
+  return verify_batch_common(ctx, __func__, set->impl_id, scheme, format, n, Keys(set, key_idx), sigs, msgs, msg_off, status_out);
 }
 
 int blsgpu_verify_batch_grouped_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t n, const uint32_t* key_idx, const uint8_t* sigs,
                                       const uint32_t* msg_idx, size_t q, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_verify_batch_grouped_keyed");
   if (!ctx) return BLSGPU_E_ARG;
-  const char* what = "blsgpu_verify_batch_grouped_keyed";
-  const KeySet* set = find_keyset(ctx, keyset, what);
-  if (!set) return BLSGPU_E_ARG;
-  return verify_grouped_common(ctx, what, set->impl_id, scheme, format, n, Keys(set, key_idx), sigs, msg_idx, q, msgs, msg_off, status_out);
+  KeySet* set = nullptr;
+  CKR(find_keyset(ctx, __func__, keyset, set));
+  return verify_grouped_common(ctx, __func__, set->impl_id, scheme, format, n, Keys(set, key_idx), sigs, msg_idx, q, msgs, msg_off, status_out);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -2519,13 +2488,10 @@ int blsgpu_sum_points(blsgpu_ctx* ctx, int group, int format, size_t n, const ui
   if (!ctx) return BLSGPU_E_ARG;
   int64_t dummy;
   if (!bad_index_out) bad_index_out = &dummy;
-  if ((group != 1 && group != 2) || (format != 0 && format != 1) || !out || !status_out || (n && !points)) {
-    ctx->err = "blsgpu_sum_points: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if ((group != 1 && group != 2) || (format != 0 && format != 1) || !out || !status_out || (n && !points)) return arg_error(ctx, __func__, "bad arguments");
   CKR(set_device(ctx));
   auto one = [&](blsgpu_ctx* c, size_t cnt, const uint8_t* pts, uint8_t* o, uint8_t* st, int64_t* bad) {
-    return group == 1 ? sum_points_impl<G1Aff>(c, format, cnt, pts, o, st, bad) : sum_points_impl<G2Aff>(c, format, cnt, pts, o, st, bad);
+    return with_group(group, [&](auto G) { return sum_points_impl<typename decltype(G)::type>(c, format, cnt, pts, o, st, bad); });
   };
   const size_t ndev = 1 + ctx->peers.size(), L = group == 1 ? 48 : 96;
   if (ndev == 1 || n < SHARD_MIN_POINTS * ndev) return one(ctx, n, points, out, status_out, bad_index_out);
@@ -2553,8 +2519,7 @@ static int hash_batch_impl(blsgpu_ctx* ctx, size_t n, const uint8_t* msgs, const
   CKR(ensure_arena(ctx, msg_bytes + (n + 1) * 8 + n * (sizeof(A) + L + sizeof(typename PtInfo<A>::Jac)) + 8 * 256));
   uint8_t* d_msgs;
   uint64_t* d_off;
-  CKR(upload(ctx, d_msgs, msgs, msg_bytes));
-  CKR(upload(ctx, d_off, msg_off, n + 1));
+  CKR(upload_records(ctx, msgs, msg_off, n, d_msgs, d_off));
   A* d_h = ctx->arena.take<A>(n);
   uint8_t* d_out = ctx->arena.take<uint8_t>(n * L);
   CKR((hash_points<A, G1Aff>(ctx, n, (const uint8_t*)d_msgs, (const uint64_t*)d_off, 0, (const G1Aff*)nullptr, (const uint8_t*)nullptr,
@@ -2569,18 +2534,16 @@ int blsgpu_hash_to_curve_batch(blsgpu_ctx* ctx, int group, size_t n, const uint8
                                size_t dst_len, uint8_t* out) {
   NVTX_RANGE("blsgpu_hash_to_curve_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  if ((group != 1 && group != 2) || !msg_off || !dst || dst_len == 0 || dst_len > 63 || (n && !out)) {
-    ctx->err = "blsgpu_hash_to_curve_batch: bad arguments (dst_len must be 1..63)";
-    return BLSGPU_E_ARG;
-  }
+  if ((group != 1 && group != 2) || !dst || dst_len == 0 || dst_len > 63 || (n && !out))
+    return arg_error(ctx, __func__, "bad arguments (dst_len must be 1..63)");
+  CKR(check_records(ctx, __func__, "msgs", msgs, "msg_off", msg_off, n));
   if (n == 0) return BLSGPU_OK;
-  CHECK_OFFSETS(msg_off, n, "blsgpu_hash_to_curve_batch");
   CKR(set_device(ctx));
   DstParam d;
   memset(d.b, 0, sizeof d.b);
   memcpy(d.b, dst, dst_len);
   d.len = (uint32_t)dst_len;
-  return group == 1 ? hash_batch_impl<G1Aff>(ctx, n, msgs, msg_off, d, out) : hash_batch_impl<G2Aff>(ctx, n, msgs, msg_off, d, out);
+  return with_group(group, [&](auto G) { return hash_batch_impl<typename decltype(G)::type>(ctx, n, msgs, msg_off, d, out); });
 }
 
 template <class A>
@@ -2604,23 +2567,16 @@ int blsgpu_recode_points(blsgpu_ctx* ctx, int group, int format_in, int format_o
                          uint8_t* status_out) {
   NVTX_RANGE("blsgpu_recode_points");
   if (!ctx) return BLSGPU_E_ARG;
-  if ((group != 1 && group != 2) || (format_in | format_out) & ~1 || (n && (!in || !out || !status_out))) {
-    ctx->err = "blsgpu_recode_points: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if ((group != 1 && group != 2) || (format_in | format_out) & ~1 || (n && (!in || !out || !status_out))) return arg_error(ctx, __func__, "bad arguments");
   if (n == 0) return BLSGPU_OK;
   CKR(set_device(ctx));
-  return group == 1 ? recode_impl<G1Aff>(ctx, format_in, format_out, n, in, out, status_out)
-                    : recode_impl<G2Aff>(ctx, format_in, format_out, n, in, out, status_out);
+  return with_group(group, [&](auto G) { return recode_impl<typename decltype(G)::type>(ctx, format_in, format_out, n, in, out, status_out); });
 }
 
 int blsgpu_fp_mul_batch(blsgpu_ctx* ctx, int variant, size_t n, const uint8_t* a, const uint8_t* b, uint8_t* out) {
   NVTX_RANGE("blsgpu_fp_mul_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  if ((variant != 0 && variant != 1) || (n && (!a || !b || !out))) {
-    ctx->err = "blsgpu_fp_mul_batch: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if ((variant != 0 && variant != 1) || (n && (!a || !b || !out))) return arg_error(ctx, __func__, "bad arguments");
   if (n == 0) return BLSGPU_OK;
   CKR(set_device(ctx));
   CKR(ensure_arena(ctx, 3 * n * 48 + 4 * 256));
@@ -2637,10 +2593,7 @@ int blsgpu_fp_mul_batch(blsgpu_ctx* ctx, int variant, size_t n, const uint8_t* a
 int blsgpu_pairing_product_is_one(blsgpu_ctx* ctx, size_t n, const uint8_t* g1_points, const uint8_t* g2_points, int* is_one_out) {
   NVTX_RANGE("blsgpu_pairing_product_is_one");
   if (!ctx) return BLSGPU_E_ARG;
-  if (!is_one_out || (n && (!g1_points || !g2_points))) {
-    ctx->err = "blsgpu_pairing_product_is_one: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if (!is_one_out || (n && (!g1_points || !g2_points))) return arg_error(ctx, __func__, "bad arguments");
   if (n == 0) {
     *is_one_out = 1;
     return BLSGPU_OK;
@@ -2662,10 +2615,7 @@ int blsgpu_pairing_product_is_one(blsgpu_ctx* ctx, size_t n, const uint8_t* g1_p
   CK(cudaMemcpyAsync(st.data(), d_st, 2 * n, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   for (uint8_t s : st)
-    if (s != BLSGPU_ST_OK) {
-      ctx->err = "blsgpu_pairing_product_is_one: undecodable point";
-      return BLSGPU_E_ARG;
-    }
+    if (s != BLSGPU_ST_OK) return arg_error(ctx, __func__, "undecodable point");
   LAUNCH(k_miller_pairs, blocks_for(n), TPB, n, (const G1Aff*)d_p, (const G2Aff*)d_q, d_F);
   CKR(reduce_levels(ctx, lv, 0, d_F, (PtInfo<G1Aff>::Jac*)nullptr));
   LAUNCH(k_final_is_one, 1, 32, (const Fp12*)(d_F + lv.back().off), d_ok);
@@ -2681,12 +2631,9 @@ int blsgpu_testdata_sign(blsgpu_ctx* ctx, int impl_id, int scheme, size_t n, con
   NVTX_RANGE("blsgpu_testdata_sign");
   if (!ctx) return BLSGPU_E_ARG;
   const bool pop_proof = scheme == 3;  // proof of possession: message = the key's own bytes, BLS_POP_ DST
-  if (!args_ok(impl_id, pop_proof ? 2 : scheme, 1) || (n && (!scalars32 || !msg_off || !out_pks || !out_sigs))) {
-    ctx->err = "blsgpu_testdata_sign: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if (!args_ok(impl_id, pop_proof ? 2 : scheme, 1) || (n && (!scalars32 || !out_pks || !out_sigs))) return arg_error(ctx, __func__, "bad arguments");
   if (n == 0) return BLSGPU_OK;
-  CHECK_OFFSETS(msg_off, n, "blsgpu_testdata_sign");
+  CKR(check_records(ctx, __func__, "msgs", msgs, "msg_off", msg_off, n));
   CKR(set_device(ctx));
   size_t pk_len = impl_id == 2 ? 48 : 96, sig_len = impl_id == 2 ? 96 : 48;
   size_t msg_bytes = (size_t)msg_off[n];
@@ -2694,8 +2641,7 @@ int blsgpu_testdata_sign(blsgpu_ctx* ctx, int impl_id, int scheme, size_t n, con
   uint8_t *d_k, *d_m;
   uint64_t* d_off;
   CKR(upload(ctx, d_k, scalars32, n * 32));
-  CKR(upload(ctx, d_m, msgs, msg_bytes));
-  CKR(upload(ctx, d_off, msg_off, n + 1));
+  CKR(upload_records(ctx, msgs, msg_off, n, d_m, d_off));
   uint8_t* d_pk = ctx->arena.take<uint8_t>(n * pk_len);
   uint8_t* d_sig = ctx->arena.take<uint8_t>(n * sig_len);
   DstParam dst;
@@ -2936,7 +2882,7 @@ int verify_secure_impl(blsgpu_ctx* ctx, int scheme, int format, size_t q, const 
   typedef typename ImplT<IMPL>::SigAff SigA;
   typedef typename ImplT<IMPL>::PkJac PkJ;
   const size_t Lp = PtInfo<PkA>::LEN, Ls = PtInfo<SigA>::LEN;
-  const size_t M = (size_t)key_off[q], msg_bytes = (size_t)msg_off[q];
+  const size_t M = (size_t)key_off[q], msg_bytes = (size_t)(msg_off[q] - msg_off[0]);
   size_t head = M * (Lp + sizeof(PkA) + 2) + q * (Ls + 2 * sizeof(SigA) + sizeof(PkA) + sizeof(PkJ) + 8) + msg_bytes + (q + 1) * 8 +
                 secure_plan_bytes(ctx, q, M, sizeof(PkJ)) + 32 * 256;
   CKR(ensure_verify_arena<IMPL>(ctx, q, head));
@@ -2946,8 +2892,7 @@ int verify_secure_impl(blsgpu_ctx* ctx, int scheme, int format, size_t q, const 
   uint8_t *d_sigb, *d_msgs;
   uint64_t* d_moff;
   CKR(upload(ctx, d_sigb, sigs, q * Ls));
-  CKR(upload(ctx, d_msgs, msgs, msg_bytes));
-  CKR(upload(ctx, d_moff, msg_off, q + 1));
+  CKR(upload_records(ctx, msgs, msg_off, q, d_msgs, d_moff));
   SigA* d_sig = ctx->arena.take<SigA>(q);
   uint8_t* d_stsig = ctx->arena.take<uint8_t>(q);
   uint8_t* d_zero = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
@@ -3090,27 +3035,63 @@ int ensure_secure_view(blsgpu_ctx* ctx, KeySet& s, int format) {
   return BLSGPU_OK;
 }
 
-// the argument checks of both keyed secure calls (those of the unkeyed calls, on the set's impl, plus the set id and every
-// key index), then the set's secure view in `format`.  *ko: key_off rebased to 0, *idx: key_idx from the first member.
-int secure_keyed_args(blsgpu_ctx* ctx, const char* what, uint64_t keyset, int scheme, int format, size_t q, const uint64_t* key_off,
-                      const uint32_t* key_idx, bool args_present, KeySet** set_out, std::vector<uint64_t>* ko, const uint32_t** idx) {
-  KeySet* set = find_keyset(ctx, keyset, what);
-  if (!set) return BLSGPU_E_ARG;
-  if (!args_ok(set->impl_id, scheme, format) || (q && (!key_off || !args_present)) || (q && key_off[q] > key_off[0] && !key_idx) ||
-      (set->impl_id == 1 && format == 0)) {
-    ctx->err = std::string(what) + ": bad arguments (Legacy mode exists only for Bls12381G2Impl)";
-    return BLSGPU_E_ARG;
+// The secure calls and their keyed forms.  A keyed call runs on the first device over the set's secure view in `format`;
+// the unkeyed calls cut their quorums over the devices of the context (SURVEY 8e, cfg 5): contiguous runs, balanced by
+// member count.  f(device context, quorums, key_off from 0, keys of the first member, quorum offset) runs a set of quorums.
+template <int IMPL, class F>
+int secure_route(blsgpu_ctx* ctx, int format, size_t q, const std::vector<uint64_t>& ko, const Keys& keys, const F& f) {
+  if (keys.set) {
+    CKR((ensure_secure_view<typename ImplT<IMPL>::PkAff>(ctx, *keys.set, format)));
+    return f(ctx, q, ko.data(), keys, (size_t)0);
   }
+  const size_t ndev = 1 + ctx->peers.size();
+  if (ndev == 1 || q < 2 * ndev || ko[q] < SHARD_MIN_ITEMS * ndev) return f(ctx, q, ko.data(), keys, (size_t)0);
+  return run_cut(ctx, q, ko.data(), [&](blsgpu_ctx* c, size_t lo, size_t hi) {
+    const std::vector<uint64_t> run = rebased(ko.data(), lo, hi);
+    return f(c, hi - lo, run.data(), Keys(keys.bytes + ko[lo] * PtInfo<typename ImplT<IMPL>::PkAff>::LEN), lo);
+  });
+}
+
+// the argument rules the secure calls share: Legacy only for Bls12381G2Impl, key_off (at most 2^32 - 16 members), the keys.
+// ko: key_off from 0; keys: from the first member on.
+int check_secure(blsgpu_ctx* ctx, const char* what, int impl_id, int scheme, int format, size_t q, const uint64_t* key_off, Keys& keys,
+                 bool outputs, std::vector<uint64_t>& ko) {
+  if (!args_ok(impl_id, scheme, format) || (q && !outputs) || (impl_id == 1 && format == 0))
+    return arg_error(ctx, what, "bad arguments (Legacy mode exists only for Bls12381G2Impl)");
   if (q == 0) return BLSGPU_OK;
-  if (!key_offsets_ok(key_off, q)) {
-    ctx->err = std::string(what) + ": key_off must be non-decreasing and below 2^32";
-    return BLSGPU_E_ARG;
-  }
-  *ko = rebased(key_off, 0, q);
-  *idx = key_idx ? key_idx + key_off[0] : nullptr;
-  if (!key_idx_ok(ctx, what, Keys(set, *idx), (size_t)(*ko)[q])) return BLSGPU_E_ARG;
-  *set_out = set;
-  return BLSGPU_OK;
+  CKR(check_sets(ctx, what, "key_off", key_off, q, MEMBERS_CAP, ko));
+  return check_keys(ctx, what, impl_id, keys, key_off[0], ko[q]);
+}
+
+int verify_secure_common(blsgpu_ctx* ctx, const char* what, int impl_id, int scheme, int format, size_t q, const uint64_t* key_off, Keys keys,
+                         const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
+  std::vector<uint64_t> ko;
+  CKR(check_secure(ctx, what, impl_id, scheme, format, q, key_off, keys, sigs && status_out, ko));
+  if (q == 0) return BLSGPU_OK;
+  CKR(check_records(ctx, what, "msgs", msgs, "msg_off", msg_off, q));
+  CKR(set_device(ctx));
+  const size_t sig_len = impl_id == 2 ? 96 : 48;
+  return with_impl(impl_id, [&](auto I) {
+    return secure_route<I>(ctx, format, q, ko, keys, [&](blsgpu_ctx* c, size_t cnt, const uint64_t* k, const Keys& ks, size_t lo) {
+      return verify_secure_impl<I>(c, scheme, format, cnt, k, ks, sigs + lo * sig_len, msgs, msg_off + lo, status_out + lo);
+    });
+  });
+}
+
+int aggregate_secure_common(blsgpu_ctx* ctx, const char* what, int impl_id, int format, size_t q, const uint64_t* key_off, Keys keys,
+                            const uint8_t* member_sigs, uint8_t* out_sigs, uint8_t* status_out) {
+  std::vector<uint64_t> ko;
+  CKR(check_secure(ctx, what, impl_id, 0, format, q, key_off, keys, out_sigs && status_out, ko));
+  if (q == 0) return BLSGPU_OK;
+  const size_t sig_len = impl_id == 2 ? 96 : 48;
+  if (member_sigs) member_sigs += key_off[0] * sig_len;
+  CKR(check_buffer(ctx, what, "member_sigs", member_sigs, ko[q]));
+  CKR(set_device(ctx));
+  return with_impl(impl_id, [&](auto I) {
+    return secure_route<I>(ctx, format, q, ko, keys, [&](blsgpu_ctx* c, size_t cnt, const uint64_t* k, const Keys& ks, size_t lo) {
+      return aggregate_secure_impl<I>(c, format, cnt, k, ks, member_sigs + ko[lo] * sig_len, out_sigs + lo * sig_len, status_out + lo);
+    });
+  });
 }
 
 }  // namespace
@@ -3119,58 +3100,14 @@ int blsgpu_verify_secure_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int for
                                const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_verify_secure_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  if (!args_ok(impl_id, scheme, format) || (q && (!key_off || !sigs || !msg_off || !status_out)) || (q && key_off[q] && !pks) ||
-      (impl_id == 1 && format == 0)) {
-    ctx->err = "blsgpu_verify_secure_batch: bad arguments (Legacy mode exists only for Bls12381G2Impl)";
-    return BLSGPU_E_ARG;
-  }
-  if (q == 0) return BLSGPU_OK;
-  if (!key_offsets_ok(key_off, q)) {
-    ctx->err = "blsgpu_verify_secure_batch: key_off must be non-decreasing and below 2^32";
-    return BLSGPU_E_ARG;
-  }
-  CHECK_OFFSETS(msg_off, q, "blsgpu_verify_secure_batch");
-  CKR(set_device(ctx));
-  auto one = [&](blsgpu_ctx* c, size_t cnt, const uint64_t* ko, const uint8_t* pk, const uint8_t* sg, const uint8_t* ms, const uint64_t* mo,
-                 uint8_t* st) {
-    return with_impl(impl_id, [&](auto I) { return verify_secure_impl<I>(c, scheme, format, cnt, ko, pk, sg, ms, mo, st); });
-  };
-  const size_t ndev = 1 + ctx->peers.size();
-  if (ndev == 1 || q < 2 * ndev || key_off[q] - key_off[0] < SHARD_MIN_ITEMS * ndev) return one(ctx, q, key_off, pks, sigs, msgs, msg_off, status_out);
-  // quorums are independent (SURVEY 8e, cfg 5): contiguous runs of quorums per device, balanced by member count
-  const size_t pk_len = impl_id == 2 ? 48 : 96, sig_len = impl_id == 2 ? 96 : 48;
-  return run_cut(ctx, q, key_off, [&](blsgpu_ctx* c, size_t lo, size_t hi) {
-    const std::vector<uint64_t> ko = rebased(key_off, lo, hi), mo = rebased(msg_off, lo, hi);
-    return one(c, hi - lo, ko.data(), pks ? pks + key_off[lo] * pk_len : nullptr, sigs + lo * sig_len, msgs ? msgs + msg_off[lo] : nullptr,
-               mo.data(), status_out + lo);
-  });
+  return verify_secure_common(ctx, __func__, impl_id, scheme, format, q, key_off, pks, sigs, msgs, msg_off, status_out);
 }
 
 int blsgpu_aggregate_secure_batch(blsgpu_ctx* ctx, int impl_id, int format, size_t q, const uint64_t* key_off, const uint8_t* pks,
                                   const uint8_t* member_sigs, uint8_t* out_sigs, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_aggregate_secure_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  if (!args_ok(impl_id, 0, format) || (q && (!key_off || !out_sigs || !status_out)) || (q && key_off[q] && (!pks || !member_sigs)) ||
-      (impl_id == 1 && format == 0)) {
-    ctx->err = "blsgpu_aggregate_secure_batch: bad arguments (Legacy mode exists only for Bls12381G2Impl)";
-    return BLSGPU_E_ARG;
-  }
-  if (q == 0) return BLSGPU_OK;
-  if (!key_offsets_ok(key_off, q)) {
-    ctx->err = "blsgpu_aggregate_secure_batch: key_off must be non-decreasing and below 2^32";
-    return BLSGPU_E_ARG;
-  }
-  CKR(set_device(ctx));
-  auto one = [&](blsgpu_ctx* c, size_t cnt, const uint64_t* ko, const uint8_t* pk, const uint8_t* ms, uint8_t* o, uint8_t* st) {
-    return with_impl(impl_id, [&](auto I) { return aggregate_secure_impl<I>(c, format, cnt, ko, pk, ms, o, st); });
-  };
-  const size_t ndev = 1 + ctx->peers.size();
-  if (ndev == 1 || q < 2 * ndev || key_off[q] - key_off[0] < SHARD_MIN_ITEMS * ndev) return one(ctx, q, key_off, pks, member_sigs, out_sigs, status_out);
-  const size_t pk_len = impl_id == 2 ? 48 : 96, sig_len = impl_id == 2 ? 96 : 48;
-  return run_cut(ctx, q, key_off, [&](blsgpu_ctx* c, size_t lo, size_t hi) {
-    const std::vector<uint64_t> ko = rebased(key_off, lo, hi);
-    return one(c, hi - lo, ko.data(), pks + key_off[lo] * pk_len, member_sigs + key_off[lo] * sig_len, out_sigs + lo * sig_len, status_out + lo);
-  });
+  return aggregate_secure_common(ctx, __func__, impl_id, format, q, key_off, pks, member_sigs, out_sigs, status_out);
 }
 
 int blsgpu_verify_secure_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t q, const uint64_t* key_off,
@@ -3178,38 +3115,18 @@ int blsgpu_verify_secure_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int schem
                                      uint8_t* status_out) {
   NVTX_RANGE("blsgpu_verify_secure_batch_keyed");
   if (!ctx) return BLSGPU_E_ARG;
-  const char* what = "blsgpu_verify_secure_batch_keyed";
   KeySet* set = nullptr;
-  std::vector<uint64_t> ko;
-  const uint32_t* idx = nullptr;
-  CKR(secure_keyed_args(ctx, what, keyset, scheme, format, q, key_off, key_idx, sigs && msg_off && status_out, &set, &ko, &idx));
-  if (q == 0) return BLSGPU_OK;
-  CHECK_OFFSETS(msg_off, q, what);
-  CKR(set_device(ctx));
-  return with_impl(set->impl_id, [&](auto I) {
-    CKR((ensure_secure_view<typename ImplT<I>::PkAff>(ctx, *set, format)));
-    return verify_secure_impl<I>(ctx, scheme, format, q, ko.data(), Keys(set, idx), sigs, msgs, msg_off, status_out);
-  });
+  CKR(find_keyset(ctx, __func__, keyset, set));
+  return verify_secure_common(ctx, __func__, set->impl_id, scheme, format, q, key_off, Keys(set, key_idx), sigs, msgs, msg_off, status_out);
 }
 
 int blsgpu_aggregate_secure_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int format, size_t q, const uint64_t* key_off,
                                         const uint32_t* key_idx, const uint8_t* member_sigs, uint8_t* out_sigs, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_aggregate_secure_batch_keyed");
   if (!ctx) return BLSGPU_E_ARG;
-  const char* what = "blsgpu_aggregate_secure_batch_keyed";
   KeySet* set = nullptr;
-  std::vector<uint64_t> ko;
-  const uint32_t* idx = nullptr;
-  CKR(secure_keyed_args(ctx, what, keyset, 0, format, q, key_off, key_idx, out_sigs && status_out && (!key_off || key_off[q] == key_off[0] || member_sigs),
-                        &set, &ko, &idx));
-  if (q == 0) return BLSGPU_OK;
-  CKR(set_device(ctx));
-  return with_impl(set->impl_id, [&](auto I) {
-    CKR((ensure_secure_view<typename ImplT<I>::PkAff>(ctx, *set, format)));
-    const size_t Ls = PtInfo<typename ImplT<I>::SigAff>::LEN;
-    return aggregate_secure_impl<I>(ctx, format, q, ko.data(), Keys(set, idx), member_sigs ? member_sigs + key_off[0] * Ls : nullptr, out_sigs,
-                                    status_out);
-  });
+  CKR(find_keyset(ctx, __func__, keyset, set));
+  return aggregate_secure_common(ctx, __func__, set->impl_id, format, q, key_off, Keys(set, key_idx), member_sigs, out_sigs, status_out);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -3312,8 +3229,7 @@ int verify_multisig_impl(blsgpu_ctx* ctx, int scheme, int format, size_t q, cons
   uint8_t *d_sigb, *d_msgs;
   uint64_t* d_moff;
   CKR(upload(ctx, d_sigb, sigs, q * Ls));
-  CKR(upload(ctx, d_msgs, msgs, msg_bytes));
-  CKR(upload(ctx, d_moff, msg_off, q + 1));
+  CKR(upload_records(ctx, msgs, msg_off, q, d_msgs, d_moff));
   SigA* d_sig = ctx->arena.take<SigA>(q);
   uint8_t* d_stsig = ctx->arena.take<uint8_t>(q);
   uint8_t* d_status = ctx->arena.take<uint8_t>(q);
@@ -3366,29 +3282,16 @@ int sum_points_batch_impl(blsgpu_ctx* ctx, int format, size_t q, const uint64_t*
   return BLSGPU_OK;
 }
 
-// the argument checks of both multi-signature calls (the secure calls' rules; both formats for both impls, as
-// blsgpu_verify_batch), then the pipeline with key_off rebased to 0 and the keys from the first member on
+// both multi-signature calls (both formats for both impls, as blsgpu_verify_batch): the pipeline sees key_off from 0 and the
+// keys from the first member on
 int verify_multisig_common(blsgpu_ctx* ctx, const char* what, int impl_id, int scheme, int format, size_t q, const uint64_t* key_off, Keys keys,
                            const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
-  const void* members = keys.set ? (const void*)keys.idx : (const void*)keys.bytes;
-  if (!args_ok(impl_id, scheme, format) || (q && (!key_off || !sigs || !msg_off || !status_out)) || (q && key_off[q] > key_off[0] && !members)) {
-    ctx->err = std::string(what) + ": bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if (!args_ok(impl_id, scheme, format) || (q && (!sigs || !status_out))) return arg_error(ctx, what, "bad arguments");
   if (q == 0) return BLSGPU_OK;
-  if (!key_offsets_ok(key_off, q)) {
-    ctx->err = std::string(what) + ": key_off must be non-decreasing and below 2^32";
-    return BLSGPU_E_ARG;
-  }
-  CHECK_OFFSETS(msg_off, q, what);
-  if (msg_off[q] > msg_off[0] && !msgs) {
-    ctx->err = std::string(what) + ": msgs is null";
-    return BLSGPU_E_ARG;
-  }
-  const std::vector<uint64_t> ko = rebased(key_off, 0, q);
-  if (keys.set && keys.idx) keys.idx += key_off[0];
-  if (!keys.set && keys.bytes) keys.bytes += key_off[0] * (impl_id == 2 ? 48 : 96);
-  if (!key_idx_ok(ctx, what, keys, (size_t)ko[q])) return BLSGPU_E_ARG;
+  std::vector<uint64_t> ko;
+  CKR(check_sets(ctx, what, "key_off", key_off, q, MEMBERS_CAP, ko));
+  CKR(check_keys(ctx, what, impl_id, keys, key_off[0], ko[q]));
+  CKR(check_records(ctx, what, "msgs", msgs, "msg_off", msg_off, q));
   CKR(set_device(ctx));
   return with_impl(impl_id, [&](auto I) { return verify_multisig_impl<I>(ctx, scheme, format, q, ko.data(), keys, sigs, msgs, msg_off, status_out); });
 }
@@ -3399,7 +3302,7 @@ int blsgpu_verify_multisig_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int f
                                  const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_verify_multisig_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  return verify_multisig_common(ctx, "blsgpu_verify_multisig_batch", impl_id, scheme, format, q, key_off, Keys(pks), sigs, msgs, msg_off, status_out);
+  return verify_multisig_common(ctx, __func__, impl_id, scheme, format, q, key_off, pks, sigs, msgs, msg_off, status_out);
 }
 
 int blsgpu_verify_multisig_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t q, const uint64_t* key_off,
@@ -3407,32 +3310,25 @@ int blsgpu_verify_multisig_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int sch
                                        uint8_t* status_out) {
   NVTX_RANGE("blsgpu_verify_multisig_batch_keyed");
   if (!ctx) return BLSGPU_E_ARG;
-  const char* what = "blsgpu_verify_multisig_batch_keyed";
-  const KeySet* set = find_keyset(ctx, keyset, what);
-  if (!set) return BLSGPU_E_ARG;
-  return verify_multisig_common(ctx, what, set->impl_id, scheme, format, q, key_off, Keys(set, key_idx), sigs, msgs, msg_off, status_out);
+  KeySet* set = nullptr;
+  CKR(find_keyset(ctx, __func__, keyset, set));
+  return verify_multisig_common(ctx, __func__, set->impl_id, scheme, format, q, key_off, Keys(set, key_idx), sigs, msgs, msg_off, status_out);
 }
 
 int blsgpu_sum_points_batch(blsgpu_ctx* ctx, int group, int format, size_t q, const uint64_t* set_off, const uint8_t* points, uint8_t* out,
                             uint8_t* status_out, int64_t* bad_index_out) {
   NVTX_RANGE("blsgpu_sum_points_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  const char* what = "blsgpu_sum_points_batch";
-  if ((group != 1 && group != 2) || (format != 0 && format != 1) || (q && (!set_off || !out || !status_out)) ||
-      (q && set_off[q] > set_off[0] && !points)) {
-    ctx->err = std::string(what) + ": bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if ((group != 1 && group != 2) || (format != 0 && format != 1) || (q && (!out || !status_out))) return arg_error(ctx, __func__, "bad arguments");
   if (q == 0) return BLSGPU_OK;
-  if (!key_offsets_ok(set_off, q)) {
-    ctx->err = std::string(what) + ": set_off must be non-decreasing and below 2^32";
-    return BLSGPU_E_ARG;
-  }
-  const std::vector<uint64_t> so = rebased(set_off, 0, q);
-  const uint8_t* pts = points ? points + set_off[0] * (group == 1 ? 48 : 96) : nullptr;
+  std::vector<uint64_t> so;
+  CKR(check_sets(ctx, __func__, "set_off", set_off, q, MEMBERS_CAP, so));
+  if (points) points += set_off[0] * (group == 1 ? 48 : 96);
+  CKR(check_buffer(ctx, __func__, "points", points, so[q]));
   CKR(set_device(ctx));
-  return group == 1 ? sum_points_batch_impl<G1Aff>(ctx, format, q, so.data(), pts, out, status_out, bad_index_out)
-                    : sum_points_batch_impl<G2Aff>(ctx, format, q, so.data(), pts, out, status_out, bad_index_out);
+  return with_group(group, [&](auto G) {
+    return sum_points_batch_impl<typename decltype(G)::type>(ctx, format, q, so.data(), points, out, status_out, bad_index_out);
+  });
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -3522,15 +3418,14 @@ int blsgpu_combine_shares_batch(blsgpu_ctx* ctx, int group, size_t q, const uint
                                 uint8_t* status_out) {
   NVTX_RANGE("blsgpu_combine_shares_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  if ((group != 1 && group != 2) || (q && (!share_off || !out || !status_out)) || (q && share_off[q] && !shares)) {
-    ctx->err = "blsgpu_combine_shares_batch: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if ((group != 1 && group != 2) || (q && (!out || !status_out))) return arg_error(ctx, __func__, "bad arguments");
   if (q == 0) return BLSGPU_OK;
-  CHECK_OFFSETS(share_off, q, "blsgpu_combine_shares_batch");
+  std::vector<uint64_t> so;
+  CKR(check_sets(ctx, __func__, "share_off", share_off, q, NO_CAP, so));
+  if (shares) shares += share_off[0] * (32 + (group == 1 ? 48 : 96));
+  CKR(check_buffer(ctx, __func__, "shares", shares, so[q]));
   CKR(set_device(ctx));
-  return group == 1 ? combine_shares_impl<G1Aff>(ctx, q, share_off, shares, out, status_out)
-                    : combine_shares_impl<G2Aff>(ctx, q, share_off, shares, out, status_out);
+  return with_group(group, [&](auto G) { return combine_shares_impl<typename decltype(G)::type>(ctx, q, so.data(), shares, out, status_out); });
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -3540,11 +3435,8 @@ int blsgpu_verify_batch_wire(blsgpu_ctx* ctx, int impl_id, size_t n, const uint8
                              const uint64_t* msg_off, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_verify_batch_wire");
   if (!ctx) return BLSGPU_E_ARG;
-  if ((impl_id != 1 && impl_id != 2) || (n && (!pks || !tagged_sigs || !msg_off || !status_out))) {
-    ctx->err = "blsgpu_verify_batch_wire: bad arguments";
-    return BLSGPU_E_ARG;
-  }
-  CHECK_OFFSETS(msg_off, n, "blsgpu_verify_batch_wire");
+  if ((impl_id != 1 && impl_id != 2) || (n && (!pks || !tagged_sigs || !status_out))) return arg_error(ctx, __func__, "bad arguments");
+  CKR(check_records(ctx, __func__, "msgs", msgs, "msg_off", msg_off, n));
   const size_t pk_len = impl_id == 2 ? 48 : 96, rec = (impl_id == 2 ? 96 : 48) + 1;
   std::vector<uint64_t> pk_off(n + 1), sig_off(n + 1);
   for (size_t i = 0; i <= n; i++) {
@@ -3560,10 +3452,7 @@ int blsgpu_verify_share_batch(blsgpu_ctx* ctx, int impl_id, int scheme, size_t n
                               const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_verify_share_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  if (!args_ok(impl_id, scheme, 1) || (n && (!pk_shares || !sig_shares || !msg_off || !status_out))) {
-    ctx->err = "blsgpu_verify_share_batch: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if (!args_ok(impl_id, scheme, 1) || (n && (!pk_shares || !sig_shares || !msg_off || !status_out))) return arg_error(ctx, __func__, "bad arguments");
   if (n == 0) return BLSGPU_OK;
   static const uint8_t R_BE[32] = {0x73, 0xed, 0xa7, 0x53, 0x29, 0x9d, 0x7d, 0x48, 0x33, 0x39, 0xd8, 0x08, 0x09, 0xa1, 0xd8, 0x05,
                                    0x53, 0xbd, 0xa4, 0x02, 0xff, 0xfe, 0x5b, 0xfe, 0xff, 0xff, 0xff, 0xff, 0x00, 0x00, 0x00, 0x01};
@@ -3576,7 +3465,7 @@ int blsgpu_verify_share_batch(blsgpu_ctx* ctx, int impl_id, int scheme, size_t n
     memcpy(&p[i * pk_len], pr + 32, pk_len);
     memcpy(&g[i * sig_len], sr + 32, sig_len);
   }
-  CKR(blsgpu_verify_batch(ctx, impl_id, scheme, 1, n, p.data(), g.data(), msgs, msg_off, status_out));
+  CKR(verify_batch_common(ctx, __func__, impl_id, scheme, 1, n, p.data(), g.data(), msgs, msg_off, status_out));
   for (size_t i = 0; i < n; i++)
     if (bad_id[i]) status_out[i] = BLSGPU_ST_DESERIALIZE;
   return BLSGPU_OK;
@@ -3587,14 +3476,17 @@ int blsgpu_pairing_check_batch(blsgpu_ctx* ctx, size_t q, const uint64_t* pair_o
                                uint8_t* ok_out, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_pairing_check_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  if (q && (!pair_off || !ok_out || !status_out || (pair_off[q] && (!g1_points || !g2_points)))) {
-    ctx->err = "blsgpu_pairing_check_batch: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if (q && (!ok_out || !status_out)) return arg_error(ctx, __func__, "bad arguments");
   if (q == 0) return BLSGPU_OK;
-  CHECK_OFFSETS(pair_off, q, "blsgpu_pairing_check_batch");
+  std::vector<uint64_t> po;
+  CKR(check_sets(ctx, __func__, "pair_off", pair_off, q, NO_CAP, po));
+  const size_t M = (size_t)po[q];
+  if (g1_points) g1_points += pair_off[0] * 48;
+  if (g2_points) g2_points += pair_off[0] * 96;
+  CKR(check_buffer(ctx, __func__, "g1_points", g1_points, M));
+  CKR(check_buffer(ctx, __func__, "g2_points", g2_points, M));
+  pair_off = po.data();
   CKR(set_device(ctx));
-  const size_t M = (size_t)pair_off[q];
   CKR(ensure_arena(ctx, M * (48 + 96 + sizeof(G1Aff) + sizeof(G2Aff) + sizeof(Fp12) + 2) + (q + 1) * 9 + 16 * 256));
   uint8_t *d_a, *d_b;
   uint64_t* d_off;
@@ -3634,12 +3526,9 @@ int blsgpu_signcrypt_valid_batch(blsgpu_ctx* ctx, int impl_id, int scheme, size_
                                  const uint8_t* v_bytes, const uint64_t* v_off, uint8_t* ok_out, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_signcrypt_valid_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  if (!args_ok(impl_id, scheme, 1) || (n && (!u_points || !w_points || !v_off || !ok_out || !status_out))) {
-    ctx->err = "blsgpu_signcrypt_valid_batch: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if (!args_ok(impl_id, scheme, 1) || (n && (!u_points || !w_points || !ok_out || !status_out))) return arg_error(ctx, __func__, "bad arguments");
   if (n == 0) return BLSGPU_OK;
-  CHECK_OFFSETS(v_off, n, "blsgpu_signcrypt_valid_batch");
+  CKR(check_records(ctx, __func__, "v_bytes", v_bytes, "v_off", v_off, n));
   DstParam dst;
   make_dst(dst, impl_id, scheme, false);
   CKR(verify_host_common(ctx, impl_id, 1, dst, 1, n, u_points, w_points, v_bytes, v_off, status_out));
@@ -3687,8 +3576,7 @@ int pok_verify_impl(blsgpu_ctx* ctx, int scheme, size_t n, const uint8_t* commit
   CKR(upload(ctx, d_pkb, pks, n * Lp));
   CKR(upload(ctx, d_y, ys, n * 32));
   CKR(upload(ctx, d_yf, yflag.data(), n));
-  CKR(upload(ctx, d_msgs, msgs, msg_bytes));
-  CKR(upload(ctx, d_moff, msg_off, n + 1));
+  CKR(upload_records(ctx, msgs, msg_off, n, d_msgs, d_moff));
   SigA* d_cm = ctx->arena.take<SigA>(n);
   SigA* d_pr = ctx->arena.take<SigA>(n);
   SigA* d_a = ctx->arena.take<SigA>(n);
@@ -3730,8 +3618,7 @@ int signcrypt_share_impl(blsgpu_ctx* ctx, int scheme, size_t n, const uint8_t* s
   CKR(upload(ctx, d_pkb, pks, n * Lp));
   CKR(upload(ctx, d_ub, us, n * Lp));
   CKR(upload(ctx, d_wb, ws, n * Ls));
-  CKR(upload(ctx, d_v, v_bytes, v_total));
-  CKR(upload(ctx, d_voff, v_off, n + 1));
+  CKR(upload_records(ctx, v_bytes, v_off, n, d_v, d_voff));
   PkA* d_sh = ctx->arena.take<PkA>(n);
   PkA* d_pk = ctx->arena.take<PkA>(n);
   PkA* d_u = ctx->arena.take<PkA>(n);
@@ -3772,12 +3659,9 @@ int blsgpu_pok_verify_batch(blsgpu_ctx* ctx, int impl_id, int scheme, size_t n, 
                             const uint8_t* pks, const uint8_t* challenges32, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_pok_verify_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  if (!args_ok(impl_id, scheme, 1) || (n && (!commitments || !proofs || !pks || !challenges32 || !msg_off || !status_out))) {
-    ctx->err = "blsgpu_pok_verify_batch: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if (!args_ok(impl_id, scheme, 1) || (n && (!commitments || !proofs || !pks || !challenges32 || !status_out))) return arg_error(ctx, __func__, "bad arguments");
   if (n == 0) return BLSGPU_OK;
-  CHECK_OFFSETS(msg_off, n, "blsgpu_pok_verify_batch");
+  CKR(check_records(ctx, __func__, "msgs", msgs, "msg_off", msg_off, n));
   CKR(set_device(ctx));
   return with_impl(impl_id, [&](auto I) { return pok_verify_impl<I>(ctx, scheme, n, commitments, proofs, pks, challenges32, msgs, msg_off, status_out); });
 }
@@ -3787,12 +3671,10 @@ int blsgpu_signcrypt_verify_share_batch(blsgpu_ctx* ctx, int impl_id, int scheme
                                         uint8_t* ok_out, uint8_t* status_out) {
   NVTX_RANGE("blsgpu_signcrypt_verify_share_batch");
   if (!ctx) return BLSGPU_E_ARG;
-  if (!args_ok(impl_id, scheme, 1) || (n && (!shares || !pk_shares || !u_points || !w_points || !v_off || !ok_out || !status_out))) {
-    ctx->err = "blsgpu_signcrypt_verify_share_batch: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if (!args_ok(impl_id, scheme, 1) || (n && (!shares || !pk_shares || !u_points || !w_points || !ok_out || !status_out)))
+    return arg_error(ctx, __func__, "bad arguments");
   if (n == 0) return BLSGPU_OK;
-  CHECK_OFFSETS(v_off, n, "blsgpu_signcrypt_verify_share_batch");
+  CKR(check_records(ctx, __func__, "v_bytes", v_bytes, "v_off", v_off, n));
   CKR(set_device(ctx));
   return with_impl(impl_id, [&](auto I) {
     return signcrypt_share_impl<I>(ctx, scheme, n, shares, pk_shares, u_points, w_points, v_bytes, v_off, ok_out, status_out);
@@ -3808,19 +3690,12 @@ int blsgpu_verify_batch_records(blsgpu_ctx* ctx, int impl_id, int format, int sc
   NVTX_RANGE("blsgpu_verify_batch_records");
   if (!ctx) return BLSGPU_E_ARG;
   const bool tagged = scheme_or_tagged < 0;
-  if ((impl_id != 1 && impl_id != 2) || (format != 0 && format != 1) || scheme_or_tagged > 2 ||
-      (n && (!pk_off || !sig_off || !msg_off || !status_out))) {
-    ctx->err = "blsgpu_verify_batch_records: bad arguments";
-    return BLSGPU_E_ARG;
-  }
+  if ((impl_id != 1 && impl_id != 2) || (format != 0 && format != 1) || scheme_or_tagged > 2 || (n && !status_out))
+    return arg_error(ctx, __func__, "bad arguments");
   if (n == 0) return BLSGPU_OK;
-  CHECK_OFFSETS(pk_off, n, "blsgpu_verify_batch_records");
-  CHECK_OFFSETS(sig_off, n, "blsgpu_verify_batch_records");
-  CHECK_OFFSETS(msg_off, n, "blsgpu_verify_batch_records");
-  if ((!pk_bytes && pk_off[n] > pk_off[0]) || (!sig_bytes && sig_off[n] > sig_off[0]) || (!msgs && msg_off[n] > msg_off[0])) {
-    ctx->err = "blsgpu_verify_batch_records: pk_bytes, sig_bytes or msgs is null";
-    return BLSGPU_E_ARG;
-  }
+  CKR(check_records(ctx, __func__, "pk_bytes", pk_bytes, "pk_off", pk_off, n));
+  CKR(check_records(ctx, __func__, "sig_bytes", sig_bytes, "sig_off", sig_off, n));
+  CKR(check_records(ctx, __func__, "msgs", msgs, "msg_off", msg_off, n));
   const size_t pk_len = impl_id == 2 ? 48 : 96, sig_len = impl_id == 2 ? 96 : 48;
   // InvalidLength (public_key.rs:159-164, signature.rs:236-241) and the serde_bare tag (signature.rs:120-126) per record;
   // well-formed records are regrouped by scheme and go through blsgpu_verify_batch in `format`

@@ -19,6 +19,22 @@
  *   return  : 0 on success or a negative BLSGPU_E_* engine error; per-item outcomes go to status_out (BLSGPU_ST_*),
  *             which reproduce the reference's BlsResult for that item
  *   threads : one call at a time per context; contexts are independent
+ *
+ * Arguments (every entry point).  A call that breaks these rules returns BLSGPU_E_ARG before any device work (only the
+ * decoded contents of blsgpu_pairing_product_is_one and blsgpu_final_exp_is_one are refused later); blsgpu_last_error names
+ * the entry point, and the context stays usable.
+ *   empty batches : a call over no items (n = 0 or q = 0) returns 0, and the buffers of the items it has not may be NULL.
+ *                   The calls with a result even for no items (blsgpu_aggregate_verify, blsgpu_sum_points,
+ *                   blsgpu_miller_partial, blsgpu_pairing_product_is_one) still need the buffers of that result, and the
+ *                   msg_off of blsgpu_aggregate_verify, blsgpu_hash_to_curve_batch and blsgpu_verify_batch_wire its one entry
+ *   offsets       : an offset array has one entry more than it delimits; its entries are non-decreasing and every record
+ *                   (a message, a set of members) is below 2^32 bytes or members.  Records are located from off[0] on, so a
+ *                   slice of a larger buffer may be passed as is.  Calls that count members in 32 bits (grouped, multi-
+ *                   signature, aggregate-batch and key-set calls, secure aggregation) take at most 2^32 - 16 members:
+ *                   off[q] - off[0]
+ *   null buffers  : a buffer may be NULL only when it holds no bytes: a NULL msgs with messages that span bytes is refused
+ *   key sets      : keyed calls name keys by uint32 index into a set of this context (blsgpu_keyset_create); an id this
+ *                   context does not hold and an index at or above the set's size are refused
  */
 #ifndef BLSGPU_H
 #define BLSGPU_H
@@ -108,7 +124,7 @@ int blsgpu_verify_batch_dev(blsgpu_ctx* ctx, int impl_id, int scheme, int format
  * (items need not be sorted, a message may have any number of items, including none).  status_out[i] is exactly what
  * blsgpu_verify_batch returns for item i with its own copy of the message.  Basic and ProofOfPossession hash each message
  * once and run one Miller loop per run of up to 96 items of one message; MessageAugmentation hashes pk || msg, so it runs
- * blsgpu_verify_batch's pipeline on per-item messages.  msg_idx[i] >= q, at most 2^32 - 16 items.  First device only. */
+ * blsgpu_verify_batch's pipeline on per-item messages.  msg_idx[i] >= q is BLSGPU_E_ARG.  First device only. */
 int blsgpu_verify_batch_grouped(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t n, const uint8_t* pks,
                                 const uint8_t* sigs, const uint32_t* msg_idx, size_t q, const uint8_t* msgs,
                                 const uint64_t* msg_off, uint8_t* status_out);
@@ -123,13 +139,13 @@ int blsgpu_verify_batch_grouped(blsgpu_ctx* ctx, int impl_id, int scheme, int fo
  * status_out[i] (may be NULL): BLSGPU_ST_OK, DESERIALIZE or LEGACY_FORMAT for key i.  Keys that fail to decode stay in
  * the set, so that items naming them get exactly the status blsgpu_verify_batch gives for those bytes.
  * *keyset_out: a non-zero id, unique in the process (never reused).  n = 0 makes an empty set; at most 2^32 - 16 keys.
- * Synchronises before returning; on BLSGPU_E_ALLOC or BLSGPU_E_CUDA no set is created.  An id this context does not hold
- * (destroyed, or another context's) is BLSGPU_E_ARG in every call below.  blsgpu_ctx_destroy frees the sets still alive. */
+ * Synchronises before returning; on BLSGPU_E_ALLOC or BLSGPU_E_CUDA no set is created.  A destroyed set's id is refused like
+ * any id this context does not hold.  blsgpu_ctx_destroy frees the sets still alive. */
 int blsgpu_keyset_create(blsgpu_ctx* ctx, int impl_id, int format, size_t n, const uint8_t* pks, uint8_t* status_out,
                          uint64_t* keyset_out);
 int blsgpu_keyset_destroy(blsgpu_ctx* ctx, uint64_t keyset);
 /* blsgpu_verify_batch with pks[i] = the bytes key key_idx[i] of the set was created from; `format` is that of sigs only.
- * key_idx[i] at or above the set's size is BLSGPU_E_ARG.  No key is decoded: the keys are gathered from the set. */
+ * No key is decoded: the keys are gathered from the set. */
 int blsgpu_verify_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t n, const uint32_t* key_idx,
                               const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out);
 /* blsgpu_verify_batch_grouped with pks[i] = the bytes of key key_idx[i] */
@@ -170,8 +186,8 @@ int blsgpu_aggregate_verify(blsgpu_ctx* ctx, int impl_id, int scheme, int format
                             const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* sig, uint8_t* status_out,
                             int64_t index_out[2]);
 /* q x AggregateSignature::verify (reference src/aggregate_signature.rs:230-239 -> sig_core.rs:149-178, sig_basic.rs:41-64 |
- * sig_aug.rs:27-38 | sig_pop.rs:52-58).  Aggregate j owns pairs set_off[j]..set_off[j+1]-1 of pks / msgs (set_off has q+1
- * non-decreasing entries, like key_off of blsgpu_verify_secure_batch); msg_off has set_off[q]+1 entries, one message per pair;
+ * sig_aug.rs:27-38 | sig_pop.rs:52-58).  Aggregate j owns pairs set_off[j]..set_off[j+1]-1 of pks / msgs; msg_off holds
+ * one message per pair (entries set_off[0] .. set_off[q]);
  * sigs holds q aggregate signatures.  status_out[j] and index_out[2j..2j+1] (index_out may be NULL) mean exactly what
  * blsgpu_aggregate_verify returns for aggregate j alone; indices are positions INSIDE aggregate j.  Duplicate messages
  * (Basic) are looked for within an aggregate only.  One pipeline and one final exponentiation serve the whole call: every
@@ -211,9 +227,7 @@ int blsgpu_aggregate_secure_batch(blsgpu_ctx* ctx, int impl_id, int format, size
  * set encoded in the call's `format`, as the reference's *_with_mode on already-parsed keys: when `format` is the set's,
  * those are the bytes the set was created from, and every status and output byte equals the unkeyed call's on them.  A set
  * may be used in either format.  A key that failed to decode at creation gives its quorum the status it was created with
- * (the first bad key in member order decides).  The argument rules are the unkeyed calls'; an id this context does not hold
- * and a key_idx entry at or above the set's size are BLSGPU_E_ARG.  No key is decoded, and no member's key bytes cross the
- * bus: the call uploads key_off and key_idx (4 bytes per member) and sorts the quorums on the device.
+ * (the first bad key in member order decides).  No key is decoded, and no member's key bytes cross the bus: the call uploads key_off and key_idx (4 bytes per member) and sorts the quorums on the device.
  * Secure view: the first keyed secure call in a format builds, once per set and format, every key's encoding in that format
  * and its rank in byte order: 52 bytes per key of impl_id 2 and 100 of impl_id 1 on the device, 4 per key on the host.  The
  * build encodes on the device and sorts on the host (once, O(n log n) for n keys); the view lives until the set is
@@ -228,8 +242,7 @@ int blsgpu_aggregate_secure_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int fo
 /* ---- multi-signatures over signer subsets ------------------------------------------------------------------------
  * q x MultiSignature::verify(MultiPublicKey::from_public_keys(keys of set j), msg_j)  (reference src/multi_signature.rs:127-135,
  * src/multi_public_key.rs:79-83, src/traits/pk_multi.rs:7-13 -> core_verify sig_core.rs:120-146).  Set j owns keys
- * key_off[j] .. key_off[j+1]-1 of pks (key_off: q+1 non-decreasing entries below 2^32, as blsgpu_verify_secure_batch); one
- * signature and one message per set.
+ * key_off[j] .. key_off[j+1]-1 of pks; one signature and one message per set.
  * status_out[j] is exactly blsgpu_sum_points(pk group, format, keys of set j) followed by blsgpu_verify_batch(impl, scheme,
  * format, [that sum], [sig_j], [msg_j]): the first key of the set (in member order) that fails to decode, else the
  * signature's decode error, else SIG_IDENTITY, else PK_IDENTITY when the sum is the identity (an empty set, P and -P, only
@@ -238,13 +251,12 @@ int blsgpu_aggregate_secure_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int fo
  * The key sums are one segmented sum on the device, balanced by member count (chunks of 16 members of one set, then levels
  * of ranges of 16 partial sums), recorded as BLSGPU_STAGE_DECODE_PK together with the keys' decode; the q (sum, signature,
  * message) triples then take blsgpu_verify_batch's pipeline (one random-linear-combination check, bisection on failure).
- * At most 2^32 - 16 members per call; q = 0 is OK.  First device only. */
+ * First device only. */
 int blsgpu_verify_multisig_batch(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t q, const uint64_t* key_off,
                                  const uint8_t* pks, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off,
                                  uint8_t* status_out);
-/* the same with set j's keys = keys key_idx[key_off[j] .. key_off[j+1]) of a key set; `format` is that of sigs only.  An id
- * this context does not hold and a key_idx entry at or above the set's size are BLSGPU_E_ARG; a key that failed to decode
- * at creation gives its set the status it was created with.  No key is decoded: 4 bytes per member cross the bus. */
+/* the same with set j's keys = keys key_idx[key_off[j] .. key_off[j+1]) of a key set; `format` is that of sigs only.  A key
+ * that failed to decode at creation gives its set the status it was created with.  No key is decoded: 4 bytes per member cross the bus. */
 int blsgpu_verify_multisig_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t q,
                                        const uint64_t* key_off, const uint32_t* key_idx, const uint8_t* sigs,
                                        const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out);

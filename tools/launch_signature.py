@@ -146,6 +146,92 @@ def main():
     pk_rec[3] = pk_rec[3][:47]
     line("verify_batch_records tagged", eng.verify_batch_records(2, 1, -1, pk_rec, tagged, msgs))
     line("verify_batch_records raw", eng.verify_batch_records(2, 1, 0, pk_rec, [t[1:] for t in tagged], msgs))
+
+    # the remaining entry points, appended so that every line above (and the random draws behind it) stays as it was
+    # keyed verify: 300 items naming keys of a set of 1000
+    ks = eng.key_set(2, pks[:48 * 1000])
+    kidx = np.array(rnd.sample(range(1000), 300), dtype=np.uint32)
+    kd, ko = B.pack_messages([bytes(data[off[k]:off[k + 1]]) for k in kidx])
+    ksg = sigs.reshape(-1, 96)[kidx].reshape(-1)
+    line.last = eng.launch_count()
+    for tag, bad in [("valid", []), ("bad", sorted(rnd.sample(range(300), 3)))]:
+        line(f"verify_batch_keyed n=300 {tag}", eng.verify_batch_keyed_packed(ks, 0, kidx, spoil(ksg, 96, bad), kd, ko))
+
+    # 210 keys, key i signs message i % 7 (Basic and MessageAugmentation): grouped, multisig and secure calls over them
+    gq, gn = 7, 210
+    gd, go = B.pack_messages([b"grp-%d" % (i % gq) for i in range(gn)])
+    gm = [b"grp-%d" % j for j in range(gq)]
+    gk = keys(rnd, gn)
+    gpk, gsig = eng.testdata_sign(2, 0, gk, gd, go)
+    _, gsig_aug = eng.testdata_sign(2, 1, gk, gd, go)
+    gks = eng.key_set(2, gpk)
+    midx = np.arange(gn, dtype=np.uint32) % gq
+    all_idx = np.arange(gn, dtype=np.uint32)
+    gmd, gmo = B.pack_messages(gm)
+    line.last = eng.launch_count()
+    for scheme, sg in [(0, gsig), (1, gsig_aug)]:
+        for tag, bad in [("valid", []), ("bad", sorted(rnd.sample(range(gn), 3)))]:
+            s = spoil(sg, 96, bad)
+            line(f"verify_batch_grouped scheme={scheme} {tag}", eng.verify_batch_grouped_packed(2, scheme, gpk, s, midx, gmd, gmo))
+            line(f"verify_batch_grouped_keyed scheme={scheme} {tag}", eng.verify_batch_grouped_keyed_packed(gks, scheme, all_idx, s, midx, gmd, gmo))
+
+    # quorum j = the keys of message j, with its members in key order; multi-signatures are their signatures' sums
+    members = np.concatenate([np.arange(j, gn, gq) for j in range(gq)]).astype(np.uint32)
+    qoff = np.arange(gq + 1, dtype=np.uint64) * np.uint64(gn // gq)
+    mpk = gpk.reshape(-1, 48)[members].reshape(-1)
+    msg_sigs = gsig.reshape(-1, 96)[members].reshape(-1)
+    st, bad_idx, msums = eng.sum_points_batch_packed(2, qoff, msg_sigs)
+    line("sum_points_batch", st, bad_idx, msums)
+    broken = msg_sigs.copy()
+    broken[96 * 40] ^= 0x01
+    line("sum_points_batch bad point", *eng.sum_points_batch_packed(2, qoff, broken))
+    for tag, sw in [("valid", []), ("bad", [2, 5])]:
+        ms = spoil(msums, 96, sw)
+        line(f"verify_multisig_batch {tag}", eng.verify_multisig_batch_packed(2, 0, qoff, mpk, ms, gmd, gmo))
+        line(f"verify_multisig_batch_keyed {tag}", eng.verify_multisig_batch_keyed_packed(gks, 0, qoff, members, ms, gmd, gmo))
+
+    # secure aggregation over the same quorums: the aggregates verify; then two of them swapped
+    st, secure = eng.aggregate_secure_batch_packed(2, qoff, mpk, msg_sigs)
+    line("aggregate_secure_batch", st, secure)
+    st, secure_k = eng.aggregate_secure_batch_keyed_packed(gks, qoff, members, msg_sigs)
+    line("aggregate_secure_batch_keyed", st, secure_k)
+    for tag, sw in [("valid", []), ("bad", [1, 4])]:
+        ss = spoil(secure, 96, sw)
+        line(f"verify_secure_batch quorums {tag}", eng.verify_secure_batch_packed(2, 0, qoff, mpk, ss, gmd, gmo))
+        line(f"verify_secure_batch_keyed {tag}", eng.verify_secure_batch_keyed_packed(gks, 0, qoff, members, ss, gmd, gmo))
+
+    # threshold shares of f(x) = a0 + a1 x: five shares per set, then a set with a repeated identifier
+    a0, a1 = rnd.randrange(1, O.R), rnd.randrange(1, O.R)
+    xs = list(range(1, 6))
+    sh_k = np.frombuffer(b"".join(((a0 + a1 * x) % O.R).to_bytes(32, "big") for x in xs), dtype=np.uint8)
+    sd, so = B.pack_messages([b"share"] * len(xs))
+    sh_pk, _ = eng.testdata_sign(2, 0, sh_k, sd, so)
+    line.last = eng.launch_count()
+    recs = [x.to_bytes(32, "big") + bytes(sh_pk[48 * i:48 * i + 48]) for i, x in enumerate(xs)]
+    line("combine_shares_batch", *eng.combine_shares_batch(1, [recs, recs[:3], recs[:2] + recs[1:2]]))
+
+    # pairing_check_batch: e(P, Q) e(-P, Q) == 1, and a lone e(P, Q)
+    p0, q0 = bytes(pks[:48]), bytes(sigs[:96])
+    neg = bytes([p0[0] ^ 0x20]) + p0[1:]
+    line("pairing_check_batch", *eng.pairing_check_batch([[(p0, q0), (neg, q0)], [(p0, q0)], []]))
+
+    # the other public checks and building blocks, on the batch's keys and signatures (their statuses are rejections)
+    n = 48
+    pk_l = [bytes(pks[48 * i:48 * i + 48]) for i in range(n)]
+    sig_l = [bytes(sigs[96 * i:96 * i + 96]) for i in range(n)]
+    msgs = [bytes(data[off[i]:off[i + 1]]) for i in range(n)]
+    ys = [rnd.randrange(1, O.R).to_bytes(32, "big") for _ in range(n)]
+    line("pok_verify_batch", eng.pok_verify_batch(2, 0, sig_l, sig_l[1:] + sig_l[:1], pk_l, ys, msgs))
+    line("signcrypt_valid_batch", *eng.signcrypt_valid_batch(2, 0, pk_l, sig_l, msgs))
+    line("signcrypt_verify_share_batch", *eng.signcrypt_verify_share_batch(2, 0, pk_l, pk_l[1:] + pk_l[:1], pk_l, sig_l, msgs))
+    line("hash_to_curve_batch", np.frombuffer(b"".join(eng.hash_to_curve_batch(2, msgs, b"launch-signature-dst")), dtype=np.uint8))
+    st, out = eng.recode_points(1, pk_l, 1, 0)
+    line("recode_points", st, np.frombuffer(b"".join(out), dtype=np.uint8))
+    ids = [rnd.randrange(1, O.R).to_bytes(32, "big") for _ in range(n)]
+    pk_sh = [ids[i] + pk_l[i] for i in range(n)]
+    for tag, sl_ in [("valid", sig_l), ("bad", sig_l[:5] + [sig_l[6]] + sig_l[6:])]:
+        sig_sh = [ids[i] + sl_[i] for i in range(n)]
+        line(f"verify_share_batch {tag}", eng.verify_share_batch(2, 0, pk_sh, sig_sh, msgs))
     eng.close()
 
 

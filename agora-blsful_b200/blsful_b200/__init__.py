@@ -120,6 +120,8 @@ def load_library() -> ctypes.CDLL:
         "blsgpu_verify_batch_grouped": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u8p, u8p, vp, c.c_size_t, u8p, u64p, u8p]),
         "blsgpu_keyset_create": (c.c_int, [vp, c.c_int, c.c_int, c.c_size_t, u8p, u8p, c.POINTER(c.c_uint64)]),
         "blsgpu_keyset_destroy": (c.c_int, [vp, c.c_uint64]),
+        "blsgpu_keyset_update": (c.c_int, [vp, c.c_uint64, c.c_int, c.c_size_t, vp, u8p, u8p]),
+        "blsgpu_keyset_append": (c.c_int, [vp, c.c_uint64, c.c_int, c.c_size_t, u8p, u8p]),
         "blsgpu_verify_batch_keyed": (c.c_int, [vp, c.c_uint64, c.c_int, c.c_int, c.c_size_t, vp, u8p, u8p, u64p, u8p]),
         "blsgpu_verify_batch_grouped_keyed": (c.c_int, [vp, c.c_uint64, c.c_int, c.c_int, c.c_size_t, vp, u8p, vp, c.c_size_t, u8p, u64p, u8p]),
         "blsgpu_miller_partial": (c.c_int, [vp, c.c_int, c.c_int, c.c_int, c.c_size_t, u8p, u8p, u8p, u64p, u8p, u8p]),
@@ -168,7 +170,7 @@ EXPORTED_SYMBOLS = [
     "blsgpu_ctx_create", "blsgpu_ctx_destroy", "blsgpu_last_error", "blsgpu_ctx_set_rlc_salt", "blsgpu_ctx_set_rlc_bits",
     "blsgpu_ctx_set_stream",
     "blsgpu_verify_batch", "blsgpu_verify_batch_grouped",
-    "blsgpu_keyset_create", "blsgpu_keyset_destroy", "blsgpu_verify_batch_keyed", "blsgpu_verify_batch_grouped_keyed",
+    "blsgpu_keyset_create", "blsgpu_keyset_destroy", "blsgpu_keyset_update", "blsgpu_keyset_append", "blsgpu_verify_batch_keyed", "blsgpu_verify_batch_grouped_keyed",
     "blsgpu_miller_partial", "blsgpu_final_exp_is_one", "blsgpu_partial_finish",
     "blsgpu_verify_batch_dev", "blsgpu_pop_verify_batch", "blsgpu_aggregate_verify", "blsgpu_aggregate_verify_batch", "blsgpu_sum_points",
     "blsgpu_verify_secure_batch", "blsgpu_aggregate_secure_batch",
@@ -375,6 +377,30 @@ class Engine:
         self._check(self._lib.blsgpu_keyset_create(self._ctx, impl_id, fmt, n, _ptr(pk), _ptr(status), ctypes.byref(ident)),
                     "blsgpu_keyset_create")
         return KeySet(self, impl_id, ident.value, status)
+
+    def update_key_set(self, keys: KeySet, key_idx, pks, fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """Key key_idx[i] of `keys` becomes pks[i], decoded in fmt (blsgpu_keyset_update): the set keeps its id and every
+        other key.  Returns the k decode statuses, which keys.status takes over."""
+        pk = _pack_points(pks, pk_len(keys.impl_id), "public key")
+        idx = np.ascontiguousarray(key_idx, dtype=np.uint32).reshape(-1)
+        k = pk.size // pk_len(keys.impl_id)
+        if idx.size != k:
+            raise BlsError(ST_MISMATCHED_LENGTHS)
+        status = np.zeros(k, dtype=np.uint8)
+        self._check(self._lib.blsgpu_keyset_update(self._ctx, keys.id, fmt, k, _ptr(idx), _ptr(pk), _ptr(status)), "blsgpu_keyset_update")
+        keys.status = keys.status.copy()
+        keys.status[idx] = status
+        return status
+
+    def append_key_set(self, keys: KeySet, pks, fmt: int = SerializationFormat.Modern) -> np.ndarray:
+        """Appends pks, decoded in fmt, to `keys` (blsgpu_keyset_append): they take indices len(keys) onwards.  Returns their
+        decode statuses, which keys.status takes over."""
+        pk = _pack_points(pks, pk_len(keys.impl_id), "public key")
+        k = pk.size // pk_len(keys.impl_id)
+        status = np.zeros(k, dtype=np.uint8)
+        self._check(self._lib.blsgpu_keyset_append(self._ctx, keys.id, fmt, k, _ptr(pk), _ptr(status)), "blsgpu_keyset_append")
+        keys.status = np.concatenate([keys.status, status])
+        return status
 
     def verify_batch_keyed(self, keys: KeySet, scheme: int, key_idx, sigs, msgs: Sequence[bytes],
                            fmt: int = SerializationFormat.Modern) -> np.ndarray:

@@ -117,12 +117,14 @@ struct PendingSlice {
 
 // public keys decoded once (blsgpu_keyset_create): n affine points of the impl's key group and their decode statuses, in a
 // device allocation of their own on the first device (apart from the arena, so that regrowing the arena keeps them)
-// The secure view of a key set in one format (ensure_secure_view, built by the first keyed secure call in that format):
+// The secure view of a key set in one format (ensure_secure_view, built by the first keyed secure call in that format, and
+// kept current by the set's updates and appends, keyset_change_impl):
 // every key re-encoded in the format, and its dense rank in memcmp order of those encodings (equal bytes, equal rank).
 struct SecureView {
   uint8_t* enc = nullptr;            // device, n encodings
   uint32_t* rank = nullptr;          // device, n ranks
   std::vector<uint32_t> host_rank;  // the same ranks, for quorums the host plans
+  size_t ranks = 0;                 // distinct encodings (the largest rank + 1)
 };
 struct KeySet {
   int impl_id = 0;
@@ -2386,6 +2388,172 @@ int keyset_create_impl(blsgpu_ctx* ctx, int impl_id, int format, size_t n, const
   *keyset_out = id;
   return BLSGPU_OK;
 }
+
+// The dense ranks of a secure view after some of its keys change, equal to those a fresh ensure_secure_view gives over the
+// final encodings.  h: the old ranks of the n keys, over `ranks` distinct encodings.  Key idx[j] (j < k; at or above n for
+// an appended key) takes encoding enc[j] (L bytes), which k_rank_search placed at pos[j] = 2 * lb + eq among the old ranks.
+// Two kept keys are equal iff their old ranks are; a new key equals the keys of old rank lb when eq is set, and otherwise
+// lies between old ranks lb - 1 and lb; new keys are ordered among themselves by memcmp.  An old rank that neither a kept
+// key nor an equal new key holds disappears.  out: the n1 new ranks; returns the new count of distinct encodings.
+// O(n + ranks) integer work, and a sort of the k new keys.
+size_t merge_ranks(const std::vector<uint32_t>& h, size_t ranks, size_t n1, size_t k, const uint32_t* idx, const uint8_t* enc,
+                   const uint64_t* pos, size_t L, std::vector<uint32_t>& out) {
+  const size_t n = h.size();
+  std::vector<uint8_t> kept(n, 1), alive(ranks, 0);
+  for (size_t j = 0; j < k; j++)
+    if (idx[j] < n) kept[idx[j]] = 0;
+  for (size_t i = 0; i < n; i++)
+    if (kept[i]) alive[h[i]] = 1;
+  std::vector<uint32_t> ord(k);
+  for (size_t j = 0; j < k; j++) ord[j] = (uint32_t)j;
+  // by lb, then by bytes: the new keys equal to rank lb come after those below it
+  std::sort(ord.begin(), ord.end(), [&](uint32_t a, uint32_t b) {
+    if (pos[a] >> 1 != pos[b] >> 1) return pos[a] >> 1 < pos[b] >> 1;
+    return memcmp(enc + (size_t)a * L, enc + (size_t)b * L, L) < 0;
+  });
+  std::vector<uint32_t> remap(ranks), fresh(k);
+  size_t c = 0, p = 0;
+  for (size_t r = 0; r <= ranks; r++) {
+    const uint8_t* last = nullptr;  // the previous new encoding below old rank r
+    for (; p < k && pos[ord[p]] >> 1 == r && !(pos[ord[p]] & 1); p++) {
+      const uint8_t* e = enc + (size_t)ord[p] * L;
+      if (!last || memcmp(last, e, L) != 0) c++;
+      fresh[ord[p]] = (uint32_t)(c - 1);
+      last = e;
+    }
+    if (r == ranks) break;
+    bool held = alive[r];
+    for (; p < k && pos[ord[p]] >> 1 == r; p++) {  // equal to old rank r
+      fresh[ord[p]] = (uint32_t)c;
+      held = true;
+    }
+    if (held) remap[r] = (uint32_t)c++;
+  }
+  out.resize(n1);
+  for (size_t i = 0; i < n; i++)
+    if (kept[i]) out[i] = remap[h[i]];
+  for (size_t j = 0; j < k; j++) out[idx[j]] = fresh[j];
+  return c;
+}
+
+// k keys of set s change (blsgpu_keyset_update: key_idx are distinct indices below n) or are appended (append: key_idx =
+// n .. n + k - 1).  The keys are decoded into arena scratch, and for every live secure view encoded in its format and placed
+// among its ranks by a binary search; the new ranks are merged on the host (merge_ranks).  Only then is the set written: an
+// append first allocates every array at the size n + k and copies the old contents device to device, then the points,
+// statuses and encodings are scattered to key_idx and the ranks uploaded.  The old arrays of an append are freed last.
+template <class PkA>
+int keyset_change_impl(blsgpu_ctx* ctx, KeySet& s, int format, size_t k, const uint32_t* key_idx, const uint8_t* pks, uint8_t* status_out,
+                       bool append) {
+  constexpr int L = PtInfo<PkA>::LEN;
+  const size_t n = s.n, n1 = append ? n + k : n;
+  bool live[2];
+  size_t need = Arena::bytes<uint8_t>(k * L) + Arena::bytes<uint32_t>(k) + Arena::bytes<PkA>(k) + Arena::bytes<uint8_t>(k);
+  for (int f = 0; f < 2; f++) {
+    live[f] = s.view[f].enc != nullptr;
+    if (live[f]) need += Arena::bytes<uint8_t>(k * L) + Arena::bytes<uint64_t>(k) + Arena::bytes<uint32_t>(std::max<size_t>(s.view[f].ranks, 1));
+  }
+  CKR(ensure_arena(ctx, need));
+  uint8_t* d_bytes;
+  uint32_t* d_idx;
+  CKR(upload(ctx, d_bytes, pks, k * L));
+  CKR(upload(ctx, d_idx, key_idx, k));
+  PkA* d_pts = ctx->arena.take<PkA>(k);
+  uint8_t* d_st = ctx->arena.take<uint8_t>(k);
+  CKR((decode_points<PkA>(ctx, k, (const uint8_t*)d_bytes, format, d_pts, d_st)));
+  if (status_out) CK(cudaMemcpyAsync(status_out, d_st, k, cudaMemcpyDeviceToHost, ctx->stream));
+  uint8_t* d_enc[2] = {nullptr, nullptr};
+  std::vector<uint8_t> enc[2];
+  std::vector<uint64_t> pos[2];
+  for (int f = 0; f < 2; f++) {
+    if (!live[f]) continue;
+    const SecureView& v = s.view[f];
+    d_enc[f] = ctx->arena.take<uint8_t>(k * L);
+    uint64_t* d_pos = ctx->arena.take<uint64_t>(k);
+    uint32_t* d_rep = ctx->arena.take<uint32_t>(std::max<size_t>(v.ranks, 1));
+    LAUNCH((k_encode<PkA>), blocks_for(k), TPB, k, (const PkA*)d_pts, f, d_enc[f]);
+    if (n) LAUNCH(k_rank_reps, blocks_for(n), TPB, n, (const uint32_t*)v.rank, d_rep);
+    LAUNCH((k_rank_search<L>), blocks_for(k), TPB, k, (const uint8_t*)d_enc[f], (const uint8_t*)v.enc, (const uint32_t*)d_rep, v.ranks, d_pos);
+    enc[f].resize(k * L);
+    pos[f].resize(k);
+    CK(cudaMemcpyAsync(enc[f].data(), d_enc[f], k * L, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(pos[f].data(), d_pos, k * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  CK(cudaStreamSynchronize(ctx->stream));
+  std::vector<uint32_t> rank[2];
+  size_t ranks[2] = {0, 0};
+  for (int f = 0; f < 2; f++)
+    if (live[f]) ranks[f] = merge_ranks(s.view[f].host_rank, s.view[f].ranks, n1, k, key_idx, enc[f].data(), pos[f].data(), L, rank[f]);
+
+  KeySet g;  // the device arrays written: the set's own, or for an append the grown ones
+  if (!append) {
+    g.pts = s.pts;
+    g.st = s.st;
+    for (int f = 0; f < 2; f++) {
+      g.view[f].enc = s.view[f].enc;
+      g.view[f].rank = s.view[f].rank;
+    }
+  }
+  const int r = [&]() -> int {
+    if (append) {
+      CK(cudaMalloc(&g.pts, n1 * sizeof(PkA)));
+      CK(cudaMalloc(&g.st, n1));
+      for (int f = 0; f < 2; f++) {
+        if (!live[f]) continue;
+        CK(cudaMalloc(&g.view[f].enc, n1 * L));
+        CK(cudaMalloc(&g.view[f].rank, n1 * 4));
+      }
+      if (n) {
+        CK(cudaMemcpyAsync(g.pts, s.pts, n * sizeof(PkA), cudaMemcpyDeviceToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(g.st, s.st, n, cudaMemcpyDeviceToDevice, ctx->stream));
+        for (int f = 0; f < 2; f++)
+          if (live[f]) CK(cudaMemcpyAsync(g.view[f].enc, s.view[f].enc, n * L, cudaMemcpyDeviceToDevice, ctx->stream));
+      }
+    }
+    LAUNCH((k_scatter_keys<PkA>), blocks_for(k), TPB, k, (const uint32_t*)d_idx, (const PkA*)d_pts, (const uint8_t*)d_st, (PkA*)g.pts, g.st);
+    for (int f = 0; f < 2; f++) {
+      if (!live[f]) continue;
+      LAUNCH((k_scatter_enc<L>), blocks_for(k), TPB, k, (const uint32_t*)d_idx, (const uint8_t*)d_enc[f], g.view[f].enc);
+      CK(cudaMemcpyAsync(g.view[f].rank, rank[f].data(), n1 * 4, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    CK(cudaStreamSynchronize(ctx->stream));
+    return BLSGPU_OK;
+  }();
+  if (r != BLSGPU_OK) {
+    if (append) {  // the set keeps its old arrays
+      free_keyset(g);
+      (void)cudaGetLastError();
+    }
+    return r;
+  }
+  if (append) {
+    free_keyset(s);
+    s.pts = g.pts;
+    s.st = g.st;
+    s.n = n1;
+  }
+  for (int f = 0; f < 2; f++) {
+    if (!live[f]) continue;
+    s.view[f].enc = g.view[f].enc;
+    s.view[f].rank = g.view[f].rank;
+    s.view[f].host_rank = std::move(rank[f]);
+    s.view[f].ranks = ranks[f];
+  }
+  return BLSGPU_OK;
+}
+
+// the k target keys of an update: each below the set's size, none named twice
+int check_update_keys(blsgpu_ctx* ctx, const char* what, KeySet* set, size_t k, const uint32_t* key_idx) {
+  Keys keys(set, key_idx);
+  CKR(check_keys(ctx, what, set->impl_id, keys, 0, k));
+  std::vector<std::pair<uint32_t, uint32_t>> o(k);  // (key, position)
+  for (size_t i = 0; i < k; i++) o[i] = {key_idx[i], (uint32_t)i};
+  std::sort(o.begin(), o.end());
+  for (size_t i = 1; i < k; i++)
+    if (o[i].first == o[i - 1].first)
+      return arg_error(ctx, what, "key_idx[" + std::to_string(o[i - 1].second) + "] and key_idx[" + std::to_string(o[i].second) +
+                                      "] both name key " + std::to_string(o[i].first));
+  return BLSGPU_OK;
+}
 }  // namespace
 
 int blsgpu_verify_batch_grouped(blsgpu_ctx* ctx, int impl_id, int scheme, int format, size_t n, const uint8_t* pks, const uint8_t* sigs,
@@ -2418,6 +2586,39 @@ int blsgpu_keyset_destroy(blsgpu_ctx* ctx, uint64_t keyset) {
   ctx->keysets.erase(keyset);
   CK(e);
   return BLSGPU_OK;
+}
+
+int blsgpu_keyset_update(blsgpu_ctx* ctx, uint64_t keyset, int format, size_t k, const uint32_t* key_idx, const uint8_t* pks,
+                         uint8_t* status_out) {
+  NVTX_RANGE("blsgpu_keyset_update");
+  if (!ctx) return BLSGPU_E_ARG;
+  KeySet* set = nullptr;
+  CKR(find_keyset(ctx, __func__, keyset, set));
+  if (format != 0 && format != 1) return arg_error(ctx, __func__, "bad arguments");
+  CKR(check_buffer(ctx, __func__, "pks", pks, k));
+  CKR(check_update_keys(ctx, __func__, set, k, key_idx));
+  if (k == 0) return BLSGPU_OK;
+  CKR(set_device(ctx));
+  return with_impl(set->impl_id, [&](auto I) {
+    return keyset_change_impl<typename ImplT<I>::PkAff>(ctx, *set, format, k, key_idx, pks, status_out, false);
+  });
+}
+
+int blsgpu_keyset_append(blsgpu_ctx* ctx, uint64_t keyset, int format, size_t k, const uint8_t* pks, uint8_t* status_out) {
+  NVTX_RANGE("blsgpu_keyset_append");
+  if (!ctx) return BLSGPU_E_ARG;
+  KeySet* set = nullptr;
+  CKR(find_keyset(ctx, __func__, keyset, set));
+  if (format != 0 && format != 1) return arg_error(ctx, __func__, "bad arguments");
+  CKR(check_buffer(ctx, __func__, "pks", pks, k));
+  if (k > MEMBERS_CAP - set->n) return arg_error(ctx, __func__, "at most 2^32 - 16 keys per set");
+  if (k == 0) return BLSGPU_OK;
+  std::vector<uint32_t> idx(k);
+  for (size_t i = 0; i < k; i++) idx[i] = (uint32_t)(set->n + i);
+  CKR(set_device(ctx));
+  return with_impl(set->impl_id, [&](auto I) {
+    return keyset_change_impl<typename ImplT<I>::PkAff>(ctx, *set, format, k, idx.data(), pks, status_out, true);
+  });
 }
 
 int blsgpu_verify_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t n, const uint32_t* key_idx, const uint8_t* sigs,
@@ -3020,6 +3221,7 @@ int ensure_secure_view(blsgpu_ctx* ctx, KeySet& s, int format) {
         if (i && (o[i].first != o[i - 1].first || memcmp(&enc[(size_t)o[i].second * L], &enc[(size_t)o[i - 1].second * L], L) != 0)) rk++;
         nv.host_rank[o[i].second] = rk;
       }
+      nv.ranks = (size_t)rk + 1;
       CK(cudaMemcpyAsync(nv.rank, nv.host_rank.data(), n * 4, cudaMemcpyHostToDevice, ctx->stream));
       CK(cudaStreamSynchronize(ctx->stream));
     }

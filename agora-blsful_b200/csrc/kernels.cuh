@@ -192,6 +192,59 @@ __global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_gather_keys(size_t n, c
   st[i] = set_st[k];
 }
 
+// ---- key-set updates (blsgpu_keyset_update / blsgpu_keyset_append) ------------------------------------------------------
+// the inverse of k_gather_keys: key key_idx[i] of the set takes decoded point i and its status (the indices are distinct)
+template <class A>
+__global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_scatter_keys(size_t n, const uint32_t* __restrict__ key_idx, const A* __restrict__ pts,
+                                                      const uint8_t* __restrict__ st, A* __restrict__ set_pts, uint8_t* __restrict__ set_st) {
+  size_t i = BLS_TID();
+  if (i >= n) return;
+  const uint32_t k = key_idx[i];
+  set_pts[k] = pts[i];
+  set_st[k] = st[i];
+}
+// the same for a secure view's encodings of L bytes
+template <int L>
+__global__ void __launch_bounds__(128) k_scatter_enc(size_t n, const uint32_t* __restrict__ key_idx, const uint8_t* __restrict__ enc,
+                                                     uint8_t* __restrict__ view_enc) {
+  size_t i = BLS_TID();
+  if (i >= n) return;
+  const size_t k = key_idx[i];
+  for (int b = 0; b < L; b++) view_enc[k * L + b] = enc[i * L + b];
+}
+// rep[r] = a key of dense rank r in a secure view (keys of one rank have equal encodings, so any of them will do)
+__global__ void __launch_bounds__(128) k_rank_reps(size_t n, const uint32_t* __restrict__ rank, uint32_t* __restrict__ rep) {
+  size_t i = BLS_TID();
+  if (i >= n) return;
+  rep[rank[i]] = (uint32_t)i;
+}
+// where encoding i of the n new ones falls among the `ranks` distinct encodings of a secure view (rep: one key per rank, in
+// memcmp order of their encodings view_enc): pos[i] = 2 * lb + eq, lb = the number of ranks whose encoding is below it, eq
+// = 1 when the encoding of rank lb equals it
+template <int L>
+__global__ void __launch_bounds__(128) k_rank_search(size_t n, const uint8_t* __restrict__ enc, const uint8_t* __restrict__ view_enc,
+                                                     const uint32_t* __restrict__ rep, size_t ranks, uint64_t* __restrict__ pos) {
+  size_t i = BLS_TID();
+  if (i >= n) return;
+  uint8_t e[L];
+  for (int b = 0; b < L; b++) e[b] = enc[i * L + b];
+  auto cmp = [&](size_t r) {  // memcmp(view encoding of rank r, e)
+    const uint8_t* v = view_enc + (size_t)rep[r] * L;
+    for (int b = 0; b < L; b++)
+      if (v[b] != e[b]) return v[b] < e[b] ? -1 : 1;
+    return 0;
+  };
+  size_t lo = 0, hi = ranks;
+  while (lo < hi) {
+    const size_t mid = lo + (hi - lo) / 2;
+    if (cmp(mid) < 0)
+      lo = mid + 1;
+    else
+      hi = mid;
+  }
+  pos[i] = 2 * (uint64_t)lo + (lo < ranks && cmp(lo) == 0 ? 1 : 0);
+}
+
 // affine points -> compressed bytes in `format`
 template <class A>
 __global__ void __launch_bounds__(128, BLS_MIN_BLOCKS) k_encode(size_t n, const A* __restrict__ in, int format, uint8_t* __restrict__ out) {

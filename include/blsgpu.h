@@ -144,6 +144,31 @@ int blsgpu_verify_batch_grouped(blsgpu_ctx* ctx, int impl_id, int scheme, int fo
 int blsgpu_keyset_create(blsgpu_ctx* ctx, int impl_id, int format, size_t n, const uint8_t* pks, uint8_t* status_out,
                          uint64_t* keyset_out);
 int blsgpu_keyset_destroy(blsgpu_ctx* ctx, uint64_t keyset);
+/* Changing a set in place: the set keeps its id and the indices of the keys that did not change, and the work is that of
+ * the k changed keys (their decode, and for each live secure view their encoding and a binary search among the set's keys)
+ * plus an O(n) pass over 4-byte ranks on the host and their upload.
+ *   equivalence : after any sequence of creates, updates and appends, every keyed call returns byte for byte what it returns
+ *                 on a set created from the final key bytes (statuses, aggregates and indices, in both formats).  "The bytes
+ *                 a key of the set was created from" in the keyed calls below means the bytes it was last given.
+ *   format      : each call has its own `format`, as blsgpu_keyset_create; a key's status is the one the format that last
+ *                 decoded it gave.  A key that fails to decode stays in the set with that status, as at creation.
+ *   refused     : with BLSGPU_E_ARG before any device work, the set unchanged: an id this context does not hold, a NULL pks
+ *                 or key_idx with k > 0, a key_idx[i] at or above the set's size, an index named twice in one update (both
+ *                 positions are named in blsgpu_last_error), an append past 2^32 - 16 keys.  k = 0 returns 0.
+ *   failures    : on BLSGPU_E_ALLOC the set is unchanged (the keys are decoded into scratch, and an append allocates the
+ *                 grown set, before anything is written into the set).  A set that meets BLSGPU_E_CUDA can only be destroyed.
+ *   secure views: live views are kept current, so that the next keyed secure call does not rebuild them.  The view's memory
+ *                 per key is unchanged.
+ * Both calls end a pending blsgpu_miller_partial slice, synchronise before returning and run on the first device only.
+ *
+ * Key key_idx[i] of the set becomes the key decoded from pks[i] (k compressed keys of the set's impl in `format`).
+ * status_out[i] (may be NULL): BLSGPU_ST_OK, DESERIALIZE or LEGACY_FORMAT, exactly what blsgpu_keyset_create gives for
+ * those bytes. */
+int blsgpu_keyset_update(blsgpu_ctx* ctx, uint64_t keyset, int format, size_t k, const uint32_t* key_idx,
+                         const uint8_t* pks, uint8_t* status_out);
+/* k keys appended: a set of n keys gives them indices n .. n + k - 1 (statuses as blsgpu_keyset_update).  The set's
+ * device arrays are reallocated at the exact new size: the old ones are copied device to device, then freed. */
+int blsgpu_keyset_append(blsgpu_ctx* ctx, uint64_t keyset, int format, size_t k, const uint8_t* pks, uint8_t* status_out);
 /* blsgpu_verify_batch with pks[i] = the bytes key key_idx[i] of the set was created from; `format` is that of sigs only.
  * No key is decoded: the keys are gathered from the set. */
 int blsgpu_verify_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t n, const uint32_t* key_idx,
@@ -231,7 +256,7 @@ int blsgpu_aggregate_secure_batch(blsgpu_ctx* ctx, int impl_id, int format, size
  * Secure view: the first keyed secure call in a format builds, once per set and format, every key's encoding in that format
  * and its rank in byte order: 52 bytes per key of impl_id 2 and 100 of impl_id 1 on the device, 4 per key on the host.  The
  * build encodes on the device and sorts on the host (once, O(n log n) for n keys); the view lives until the set is
- * destroyed.  First device only. */
+ * destroyed, and blsgpu_keyset_update / blsgpu_keyset_append keep it current.  First device only. */
 int blsgpu_verify_secure_batch_keyed(blsgpu_ctx* ctx, uint64_t keyset, int scheme, int format, size_t q,
                                      const uint64_t* key_off, const uint32_t* key_idx, const uint8_t* sigs,
                                      const uint8_t* msgs, const uint64_t* msg_off, uint8_t* status_out);

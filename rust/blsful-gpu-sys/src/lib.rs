@@ -58,6 +58,10 @@ extern "C" {
     pub fn blsgpu_keyset_create(ctx: *mut blsgpu_ctx, impl_id: c_int, format: c_int, n: usize, pks: *const u8,
         status_out: *mut u8 /* [n] or null */, keyset_out: *mut u64) -> c_int;
     pub fn blsgpu_keyset_destroy(ctx: *mut blsgpu_ctx, keyset: u64) -> c_int;
+    pub fn blsgpu_keyset_update(ctx: *mut blsgpu_ctx, keyset: u64, format: c_int, k: usize, key_idx: *const u32, pks: *const u8,
+        status_out: *mut u8 /* [k] or null */) -> c_int;
+    pub fn blsgpu_keyset_append(ctx: *mut blsgpu_ctx, keyset: u64, format: c_int, k: usize, pks: *const u8,
+        status_out: *mut u8 /* [k] or null */) -> c_int;
     pub fn blsgpu_verify_batch_keyed(ctx: *mut blsgpu_ctx, keyset: u64, scheme: c_int, format: c_int, n: usize,
         key_idx: *const u32, sigs: *const u8, msgs: *const u8, msg_off: *const u64, status_out: *mut u8) -> c_int;
     pub fn blsgpu_verify_batch_grouped_keyed(ctx: *mut blsgpu_ctx, keyset: u64, scheme: c_int, format: c_int, n: usize,

@@ -7,6 +7,7 @@
 //! |---|---|
 //! | [`Engine::verify_batch`] | `Signature::verify` (src/signature.rs:130-138) |
 //! | [`Engine::verify_batch_keyed`] / [`Engine::verify_batch_grouped_keyed`] | `Signature::verify` against keys decoded once into a [`KeySet`] |
+//! | [`Engine::update_key_set`] / [`Engine::append_key_set`] | a [`KeySet`] changed in place: keys replaced by index or appended, the set's id and other indices kept |
 //! | [`Engine::verify_secure_batch_keyed_with_mode`] / [`Engine::aggregate_secure_batch_keyed_with_mode`] | `verify_secure_with_mode` / `aggregate_secure_with_mode` over quorum members named by index into a [`KeySet`] |
 //! | [`Engine::pop_verify_batch`] | `ProofOfPossession::verify` (src/proof_of_possession.rs:77-81) |
 //! | [`Engine::aggregate_verify`] | `AggregateSignature::verify` (src/aggregate_signature.rs:230-239) |
@@ -447,6 +448,53 @@ impl Engine {
         let rc = unsafe { sys::blsgpu_keyset_create(self.ctx, C::IMPL_ID, format_id(format), n, pks.as_ptr(), status.as_mut_ptr(), &mut id) };
         self.check(rc)?;
         Ok((KeySet { id, len: n, _impl: PhantomData }, status))
+    }
+
+    /// Key `key_idx[i]` of `keys` becomes `pks[i]`, in place: the set keeps its id and every other key, and its secure
+    /// views stay current.  An index at or past the end of the set, or named twice, is an `EngineError` (`BLSGPU_E_ARG`)
+    /// that leaves the set unchanged.
+    pub fn update_key_set<C: GpuImpl>(&mut self, keys: &mut KeySet<C>, key_idx: &[u32], pks: &[PublicKey<C>]) -> EngineResult<()> {
+        let bytes = pack_points(pks.iter().map(|p| p.0), C::PK_BYTES);
+        self.update_key_set_bytes(keys, SerializationFormat::Modern, key_idx, &bytes).map(|_| ())
+    }
+
+    /// The byte form of [`Engine::update_key_set`]: keys serialised in `format`, with one status per key, as
+    /// [`Engine::key_set_bytes`] gives for those bytes.
+    pub fn update_key_set_bytes<C: GpuImpl>(
+        &mut self,
+        keys: &mut KeySet<C>,
+        format: SerializationFormat,
+        key_idx: &[u32],
+        pks: &[u8],
+    ) -> EngineResult<Vec<u8>> {
+        if pks.len() % C::PK_BYTES != 0 || pks.len() / C::PK_BYTES != key_idx.len() {
+            return Err(EngineError { code: sys::BLSGPU_E_ARG, message: "update_key_set_bytes: one whole key per index".into() });
+        }
+        let mut status = vec![0u8; key_idx.len()];
+        let rc = unsafe {
+            sys::blsgpu_keyset_update(self.ctx, keys.id, format_id(format), key_idx.len(), key_idx.as_ptr(), pks.as_ptr(), status.as_mut_ptr())
+        };
+        self.check(rc)?;
+        Ok(status)
+    }
+
+    /// Appends `pks` to `keys`: they take indices `keys.len()` onwards, and the set keeps its id.
+    pub fn append_key_set<C: GpuImpl>(&mut self, keys: &mut KeySet<C>, pks: &[PublicKey<C>]) -> EngineResult<()> {
+        let bytes = pack_points(pks.iter().map(|p| p.0), C::PK_BYTES);
+        self.append_key_set_bytes(keys, SerializationFormat::Modern, &bytes).map(|_| ())
+    }
+
+    /// The byte form of [`Engine::append_key_set`]: keys serialised in `format`, with one status per key.
+    pub fn append_key_set_bytes<C: GpuImpl>(&mut self, keys: &mut KeySet<C>, format: SerializationFormat, pks: &[u8]) -> EngineResult<Vec<u8>> {
+        if pks.len() % C::PK_BYTES != 0 {
+            return Err(EngineError { code: sys::BLSGPU_E_ARG, message: "append_key_set_bytes: not a whole number of keys".into() });
+        }
+        let k = pks.len() / C::PK_BYTES;
+        let mut status = vec![0u8; k];
+        let rc = unsafe { sys::blsgpu_keyset_append(self.ctx, keys.id, format_id(format), k, pks.as_ptr(), status.as_mut_ptr()) };
+        self.check(rc)?;
+        keys.len += k;
+        Ok(status)
     }
 
     /// Frees the device memory of a key set now (dropping the engine frees every set it still holds).

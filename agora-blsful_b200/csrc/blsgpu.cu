@@ -79,8 +79,8 @@ constexpr size_t REDUCE_WIDE_MAX = 4096;
 // bump allocator over one device buffer, regrown between calls
 struct Arena {
   uint8_t* base = nullptr;
-  size_t cap = 0, off = 0;
-  bool over = false;  // a take ran past the capacity the entry point sized: every later launch is refused (ARENA_OK)
+  size_t cap = 0, budget = 0, off = 0;  // budget: the bytes the call counted its takes to need (cap may hold more)
+  bool over = false;  // a take ran past the call's budget: every later launch is refused (ARENA_OK)
   template <class T>
   static size_t bytes(size_t count) {
     return (count * sizeof(T) + 255) & ~size_t(255);
@@ -89,19 +89,36 @@ struct Arena {
   T* take(size_t count) {
     T* p = reinterpret_cast<T*>(base + off);
     off += bytes<T>(count);
-    if (off > cap) over = true;
+    if (off > budget) over = true;
     return p;
   }
 };
-// counts what a sequence of Arena takes occupies, without memory: budgets derived from the takes themselves
+// counts what a sequence of Arena takes occupies at its peak, without memory: every budget is its takes counted
 struct ArenaSize {
-  size_t off = 0;
+  size_t off = 0, peak = 0;
   template <class T>
   T* take(size_t count) {
     off += Arena::bytes<T>(count);
+    peak = std::max(peak, off);
     return nullptr;
   }
 };
+// `count` T of scratch handed back to the arena at once: later takes reuse it, which is safe for work ordered after its
+// last reader on one stream
+template <class T, class A>
+T* take_back(A& a, size_t count) {
+  const size_t mark = a.off;
+  T* p = a.template take<T>(count);
+  a.off = mark;
+  return p;
+}
+// the peak of the takes that takes(a) makes
+template <class Takes>
+size_t counted(const Takes& takes) {
+  ArenaSize a;
+  takes(a);
+  return a.peak;
+}
 
 struct Level {
   size_t off, cnt;
@@ -147,8 +164,7 @@ struct blsgpu_ctx {
   std::vector<int> devices;
   std::unique_ptr<PendingSlice> pending;  // invalidated by every call that re-plans the arena
   std::unordered_map<uint64_t, KeySet> keysets;  // by id: ids come from a process-wide counter and are never reused
-  uint8_t* fold_scratch = nullptr;        // small device buffer of the fold (blsgpu_final_exp_is_one), apart from the arena
-  size_t fold_cap = 0;
+  Arena fold;  // small device buffer of the fold (blsgpu_final_exp_is_one, fold_roots), apart from the arena
   std::vector<blsgpu_ctx*> peers;  // one single-device context per further device (devices[1..]); see verify_host_common
   cudaStream_t stream = nullptr;
   cudaStream_t own_stream = nullptr;
@@ -181,10 +197,12 @@ struct blsgpu_ctx {
 
 namespace {
 
+// an arena of at least `bytes`, the call's budget (an ArenaSize count of its takes)
 int ensure_arena(blsgpu_ctx* ctx, size_t bytes) {
   ctx->pending.reset();  // the arena is about to be handed out again
   ctx->arena.off = 0;
   ctx->arena.over = false;
+  ctx->arena.budget = bytes;
   if (ctx->arena.cap >= bytes) return BLSGPU_OK;
   if (ctx->arena.base) CK(cudaFree(ctx->arena.base));  // the device may not hold the old and the new arena at once
   ctx->arena.base = nullptr;
@@ -250,7 +268,7 @@ int check_launch(blsgpu_ctx* ctx, const char* what) {
 }
 #define ARENA_OK()                                                          \
   do {                                                                      \
-    if (ctx->arena.over) {                                                  \
+    if (ctx->arena.over || ctx->fold.over) {                                \
       ctx->err = "internal: device scratch arena sized too small";          \
       return BLSGPU_E_ALLOC;                                                \
     }                                                                       \
@@ -270,6 +288,15 @@ int check_launch(blsgpu_ctx* ctx, const char* what) {
     kernel_end(ctx, km_, ctx->stream);                          \
     CKR(check_launch(ctx, #name));                              \
   } while (0)
+
+// sizes the arena for the takes that takes(a) makes, then makes them on it
+template <class Takes>
+int arena_takes(blsgpu_ctx* ctx, const Takes& takes) {
+  CKR(ensure_arena(ctx, counted(takes)));
+  takes(ctx->arena);
+  ARENA_OK();
+  return BLSGPU_OK;
+}
 
 size_t kernel_begin(blsgpu_ctx* ctx, int id, cudaStream_t stream);
 void kernel_end(blsgpu_ctx* ctx, size_t k, cudaStream_t stream);
@@ -410,6 +437,33 @@ SegLevels seg_levels(std::vector<size_t> cnt) {
 // product of Miller values (root of the product tree) and its sum of r_i sig_i in device memory; pipeline_check decides
 // F * e(-g, S) == 1 for this slice alone; pipeline_bisect finds the exact failures of a slice whose check failed.
 // -----------------------------------------------------------------------------------------------------------------
+// The bucket multi-scalar multiplication S = sum r_i sig_i over n items, r_i = rlc_scalar(root, i) (0 for an item whose
+// status is not OK): its window plan, and its takes
+struct MsmPlan {
+  int c, nwin;
+  size_t nbuckets, nchunks;
+  std::vector<Level> lm;  // the tree over the chunk sums
+  MsmPlan(size_t n, int rbits) : c(msm_window_bits(n, rbits)), nwin((rbits + c - 1) / c) {
+    nbuckets = ((size_t)1 << c) * nwin;
+    nchunks = nbuckets / MSM_CHUNK;
+    lm = make_levels(nchunks);
+  }
+};
+template <class SigJ>
+struct MsmScratch {
+  RlcScalar* r = nullptr;
+  uint32_t *cnt = nullptr, *sorted = nullptr;  // cnt: histograms, offsets, cursors
+  SigJ *B = nullptr, *V = nullptr;
+};
+template <class SigJ, class A>
+void take_msm(A& a, size_t n, const MsmPlan& m, MsmScratch<SigJ>& s) {
+  s.r = a.template take<RlcScalar>(n);
+  s.cnt = a.template take<uint32_t>(3 * m.nbuckets);
+  s.sorted = a.template take<uint32_t>((size_t)m.nwin * n);
+  s.B = a.template take<SigJ>(m.nbuckets);
+  s.V = a.template take<SigJ>(levels_total(m.lm));
+}
+
 // blocks of the node-level bucket method of the failure path (a warp per level-1 node, four per block)
 size_t node_msm_blocks(const blsgpu_ctx* ctx, size_t n1) { return std::max<size_t>(1, std::min<size_t>((n1 + 3) / 4, (size_t)ctx->sm_count * 4)); }
 constexpr size_t PROBE_SMALL = 16;  // probes the dedicated scratch holds (the root check; small batches' bisection levels)
@@ -425,8 +479,12 @@ struct Pipe {
   uint8_t* d_status = nullptr;
   Fp12* d_F = nullptr;
   SigJ *d_S = nullptr, *d_Sitem = nullptr, *d_msm_root = nullptr;
-  RlcScalar* d_r = nullptr;  // the scalars of the bucket path (use_msm)
-  Digest* d_root = nullptr;
+  MsmScratch<SigJ> msm;  // the bucket path (use_msm); its scalars msm.r are kept for the failure path
+  Digest *d_dig = nullptr, *d_root = nullptr;
+  // the failure path's node bucket method (by_nodes): bucket scratch, window sums of the level-1 nodes, item / group lists
+  bool by_nodes = false;
+  SigJ *node_buckets = nullptr, *node_W = nullptr;
+  uint32_t* d_list = nullptr;
   uint8_t* d_ok = nullptr;
   uint32_t* d_idx = nullptr;
   // probe scratch: a small dedicated one, and (after the Miller stage) the first line buffer for levels with many probes
@@ -437,8 +495,9 @@ struct Pipe {
   SLineRec* x_lines = nullptr;
   Fp12* x_T = nullptr;
   size_t x_cap = 0;            // probes per launch the point / status / T scratch holds
-  M6Arg* big_args = nullptr;   // line buffer 0 of the Miller stage, free once the stage is done
-  SLineRec* big_lines = nullptr;
+  // the line buffers of the Miller stage (take_lines); buffer 0 is free for the probes once the stage is done
+  M6Arg* m6_args[2] = {nullptr, nullptr};
+  SLineRec* m6_lines[2] = {nullptr, nullptr};
   size_t big_items = 0;
   bool root_T_ready = false;   // T = ML(-g, S_root) already computed beside the Miller stage (x_T[0])
   const Fp12* rootF() const { return d_F + lv.back().off; }
@@ -453,7 +512,7 @@ struct Pipe {
 // most one node per leaf)
 size_t probe_cap(size_t leaves) { return std::max<size_t>(PROBE_SMALL, std::min<size_t>(leaves, 4096) + 16); }
 // The probe scratch of P for `cap` probes per launch: indices and verdicts, the points and statuses of six pairs per probe,
-// the T values, and the Miller buffers of one small round.  A takes from an Arena, or counts bytes (ArenaSize: probe_scratch_bytes).
+// the T values, and the Miller buffers of one small round.  A takes from an Arena, or counts bytes (ArenaSize).
 template <class PkA, class SigA, class A>
 void take_probe_scratch(A& a, Pipe<PkA, SigA>& P, size_t cap) {
   const size_t small = std::min(cap, PROBE_SMALL);
@@ -467,12 +526,16 @@ void take_probe_scratch(A& a, Pipe<PkA, SigA>& P, size_t cap) {
   P.x_args = a.template take<M6Arg>(6 * small);
   P.x_lines = a.template take<SLineRec>(6 * small * M6_LINE_RECS);
 }
-template <class PkA, class SigA>
-size_t probe_scratch_bytes(size_t cap) {
-  ArenaSize a;
-  Pipe<PkA, SigA> P;
-  take_probe_scratch(a, P, cap);
-  return a.off;
+// The line buffers of a Miller stage over n items in passes of `chunk` (miller_stage): one, or two when the stage takes
+// several passes.  chunk 0 takes none: a call's takes counted with chunk 0 are what plan_m6_chunk plans the passes around.
+template <class PkA, class SigA, class A>
+void take_lines(A& a, Pipe<PkA, SigA>& P, size_t n, size_t chunk) {
+  if (chunk == 0) return;
+  P.big_items = std::max<size_t>(std::min(n, chunk), 6 * PROBE_SMALL);
+  for (int b = 0; b < (n > chunk ? 2 : 1); b++) {
+    P.m6_args[b] = a.template take<M6Arg>(P.big_items);
+    P.m6_lines[b] = a.template take<SLineRec>(P.big_items * M6_LINE_RECS);
+  }
 }
 // dynamic shared memory of the probe kernels, per device and per call (microseconds): a context per device may run this
 // from several host threads
@@ -570,7 +633,7 @@ int probe_rounds(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, const std::vector<uint32_t
     const size_t cnt = std::min(per, idx.size() - lo);
     CK(cudaMemcpyAsync(P.d_idx, idx.data() + lo, cnt * 4, cudaMemcpyHostToDevice, ctx->stream));
     CKR(fill(cnt));
-    CKR((probe_miller<PkA, SigA>(ctx, P, ctx->stream, cnt, big ? P.big_args : P.x_args, big ? P.big_lines : P.x_lines)));
+    CKR((probe_miller<PkA, SigA>(ctx, P, ctx->stream, cnt, big ? P.m6_args[0] : P.x_args, big ? P.m6_lines[0] : P.x_lines)));
     CKR((probe_final<PkA, SigA>(ctx, P, cnt, F ? P.d_idx : nullptr, F, P.d_ok)));
     CKR(after(lo, cnt));
     CK(cudaStreamSynchronize(ctx->stream));
@@ -596,24 +659,16 @@ int probe_level(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, const std::vector<uint32_t>
 
 // The Miller stage over n items: F[g] = prod over the items of group g of ML(r pk, H), after ctx->ev_fork.  prep(stream, cn,
 // base, args) launches the kernel that fills the M6Arg records of items [base, base + cn).  The line stream is 39 KB per item:
-// batches beyond one pass (ctx->m6_chunk) go through in chunks with two line buffers, chunk c's lines produced on side
-// stream 0 while chunk c-1's accumulator consumes the other buffer on side stream 1.  Line buffer 0 is left in P.big_* for
-// the probes of the failure path.
+// batches beyond one pass (ctx->m6_chunk) go through in chunks with two line buffers (P.m6_*, taken by take_lines with the
+// same chunk), chunk c's lines produced on side stream 0 while chunk c-1's accumulator consumes the other buffer on side
+// stream 1.
 template <class PkA, class SigA, class Prep>
 int miller_stage(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t n, const PkA* d_pk, const SigA* d_h, const uint8_t* d_status, Fp12* d_F,
                  const Prep& prep) {
   const size_t M6_CHUNK = ctx->m6_chunk;  // planned by the entry point together with the arena size (plan_m6_chunk)
-  const size_t chunk = std::max<size_t>(std::min(n, M6_CHUNK), 6 * PROBE_SMALL);
   const int nbuf = n > M6_CHUNK ? 2 : 1;
-  M6Arg* d_args[2];
-  SLineRec* d_lines[2];
-  for (int b = 0; b < nbuf; b++) {
-    d_args[b] = ctx->arena.take<M6Arg>(chunk);
-    d_lines[b] = ctx->arena.take<SLineRec>(chunk * M6_LINE_RECS);
-  }
-  P.big_args = d_args[0];
-  P.big_lines = d_lines[0];
-  P.big_items = chunk;
+  M6Arg* const* d_args = P.m6_args;
+  SLineRec* const* d_lines = P.m6_lines;
   ARENA_OK();
   CK(cudaStreamWaitEvent(ctx->side[0], ctx->ev_fork, 0));
   CK(cudaStreamWaitEvent(ctx->side[1], ctx->ev_fork, 0));
@@ -645,47 +700,18 @@ int miller_stage(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t n, const PkA* d_pk,
   return BLSGPU_OK;
 }
 
-// The bucket multi-scalar multiplication S = sum r_i sig_i over n items, r_i = rlc_scalar(root, i) (0 for an item whose
-// status is not OK): its window plan, and its takes from an Arena (or an ArenaSize: msm_bytes)
-struct MsmPlan {
-  int c, nwin;
-  size_t nbuckets, nchunks;
-  std::vector<Level> lm;  // the tree over the chunk sums
-  MsmPlan(size_t n, int rbits) : c(msm_window_bits(n, rbits)), nwin((rbits + c - 1) / c) {
-    nbuckets = ((size_t)1 << c) * nwin;
-    nchunks = nbuckets / MSM_CHUNK;
-    lm = make_levels(nchunks);
-  }
-};
-template <class SigJ, class A>
-void take_msm(A& a, size_t n, const MsmPlan& m, RlcScalar*& d_r, uint32_t*& d_cnt, uint32_t*& d_sorted, SigJ*& d_B, SigJ*& d_V) {
-  d_r = a.template take<RlcScalar>(n);
-  d_cnt = a.template take<uint32_t>(3 * m.nbuckets);  // histograms, offsets, cursors
-  d_sorted = a.template take<uint32_t>((size_t)m.nwin * n);
-  d_B = a.template take<SigJ>(m.nbuckets);
-  d_V = a.template take<SigJ>(levels_total(m.lm));
-}
-template <class SigJ>
-size_t msm_bytes(size_t n, int rbits) {
-  ArenaSize a;
-  RlcScalar* r;
-  uint32_t *cnt, *sorted;
-  SigJ *B, *V;
-  take_msm(a, n, MsmPlan(n, rbits), r, cnt, sorted, B, V);
-  return a.off;
-}
-// *r_out = the scalars (kept for the failure path and the key side of blsgpu_verify_batch_grouped), *sum_out = S
+// S = sum r_i sig_i in the scratch s (take_msm with MsmPlan(n, rbits)): s.r = the scalars (kept for the failure path and the
+// key side of blsgpu_verify_batch_grouped), *sum_out = S
 template <class SigA>
-int msm_sum(blsgpu_ctx* ctx, size_t n, const SigA* d_sig, const uint8_t* d_status, const Digest* d_root, int rbits, RlcScalar** r_out,
-            typename PtInfo<SigA>::Jac** sum_out) {
+int msm_sum(blsgpu_ctx* ctx, size_t n, const SigA* d_sig, const uint8_t* d_status, const Digest* d_root, int rbits,
+            const MsmScratch<typename PtInfo<SigA>::Jac>& s, typename PtInfo<SigA>::Jac** sum_out) {
   typedef typename PtInfo<SigA>::Jac SigJ;
   const MsmPlan m(n, rbits);
   const int c = m.c, nwin = m.nwin;
   const size_t nbuckets = m.nbuckets, nchunks = m.nchunks;
-  RlcScalar* d_r;
-  uint32_t *d_cnt, *d_sorted;
-  SigJ *d_B, *d_V;
-  take_msm(ctx->arena, n, m, d_r, d_cnt, d_sorted, d_B, d_V);
+  RlcScalar* d_r = s.r;
+  uint32_t *d_cnt = s.cnt, *d_sorted = s.sorted;
+  SigJ *d_B = s.B, *d_V = s.V;
   uint32_t *d_off = d_cnt + nbuckets, *d_cur = d_off + nbuckets;
   CK(cudaMemsetAsync(d_cnt, 0, nbuckets * sizeof(uint32_t), ctx->stream));
   LAUNCH(k_msm_count, blocks_for(n), TPB, n, (const uint8_t*)d_status, (const Digest*)d_root, rbits, c, nwin, d_r, d_cnt);
@@ -695,34 +721,59 @@ int msm_sum(blsgpu_ctx* ctx, size_t n, const SigA* d_sig, const uint8_t* d_statu
          (const uint32_t*)d_sorted, d_B);
   LAUNCH((k_msm_chunk<SigJ>), blocks_for(nchunks), TPB, nchunks, c, (const SigJ*)d_B, d_V);
   CKR(reduce_levels(ctx, m.lm, 0, nullptr, d_V));
-  *r_out = d_r;
   *sum_out = d_V + m.lm.back().off;
   return BLSGPU_OK;
 }
 
-template <class PkA, class SigA>
-int pipeline_partials(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t n, const PkA* d_pk, const SigA* d_sig, const SigA* d_h, uint8_t* d_status,
-                      bool use_rlc) {
+// Every take of the pipeline over n items (pipeline_partials): the product / sum trees, the leaf digests, the probe scratch
+// (the line records of big levels go through the Miller stage's buffer 0), the bucket MSM, the Miller line buffers for passes
+// of `chunk` items, and pipeline_bisect's scratch for the worst case it allows (every level-1 node and group failing).
+template <class PkA, class SigA, class A>
+void take_pipe(A& a, Pipe<PkA, SigA>& P, const blsgpu_ctx* ctx, size_t n, bool use_rlc, size_t chunk) {
   typedef typename PtInfo<SigA>::Jac SigJ;
   P.n = n;
   P.use_rlc = use_rlc;
+  P.rbits = use_rlc ? ctx->rlc_bits : 0;
+  P.use_msm = use_rlc && n >= MSM_MIN_ITEMS;
+  // leaves of the product/sum trees are GROUPS of 6 consecutive items (the cooperative Miller kernel's unit)
+  const size_t ng = P.ng = (n + M6_GROUP - 1) / M6_GROUP;
+  P.lv = make_levels(ng);
+  const size_t total = levels_total(P.lv);
+  P.d_F = a.template take<Fp12>(total);
+  P.d_S = a.template take<SigJ>(use_rlc ? total : 1);
+  P.d_Sitem = a.template take<SigJ>(use_rlc ? n : 1);
+  P.d_dig = a.template take<Digest>(levels_total(make_levels(n)) + 2);  // the digest tree, then [root, salt]
+  take_probe_scratch(a, P, probe_cap(ng));
+  if (P.use_msm) take_msm(a, n, MsmPlan(n, P.rbits), P.msm);
+  take_lines(a, P, n, chunk);
+  P.by_nodes = P.use_msm && P.rbits == 64 && P.lv.size() >= 3;
+  if (P.by_nodes) {
+    const size_t n1 = P.lv[1].cnt;
+    P.node_buckets = a.template take<SigJ>(node_msm_blocks(ctx, n1) * 128 * NODE_BUCKETS);
+    P.node_W = a.template take<SigJ>(n1 * 32);
+    P.d_list = a.template take<uint32_t>(n + ng);
+  }
+}
+
+// the pipeline over the n items of P (taken by take_pipe with ctx->m6_chunk)
+template <class PkA, class SigA>
+int pipeline_partials(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, const PkA* d_pk, const SigA* d_sig, const SigA* d_h, uint8_t* d_status) {
+  typedef typename PtInfo<SigA>::Jac SigJ;
+  const size_t n = P.n;
+  const bool use_rlc = P.use_rlc;
   P.d_pk = d_pk;
   P.d_sig = d_sig;
   P.d_h = d_h;
   P.d_status = d_status;
-  // leaves of the product/sum trees are GROUPS of 6 consecutive items (the cooperative Miller kernel's unit)
-  const size_t ng = P.ng = (n + M6_GROUP - 1) / M6_GROUP;
-  std::vector<Level>& lv = P.lv = make_levels(ng);
-  size_t total = levels_total(lv);
-  Fp12* d_F = P.d_F = ctx->arena.take<Fp12>(total);
-  SigJ* d_S = P.d_S = ctx->arena.take<SigJ>(use_rlc ? total : 1);
-  P.d_Sitem = ctx->arena.take<SigJ>(use_rlc ? n : 1);
-  Digest* d_dig = ctx->arena.take<Digest>(levels_total(make_levels(n)) + 2);
-  Digest* d_root = P.d_root = d_dig + levels_total(make_levels(n));  // [root, salt]
-  take_probe_scratch(ctx->arena, P, probe_cap(ng));  // the line records of big levels go through the Miller stage's buffer
+  const size_t ng = P.ng;
+  const std::vector<Level>& lv = P.lv;
+  Fp12* d_F = P.d_F;
+  SigJ* d_S = P.d_S;
+  Digest* d_dig = P.d_dig;
+  Digest* d_root = P.d_root = d_dig + levels_total(make_levels(n));
   CKR((set_probe_smem<PkA, SigA>(ctx)));
 
-  const int rbits = P.rbits = use_rlc ? ctx->rlc_bits : 0;
+  const int rbits = P.rbits;
   if (use_rlc) {
     CKR(fresh_salt(ctx));
     LAUNCH((k_leaf_digest<PkA, SigA>), blocks_for(n), TPB, n, d_pk, d_sig, d_h, d_dig);
@@ -733,8 +784,8 @@ int pipeline_partials(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P, size_t n, const PkA* 
   // run on the aux stream beside the Miller kernels.  Small batches: per-item scaling.
   // (Running the bucket kernels themselves beside the Miller stage was measured: they evict Miller blocks, +70 ms at 1M.)
   stage_mark(ctx, BLSGPU_STAGE_SCALE_SIG);
-  const bool use_msm = P.use_msm = use_rlc && n >= MSM_MIN_ITEMS;
-  if (use_msm) CKR((msm_sum<SigA>(ctx, n, d_sig, d_status, d_root, rbits, &P.d_r, &P.d_msm_root)));
+  const bool use_msm = P.use_msm;
+  if (use_msm) CKR((msm_sum<SigA>(ctx, n, d_sig, d_status, d_root, rbits, P.msm, &P.d_msm_root)));
   CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
   P.root_T_ready = false;
   if (use_msm) {
@@ -829,7 +880,7 @@ int pipeline_bisect(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P) {
   // The bucket method gave the total only.  64-bit scalars: the sums of the LEVEL-1 nodes come from a small bucket method per
   // node (k_node_msm: ~21 point operations per item), the levels above from the tree, and only the groups of level-1 nodes
   // that FAIL get per-item scalar multiplications.  Otherwise (128-bit scalars): per-item scaling of the whole batch.
-  const bool by_nodes = P.use_msm && P.rbits == 64 && lv.size() >= 3;
+  const bool by_nodes = P.by_nodes;
   if (P.use_msm && !by_nodes) {
     LAUNCH((k_scale_sig<SigA>), blocks_for(n), TPB, n, P.d_sig, P.d_status, P.d_root, P.rbits, P.d_Sitem);
     LAUNCH((k_group_sum<SigJ>), blocks_for(ng), TPB, n, (const SigJ*)P.d_Sitem, ng, P.d_S);
@@ -837,10 +888,9 @@ int pipeline_bisect(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P) {
   }
   if (by_nodes) {
     const size_t n1 = lv[1].cnt, nblocks = node_msm_blocks(ctx, n1);
-    SigJ* d_buckets = ctx->arena.take<SigJ>(nblocks * 128 * NODE_BUCKETS);
-    SigJ* d_W = ctx->arena.take<SigJ>(n1 * 32);
-    LAUNCH((k_node_msm<SigA>), (unsigned)nblocks, 128, n, n1, ng, P.d_sig, (const uint8_t*)P.d_status, (const RlcScalar*)P.d_r, d_buckets, d_W);
-    LAUNCH((k_node_combine<SigJ>), blocks_for(n1), TPB, n1, (const SigJ*)d_W, P.d_S + lv[1].off);
+    LAUNCH((k_node_msm<SigA>), (unsigned)nblocks, 128, n, n1, ng, P.d_sig, (const uint8_t*)P.d_status, (const RlcScalar*)P.msm.r, P.node_buckets,
+           P.node_W);
+    LAUNCH((k_node_combine<SigJ>), blocks_for(n1), TPB, n1, (const SigJ*)P.node_W, P.d_S + lv[1].off);
     CKR(reduce_levels(ctx, lv, 1, nullptr, P.d_S));
   }
   std::vector<uint32_t> bad;
@@ -851,8 +901,7 @@ int pipeline_bisect(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P) {
     for (uint32_t g : cand)
       for (int m = 0; m < M6_GROUP; m++)
         if ((size_t)g * M6_GROUP + m < n) its.push_back(g * M6_GROUP + m);
-    uint32_t* d_list = ctx->arena.take<uint32_t>(its.size() + cand.size());
-    ARENA_OK();
+    uint32_t* d_list = P.d_list;  // its.size() <= n, cand.size() <= ng
     CK(cudaMemcpyAsync(d_list, its.data(), its.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaMemcpyAsync(d_list + its.size(), cand.data(), cand.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
     LAUNCH((k_scale_sig_list<SigA>), blocks_for(its.size()), TPB, its.size(), (const uint32_t*)d_list, P.d_sig, (const uint8_t*)P.d_status,
@@ -892,37 +941,19 @@ int check_and_bisect(blsgpu_ctx* ctx, Pipe<PkA, SigA>& P) {
   return BLSGPU_OK;
 }
 
-// device scratch of pipeline_partials for n items, without the Miller line buffers
-template <class PkA, class SigA>
-size_t pipeline_other_bytes(size_t n) {
-  typedef typename PtInfo<SigA>::Jac SigJ;
-  size_t total = levels_total(make_levels(std::max<size_t>(n, 1)));
-  size_t gtotal = levels_total(make_levels((std::max<size_t>(n, 1) + M6_GROUP - 1) / M6_GROUP));
-  return gtotal * (sizeof(Fp12) + sizeof(SigJ)) + n * (sizeof(SigJ) + sizeof(Fp12) + sizeof(SigJ)) + total * sizeof(Digest) +
-         n * (16 + 4 * 32) + ((size_t)32 << 16) * (12 + 2 * sizeof(SigJ)) + (1 << 20) + (n + 64) * 8 + 16 * 256 + 4096 +
-         probe_scratch_bytes<PkA, SigA>(probe_cap((n + M6_GROUP - 1) / M6_GROUP)) +
-         // failure path of the bucket route: window sums of the level-1 nodes, bucket scratch of 592 x 4 warps at most, item / group lists
-         (n >= MSM_MIN_ITEMS ? (n / 96 + 2) * 32 * sizeof(SigJ) + std::min<size_t>(n / 384 + 1, 592) * 128 * NODE_BUCKETS * sizeof(SigJ) + n * 5 + 8 * 256 : 0);
-}
-size_t m6_line_bytes(size_t n, size_t chunk) {
-  return (n > chunk ? 2 : 1) * std::max<size_t>(std::min(std::max<size_t>(n, 1), chunk), 6 * PROBE_SMALL) * M6_ITEM_BYTES;
-}
-// Plans the pass size of the Miller kernels for a call over n Miller items and sizes the arena: `other` is everything the
-// call takes from the arena besides the Miller line buffers.  If the allocation fails the pass size is halved (more passes)
-// until it fits or reaches the minimum.
-int ensure_miller_arena(blsgpu_ctx* ctx, size_t n, size_t other) {
-  plan_m6_chunk(ctx, n, other);
+// Plans the pass size of the Miller kernels for a call over n Miller items and sizes the arena for takes(a, chunk), the
+// call's takes with line buffers for passes of `chunk` items (take_lines).  If the allocation fails the pass size is halved
+// (more passes) until it fits or reaches the minimum.
+template <class Takes>
+int ensure_miller_arena(blsgpu_ctx* ctx, size_t n, const Takes& takes) {
+  auto bytes = [&](size_t chunk) { return counted([&](auto& a) { takes(a, chunk); }); };
+  plan_m6_chunk(ctx, n, bytes(0));
   for (;;) {
-    const int r = ensure_arena(ctx, other + m6_line_bytes(n, ctx->m6_chunk));
+    const int r = ensure_arena(ctx, bytes(ctx->m6_chunk));
     if (r != BLSGPU_E_ALLOC || ctx->m6_chunk <= M6_CHUNK_MIN || n <= M6_CHUNK_MIN) return r;
     (void)cudaGetLastError();
     ctx->m6_chunk = std::max(M6_CHUNK_MIN, std::min(ctx->m6_chunk, n) / 2 / 120 * 120);
   }
-}
-// the same for the pipeline over n items: `head_bytes` is what the entry point takes besides the pipeline's own scratch
-template <class PkA, class SigA>
-int ensure_pipeline_arena(blsgpu_ctx* ctx, size_t n, size_t head_bytes) {
-  return ensure_miller_arena(ctx, n, head_bytes + pipeline_other_bytes<PkA, SigA>(n));
 }
 
 // compressed bytes -> affine points + per-item status: decompression (square root), then the subgroup check
@@ -951,24 +982,39 @@ int load_keys(blsgpu_ctx* ctx, size_t n, const Keys& d_keys, int format, PkA* d_
   return BLSGPU_OK;
 }
 
-// hash_to_curve of n framed messages into affine points: k_hash leaves Jacobian points in scratch that is handed back to
-// the arena at once (later takes on the same stream may reuse it), k_to_affine_batch normalises them 16 per inversion
+// the Jacobian scratch of hash_points over n messages: handed back to the arena at once, later takes reuse it
+template <class HA, class A>
+typename PtInfo<HA>::Jac* take_hash_scratch(A& a, size_t n) {
+  return take_back<typename PtInfo<HA>::Jac>(a, n);
+}
+// hash_to_curve of n framed messages into affine points: k_hash leaves Jacobian points in d_hj (take_hash_scratch),
+// k_to_affine_batch normalises them 16 per inversion
 template <class HA, class PkA>
 int hash_points(blsgpu_ctx* ctx, size_t n, const uint8_t* d_msgs, const uint64_t* d_moff, int msg_mode, const PkA* d_pk,
-                const uint8_t* d_pre, const DstParam& dst, HA* d_h) {
+                const uint8_t* d_pre, const DstParam& dst, typename PtInfo<HA>::Jac* d_hj, HA* d_h) {
   typedef typename PtInfo<HA>::Jac HJ;
-  size_t mark = ctx->arena.off;
-  HJ* d_hj = ctx->arena.take<HJ>(n);
-  if (ctx->arena.off > ctx->arena.cap) {
-    ctx->err = "hash_points: arena too small";
-    return BLSGPU_E_ALLOC;
-  }
   LAUNCH_TIMED(BLSGPU_KERNEL_HASH_MAP, (k_hash<HA, PkA>), blocks_for(n), TPB, n, d_msgs, d_moff, msg_mode, d_pk, d_pre, dst, d_hj);
   LAUNCH_TIMED(BLSGPU_KERNEL_CLEAR_COFACTOR, (k_clear_cofactor<HA>), blocks_for(n), TPB, n, d_hj);
   LAUNCH_TIMED(BLSGPU_KERNEL_TO_AFFINE, (k_to_affine_batch<HA>), blocks_for((n + TO_AFFINE_BATCH - 1) / TO_AFFINE_BATCH), TPB, n,
                (const HJ*)d_hj, d_h);
-  ctx->arena.off = mark;
   return BLSGPU_OK;
+}
+
+// the takes of verify_points_partials over n items: the message points, the hash scratch, the pipeline (take_pipe)
+template <int IMPL, class A>
+void take_verify_points(A& a, const blsgpu_ctx* ctx, size_t n, size_t chunk, typename ImplT<IMPL>::SigAff*& d_h,
+                        typename PtInfo<typename ImplT<IMPL>::SigAff>::Jac*& d_hj, Pipe<typename ImplT<IMPL>::PkAff, typename ImplT<IMPL>::SigAff>& P) {
+  d_h = a.template take<typename ImplT<IMPL>::SigAff>(n);
+  d_hj = take_hash_scratch<typename ImplT<IMPL>::SigAff>(a, n);
+  take_pipe(a, P, ctx, n, true, chunk);
+}
+// the same counted, for the budget of a call that ends in verify_points_partials
+template <int IMPL, class A>
+void take_verify_points(A& a, const blsgpu_ctx* ctx, size_t n, size_t chunk) {
+  typename ImplT<IMPL>::SigAff* d_h;
+  typename PtInfo<typename ImplT<IMPL>::SigAff>::Jac* d_hj;
+  Pipe<typename ImplT<IMPL>::PkAff, typename ImplT<IMPL>::SigAff> P;
+  take_verify_points<IMPL>(a, ctx, n, chunk, d_h, d_hj, P);
 }
 
 // verify over decoded points: per-item pre-status, hash_to_curve of the framed message, pairing pipeline
@@ -978,11 +1024,13 @@ int verify_points_partials(blsgpu_ctx* ctx, Pipe<typename ImplT<IMPL>::PkAff, ty
                            const uint8_t* d_stsig, const uint8_t* d_msgs, const uint64_t* d_moff, uint8_t* d_status_out) {
   typedef typename ImplT<IMPL>::PkAff PkA;
   typedef typename ImplT<IMPL>::SigAff SigA;
-  SigA* d_h = ctx->arena.take<SigA>(n);
+  SigA* d_h;
+  typename PtInfo<SigA>::Jac* d_hj;
+  take_verify_points<IMPL>(ctx->arena, ctx, n, ctx->m6_chunk, d_h, d_hj, P);
   LAUNCH((k_prestatus<PkA, SigA>), blocks_for(n), TPB, n, d_stpk, d_stsig, d_pk, d_sig, d_status_out);
   stage_mark(ctx, BLSGPU_STAGE_HASH);
-  CKR((hash_points<SigA, PkA>(ctx, n, d_msgs, d_moff, msg_mode, d_pk, (const uint8_t*)d_status_out, dst, d_h)));
-  return pipeline_partials<PkA, SigA>(ctx, P, n, d_pk, d_sig, d_h, d_status_out, true);
+  CKR((hash_points<SigA, PkA>(ctx, n, d_msgs, d_moff, msg_mode, d_pk, (const uint8_t*)d_status_out, dst, d_hj, d_h)));
+  return pipeline_partials<PkA, SigA>(ctx, P, d_pk, d_sig, d_h, d_status_out);
 }
 template <int IMPL>
 int verify_points(blsgpu_ctx* ctx, int msg_mode, const DstParam& dst, size_t n, const typename ImplT<IMPL>::PkAff* d_pk,
@@ -997,16 +1045,38 @@ int verify_points(blsgpu_ctx* ctx, int msg_mode, const DstParam& dst, size_t n, 
 
 // verify over device-resident inputs: compressed signatures, keys as bytes or key-set indices.  msg_mode: 0 msg, 1 pk||msg,
 // 2 pk bytes (PoP).  verify_dev_partials stops after the slice's partial results (its product of Miller values and sum of r_i sig_i).
+// n decoded keys and signatures and their statuses
+template <int IMPL>
+struct Decoded {
+  typename ImplT<IMPL>::PkAff* pk = nullptr;
+  typename ImplT<IMPL>::SigAff* sig = nullptr;
+  uint8_t *stpk = nullptr, *stsig = nullptr;
+};
+template <int IMPL, class A>
+void take_decoded(A& a, size_t n, Decoded<IMPL>& D) {
+  D.pk = a.template take<typename ImplT<IMPL>::PkAff>(n);
+  D.sig = a.template take<typename ImplT<IMPL>::SigAff>(n);
+  D.stpk = a.template take<uint8_t>(n);
+  D.stsig = a.template take<uint8_t>(n);
+}
+// the takes of verify_dev_partials over n items counted, for the budget of a call that ends in it
+template <int IMPL, class A>
+void take_verify_dev(A& a, const blsgpu_ctx* ctx, size_t n, size_t chunk) {
+  Decoded<IMPL> D;
+  take_decoded(a, n, D);
+  take_verify_points<IMPL>(a, ctx, n, chunk);
+}
 template <int IMPL>
 int verify_dev_partials(blsgpu_ctx* ctx, Pipe<typename ImplT<IMPL>::PkAff, typename ImplT<IMPL>::SigAff>& P, int msg_mode, const DstParam& dst,
                         int format, size_t n, const Keys& d_keys, const uint8_t* d_sigs, const uint8_t* d_msgs, const uint64_t* d_moff,
                         uint8_t* d_status_out) {
   typedef typename ImplT<IMPL>::PkAff PkA;
   typedef typename ImplT<IMPL>::SigAff SigA;
-  PkA* d_pk = ctx->arena.take<PkA>(n);
-  SigA* d_sig = ctx->arena.take<SigA>(n);
-  uint8_t* d_stpk = ctx->arena.take<uint8_t>(n);
-  uint8_t* d_stsig = ctx->arena.take<uint8_t>(n);
+  Decoded<IMPL> D;
+  take_decoded(ctx->arena, n, D);
+  PkA* d_pk = D.pk;
+  SigA* d_sig = D.sig;
+  uint8_t *d_stpk = D.stpk, *d_stsig = D.stsig;
   stage_reset(ctx);
   stage_mark(ctx, BLSGPU_STAGE_DECODE_PK);
   CKR((load_keys<PkA>(ctx, n, d_keys, format, d_pk, d_stpk)));
@@ -1028,37 +1098,46 @@ int verify_dev(blsgpu_ctx* ctx, int msg_mode, const DstParam& dst, int format, s
 // d_F[k], d_S[k] on this context's device: is  prod F_j * e(-g, sum S_j)  == 1 ?   One product/sum launch, one cooperative
 // probe, one six-lane final exponentiation - the "host multiplies the partials and runs a single final exponentiation" step
 // of the north star, executed on a GPU because the engine has no CPU arithmetic.
-// A over the fold scratch of at least `bytes` (a small device buffer apart from the arena, regrown between calls)
-int fold_arena(blsgpu_ctx* ctx, size_t bytes, Arena& A) {
-  if (ctx->fold_cap < bytes) {
-    if (ctx->fold_scratch) CK(cudaFree(ctx->fold_scratch));
-    ctx->fold_scratch = nullptr;
-    ctx->fold_cap = 0;
-    CK(cudaMalloc(&ctx->fold_scratch, bytes));
-    ctx->fold_cap = bytes;
+// fold_check's takes: the product / sum of the partial results, and the probe scratch (only that of P is used)
+template <class PkA, class SigA, class A>
+void take_fold_check(A& a, Pipe<PkA, SigA>& P, Fp12*& d_Froot, typename PtInfo<SigA>::Jac*& d_Sroot) {
+  d_Froot = a.template take<Fp12>(1);
+  d_Sroot = a.template take<typename PtInfo<SigA>::Jac>(1);
+  take_probe_scratch(a, P, 1);
+}
+// Sizes the fold scratch (a small device buffer apart from the arena, regrown between calls) for head(a) followed by
+// fold_check's takes, and makes head's takes from it.
+template <class PkA, class SigA, class Head>
+int fold_takes(blsgpu_ctx* ctx, const Head& head) {
+  const size_t bytes = counted([&](auto& a) {
+    head(a);
+    Pipe<PkA, SigA> P;
+    Fp12* F;
+    typename PtInfo<SigA>::Jac* S;
+    take_fold_check(a, P, F, S);
+  });
+  Arena& A = ctx->fold;
+  if (A.cap < bytes) {
+    if (A.base) CK(cudaFree(A.base));
+    A.base = nullptr;
+    A.cap = 0;
+    CK(cudaMalloc(&A.base, bytes));
+    A.cap = bytes;
   }
-  A = Arena();
-  A.base = ctx->fold_scratch;
-  A.cap = ctx->fold_cap;
+  A.off = 0;
+  A.budget = bytes;
+  A.over = false;
+  head(A);
+  ARENA_OK();
   return BLSGPU_OK;
 }
 template <class PkA, class SigA>
-size_t fold_bytes(size_t k) {
+int fold_check(blsgpu_ctx* ctx, size_t k, const Fp12* d_F, const typename PtInfo<SigA>::Jac* d_S, bool* ok_out) {
   typedef typename PtInfo<SigA>::Jac SigJ;
-  return (k + 2) * (sizeof(Fp12) + sizeof(SigJ) + sizeof(SigA) + PtInfo<SigA>::LEN + 600) + probe_scratch_bytes<PkA, SigA>(1) +
-         2 * sizeof(Fp12) + 64 * 256;
-}
-template <class PkA, class SigA>
-int fold_check(blsgpu_ctx* ctx, Arena& A, size_t k, const Fp12* d_F, const typename PtInfo<SigA>::Jac* d_S, bool* ok_out) {
-  typedef typename PtInfo<SigA>::Jac SigJ;
-  Pipe<PkA, SigA> P;  // only its probe scratch is used
-  Fp12* d_Froot = A.take<Fp12>(1);
-  SigJ* d_Sroot = A.take<SigJ>(1);
-  take_probe_scratch(A, P, 1);
-  if (A.over) {
-    ctx->err = "internal: fold scratch sized too small";
-    return BLSGPU_E_ALLOC;
-  }
+  Pipe<PkA, SigA> P;
+  Fp12* d_Froot;
+  SigJ* d_Sroot;
+  take_fold_check(ctx->fold, P, d_Froot, d_Sroot);
   CKR((set_probe_smem<PkA, SigA>(ctx)));
   if (k > 16) {
     ctx->err = "fold: at most 16 partial results";
@@ -1080,27 +1159,17 @@ template <class PkA, class SigA>
 int fold_roots(blsgpu_ctx* ctx, const std::vector<const Pipe<PkA, SigA>*>& P, bool* ok_out) {
   typedef typename PtInfo<SigA>::Jac SigJ;
   const size_t ndev = P.size();
-  Arena A;
-  CKR(fold_arena(ctx, fold_bytes<PkA, SigA>(ndev), A));
-  Fp12* d_Fk = A.take<Fp12>(ndev);
-  SigJ* d_Sk = A.take<SigJ>(ndev);
+  Fp12* d_Fk;
+  SigJ* d_Sk;
+  CKR((fold_takes<PkA, SigA>(ctx, [&](auto& a) {
+    d_Fk = a.template take<Fp12>(ndev);
+    d_Sk = a.template take<SigJ>(ndev);
+  })));
   for (size_t d = 0; d < ndev; d++) {
     CK(cudaMemcpyPeerAsync(d_Fk + d, ctx->devices[0], P[d]->rootF(), ctx->devices[d], sizeof(Fp12), ctx->stream));
     CK(cudaMemcpyPeerAsync(d_Sk + d, ctx->devices[0], P[d]->rootS(), ctx->devices[d], sizeof(SigJ), ctx->stream));
   }
-  return fold_check<PkA, SigA>(ctx, A, ndev, d_Fk, d_Sk, ok_out);
-}
-
-// what verify_dev takes from the arena before the pipeline's own scratch
-template <int IMPL>
-size_t verify_head_bytes(size_t n) {
-  typedef typename ImplT<IMPL>::PkAff PkA;
-  typedef typename ImplT<IMPL>::SigAff SigA;
-  return n * (sizeof(PkA) + 2 * sizeof(SigA) + 2) + 8 * 256;
-}
-template <int IMPL>
-int ensure_verify_arena(blsgpu_ctx* ctx, size_t n, size_t head_bytes) {
-  return ensure_pipeline_arena<typename ImplT<IMPL>::PkAff, typename ImplT<IMPL>::SigAff>(ctx, n, head_bytes + verify_head_bytes<IMPL>(n));
+  return fold_check<PkA, SigA>(ctx, ndev, d_Fk, d_Sk, ok_out);
 }
 
 bool args_ok(int impl_id, int scheme, int format) {
@@ -1191,35 +1260,42 @@ int check_keys(blsgpu_ctx* ctx, const char* what, int impl_id, Keys& keys, uint6
   return BLSGPU_OK;
 }
 
+// the device copy of `count` host T (take_up, then upload)
+template <class T, class A>
+T* take_up(A& a, size_t count) {
+  return a.template take<T>(std::max<size_t>(count, 1));
+}
 template <class T>
-int upload(blsgpu_ctx* ctx, T*& d, const T* h, size_t count) {
-  d = ctx->arena.take<T>(std::max<size_t>(count, 1));
+int upload(blsgpu_ctx* ctx, const T* d, const T* h, size_t count) {
   ARENA_OK();
-  if (count) CK(cudaMemcpyAsync(d, h, count * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
+  if (count) CK(cudaMemcpyAsync((void*)d, h, count * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
   return BLSGPU_OK;
 }
 // checked ragged records on the device as records from byte 0: the bytes off[0] .. off[n] and the offsets rebased to 0 (the
 // caller's offsets go up as they are when they start at 0: no host copy)
-int upload_records(blsgpu_ctx* ctx, const uint8_t* buf, const uint64_t* off, size_t n, uint8_t*& d_buf, uint64_t*& d_off) {
+template <class A>
+void take_records(A& a, const uint64_t* off, size_t n, uint8_t*& d_buf, uint64_t*& d_off) {
+  d_buf = take_up<uint8_t>(a, (size_t)(off[n] - off[0]));
+  d_off = take_up<uint64_t>(a, n + 1);
+}
+int upload_records(blsgpu_ctx* ctx, const uint8_t* buf, const uint64_t* off, size_t n, uint8_t* d_buf, uint64_t* d_off) {
   CKR(upload(ctx, d_buf, off[n] > off[0] ? buf + off[0] : buf, (size_t)(off[n] - off[0])));
   if (off[0] == 0) return upload(ctx, d_off, off, n + 1);
   const std::vector<uint64_t> r = rebased(off, 0, n);
   return upload(ctx, d_off, r.data(), n + 1);
 }
-// the keys of a call on the device: its compressed key bytes, or its key indices, uploaded to the arena
-template <class PkA>
-int upload_keys(blsgpu_ctx* ctx, size_t n, const Keys& keys, Keys& d_keys) {
+// the keys of a call on the device: its compressed key bytes, or its key indices, in the arena
+template <class PkA, class A>
+void take_keys(A& a, size_t n, const Keys& keys, Keys& d_keys) {
   d_keys = keys;
-  if (keys.set) {
-    uint32_t* d_idx;
-    CKR(upload(ctx, d_idx, keys.idx, n));
-    d_keys.idx = d_idx;
-  } else {
-    uint8_t* d_pks;
-    CKR(upload(ctx, d_pks, keys.bytes, n * PtInfo<PkA>::LEN));
-    d_keys.bytes = d_pks;
-  }
-  return BLSGPU_OK;
+  if (keys.set)
+    d_keys.idx = take_up<uint32_t>(a, n);
+  else
+    d_keys.bytes = take_up<uint8_t>(a, n * PtInfo<PkA>::LEN);
+}
+template <class PkA>
+int upload_keys(blsgpu_ctx* ctx, size_t n, const Keys& keys, const Keys& d_keys) {
+  return keys.set ? upload(ctx, d_keys.idx, keys.idx, n) : upload(ctx, d_keys.bytes, keys.bytes, n * PtInfo<PkA>::LEN);
 }
 
 int set_device(blsgpu_ctx* ctx) {
@@ -1314,7 +1390,7 @@ void blsgpu_ctx_destroy(blsgpu_ctx* ctx) {
   ctx->pending.reset();
   for (const auto& ks : ctx->keysets) free_keyset(ks.second);
   if (ctx->arena.base) cudaFree(ctx->arena.base);
-  if (ctx->fold_scratch) cudaFree(ctx->fold_scratch);
+  if (ctx->fold.base) cudaFree(ctx->fold.base);
   for (int i = 0; i <= BLSGPU_STAGE_COUNT; i++) cudaEventDestroy(ctx->ev[i]);
   for (const blsgpu_ctx::KernelMark& m : ctx->kmarks) {
     cudaEventDestroy(m.begin);
@@ -1389,29 +1465,45 @@ int blsgpu_verify_batch_dev(blsgpu_ctx* ctx, int impl_id, int scheme, int format
   make_dst(dst, impl_id, scheme, false);
   int mode = scheme == 1 ? 1 : 0;
   return with_impl(impl_id, [&](auto I) {
-    CKR(ensure_verify_arena<I>(ctx, n, 0));
+    CKR(ensure_miller_arena(ctx, n, [&](auto& a, size_t chunk) { take_verify_dev<decltype(I)::value>(a, ctx, n, chunk); }));
     return verify_dev<I>(ctx, mode, dst, format, n, pks_dev, sigs_dev, msgs_dev, msg_off_dev, status_out_dev);
   });
 }
 
 namespace {
-// host buffers of one slice -> its partial results (state in P, statuses so far in *d_st_out); the stream is synchronised
-template <int IMPL>
+// takes that make none (the tail of a call that takes nothing after its last step)
+struct NoTakes {
+  template <class A>
+  void operator()(A&) const {}
+};
+// host buffers of one slice -> its partial results (state in P, statuses so far in *d_st_out); the stream is synchronised.
+// The arena is sized for tail(a) as well: the takes the caller makes after this.
+template <int IMPL, class Tail = NoTakes>
 int host_partials(blsgpu_ctx* ctx, Pipe<typename ImplT<IMPL>::PkAff, typename ImplT<IMPL>::SigAff>& P, int msg_mode, const DstParam& dst, int format,
-                  size_t n, const Keys& keys, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off, uint8_t** d_st_out) {
+                  size_t n, const Keys& keys, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* msg_off, uint8_t** d_st_out,
+                  const Tail& tail = Tail()) {
   CKR(set_device(ctx));
-  const size_t pk_len = IMPL == 2 ? 48 : 96, sig_len = IMPL == 2 ? 96 : 48;
-  size_t msg_bytes = msg_off ? (size_t)(msg_off[n] - msg_off[0]) : 0;
-  size_t in_bytes = n * (pk_len + sig_len + 1) + msg_bytes + (n + 1) * 8 + 16 * 256 + 8192;  // key bytes or (fewer) key indices
-  CKR(ensure_verify_arena<IMPL>(ctx, n, in_bytes));
-  uint8_t *d_sigs, *d_msgs;
+  const size_t sig_len = IMPL == 2 ? 96 : 48;
+  const std::vector<uint64_t> no_msgs(msg_off ? 0 : n + 1, 0);  // PoP: every message empty
+  if (!msg_off) msg_off = no_msgs.data();
+  uint8_t *d_sigs, *d_msgs, *d_st;
   uint64_t* d_off;
   Keys d_keys;
+  auto head = [&](auto& a) {
+    take_keys<typename ImplT<IMPL>::PkAff>(a, n, keys, d_keys);
+    d_sigs = take_up<uint8_t>(a, n * sig_len);
+    take_records(a, msg_off, n, d_msgs, d_off);
+    d_st = a.template take<uint8_t>(n);
+  };
+  CKR(ensure_miller_arena(ctx, n, [&](auto& a, size_t chunk) {
+    head(a);
+    take_verify_dev<IMPL>(a, ctx, n, chunk);
+    tail(a);
+  }));
+  head(ctx->arena);
   CKR(upload_keys<typename ImplT<IMPL>::PkAff>(ctx, n, keys, d_keys));
   CKR(upload(ctx, d_sigs, sigs, n * sig_len));
-  const std::vector<uint64_t> no_msgs(msg_off ? 0 : n + 1, 0);  // PoP: every message empty
-  CKR(upload_records(ctx, msgs, msg_off ? msg_off : no_msgs.data(), n, d_msgs, d_off));
-  uint8_t* d_st = ctx->arena.take<uint8_t>(n);
+  CKR(upload_records(ctx, msgs, msg_off, n, d_msgs, d_off));
   *d_st_out = d_st;
   CKR((verify_dev_partials<IMPL>(ctx, P, msg_mode, dst, format, n, d_keys, d_sigs, d_msgs, d_off, d_st)));
   CK(cudaStreamSynchronize(ctx->stream));
@@ -1555,10 +1647,15 @@ int miller_partial_impl(blsgpu_ctx* ctx, int msg_mode, const DstParam& dst, int 
   const size_t Ls = PtInfo<SigA>::LEN;
   std::unique_ptr<PendingImpl<IMPL>> pend(new PendingImpl<IMPL>());
   pend->n = n;
-  CKR((host_partials<IMPL>(ctx, pend->P, msg_mode, dst, format, n, pks, sigs, msgs, msg_off, &pend->d_st)));
-  uint8_t* d_gt = ctx->arena.take<uint8_t>(576);
-  SigA* d_aff = ctx->arena.take<SigA>(1);
-  uint8_t* d_enc = ctx->arena.take<uint8_t>(Ls);
+  uint8_t *d_gt, *d_enc;
+  SigA* d_aff;
+  auto tail = [&](auto& a) {
+    d_gt = a.template take<uint8_t>(576);
+    d_aff = a.template take<SigA>(1);
+    d_enc = a.template take<uint8_t>(Ls);
+  };
+  CKR((host_partials<IMPL>(ctx, pend->P, msg_mode, dst, format, n, pks, sigs, msgs, msg_off, &pend->d_st, tail)));
+  tail(ctx->arena);
   LAUNCH(k_fp12_to_bytes, 1, 32, (size_t)1, pend->P.rootF(), d_gt);
   LAUNCH((k_to_affine<SigA>), 1, 32, (size_t)1, (const SigJ*)pend->P.rootS(), d_aff);
   LAUNCH((k_encode<SigA>), 1, 32, (size_t)1, (const SigA*)d_aff, 1, d_enc);
@@ -1574,18 +1671,18 @@ int fold_bytes_impl(blsgpu_ctx* ctx, const char* what, size_t k, const uint8_t* 
   typedef typename ImplT<IMPL>::SigAff SigA;
   typedef typename PtInfo<SigA>::Jac SigJ;
   const size_t Ls = PtInfo<SigA>::LEN;
-  Arena A;
-  CKR(fold_arena(ctx, fold_bytes<PkA, SigA>(k), A));
-  uint8_t* d_gt = A.take<uint8_t>(576 * k);
-  uint8_t* d_sb = A.take<uint8_t>(Ls * k);
-  Fp12* d_Fk = A.take<Fp12>(k);
-  SigA* d_aff = A.take<SigA>(k);
-  SigJ* d_Sk = A.take<SigJ>(k);
-  uint8_t* d_flag = A.take<uint8_t>(2 * k);
-  if (A.over) {
-    ctx->err = "internal: fold scratch sized too small";
-    return BLSGPU_E_ALLOC;
-  }
+  uint8_t *d_gt, *d_sb, *d_flag;
+  Fp12* d_Fk;
+  SigA* d_aff;
+  SigJ* d_Sk;
+  CKR((fold_takes<PkA, SigA>(ctx, [&](auto& a) {
+    d_gt = a.template take<uint8_t>(576 * k);
+    d_sb = a.template take<uint8_t>(Ls * k);
+    d_Fk = a.template take<Fp12>(k);
+    d_aff = a.template take<SigA>(k);
+    d_Sk = a.template take<SigJ>(k);
+    d_flag = a.template take<uint8_t>(2 * k);
+  })));
   CK(cudaMemcpyAsync(d_gt, gts, 576 * k, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(d_sb, sums, Ls * k, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemsetAsync(d_flag, 0, 2 * k, ctx->stream));
@@ -1598,7 +1695,7 @@ int fold_bytes_impl(blsgpu_ctx* ctx, const char* what, size_t k, const uint8_t* 
   for (uint8_t f : flag)
     if (f) return arg_error(ctx, what, "a partial result is not a canonical field element / group element");
   bool ok = false;
-  CKR((fold_check<PkA, SigA>(ctx, A, k, d_Fk, d_Sk, &ok)));
+  CKR((fold_check<PkA, SigA>(ctx, k, d_Fk, d_Sk, &ok)));
   *ok_out = ok ? 1 : 0;
   return BLSGPU_OK;
 }
@@ -1675,6 +1772,7 @@ struct AggSlice {
   SigA *d_sig = nullptr, *d_h = nullptr;
   uint8_t *d_msgs = nullptr, *d_status = nullptr;
   uint64_t* d_off = nullptr;
+  typename PtInfo<SigA>::Jac* d_hj = nullptr;
   Pipe<PkA, SigA> P;
 };
 // (1) st_out[n] and inf_out[n] get the slice's decode statuses and identity flags; with `sig` also st_out[n] / inf_out[n]
@@ -1686,20 +1784,24 @@ static int agg_decode(blsgpu_ctx* ctx, AggSlice<IMPL>& S, int format, size_t n, 
   typedef typename ImplT<IMPL>::SigAff SigA;
   const size_t pk_len = PtInfo<PkA>::LEN, sig_len = PtInfo<SigA>::LEN;
   S.n = n;
-  size_t msg_bytes = (size_t)(msg_off[n] - msg_off[0]);
-  size_t head = n * (pk_len + sizeof(PkA) + sizeof(SigA) + 2) + msg_bytes + (n + 1) * 8 + sig_len + sizeof(SigA) + 16 * 256 +
-                std::max<size_t>(n, 1) * sizeof(typename PtInfo<SigA>::Jac);
-  CKR((ensure_pipeline_arena<PkA, SigA>(ctx, std::max<size_t>(n, 1), head)));
-  uint8_t *d_pks, *d_sigb;
+  uint8_t *d_pks, *d_sigb, *d_stpk;
+  // every take of the slice: its inputs and decoded points here, the hash scratch and the pipeline for agg_partials
+  auto takes = [&](auto& a, size_t chunk) {
+    d_pks = take_up<uint8_t>(a, n * pk_len);
+    take_records(a, msg_off, n, S.d_msgs, S.d_off);
+    d_sigb = a.template take<uint8_t>(sig_len);
+    S.d_pk = a.template take<PkA>(std::max<size_t>(n, 1));
+    S.d_sig = a.template take<SigA>(1);
+    S.d_h = a.template take<SigA>(std::max<size_t>(n, 1));
+    d_stpk = a.template take<uint8_t>(n + 1);
+    S.d_status = a.template take<uint8_t>(std::max<size_t>(n, 1));
+    S.d_hj = take_hash_scratch<SigA>(a, n);
+    take_pipe(a, S.P, ctx, n, false, chunk);
+  };
+  CKR(ensure_miller_arena(ctx, n, takes));
+  takes(ctx->arena, ctx->m6_chunk);
   CKR(upload(ctx, d_pks, pks, n * pk_len));
   CKR(upload_records(ctx, msgs, msg_off, n, S.d_msgs, S.d_off));
-  d_sigb = ctx->arena.take<uint8_t>(sig_len);
-  S.d_pk = ctx->arena.take<PkA>(std::max<size_t>(n, 1));
-  S.d_sig = ctx->arena.take<SigA>(1);
-  S.d_h = ctx->arena.take<SigA>(std::max<size_t>(n, 1));
-  uint8_t* d_stpk = ctx->arena.take<uint8_t>(n + 1);
-  S.d_status = ctx->arena.take<uint8_t>(std::max<size_t>(n, 1));
-  ARENA_OK();
   stage_reset(ctx);
   if (n) CKR((decode_points<PkA>(ctx, n, (const uint8_t*)d_pks, format, S.d_pk, d_stpk)));
   if (sig) {
@@ -1775,8 +1877,8 @@ static int agg_partials(blsgpu_ctx* ctx, AggSlice<IMPL>& S, int scheme) {
   make_dst(dst, IMPL, scheme, false);
   CK(cudaMemsetAsync(S.d_status, 0, S.n, ctx->stream));
   CKR((hash_points<SigA, PkA>(ctx, S.n, (const uint8_t*)S.d_msgs, (const uint64_t*)S.d_off, scheme == 1 ? 1 : 0, (const PkA*)S.d_pk,
-                              (const uint8_t*)nullptr, dst, S.d_h)));
-  return pipeline_partials<PkA, SigA>(ctx, S.P, S.n, S.d_pk, S.d_sig, S.d_h, S.d_status, false);
+                              (const uint8_t*)nullptr, dst, S.d_hj, S.d_h)));
+  return pipeline_partials<PkA, SigA>(ctx, S.P, S.d_pk, S.d_sig, S.d_h, S.d_status);
 }
 template <int IMPL>
 static int aggregate_verify_impl(blsgpu_ctx* ctx, int scheme, int format, size_t n, const uint8_t* pks, const uint8_t* msgs,
@@ -1881,23 +1983,49 @@ static int aggregate_batch_impl(blsgpu_ctx* ctx, int scheme, int format, size_t 
   Pipe<PkA, SigA> P;
   P.lv = make_levels(q);
   const size_t qtotal = levels_total(P.lv), ndig = levels_total(make_levels(np + q));
-  size_t head = np * (Lp + sizeof(PkA) + sizeof(SigA) + 2) + msg_bytes + (np + 1) * 8 + q * (Ls + sizeof(SigA) + 2) + (q + 1) * 8 +
-                np * sizeof(SigJ) + (ndig + 2) * sizeof(Digest) + nslots * (sizeof(PkA) + sizeof(SigA) + 1 + 4) + ng * 4 +
-                seg_off.size() * 4 + seg_total * sizeof(Fp12) + qtotal * (sizeof(Fp12) + sizeof(SigJ)) +
-                probe_scratch_bytes<PkA, SigA>(probe_cap(q)) + 40 * 256;
-  CKR((ensure_pipeline_arena<PkA, SigA>(ctx, nslots, head)));
-  stage_reset(ctx);
-  uint8_t *d_pkb, *d_sigb, *d_msgs;
+  uint8_t *d_pkb, *d_sigb, *d_msgs, *d_st, *d_pair_pre, *d_agg_pre, *d_pres;
   uint64_t *d_moff, *d_soff;
+  uint32_t *d_src, *d_gset, *d_segoff;
+  PkA *d_pk, *d_pks;
+  SigA *d_sig, *d_h, *d_hs;
+  SigJ* d_hj;
+  Digest* d_dig;
+  Fp12* d_Fseg;
+  auto takes = [&](auto& a, size_t chunk) {
+    d_pkb = take_up<uint8_t>(a, np * Lp);
+    d_sigb = take_up<uint8_t>(a, q * Ls);
+    d_msgs = take_up<uint8_t>(a, msg_bytes);
+    d_moff = take_up<uint64_t>(a, np + 1);
+    d_soff = take_up<uint64_t>(a, q + 1);
+    d_pk = a.template take<PkA>(std::max<size_t>(np, 1));
+    d_sig = a.template take<SigA>(q);
+    d_st = a.template take<uint8_t>(np + q);  // decode statuses: the pks, then the signatures
+    d_pair_pre = take_up<uint8_t>(a, np);
+    d_agg_pre = take_up<uint8_t>(a, q);
+    d_src = take_up<uint32_t>(a, nslots);
+    d_gset = take_up<uint32_t>(a, ng);
+    d_segoff = take_up<uint32_t>(a, seg_off.size());
+    d_h = a.template take<SigA>(std::max<size_t>(np, 1));
+    d_hj = take_hash_scratch<SigA>(a, np);
+    d_dig = a.template take<Digest>(ndig + 2);
+    d_pks = a.template take<PkA>(nslots);
+    d_hs = a.template take<SigA>(nslots);
+    d_pres = a.template take<uint8_t>(nslots);
+    // the pipe of the set tree: leaves (F_j, S_j), probe scratch, the Miller stage's line buffers
+    P.d_F = a.template take<Fp12>(qtotal);
+    P.d_S = a.template take<SigJ>(qtotal);
+    take_probe_scratch(a, P, probe_cap(q));
+    d_Fseg = a.template take<Fp12>(std::max<size_t>(seg_total, 1));
+    take_lines(a, P, nslots, chunk);
+  };
+  CKR(ensure_miller_arena(ctx, nslots, takes));
+  takes(ctx->arena, ctx->m6_chunk);
+  stage_reset(ctx);
   CKR(upload(ctx, d_pkb, pks, np * Lp));
   CKR(upload(ctx, d_sigb, sigs, q * Ls));
   CKR(upload(ctx, d_msgs, msgs, msg_bytes));
   CKR(upload(ctx, d_moff, msg_off, np + 1));
   CKR(upload(ctx, d_soff, set_off, q + 1));
-  PkA* d_pk = ctx->arena.take<PkA>(std::max<size_t>(np, 1));
-  SigA* d_sig = ctx->arena.take<SigA>(q);
-  uint8_t* d_st = ctx->arena.take<uint8_t>(np + q);  // decode statuses: the pks, then the signatures
-  ARENA_OK();
   stage_mark(ctx, BLSGPU_STAGE_DECODE_PK);
   if (np) CKR((decode_points<PkA>(ctx, np, (const uint8_t*)d_pkb, format, d_pk, d_st, BLSGPU_KERNEL_DECODE_PK)));
   stage_mark(ctx, BLSGPU_STAGE_DECODE_SIG);
@@ -1939,8 +2067,6 @@ static int aggregate_batch_impl(blsgpu_ctx* ctx, int scheme, int format, size_t 
     stage_collect(ctx);
     return BLSGPU_OK;
   }
-  uint8_t *d_pair_pre, *d_agg_pre;
-  uint32_t *d_src, *d_gset, *d_segoff;
   CKR(upload(ctx, d_pair_pre, pair_pre.data(), np));
   CKR(upload(ctx, d_agg_pre, agg_pre.data(), q));
   CKR(upload(ctx, d_src, slot_src.data(), nslots));
@@ -1948,22 +2074,16 @@ static int aggregate_batch_impl(blsgpu_ctx* ctx, int scheme, int format, size_t 
   CKR(upload(ctx, d_segoff, seg_off.data(), seg_off.size()));
   DstParam dst;
   make_dst(dst, IMPL, scheme, false);
-  SigA* d_h = ctx->arena.take<SigA>(std::max<size_t>(np, 1));
   stage_mark(ctx, BLSGPU_STAGE_HASH);
   CKR((hash_points<SigA, PkA>(ctx, np, (const uint8_t*)d_msgs, (const uint64_t*)d_moff, scheme == 1 ? 1 : 0, (const PkA*)d_pk,
-                              (const uint8_t*)d_pair_pre, dst, d_h)));
+                              (const uint8_t*)d_pair_pre, dst, d_hj, d_h)));
   // the scalars: r_j = rlc_scalar(root, j), root = 16-ary SHA-256 tree over every pk, hashed message, signature and range
-  Digest* d_dig = ctx->arena.take<Digest>(ndig + 2);
   Digest* d_root = d_dig + ndig;  // [root, salt]
   CKR(fresh_salt(ctx));
   LAUNCH((k_agg_leaf_digest<PkA, SigA>), blocks_for(np + q), TPB, np, q, (const PkA*)d_pk, (const SigA*)d_h, (const SigA*)d_sig,
          (const uint64_t*)d_soff, d_dig);
   CKR(digest_root(ctx, np + q, d_dig, d_root));
-  PkA* d_pks = ctx->arena.take<PkA>(nslots);
-  SigA* d_hs = ctx->arena.take<SigA>(nslots);
-  uint8_t* d_pres = ctx->arena.take<uint8_t>(nslots);
   LAUNCH((k_agg_slots<PkA, SigA>), blocks_for(nslots), TPB, nslots, (const uint32_t*)d_src, (const PkA*)d_pk, (const SigA*)d_h, d_pks, d_hs, d_pres);
-  // the pipe of the set tree: leaves (F_j, S_j), probe scratch
   P.n = nslots;
   P.ng = q;
   P.use_rlc = true;
@@ -1973,10 +2093,6 @@ static int aggregate_batch_impl(blsgpu_ctx* ctx, int scheme, int format, size_t 
   P.d_h = d_hs;
   P.d_status = d_pres;
   P.d_root = d_root;
-  P.d_F = ctx->arena.take<Fp12>(qtotal);
-  P.d_S = ctx->arena.take<SigJ>(qtotal);
-  take_probe_scratch(ctx->arena, P, probe_cap(q));
-  Fp12* d_Fseg = ctx->arena.take<Fp12>(std::max<size_t>(seg_total, 1));
   CKR((set_probe_smem<PkA, SigA>(ctx)));
   stage_mark(ctx, BLSGPU_STAGE_SCALE_SIG);
   LAUNCH((k_scale_sig<SigA>), blocks_for(q), TPB, q, (const SigA*)d_sig, (const uint8_t*)d_agg_pre, (const Digest*)d_root, rbits, P.d_S);
@@ -2073,6 +2189,7 @@ struct Grouped {
   GLeaf* leaves;
   PkA* pk;
   SigA *sig, *hq, *hl;  // hq: per message, hl: per leaf
+  SigJ* hj;             // hash_points' scratch
   Digest* dig;          // leaf digests, their tree, [root, salt]
   RlcScalar* r;         // the scalars of the per-item route (the bucket route's come from msm_sum)
   SigJ* s_item;         // per-item route: r_i sig_i and the tree over them
@@ -2082,9 +2199,9 @@ struct Grouped {
   SigA* s_aff;
   Pipe<PkA, SigA> P;  // the tree over the Miller groups of leaves
 };
-// every take of the grouped pipeline but the bucket MSM's (msm_sum) and the Miller line buffers (miller_stage)
+// every take of the grouped pipeline, with Miller line buffers for passes of `chunk` leaves
 template <class PkA, class SigA, class A>
-void take_grouped(A& a, Grouped<PkA, SigA>& G) {
+void take_grouped(A& a, Grouped<PkA, SigA>& G, int rbits, size_t chunk) {
   typedef typename Grouped<PkA, SigA>::PkJ PkJ;
   typedef typename Grouped<PkA, SigA>::SigJ SigJ;
   const size_t n = G.n, nl = G.nl, ng = (nl + M6_GROUP - 1) / M6_GROUP, ndig = levels_total(make_levels(n));
@@ -2107,6 +2224,7 @@ void take_grouped(A& a, Grouped<PkA, SigA>& G) {
   G.stsig = a.template take<uint8_t>(n);
   G.status = a.template take<uint8_t>(n);
   G.hq = a.template take<SigA>(G.q);
+  G.hj = take_hash_scratch<SigA>(a, G.q);
   G.dig = a.template take<Digest>(ndig + 2);
   if (n < MSM_MIN_ITEMS) {
     G.r = a.template take<RlcScalar>(n);
@@ -2126,15 +2244,8 @@ void take_grouped(A& a, Grouped<PkA, SigA>& G) {
   G.P.d_F = a.template take<Fp12>(gtotal);
   G.P.d_S = a.template take<SigJ>(gtotal);
   take_probe_scratch(a, G.P, probe_cap(ng));
-}
-// the grouped pipeline's device scratch without the Miller line buffers: its takes, the bucket MSM's, and the Jacobian
-// scratch hash_points holds for the q hashes
-template <class PkA, class SigA>
-size_t grouped_bytes(Grouped<PkA, SigA> G, int rbits) {
-  ArenaSize a;
-  take_grouped(a, G);
-  return a.off + (G.n >= MSM_MIN_ITEMS ? msm_bytes<typename Grouped<PkA, SigA>::SigJ>(G.n, rbits) : 0) +
-         Arena::bytes<typename Grouped<PkA, SigA>::SigJ>(G.q) + 4 * 256;
+  if (n >= MSM_MIN_ITEMS) take_msm(a, n, MsmPlan(n, rbits), G.P.msm);
+  take_lines(a, G.P, nl, chunk);
 }
 // sum_{i in l} r_i * pts[i] into out[l] for every leaf: the bucket kernel for the big leaves, per-item scaling for the small
 template <class A, class G>
@@ -2187,8 +2298,8 @@ int verify_grouped_impl(blsgpu_ctx* ctx, int scheme, int format, size_t n, const
   G.msg_bytes = (size_t)(msg_off[q] - msg_off[0]);
   G.blocks = node_msm_blocks(ctx, G.nbig);
   const int rbits = ctx->rlc_bits;
-  CKR(ensure_miller_arena(ctx, G.nl, grouped_bytes(G, rbits)));
-  take_grouped(ctx->arena, G);
+  CKR(ensure_miller_arena(ctx, G.nl, [&](auto& a, size_t chunk) { take_grouped(a, G, rbits, chunk); }));
+  take_grouped(ctx->arena, G, rbits, ctx->m6_chunk);
   ARENA_OK();
   Pipe<PkA, SigA>& P = G.P;
   stage_reset(ctx);
@@ -2221,7 +2332,7 @@ int verify_grouped_impl(blsgpu_ctx* ctx, int scheme, int format, size_t n, const
   stage_mark(ctx, BLSGPU_STAGE_HASH);
   DstParam dst;
   make_dst(dst, IMPL, scheme, false);
-  CKR((hash_points<SigA, PkA>(ctx, q, (const uint8_t*)G.msgs, (const uint64_t*)G.moff, 0, (const PkA*)nullptr, (const uint8_t*)G.mpre, dst, G.hq)));
+  CKR((hash_points<SigA, PkA>(ctx, q, (const uint8_t*)G.msgs, (const uint64_t*)G.moff, 0, (const PkA*)nullptr, (const uint8_t*)G.mpre, dst, G.hj, G.hq)));
   CKR(fresh_salt(ctx));
   const size_t ndig = levels_total(make_levels(n));
   Digest* d_root = G.dig + ndig;
@@ -2233,7 +2344,8 @@ int verify_grouped_impl(blsgpu_ctx* ctx, int scheme, int format, size_t n, const
   RlcScalar* d_r = nullptr;
   SigJ* d_S = nullptr;
   if (n >= MSM_MIN_ITEMS) {
-    CKR((msm_sum<SigA>(ctx, n, G.sig, G.status, d_root, rbits, &d_r, &d_S)));
+    CKR((msm_sum<SigA>(ctx, n, G.sig, G.status, d_root, rbits, P.msm, &d_S)));
+    d_r = P.msm.r;
   } else {
     d_r = G.r;
     const std::vector<Level> lvn = make_levels(n);
@@ -2447,36 +2559,41 @@ int keyset_change_impl(blsgpu_ctx* ctx, KeySet& s, int format, size_t k, const u
   constexpr int L = PtInfo<PkA>::LEN;
   const size_t n = s.n, n1 = append ? n + k : n;
   bool live[2];
-  size_t need = Arena::bytes<uint8_t>(k * L) + Arena::bytes<uint32_t>(k) + Arena::bytes<PkA>(k) + Arena::bytes<uint8_t>(k);
-  for (int f = 0; f < 2; f++) {
-    live[f] = s.view[f].enc != nullptr;
-    if (live[f]) need += Arena::bytes<uint8_t>(k * L) + Arena::bytes<uint64_t>(k) + Arena::bytes<uint32_t>(std::max<size_t>(s.view[f].ranks, 1));
-  }
-  CKR(ensure_arena(ctx, need));
-  uint8_t* d_bytes;
+  for (int f = 0; f < 2; f++) live[f] = s.view[f].enc != nullptr;
+  uint8_t *d_bytes, *d_st;
   uint32_t* d_idx;
+  PkA* d_pts;
+  uint8_t* d_enc[2] = {nullptr, nullptr};
+  uint64_t* d_pos[2] = {nullptr, nullptr};
+  uint32_t* d_rep[2] = {nullptr, nullptr};
+  CKR(arena_takes(ctx, [&](auto& a) {
+    d_bytes = take_up<uint8_t>(a, k * L);
+    d_idx = take_up<uint32_t>(a, k);
+    d_pts = a.template take<PkA>(k);
+    d_st = a.template take<uint8_t>(k);
+    for (int f = 0; f < 2; f++) {
+      if (!live[f]) continue;
+      d_enc[f] = a.template take<uint8_t>(k * L);
+      d_pos[f] = a.template take<uint64_t>(k);
+      d_rep[f] = a.template take<uint32_t>(std::max<size_t>(s.view[f].ranks, 1));
+    }
+  }));
   CKR(upload(ctx, d_bytes, pks, k * L));
   CKR(upload(ctx, d_idx, key_idx, k));
-  PkA* d_pts = ctx->arena.take<PkA>(k);
-  uint8_t* d_st = ctx->arena.take<uint8_t>(k);
   CKR((decode_points<PkA>(ctx, k, (const uint8_t*)d_bytes, format, d_pts, d_st)));
   if (status_out) CK(cudaMemcpyAsync(status_out, d_st, k, cudaMemcpyDeviceToHost, ctx->stream));
-  uint8_t* d_enc[2] = {nullptr, nullptr};
   std::vector<uint8_t> enc[2];
   std::vector<uint64_t> pos[2];
   for (int f = 0; f < 2; f++) {
     if (!live[f]) continue;
     const SecureView& v = s.view[f];
-    d_enc[f] = ctx->arena.take<uint8_t>(k * L);
-    uint64_t* d_pos = ctx->arena.take<uint64_t>(k);
-    uint32_t* d_rep = ctx->arena.take<uint32_t>(std::max<size_t>(v.ranks, 1));
     LAUNCH((k_encode<PkA>), blocks_for(k), TPB, k, (const PkA*)d_pts, f, d_enc[f]);
-    if (n) LAUNCH(k_rank_reps, blocks_for(n), TPB, n, (const uint32_t*)v.rank, d_rep);
-    LAUNCH((k_rank_search<L>), blocks_for(k), TPB, k, (const uint8_t*)d_enc[f], (const uint8_t*)v.enc, (const uint32_t*)d_rep, v.ranks, d_pos);
+    if (n) LAUNCH(k_rank_reps, blocks_for(n), TPB, n, (const uint32_t*)v.rank, d_rep[f]);
+    LAUNCH((k_rank_search<L>), blocks_for(k), TPB, k, (const uint8_t*)d_enc[f], (const uint8_t*)v.enc, (const uint32_t*)d_rep[f], v.ranks, d_pos[f]);
     enc[f].resize(k * L);
     pos[f].resize(k);
     CK(cudaMemcpyAsync(enc[f].data(), d_enc[f], k * L, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(pos[f].data(), d_pos, k * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(pos[f].data(), d_pos[f], k * 8, cudaMemcpyDeviceToHost, ctx->stream));
   }
   CK(cudaStreamSynchronize(ctx->stream));
   std::vector<uint32_t> rank[2];
@@ -2646,15 +2763,18 @@ static int sum_points_impl(blsgpu_ctx* ctx, int format, size_t n, const uint8_t*
   typedef typename PtInfo<A>::Jac J;
   const size_t L = PtInfo<A>::LEN;
   std::vector<Level> lv = make_levels(std::max<size_t>(n, 1));
-  size_t need = n * (L + sizeof(A) + 1) + levels_total(lv) * sizeof(J) + sizeof(A) + L + 16 * 256;
-  CKR(ensure_arena(ctx, need));
-  uint8_t* d_in;
+  uint8_t *d_in, *d_st, *d_out;
+  A *d_pts, *d_res;
+  J* d_tree;
+  CKR(arena_takes(ctx, [&](auto& a) {
+    d_in = take_up<uint8_t>(a, n * L);
+    d_pts = a.template take<A>(std::max<size_t>(n, 1));
+    d_st = a.template take<uint8_t>(std::max<size_t>(n, 1));
+    d_tree = a.template take<J>(levels_total(lv) + 1);
+    d_res = a.template take<A>(1);
+    d_out = a.template take<uint8_t>(L);
+  }));
   CKR(upload(ctx, d_in, points, n * L));
-  A* d_pts = ctx->arena.take<A>(std::max<size_t>(n, 1));
-  uint8_t* d_st = ctx->arena.take<uint8_t>(std::max<size_t>(n, 1));
-  J* d_tree = ctx->arena.take<J>(levels_total(lv) + 1);
-  A* d_res = ctx->arena.take<A>(1);
-  uint8_t* d_out = ctx->arena.take<uint8_t>(L);
   *bad_index_out = -1;
   std::vector<uint8_t> st(n);
   if (n) {
@@ -2716,15 +2836,19 @@ int blsgpu_sum_points(blsgpu_ctx* ctx, int group, int format, size_t n, const ui
 template <class A>
 static int hash_batch_impl(blsgpu_ctx* ctx, size_t n, const uint8_t* msgs, const uint64_t* msg_off, const DstParam& dst, uint8_t* out) {
   const size_t L = PtInfo<A>::LEN;
-  size_t msg_bytes = (size_t)msg_off[n];
-  CKR(ensure_arena(ctx, msg_bytes + (n + 1) * 8 + n * (sizeof(A) + L + sizeof(typename PtInfo<A>::Jac)) + 8 * 256));
-  uint8_t* d_msgs;
+  uint8_t *d_msgs, *d_out;
   uint64_t* d_off;
+  A* d_h;
+  typename PtInfo<A>::Jac* d_hj;
+  CKR(arena_takes(ctx, [&](auto& a) {
+    take_records(a, msg_off, n, d_msgs, d_off);
+    d_h = a.template take<A>(n);
+    d_out = a.template take<uint8_t>(n * L);
+    d_hj = take_hash_scratch<A>(a, n);
+  }));
   CKR(upload_records(ctx, msgs, msg_off, n, d_msgs, d_off));
-  A* d_h = ctx->arena.take<A>(n);
-  uint8_t* d_out = ctx->arena.take<uint8_t>(n * L);
   CKR((hash_points<A, G1Aff>(ctx, n, (const uint8_t*)d_msgs, (const uint64_t*)d_off, 0, (const G1Aff*)nullptr, (const uint8_t*)nullptr,
-                             dst, d_h)));
+                             dst, d_hj, d_h)));
   LAUNCH((k_encode<A>), blocks_for(n), TPB, n, (const A*)d_h, 1, d_out);
   CK(cudaMemcpyAsync(out, d_out, n * L, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
@@ -2750,12 +2874,15 @@ int blsgpu_hash_to_curve_batch(blsgpu_ctx* ctx, int group, size_t n, const uint8
 template <class A>
 static int recode_impl(blsgpu_ctx* ctx, int fin, int fout, size_t n, const uint8_t* in, uint8_t* out, uint8_t* status_out) {
   const size_t L = PtInfo<A>::LEN;
-  CKR(ensure_arena(ctx, n * (2 * L + sizeof(A) + 1) + 8 * 256));
-  uint8_t* d_in;
+  uint8_t *d_in, *d_st, *d_out;
+  A* d_pts;
+  CKR(arena_takes(ctx, [&](auto& a) {
+    d_in = take_up<uint8_t>(a, n * L);
+    d_pts = a.template take<A>(n);
+    d_st = a.template take<uint8_t>(n);
+    d_out = a.template take<uint8_t>(n * L);
+  }));
   CKR(upload(ctx, d_in, in, n * L));
-  A* d_pts = ctx->arena.take<A>(n);
-  uint8_t* d_st = ctx->arena.take<uint8_t>(n);
-  uint8_t* d_out = ctx->arena.take<uint8_t>(n * L);
   CKR((decode_points<A>(ctx, n, (const uint8_t*)d_in, fin, d_pts, d_st)));
   LAUNCH((k_encode<A>), blocks_for(n), TPB, n, (const A*)d_pts, fout, d_out);
   CK(cudaMemcpyAsync(out, d_out, n * L, cudaMemcpyDeviceToHost, ctx->stream));
@@ -2780,11 +2907,14 @@ int blsgpu_fp_mul_batch(blsgpu_ctx* ctx, int variant, size_t n, const uint8_t* a
   if ((variant != 0 && variant != 1) || (n && (!a || !b || !out))) return arg_error(ctx, __func__, "bad arguments");
   if (n == 0) return BLSGPU_OK;
   CKR(set_device(ctx));
-  CKR(ensure_arena(ctx, 3 * n * 48 + 4 * 256));
-  uint8_t *d_a, *d_b;
+  uint8_t *d_a, *d_b, *d_o;
+  CKR(arena_takes(ctx, [&](auto& ar) {
+    d_a = take_up<uint8_t>(ar, n * 48);
+    d_b = take_up<uint8_t>(ar, n * 48);
+    d_o = ar.template take<uint8_t>(n * 48);
+  }));
   CKR(upload(ctx, d_a, a, n * 48));
   CKR(upload(ctx, d_b, b, n * 48));
-  uint8_t* d_o = ctx->arena.take<uint8_t>(n * 48);
   LAUNCH(k_fp_mul, blocks_for(n), TPB, n, variant, (const uint8_t*)d_a, (const uint8_t*)d_b, d_o);
   CK(cudaMemcpyAsync(out, d_o, n * 48, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
@@ -2801,15 +2931,21 @@ int blsgpu_pairing_product_is_one(blsgpu_ctx* ctx, size_t n, const uint8_t* g1_p
   }
   CKR(set_device(ctx));
   std::vector<Level> lv = make_levels(n);
-  CKR(ensure_arena(ctx, n * (48 + 96 + sizeof(G1Aff) + sizeof(G2Aff) + 2) + levels_total(lv) * sizeof(Fp12) + 12 * 256));
-  uint8_t *d_a, *d_b;
+  uint8_t *d_a, *d_b, *d_st, *d_ok;
+  G1Aff* d_p;
+  G2Aff* d_q;
+  Fp12* d_F;
+  CKR(arena_takes(ctx, [&](auto& a) {
+    d_a = take_up<uint8_t>(a, n * 48);
+    d_b = take_up<uint8_t>(a, n * 96);
+    d_p = a.template take<G1Aff>(n);
+    d_q = a.template take<G2Aff>(n);
+    d_st = a.template take<uint8_t>(2 * n);
+    d_F = a.template take<Fp12>(levels_total(lv));
+    d_ok = a.template take<uint8_t>(1);
+  }));
   CKR(upload(ctx, d_a, g1_points, n * 48));
   CKR(upload(ctx, d_b, g2_points, n * 96));
-  G1Aff* d_p = ctx->arena.take<G1Aff>(n);
-  G2Aff* d_q = ctx->arena.take<G2Aff>(n);
-  uint8_t* d_st = ctx->arena.take<uint8_t>(2 * n);
-  Fp12* d_F = ctx->arena.take<Fp12>(levels_total(lv));
-  uint8_t* d_ok = ctx->arena.take<uint8_t>(1);
   CKR((decode_points<G1Aff>(ctx, n, (const uint8_t*)d_a, 1, d_p, d_st)));
   CKR((decode_points<G2Aff>(ctx, n, (const uint8_t*)d_b, 1, d_q, d_st + n)));
   std::vector<uint8_t> st(2 * n);
@@ -2837,14 +2973,16 @@ int blsgpu_testdata_sign(blsgpu_ctx* ctx, int impl_id, int scheme, size_t n, con
   CKR(check_records(ctx, __func__, "msgs", msgs, "msg_off", msg_off, n));
   CKR(set_device(ctx));
   size_t pk_len = impl_id == 2 ? 48 : 96, sig_len = impl_id == 2 ? 96 : 48;
-  size_t msg_bytes = (size_t)msg_off[n];
-  CKR(ensure_arena(ctx, n * (32 + 8 + pk_len + sig_len) + msg_bytes + 16 * 256));
-  uint8_t *d_k, *d_m;
+  uint8_t *d_k, *d_m, *d_pk, *d_sig;
   uint64_t* d_off;
+  CKR(arena_takes(ctx, [&](auto& a) {
+    d_k = take_up<uint8_t>(a, n * 32);
+    take_records(a, msg_off, n, d_m, d_off);
+    d_pk = a.template take<uint8_t>(n * pk_len);
+    d_sig = a.template take<uint8_t>(n * sig_len);
+  }));
   CKR(upload(ctx, d_k, scalars32, n * 32));
   CKR(upload_records(ctx, msgs, msg_off, n, d_m, d_off));
-  uint8_t* d_pk = ctx->arena.take<uint8_t>(n * pk_len);
-  uint8_t* d_sig = ctx->arena.take<uint8_t>(n * sig_len);
   DstParam dst;
   make_dst(dst, impl_id, pop_proof ? 2 : scheme, pop_proof);
   int mode = pop_proof ? 2 : scheme == 1 ? 1 : 0;
@@ -2863,8 +3001,8 @@ int blsgpu_imad_peak(blsgpu_ctx* ctx, double* mac_per_s_out) {
   NVTX_RANGE("blsgpu_imad_peak");
   if (!ctx || !mac_per_s_out) return BLSGPU_E_ARG;
   CKR(set_device(ctx));
-  CKR(ensure_arena(ctx, 4096));
-  uint64_t* d_sink = ctx->arena.take<uint64_t>(1);
+  uint64_t* d_sink;
+  CKR(arena_takes(ctx, [&](auto& a) { d_sink = a.template take<uint64_t>(1); }));
   cudaDeviceProp prop;
   CK(cudaGetDeviceProperties(&prop, ctx->devices[0]));
   const int blocks = prop.multiProcessorCount * 8, threads = 256;
@@ -2940,27 +3078,36 @@ SecurePlan make_secure_plan(size_t q, const uint64_t* key_off, const uint8_t* pk
 
 // device part shared by verify and aggregate: out_sum[j] = sum_i t_i * points[src(i)] ; zero_out[m] flags t_m == 0.
 // One bucket multi-scalar multiplication per key set: a warp per set, a lane per 8-bit window (kernels.cuh k_secure_msm).
-// The plan is on the device: d_ord indexes d_key_bytes, d_src indexes d_points.
+// The plan is on the device: d_ord indexes d_key_bytes, d_src indexes d_points.  Its scratch (take_weighted_sums): the
+// per-set digest bases, the members' window digits, the bucket scratch and the window sums.
+template <class J>
+struct WeightedSums {
+  Digest* base = nullptr;
+  int8_t* digits = nullptr;
+  J *buckets = nullptr, *W = nullptr;
+};
+template <class J, class A>
+void take_weighted_sums(A& a, const blsgpu_ctx* ctx, size_t q, size_t M, WeightedSums<J>& w) {
+  w.base = a.template take<Digest>(q);
+  w.digits = a.template take<int8_t>(std::max<size_t>(M, 1) * SECURE_WINDOWS);
+  w.buckets = a.template take<J>(secure_msm_blocks(ctx, q) * 128 * SECURE_BUCKETS);
+  w.W = a.template take<J>(q * SECURE_WINDOWS);
+}
 template <class A>
 int secure_weighted_sums(blsgpu_ctx* ctx, size_t q, size_t M, const uint64_t* d_koff, const uint32_t* d_ord, const uint32_t* d_set,
                          const uint32_t* d_pos, const uint8_t* d_key_bytes, int key_len, const uint32_t* d_src, const A* d_points,
-                         typename PtInfo<A>::Jac* d_sum, uint8_t* d_zero) {
+                         const WeightedSums<typename PtInfo<A>::Jac>& w, typename PtInfo<A>::Jac* d_sum, uint8_t* d_zero) {
   typedef typename PtInfo<A>::Jac J;
-  Digest* d_base = ctx->arena.take<Digest>(q);
-  int8_t* d_digits = ctx->arena.take<int8_t>(std::max<size_t>(M, 1) * SECURE_WINDOWS);
+  Digest* d_base = w.base;
+  int8_t* d_digits = w.digits;
   const size_t nblocks = secure_msm_blocks(ctx, q);
-  J* d_buckets = ctx->arena.take<J>(nblocks * 128 * SECURE_BUCKETS);
-  J* d_W = ctx->arena.take<J>(q * SECURE_WINDOWS);
+  J* d_buckets = w.buckets;
+  J* d_W = w.W;
   LAUNCH(k_secure_base, blocks_for(q), TPB, q, d_koff, d_ord, d_key_bytes, key_len, d_base);
   if (M) LAUNCH(k_secure_digits, blocks_for(M), TPB, M, d_set, d_pos, (const Digest*)d_base, d_digits, d_zero);
   LAUNCH((k_secure_msm<A>), (unsigned)nblocks, 128, q, d_koff, d_src, (const int8_t*)d_digits, d_points, d_buckets, d_W);
   LAUNCH((k_secure_combine<J>), blocks_for(q), TPB, q, (const J*)d_W, d_sum);
   return BLSGPU_OK;
-}
-
-size_t secure_plan_bytes(const blsgpu_ctx* ctx, size_t q, size_t M, size_t jac_size) {
-  return (q + 1) * 8 + M * (16 + SECURE_WINDOWS) + q * 32 + secure_msm_blocks(ctx, q) * 128 * SECURE_BUCKETS * jac_size +
-         (q * SECURE_WINDOWS + 2) * jac_size + 24 * 256;
 }
 
 // Quorums of at most this many members are planned by k_secure_plan_keyed in shared memory (8 bytes per member, so 32 KB:
@@ -2988,19 +3135,44 @@ struct SecureKeys {
 // on the device by the set's secure view in `format` (k_secure_plan_keyed; make_secure_plan over the ranks for quorums
 // above SECURE_PLAN_CAP), and take the keys' encodings and points from the view and the set.  with_first: the plan's
 // `first` is needed (aggregate).
+// The arena scratch of secure_keys: unkeyed, the key bytes, their points and statuses; keyed, the key indices and the
+// quorums' key statuses; both, the key offsets and the plan.
 template <class PkA>
-int secure_keys(blsgpu_ctx* ctx, int format, size_t q, const uint64_t* key_off, const Keys& keys, bool with_first, SecureKeys<PkA>& K) {
+struct SecureKeyBufs {
+  uint8_t *pkb = nullptr, *st = nullptr;
+  PkA* pk = nullptr;
+  uint64_t* koff = nullptr;
+  uint32_t *kidx = nullptr, *ord = nullptr, *set = nullptr, *pos = nullptr, *first = nullptr;
+};
+template <class PkA, class A>
+void take_secure_keys(A& a, size_t q, size_t M, const Keys& keys, bool with_first, SecureKeyBufs<PkA>& b) {
+  if (!keys.set) {
+    b.pkb = take_up<uint8_t>(a, M * PtInfo<PkA>::LEN);
+    b.pk = a.template take<PkA>(std::max<size_t>(M, 1));
+    b.st = a.template take<uint8_t>(std::max<size_t>(M, 1));
+  }
+  b.koff = take_up<uint64_t>(a, q + 1);
+  if (keys.set) b.kidx = take_up<uint32_t>(a, M);
+  b.ord = take_up<uint32_t>(a, M);
+  b.set = take_up<uint32_t>(a, M);
+  b.pos = take_up<uint32_t>(a, M);
+  if (with_first || keys.set) b.first = take_up<uint32_t>(a, M);
+  if (keys.set) b.st = a.template take<uint8_t>(q);
+}
+template <class PkA>
+int secure_keys(blsgpu_ctx* ctx, int format, size_t q, const uint64_t* key_off, const Keys& keys, bool with_first, const SecureKeyBufs<PkA>& b,
+                SecureKeys<PkA>& K) {
   const size_t M = (size_t)key_off[q], Lp = PtInfo<PkA>::LEN;
-  uint64_t* d_koff;
+  uint64_t* d_koff = b.koff;
   if (!keys.set) {
     K.host_plans.push_back(make_secure_plan(q, key_off, keys.bytes, Lp));
     const SecurePlan& pl = K.host_plans.back();
-    uint8_t* d_pkb;
+    uint8_t* d_pkb = b.pkb;
     CKR(upload(ctx, d_pkb, keys.bytes, M * Lp));
-    PkA* d_pk = ctx->arena.take<PkA>(std::max<size_t>(M, 1));
-    uint8_t* d_stpk = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
+    PkA* d_pk = b.pk;
+    uint8_t* d_stpk = b.st;
     if (M) CKR((decode_points<PkA>(ctx, M, (const uint8_t*)d_pkb, format, d_pk, d_stpk)));
-    uint32_t *d_ord, *d_set, *d_pos, *d_first = nullptr;
+    uint32_t *d_ord = b.ord, *d_set = b.set, *d_pos = b.pos, *d_first = with_first ? b.first : nullptr;
     CKR(upload(ctx, d_koff, key_off, q + 1));
     CKR(upload(ctx, d_ord, pl.ord.data(), M));
     CKR(upload(ctx, d_set, pl.set_of.data(), M));
@@ -3018,14 +3190,11 @@ int secure_keys(blsgpu_ctx* ctx, int format, size_t q, const uint64_t* key_off, 
     return BLSGPU_OK;
   }
   const SecureView& v = keys.set->view[format];
-  uint32_t* d_kidx;
+  uint32_t* d_kidx = b.kidx;
   CKR(upload(ctx, d_koff, key_off, q + 1));
   CKR(upload(ctx, d_kidx, keys.idx, M));
-  uint32_t* d_ord = ctx->arena.take<uint32_t>(std::max<size_t>(M, 1));
-  uint32_t* d_set = ctx->arena.take<uint32_t>(std::max<size_t>(M, 1));
-  uint32_t* d_pos = ctx->arena.take<uint32_t>(std::max<size_t>(M, 1));
-  uint32_t* d_first = ctx->arena.take<uint32_t>(std::max<size_t>(M, 1));
-  uint8_t* d_keyst = ctx->arena.take<uint8_t>(q);
+  uint32_t *d_ord = b.ord, *d_set = b.set, *d_pos = b.pos, *d_first = b.first;
+  uint8_t* d_keyst = b.st;
   uint32_t slots = 1;
   for (size_t j = 0; j < q; j++) {
     const uint64_t cnt = key_off[j + 1] - key_off[j];
@@ -3083,26 +3252,39 @@ int verify_secure_impl(blsgpu_ctx* ctx, int scheme, int format, size_t q, const 
   typedef typename ImplT<IMPL>::SigAff SigA;
   typedef typename ImplT<IMPL>::PkJac PkJ;
   const size_t Lp = PtInfo<PkA>::LEN, Ls = PtInfo<SigA>::LEN;
-  const size_t M = (size_t)key_off[q], msg_bytes = (size_t)(msg_off[q] - msg_off[0]);
-  size_t head = M * (Lp + sizeof(PkA) + 2) + q * (Ls + 2 * sizeof(SigA) + sizeof(PkA) + sizeof(PkJ) + 8) + msg_bytes + (q + 1) * 8 +
-                secure_plan_bytes(ctx, q, M, sizeof(PkJ)) + 32 * 256;
-  CKR(ensure_verify_arena<IMPL>(ctx, q, head));
+  const size_t M = (size_t)key_off[q];
+  SecureKeyBufs<PkA> kb;
+  WeightedSums<PkJ> ws;
+  uint8_t *d_sigb, *d_msgs, *d_stsig, *d_zero, *d_setst, *d_status;
+  uint64_t* d_moff;
+  SigA* d_sig;
+  PkJ* d_sum;
+  PkA* d_agg;
+  auto head = [&](auto& a) {
+    take_secure_keys(a, q, M, keys, false, kb);
+    d_sigb = take_up<uint8_t>(a, q * Ls);
+    take_records(a, msg_off, q, d_msgs, d_moff);
+    d_sig = a.template take<SigA>(q);
+    d_stsig = a.template take<uint8_t>(q);
+    d_zero = a.template take<uint8_t>(std::max<size_t>(M, 1));
+    d_sum = a.template take<PkJ>(q);
+    d_agg = a.template take<PkA>(q);
+    d_setst = a.template take<uint8_t>(q);
+    d_status = a.template take<uint8_t>(q);
+    take_weighted_sums(a, ctx, q, M, ws);
+  };
+  CKR(ensure_miller_arena(ctx, q, [&](auto& a, size_t chunk) {
+    head(a);
+    take_verify_points<IMPL>(a, ctx, q, chunk);
+  }));
+  head(ctx->arena);
   stage_reset(ctx);
   SecureKeys<PkA> K;
-  CKR((secure_keys<PkA>(ctx, format, q, key_off, keys, false, K)));
-  uint8_t *d_sigb, *d_msgs;
-  uint64_t* d_moff;
+  CKR((secure_keys<PkA>(ctx, format, q, key_off, keys, false, kb, K)));
   CKR(upload(ctx, d_sigb, sigs, q * Ls));
   CKR(upload_records(ctx, msgs, msg_off, q, d_msgs, d_moff));
-  SigA* d_sig = ctx->arena.take<SigA>(q);
-  uint8_t* d_stsig = ctx->arena.take<uint8_t>(q);
-  uint8_t* d_zero = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
-  PkJ* d_sum = ctx->arena.take<PkJ>(q);
-  PkA* d_agg = ctx->arena.take<PkA>(q);
-  uint8_t* d_setst = ctx->arena.take<uint8_t>(q);
-  uint8_t* d_status = ctx->arena.take<uint8_t>(q);
   CKR((decode_points<SigA>(ctx, q, (const uint8_t*)d_sigb, format, d_sig, d_stsig)));
-  CKR((secure_weighted_sums<PkA>(ctx, q, M, K.koff, K.ord, K.set, K.pos, K.key_bytes, (int)Lp, K.ord, K.pts, d_sum, d_zero)));
+  CKR((secure_weighted_sums<PkA>(ctx, q, M, K.koff, K.ord, K.set, K.pos, K.key_bytes, (int)Lp, K.ord, K.pts, ws, d_sum, d_zero)));
   LAUNCH((k_to_affine<PkA>), blocks_for(q), TPB, q, (const PkJ*)d_sum, d_agg);
   const size_t nst = K.st_per_member ? M : q;
   std::vector<uint8_t> stpk(nst), stsig(q), zero(M);
@@ -3148,22 +3330,28 @@ int aggregate_secure_impl(blsgpu_ctx* ctx, int format, size_t q, const uint64_t*
   typedef typename ImplT<IMPL>::SigJac SigJ;
   const size_t Lp = PtInfo<PkA>::LEN, Ls = PtInfo<SigA>::LEN;
   const size_t M = (size_t)key_off[q];
-  size_t need = M * (Lp + Ls + sizeof(PkA) + sizeof(SigA) + 3) + q * (Ls + sizeof(SigA) + sizeof(SigJ) + 8) +
-                secure_plan_bytes(ctx, q, M, sizeof(SigJ)) + 32 * 256;
-  CKR(ensure_arena(ctx, need));
+  SecureKeyBufs<PkA> kb;
+  WeightedSums<SigJ> ws;
+  uint8_t *d_sigb, *d_stsig, *d_zero, *d_out;
+  SigA *d_sig, *d_agg;
+  SigJ* d_sum;
+  CKR(arena_takes(ctx, [&](auto& a) {
+    take_secure_keys(a, q, M, keys, true, kb);
+    d_sigb = take_up<uint8_t>(a, M * Ls);
+    d_sig = a.template take<SigA>(std::max<size_t>(M, 1));
+    d_stsig = a.template take<uint8_t>(std::max<size_t>(M, 1));
+    d_zero = a.template take<uint8_t>(std::max<size_t>(M, 1));
+    d_sum = a.template take<SigJ>(q);
+    d_agg = a.template take<SigA>(q);
+    d_out = a.template take<uint8_t>(q * Ls);
+    take_weighted_sums(a, ctx, q, M, ws);
+  }));
   SecureKeys<PkA> K;
-  CKR((secure_keys<PkA>(ctx, format, q, key_off, keys, true, K)));
-  uint8_t* d_sigb;
+  CKR((secure_keys<PkA>(ctx, format, q, key_off, keys, true, kb, K)));
   CKR(upload(ctx, d_sigb, member_sigs, M * Ls));
-  SigA* d_sig = ctx->arena.take<SigA>(std::max<size_t>(M, 1));
-  uint8_t* d_stsig = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
-  uint8_t* d_zero = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
-  SigJ* d_sum = ctx->arena.take<SigJ>(q);
-  SigA* d_agg = ctx->arena.take<SigA>(q);
-  uint8_t* d_out = ctx->arena.take<uint8_t>(q * Ls);
   if (M) CKR((decode_points<SigA>(ctx, M, (const uint8_t*)d_sigb, format, d_sig, d_stsig)));
   // sum_i t_i * sig[first original index whose key bytes equal sorted key i]   (secure_aggregation.rs:138-153)
-  CKR((secure_weighted_sums<SigA>(ctx, q, M, K.koff, K.ord, K.set, K.pos, K.key_bytes, (int)Lp, K.first, d_sig, d_sum, d_zero)));
+  CKR((secure_weighted_sums<SigA>(ctx, q, M, K.koff, K.ord, K.set, K.pos, K.key_bytes, (int)Lp, K.first, d_sig, ws, d_sum, d_zero)));
   LAUNCH((k_to_affine<SigA>), blocks_for(q), TPB, q, (const SigJ*)d_sum, d_agg);
   LAUNCH((k_encode<SigA>), blocks_for(q), TPB, q, (const SigA*)d_agg, format, d_out);
   const size_t nst = K.st_per_member ? M : q;
@@ -3359,35 +3547,44 @@ struct SegSumPlan {
     lv = seg_levels(std::move(cnt));
   }
   size_t nchunks() const { return cset.size(); }
-  template <class J>
-  size_t bytes() const {
-    return Arena::bytes<uint32_t>(coff.size()) + Arena::bytes<uint32_t>(cset.size()) + Arena::bytes<uint32_t>(std::max<size_t>(lv.off.size(), 1)) +
-           Arena::bytes<J>(std::max<size_t>(lv.below_top(), 1)) + Arena::bytes<unsigned long long>(q) + Arena::bytes<J>(q);
-  }
 };
+// the arena scratch of seg_point_sums over a plan: the plan's chunks and level offsets, the levels' nodes, and per set its
+// first bad member and its sum
+template <class J>
+struct SegSums {
+  uint32_t *coff = nullptr, *cset = nullptr, *segoff = nullptr;
+  J *nodes = nullptr, *sum = nullptr;
+  unsigned long long* bad = nullptr;
+};
+template <class J, class A>
+void take_seg_sums(A& a, const SegSumPlan& pl, SegSums<J>& s) {
+  s.coff = take_up<uint32_t>(a, pl.coff.size());
+  s.cset = take_up<uint32_t>(a, pl.cset.size());
+  s.segoff = take_up<uint32_t>(a, pl.lv.off.size());
+  s.nodes = a.template take<J>(std::max<size_t>(pl.lv.below_top(), 1));
+  s.bad = a.template take<unsigned long long>(pl.q);
+  s.sum = a.template take<J>(pl.q);
+}
 
-// sum[j] = the sum of set j's points (the identity for an empty set), first_bad[j] = (member << 8 | status) of its first
+// s.sum[j] = the sum of set j's points (the identity for an empty set), s.bad[j] = (member << 8 | status) of its first
 // member that failed to decode or ~0 (kernels.cuh k_seg_sum_gather).  Member m's point is d_pts[d_idx[m]], or d_pts[m] when
 // d_idx is null; likewise its status in d_st.
 template <class A>
-int seg_point_sums(blsgpu_ctx* ctx, const SegSumPlan& pl, const uint32_t* d_idx, const A* d_pts, const uint8_t* d_st,
-                   typename PtInfo<A>::Jac** sum_out, unsigned long long** first_bad_out) {
+int seg_point_sums(blsgpu_ctx* ctx, const SegSumPlan& pl, const SegSums<typename PtInfo<A>::Jac>& s, const uint32_t* d_idx, const A* d_pts,
+                   const uint8_t* d_st) {
   typedef typename PtInfo<A>::Jac J;
-  uint32_t *d_coff, *d_cset, *d_segoff;
+  uint32_t *d_coff = s.coff, *d_cset = s.cset, *d_segoff = s.segoff;
   CKR(upload(ctx, d_coff, pl.coff.data(), pl.coff.size()));
   CKR(upload(ctx, d_cset, pl.cset.data(), pl.cset.size()));
   CKR(upload(ctx, d_segoff, pl.lv.off.data(), pl.lv.off.size()));
-  J* d_nodes = ctx->arena.take<J>(std::max<size_t>(pl.lv.below_top(), 1));
-  unsigned long long* d_bad = ctx->arena.take<unsigned long long>(pl.q);
-  J* d_sum = ctx->arena.take<J>(pl.q);
-  ARENA_OK();
+  J* d_nodes = s.nodes;
+  unsigned long long* d_bad = s.bad;
+  J* d_sum = s.sum;
   CK(cudaMemsetAsync(d_bad, 0xff, pl.q * sizeof(unsigned long long), ctx->stream));
   const bool levels = pl.lv.n.size() > 1;  // some set has more than one chunk
   LAUNCH((k_seg_sum_gather<A>), blocks_for(pl.nchunks()), TPB, pl.nchunks(), (const uint32_t*)d_coff, (const uint32_t*)d_cset, d_idx, d_pts, d_st,
          levels ? d_nodes : d_sum, d_bad);
   if (levels) CKR(seg_reduce_levels<J>(ctx, pl.lv, d_segoff, d_nodes, d_sum));
-  *sum_out = d_sum;
-  *first_bad_out = d_bad;
   return BLSGPU_OK;
 }
 
@@ -3401,40 +3598,47 @@ int verify_multisig_impl(blsgpu_ctx* ctx, int scheme, int format, size_t q, cons
   typedef typename ImplT<IMPL>::PkAff PkA;
   typedef typename ImplT<IMPL>::SigAff SigA;
   typedef typename ImplT<IMPL>::PkJac PkJ;
-  const size_t Lp = PtInfo<PkA>::LEN, Ls = PtInfo<SigA>::LEN;
-  const size_t M = (size_t)key_off[q], msg_bytes = (size_t)msg_off[q];
+  const size_t Ls = PtInfo<SigA>::LEN;
+  const size_t M = (size_t)key_off[q];
   const SegSumPlan pl(q, key_off);
-  const size_t head = (keys.set ? M * 4 : M * (Lp + sizeof(PkA) + 1)) + pl.bytes<PkJ>() + q * (Ls + sizeof(SigA) + sizeof(PkA) + 3) + msg_bytes +
-                      (q + 1) * 8 + 16 * 256;
-  CKR(ensure_verify_arena<IMPL>(ctx, q, head));
+  Keys d_keys;
+  PkA *d_pk = nullptr, *d_agg;
+  uint8_t *d_stpk = nullptr, *d_setst, *d_sigb, *d_msgs, *d_stsig, *d_status;
+  uint64_t* d_moff;
+  SigA* d_sig;
+  SegSums<PkJ> ss;
+  auto head = [&](auto& a) {
+    take_keys<PkA>(a, M, keys, d_keys);
+    if (!keys.set) {
+      d_pk = a.template take<PkA>(std::max<size_t>(M, 1));
+      d_stpk = a.template take<uint8_t>(std::max<size_t>(M, 1));
+    }
+    take_seg_sums(a, pl, ss);
+    d_agg = a.template take<PkA>(q);
+    d_setst = a.template take<uint8_t>(q);
+    d_sigb = take_up<uint8_t>(a, q * Ls);
+    take_records(a, msg_off, q, d_msgs, d_moff);
+    d_sig = a.template take<SigA>(q);
+    d_stsig = a.template take<uint8_t>(q);
+    d_status = a.template take<uint8_t>(q);
+  };
+  CKR(ensure_miller_arena(ctx, q, [&](auto& a, size_t chunk) {
+    head(a);
+    take_verify_points<IMPL>(a, ctx, q, chunk);
+  }));
+  head(ctx->arena);
   stage_reset(ctx);
   stage_mark(ctx, BLSGPU_STAGE_DECODE_PK);  // the key side: decode (unkeyed calls) and the segmented sums
-  Keys d_keys;
   CKR(upload_keys<PkA>(ctx, M, keys, d_keys));
-  const PkA* d_pts = keys.set ? (const PkA*)keys.set->pts : nullptr;
-  const uint8_t* d_st = keys.set ? (const uint8_t*)keys.set->st : nullptr;
-  if (!keys.set) {
-    PkA* d_pk = ctx->arena.take<PkA>(std::max<size_t>(M, 1));
-    uint8_t* d_stpk = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
-    if (M) CKR((decode_points<PkA>(ctx, M, d_keys.bytes, format, d_pk, d_stpk, BLSGPU_KERNEL_DECODE_PK)));
-    d_pts = d_pk;
-    d_st = d_stpk;
-  }
-  PkJ* d_sum;
-  unsigned long long* d_bad;
-  CKR((seg_point_sums<PkA>(ctx, pl, keys.set ? d_keys.idx : nullptr, d_pts, d_st, &d_sum, &d_bad)));
-  PkA* d_agg = ctx->arena.take<PkA>(q);
-  uint8_t* d_setst = ctx->arena.take<uint8_t>(q);
-  LAUNCH((k_to_affine_batch<PkA>), blocks_for((q + TO_AFFINE_BATCH - 1) / TO_AFFINE_BATCH), TPB, q, (const PkJ*)d_sum, d_agg);
-  LAUNCH(k_seg_first_bad_status, blocks_for(q), TPB, q, (const unsigned long long*)d_bad, d_setst);
+  const PkA* d_pts = keys.set ? (const PkA*)keys.set->pts : d_pk;
+  const uint8_t* d_st = keys.set ? (const uint8_t*)keys.set->st : d_stpk;
+  if (!keys.set && M) CKR((decode_points<PkA>(ctx, M, d_keys.bytes, format, d_pk, d_stpk, BLSGPU_KERNEL_DECODE_PK)));
+  CKR((seg_point_sums<PkA>(ctx, pl, ss, keys.set ? d_keys.idx : nullptr, d_pts, d_st)));
+  LAUNCH((k_to_affine_batch<PkA>), blocks_for((q + TO_AFFINE_BATCH - 1) / TO_AFFINE_BATCH), TPB, q, (const PkJ*)ss.sum, d_agg);
+  LAUNCH(k_seg_first_bad_status, blocks_for(q), TPB, q, (const unsigned long long*)ss.bad, d_setst);
   stage_mark(ctx, BLSGPU_STAGE_DECODE_SIG);
-  uint8_t *d_sigb, *d_msgs;
-  uint64_t* d_moff;
   CKR(upload(ctx, d_sigb, sigs, q * Ls));
   CKR(upload_records(ctx, msgs, msg_off, q, d_msgs, d_moff));
-  SigA* d_sig = ctx->arena.take<SigA>(q);
-  uint8_t* d_stsig = ctx->arena.take<uint8_t>(q);
-  uint8_t* d_status = ctx->arena.take<uint8_t>(q);
   CKR((decode_points<SigA>(ctx, q, (const uint8_t*)d_sigb, format, d_sig, d_stsig, BLSGPU_KERNEL_DECODE_SIG)));
   DstParam dst;
   make_dst(dst, IMPL, scheme, false);
@@ -3453,19 +3657,22 @@ int sum_points_batch_impl(blsgpu_ctx* ctx, int format, size_t q, const uint64_t*
   typedef typename PtInfo<A>::Jac J;
   const size_t L = PtInfo<A>::LEN, M = (size_t)set_off[q];
   const SegSumPlan pl(q, set_off);
-  CKR(ensure_arena(ctx, M * (L + sizeof(A) + 1) + pl.bytes<J>() + q * (sizeof(A) + L) + 16 * 256));
-  uint8_t* d_in;
+  uint8_t *d_in, *d_st, *d_out;
+  A *d_pts, *d_res;
+  SegSums<J> ss;
+  CKR(arena_takes(ctx, [&](auto& a) {
+    d_in = take_up<uint8_t>(a, M * L);
+    d_pts = a.template take<A>(std::max<size_t>(M, 1));
+    d_st = a.template take<uint8_t>(std::max<size_t>(M, 1));
+    take_seg_sums(a, pl, ss);
+    d_res = a.template take<A>(q);
+    d_out = a.template take<uint8_t>(q * L);
+  }));
   CKR(upload(ctx, d_in, points, M * L));
-  A* d_pts = ctx->arena.take<A>(std::max<size_t>(M, 1));
-  uint8_t* d_st = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
-  ARENA_OK();
   if (M) CKR((decode_points<A>(ctx, M, (const uint8_t*)d_in, format, d_pts, d_st)));
-  J* d_sum;
-  unsigned long long* d_bad;
-  CKR((seg_point_sums<A>(ctx, pl, nullptr, d_pts, d_st, &d_sum, &d_bad)));
-  A* d_res = ctx->arena.take<A>(q);
-  uint8_t* d_out = ctx->arena.take<uint8_t>(q * L);
-  LAUNCH((k_to_affine_batch<A>), blocks_for((q + TO_AFFINE_BATCH - 1) / TO_AFFINE_BATCH), TPB, q, (const J*)d_sum, d_res);
+  CKR((seg_point_sums<A>(ctx, pl, ss, nullptr, d_pts, d_st)));
+  unsigned long long* d_bad = ss.bad;
+  LAUNCH((k_to_affine_batch<A>), blocks_for((q + TO_AFFINE_BATCH - 1) / TO_AFFINE_BATCH), TPB, q, (const J*)ss.sum, d_res);
   LAUNCH((k_encode<A>), blocks_for(q), TPB, q, (const A*)d_res, format, d_out);
   std::vector<unsigned long long> bad(q);
   CK(cudaMemcpyAsync(out, d_out, q * L, cudaMemcpyDeviceToHost, ctx->stream));
@@ -3551,28 +3758,36 @@ static int combine_shares_impl(blsgpu_ctx* ctx, size_t q, const uint64_t* share_
       iota[i] = (uint32_t)i;
     }
   const size_t nblocks = secure_msm_blocks(ctx, q);
-  CKR(ensure_arena(ctx, M * (32 + L + 32 + sizeof(A) + SECURE_WINDOWS + 16) + q * (SECURE_WINDOWS + 2) * sizeof(J) +
-                            nblocks * 128 * SECURE_BUCKETS * sizeof(J) + q * (sizeof(A) + L + 16) + (q + 1) * 8 + 32 * 256));
-  uint8_t *d_ids, *d_pts;
-  uint32_t *d_set, *d_iota;
+  uint8_t *d_ids, *d_pts, *d_idflag, *d_stpt, *d_dup, *d_bad, *d_out;
+  uint32_t *d_set, *d_iota, *d_raw;
   uint64_t* d_off;
+  A *d_p, *d_res;
+  int8_t* d_digits;
+  J *d_buckets, *d_W, *d_sum;
+  CKR(arena_takes(ctx, [&](auto& a) {
+    d_ids = take_up<uint8_t>(a, M * 32);
+    d_pts = take_up<uint8_t>(a, M * L);
+    d_set = take_up<uint32_t>(a, M);
+    d_iota = take_up<uint32_t>(a, M);
+    d_off = take_up<uint64_t>(a, q + 1);
+    d_raw = a.template take<uint32_t>(std::max<size_t>(M, 1) * 8);
+    d_idflag = a.template take<uint8_t>(std::max<size_t>(M, 1));
+    d_stpt = a.template take<uint8_t>(std::max<size_t>(M, 1));
+    d_dup = a.template take<uint8_t>(std::max<size_t>(M, 1));
+    d_bad = a.template take<uint8_t>(q);
+    d_p = a.template take<A>(std::max<size_t>(M, 1));
+    d_digits = a.template take<int8_t>(std::max<size_t>(M, 1) * SECURE_WINDOWS);
+    d_buckets = a.template take<J>(nblocks * 128 * SECURE_BUCKETS);
+    d_W = a.template take<J>(q * SECURE_WINDOWS);
+    d_sum = a.template take<J>(q);
+    d_res = a.template take<A>(q);
+    d_out = a.template take<uint8_t>(q * L);
+  }));
   CKR(upload(ctx, d_ids, ids.data(), M * 32));
   CKR(upload(ctx, d_pts, pts.data(), M * L));
   CKR(upload(ctx, d_set, set_of.data(), M));
   CKR(upload(ctx, d_iota, iota.data(), M));
   CKR(upload(ctx, d_off, share_off, q + 1));
-  uint32_t* d_raw = ctx->arena.take<uint32_t>(std::max<size_t>(M, 1) * 8);
-  uint8_t* d_idflag = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
-  uint8_t* d_stpt = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
-  uint8_t* d_dup = ctx->arena.take<uint8_t>(std::max<size_t>(M, 1));
-  uint8_t* d_bad = ctx->arena.take<uint8_t>(q);
-  A* d_p = ctx->arena.take<A>(std::max<size_t>(M, 1));
-  int8_t* d_digits = ctx->arena.take<int8_t>(std::max<size_t>(M, 1) * SECURE_WINDOWS);
-  J* d_buckets = ctx->arena.take<J>(nblocks * 128 * SECURE_BUCKETS);
-  J* d_W = ctx->arena.take<J>(q * SECURE_WINDOWS);
-  J* d_sum = ctx->arena.take<J>(q);
-  A* d_res = ctx->arena.take<A>(q);
-  uint8_t* d_out = ctx->arena.take<uint8_t>(q * L);
   std::vector<uint8_t> idflag(M), stpt(M), dup(M), bad(q, 0);
   if (M) {
     LAUNCH(k_share_ids, blocks_for(M), TPB, M, (const uint8_t*)d_ids, d_raw, d_idflag);
@@ -3689,17 +3904,24 @@ int blsgpu_pairing_check_batch(blsgpu_ctx* ctx, size_t q, const uint64_t* pair_o
   CKR(check_buffer(ctx, __func__, "g2_points", g2_points, M));
   pair_off = po.data();
   CKR(set_device(ctx));
-  CKR(ensure_arena(ctx, M * (48 + 96 + sizeof(G1Aff) + sizeof(G2Aff) + sizeof(Fp12) + 2) + (q + 1) * 9 + 16 * 256));
-  uint8_t *d_a, *d_b;
+  uint8_t *d_a, *d_b, *d_st, *d_ok;
   uint64_t* d_off;
+  G1Aff* d_p;
+  G2Aff* d_q;
+  Fp12* d_F;
+  CKR(arena_takes(ctx, [&](auto& a) {
+    d_a = take_up<uint8_t>(a, M * 48);
+    d_b = take_up<uint8_t>(a, M * 96);
+    d_off = take_up<uint64_t>(a, q + 1);
+    d_p = a.template take<G1Aff>(std::max<size_t>(M, 1));
+    d_q = a.template take<G2Aff>(std::max<size_t>(M, 1));
+    d_st = a.template take<uint8_t>(2 * std::max<size_t>(M, 1));
+    d_F = a.template take<Fp12>(std::max<size_t>(M, 1));
+    d_ok = a.template take<uint8_t>(q);
+  }));
   CKR(upload(ctx, d_a, g1_points, M * 48));
   CKR(upload(ctx, d_b, g2_points, M * 96));
   CKR(upload(ctx, d_off, pair_off, q + 1));
-  G1Aff* d_p = ctx->arena.take<G1Aff>(std::max<size_t>(M, 1));
-  G2Aff* d_q = ctx->arena.take<G2Aff>(std::max<size_t>(M, 1));
-  uint8_t* d_st = ctx->arena.take<uint8_t>(2 * std::max<size_t>(M, 1));
-  Fp12* d_F = ctx->arena.take<Fp12>(std::max<size_t>(M, 1));
-  uint8_t* d_ok = ctx->arena.take<uint8_t>(q);
   std::vector<uint8_t> st(2 * M);
   if (M) {
     CKR((decode_points<G1Aff>(ctx, M, (const uint8_t*)d_a, 1, d_p, d_st)));
@@ -3745,10 +3967,20 @@ namespace {
 static const uint8_t R_ORDER_BE[32] = {0x73, 0xed, 0xa7, 0x53, 0x29, 0x9d, 0x7d, 0x48, 0x33, 0x39, 0xd8, 0x08, 0x09, 0xa1, 0xd8, 0x05,
                                        0x53, 0xbd, 0xa4, 0x02, 0xff, 0xfe, 0x5b, 0xfe, 0xff, 0xff, 0xff, 0xff, 0x00, 0x00, 0x00, 0x01};
 
+// the scratch of pair2_check over n items: the pairs' Miller values and the item offsets
+struct Pair2 {
+  Fp12* F = nullptr;
+  uint64_t* off = nullptr;
+};
+template <class A>
+void take_pair2(A& a, size_t n, Pair2& s) {
+  s.F = a.template take<Fp12>(2 * n);
+  s.off = a.template take<uint64_t>(n + 1);
+}
 // prod over the two pairs of every item == 1 ?  (one thread per pair / per item: these checks are low-volume)
-int pair2_check(blsgpu_ctx* ctx, size_t n, const G1Aff* d_g1, const G2Aff* d_g2, uint8_t* d_ok) {
-  Fp12* d_F = ctx->arena.take<Fp12>(2 * n);
-  uint64_t* d_off = ctx->arena.take<uint64_t>(n + 1);
+int pair2_check(blsgpu_ctx* ctx, size_t n, const Pair2& s, const G1Aff* d_g1, const G2Aff* d_g2, uint8_t* d_ok) {
+  Fp12* d_F = s.F;
+  uint64_t* d_off = s.off;
   LAUNCH(k_pair_offsets, blocks_for(n + 1), TPB, n, d_off);
   LAUNCH(k_miller_pairs, blocks_for(2 * n), TPB, 2 * n, d_g1, d_g2, d_F);
   LAUNCH(k_set_final_is_one, blocks_for(n, 64), 64, n, (const uint64_t*)d_off, (const Fp12*)d_F, d_ok);
@@ -3761,7 +3993,7 @@ int pok_verify_impl(blsgpu_ctx* ctx, int scheme, size_t n, const uint8_t* commit
   typedef typename ImplT<IMPL>::PkAff PkA;
   typedef typename ImplT<IMPL>::SigAff SigA;
   typedef typename PtInfo<SigA>::Jac SigJ;
-  const size_t Lp = PtInfo<PkA>::LEN, Ls = PtInfo<SigA>::LEN, msg_bytes = (size_t)msg_off[n];
+  const size_t Lp = PtInfo<PkA>::LEN, Ls = PtInfo<SigA>::LEN;
   std::vector<uint8_t> yflag(n);
   for (size_t i = 0; i < n; i++) {
     const uint8_t* y = ys + 32 * i;
@@ -3769,25 +4001,39 @@ int pok_verify_impl(blsgpu_ctx* ctx, int scheme, size_t n, const uint8_t* commit
     for (int b = 0; b < 32; b++) zero = zero && y[b] == 0;
     yflag[i] = memcmp(y, R_ORDER_BE, 32) >= 0 ? 1 : zero ? 2 : 0;  // Scalar parsing rejects values >= r
   }
-  CKR(ensure_arena(ctx, n * (2 * Ls + Lp + 32 + 4 * sizeof(SigA) + sizeof(PkA) + sizeof(SigJ) + 2 * (sizeof(G1Aff) + sizeof(G2Aff) + sizeof(Fp12)) + 16) +
-                            msg_bytes + (n + 1) * 16 + 40 * 256));
-  uint8_t *d_cmb, *d_prb, *d_pkb, *d_y, *d_yf, *d_msgs;
+  uint8_t *d_cmb, *d_prb, *d_pkb, *d_y, *d_yf, *d_msgs, *d_st, *d_ok;
   uint64_t* d_moff;
+  SigA *d_cm, *d_pr, *d_a;
+  PkA* d_pk;
+  SigJ* d_hj;
+  G1Aff* d_g1;
+  G2Aff* d_g2;
+  Pair2 p2;
+  CKR(arena_takes(ctx, [&](auto& a) {
+    d_cmb = take_up<uint8_t>(a, n * Ls);
+    d_prb = take_up<uint8_t>(a, n * Ls);
+    d_pkb = take_up<uint8_t>(a, n * Lp);
+    d_y = take_up<uint8_t>(a, n * 32);
+    d_yf = take_up<uint8_t>(a, n);
+    take_records(a, msg_off, n, d_msgs, d_moff);
+    d_cm = a.template take<SigA>(n);
+    d_pr = a.template take<SigA>(n);
+    d_a = a.template take<SigA>(n);
+    d_pk = a.template take<PkA>(n);
+    d_st = a.template take<uint8_t>(4 * n);
+    d_ok = a.template take<uint8_t>(n);
+    d_g1 = a.template take<G1Aff>(2 * n);
+    d_g2 = a.template take<G2Aff>(2 * n);
+    d_hj = take_hash_scratch<SigA>(a, n);
+    take_pair2(a, n, p2);
+  }));
   CKR(upload(ctx, d_cmb, commitments, n * Ls));
   CKR(upload(ctx, d_prb, proofs, n * Ls));
   CKR(upload(ctx, d_pkb, pks, n * Lp));
   CKR(upload(ctx, d_y, ys, n * 32));
   CKR(upload(ctx, d_yf, yflag.data(), n));
   CKR(upload_records(ctx, msgs, msg_off, n, d_msgs, d_moff));
-  SigA* d_cm = ctx->arena.take<SigA>(n);
-  SigA* d_pr = ctx->arena.take<SigA>(n);
-  SigA* d_a = ctx->arena.take<SigA>(n);
-  PkA* d_pk = ctx->arena.take<PkA>(n);
-  uint8_t* d_st = ctx->arena.take<uint8_t>(4 * n);
   uint8_t *d_stcm = d_st, *d_stpr = d_st + n, *d_stpk = d_st + 2 * n, *d_status = d_st + 3 * n;
-  uint8_t* d_ok = ctx->arena.take<uint8_t>(n);
-  G1Aff* d_g1 = ctx->arena.take<G1Aff>(2 * n);
-  G2Aff* d_g2 = ctx->arena.take<G2Aff>(2 * n);
   CKR((decode_points<SigA>(ctx, n, (const uint8_t*)d_cmb, 1, d_cm, d_stcm)));
   CKR((decode_points<SigA>(ctx, n, (const uint8_t*)d_prb, 1, d_pr, d_stpr)));
   CKR((decode_points<PkA>(ctx, n, (const uint8_t*)d_pkb, 1, d_pk, d_stpk)));
@@ -3795,10 +4041,10 @@ int pok_verify_impl(blsgpu_ctx* ctx, int scheme, size_t n, const uint8_t* commit
          (const uint8_t*)d_yf, (const SigA*)d_cm, (const SigA*)d_pr, (const PkA*)d_pk, d_status);
   DstParam dst;
   make_dst(dst, IMPL, scheme, false);
-  CKR((hash_points<SigA, PkA>(ctx, n, (const uint8_t*)d_msgs, (const uint64_t*)d_moff, 0, (const PkA*)d_pk, (const uint8_t*)d_status, dst, d_a)));
+  CKR((hash_points<SigA, PkA>(ctx, n, (const uint8_t*)d_msgs, (const uint64_t*)d_moff, 0, (const PkA*)d_pk, (const uint8_t*)d_status, dst, d_hj, d_a)));
   LAUNCH((k_pok_pairs<PkA, SigA>), blocks_for(n), TPB, n, (const uint8_t*)d_status, (const SigA*)d_a, (const SigA*)d_cm, (const SigA*)d_pr,
          (const PkA*)d_pk, (const uint8_t*)d_y, d_g1, d_g2);
-  CKR(pair2_check(ctx, n, d_g1, d_g2, d_ok));
+  CKR(pair2_check(ctx, n, p2, d_g1, d_g2, d_ok));
   LAUNCH(k_pok_finish, blocks_for(n), TPB, n, (const uint8_t*)d_ok, d_status);
   CK(cudaMemcpyAsync(status_out, d_status, n, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
@@ -3811,25 +4057,38 @@ int signcrypt_share_impl(blsgpu_ctx* ctx, int scheme, size_t n, const uint8_t* s
   typedef typename ImplT<IMPL>::PkAff PkA;
   typedef typename ImplT<IMPL>::SigAff SigA;
   typedef typename PtInfo<SigA>::Jac SigJ;
-  const size_t Lp = PtInfo<PkA>::LEN, Ls = PtInfo<SigA>::LEN, v_total = (size_t)v_off[n];
-  CKR(ensure_arena(ctx, n * (3 * Lp + Ls + 3 * sizeof(PkA) + 2 * sizeof(SigA) + sizeof(SigJ) + 2 * (sizeof(G1Aff) + sizeof(G2Aff) + sizeof(Fp12)) + 24) +
-                            v_total + (n + 1) * 16 + 40 * 256));
-  uint8_t *d_shb, *d_pkb, *d_ub, *d_wb, *d_v;
+  const size_t Lp = PtInfo<PkA>::LEN, Ls = PtInfo<SigA>::LEN;
+  uint8_t *d_shb, *d_pkb, *d_ub, *d_wb, *d_v, *d_st;
   uint64_t* d_voff;
+  PkA *d_sh, *d_pk, *d_u;
+  SigA *d_w, *d_wt;
+  SigJ* d_hj;
+  G1Aff* d_g1;
+  G2Aff* d_g2;
+  Pair2 p2;
+  CKR(arena_takes(ctx, [&](auto& a) {
+    d_shb = take_up<uint8_t>(a, n * Lp);
+    d_pkb = take_up<uint8_t>(a, n * Lp);
+    d_ub = take_up<uint8_t>(a, n * Lp);
+    d_wb = take_up<uint8_t>(a, n * Ls);
+    take_records(a, v_off, n, d_v, d_voff);
+    d_sh = a.template take<PkA>(n);
+    d_pk = a.template take<PkA>(n);
+    d_u = a.template take<PkA>(n);
+    d_w = a.template take<SigA>(n);
+    d_wt = a.template take<SigA>(n);
+    d_st = a.template take<uint8_t>(6 * n);
+    d_g1 = a.template take<G1Aff>(2 * n);
+    d_g2 = a.template take<G2Aff>(2 * n);
+    d_hj = take_hash_scratch<SigA>(a, n);
+    take_pair2(a, n, p2);
+  }));
   CKR(upload(ctx, d_shb, shares, n * Lp));
   CKR(upload(ctx, d_pkb, pks, n * Lp));
   CKR(upload(ctx, d_ub, us, n * Lp));
   CKR(upload(ctx, d_wb, ws, n * Ls));
   CKR(upload_records(ctx, v_bytes, v_off, n, d_v, d_voff));
-  PkA* d_sh = ctx->arena.take<PkA>(n);
-  PkA* d_pk = ctx->arena.take<PkA>(n);
-  PkA* d_u = ctx->arena.take<PkA>(n);
-  SigA* d_w = ctx->arena.take<SigA>(n);
-  SigA* d_wt = ctx->arena.take<SigA>(n);
-  uint8_t* d_st = ctx->arena.take<uint8_t>(6 * n);
   uint8_t *d_s0 = d_st, *d_s1 = d_st + n, *d_s2 = d_st + 2 * n, *d_s3 = d_st + 3 * n, *d_flag = d_st + 4 * n, *d_ok = d_st + 5 * n;
-  G1Aff* d_g1 = ctx->arena.take<G1Aff>(2 * n);
-  G2Aff* d_g2 = ctx->arena.take<G2Aff>(2 * n);
   CKR((decode_points<PkA>(ctx, n, (const uint8_t*)d_shb, 1, d_sh, d_s0)));
   CKR((decode_points<PkA>(ctx, n, (const uint8_t*)d_pkb, 1, d_pk, d_s1)));
   CKR((decode_points<PkA>(ctx, n, (const uint8_t*)d_ub, 1, d_u, d_s2)));
@@ -3846,10 +4105,10 @@ int signcrypt_share_impl(blsgpu_ctx* ctx, int scheme, size_t n, const uint8_t* s
   DstParam dst;
   make_dst(dst, IMPL, scheme, false);
   // W' = hash_to_point(u.to_bytes() || v): the pk-prefix framing with u in the key's place (compute_w, sign_crypt.rs:151-158)
-  CKR((hash_points<SigA, PkA>(ctx, n, (const uint8_t*)d_v, (const uint64_t*)d_voff, 1, (const PkA*)d_u, (const uint8_t*)d_s0, dst, d_wt)));
+  CKR((hash_points<SigA, PkA>(ctx, n, (const uint8_t*)d_v, (const uint64_t*)d_voff, 1, (const PkA*)d_u, (const uint8_t*)d_s0, dst, d_hj, d_wt)));
   LAUNCH((k_signcrypt_share_pairs<PkA, SigA>), blocks_for(n), TPB, n, (const uint8_t*)d_s0, (const SigA*)d_wt, (const PkA*)d_sh, (const PkA*)d_pk,
          (const SigA*)d_w, d_g1, d_g2, d_flag);
-  CKR(pair2_check(ctx, n, d_g1, d_g2, d_ok));
+  CKR(pair2_check(ctx, n, p2, d_g1, d_g2, d_ok));
   LAUNCH(k_and_flags, blocks_for(n), TPB, n, (const uint8_t*)d_flag, d_ok);
   CK(cudaMemcpyAsync(ok_out, d_ok, n, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
